@@ -2,6 +2,7 @@
 """Region-stage benchmark (BASELINE.json metric: region-stage images/sec; NMS us @12k boxes).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload all|rpn|voc1|train|infer|joint]
+                    [--dump-outputs DIR]
 
 The line's headline (`value`, `e2e`, `roofline`, `cpu_baseline`) is BASELINE.json configs[1]: RPN proposal layer, 9 anchors x
 38x63 map (608x1008 image, N = 21546), 12000 pre-NMS -> 2000 post-NMS at IoU 0.7, batch 64 images per GPU; one "step" = one
@@ -13,10 +14,16 @@ pass of decode + top-k + NMS over one batch of 64 synthetic images.  With the de
 Under torchrun every rank processes its own images (weak scaling; the only collective is the detection all-gather of
 `infer`); rank 0 prints ONE JSON line.  `--impl reference` times the CPU restatement of the reference (oracle/) on the
 host cores for the same configurations.
+
+`--steps K` is the number of timed steps of every workload's step loops (the per-kernel timings use their own repetition
+counts).  `--dump-outputs DIR` writes, after the timed steps, what the timed path of each workload run handed its caller in
+its last step as DIR/<workload>_<output>.npy (float32, or float64 for integer outputs); inputs are seeded, so two builds
+run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -33,6 +40,8 @@ HW = (608, 1008)
 BATCH = 64
 PRE_K, POST_K, THR = 12000, 2000, 0.7
 N_ROTATE = 8           # resident input batches cycled through so that every step reads cold data (> L2)
+DUMP_SAMPLE = 1 << 20  # --dump-outputs: an output with more elements is reduced to this many seeded positions
+DUMP_MAX_BYTES = 64 << 20
 METRIC = "region-stage images/sec (RPN+NMS+RoIPool) at 1/2/4/8 B200; NMS us @12k boxes"
 WORKLOAD = ("configs[1]: RPN proposal layer, 9 anchors x 38x63 map (608x1008), 12000 pre-NMS -> 2000 post-NMS "
             "@ IoU 0.7, batch 64 images/GPU")
@@ -83,6 +92,33 @@ def make_inputs(seed0: int, batch: int, hw=HW):
     logits = rs.standard_normal((batch, n, 2)).astype(np.float32)
     reg = (rs.standard_normal((batch, n, 4)) * 0.2).astype(np.float32)
     return logits, reg
+
+
+def dump_arrays(prefix: str, arrays: dict) -> dict:
+    """Host copies of one step's outputs for --dump-outputs: floating-point outputs as float32 (float64 stays float64),
+    integer ones as float64 (exact).  An output of more than DUMP_SAMPLE elements is reduced to its elements at seeded
+    positions of the flattened array (name suffix `_sample`), the same positions in every run."""
+    import torch
+    out = {}
+    for key, t in arrays.items():
+        t = torch.as_tensor(t).detach()
+        name = f"{prefix}_{key}"
+        if t.numel() > DUMP_SAMPLE:
+            pos = np.unique(np.random.RandomState(0).randint(0, t.numel(), DUMP_SAMPLE))
+            t = t.reshape(-1)[torch.from_numpy(pos).to(t.device)]
+            name += "_sample"
+        wide = t.dtype == torch.float64 or not t.is_floating_point()
+        out[name] = t.to(torch.float64 if wide else torch.float32).cpu().numpy()
+    return out
+
+
+def write_outputs(dumps: dict, out_dir: str):
+    total = sum(a.nbytes for a in dumps.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"bench.py: --dump-outputs: {total / 2**20:.1f} MB of outputs, more than {DUMP_MAX_BYTES >> 20} MB")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in dumps.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------ CPU arm (oracle port)
@@ -251,6 +287,7 @@ class ClockSampler:
             self.p = subprocess.Popen(["nvidia-smi", "-i", str(gpu_index), f"--query-gpu={self.Q}",
                                        "--format=csv,noheader,nounits", "-lms", "50"], stdout=self.f,
                                       stderr=subprocess.DEVNULL)
+            atexit.register(self.stop)        # a run that fails must not leave nvidia-smi behind
         except Exception:
             self.p = None
 
@@ -258,11 +295,12 @@ class ClockSampler:
         out = {"sm_mhz": None, "sm_max_mhz": None, "reasons": []}
         if self.p is None:
             return out
-        self.p.terminate()
+        p, self.p = self.p, None
+        p.terminate()
         try:
-            self.p.wait(timeout=5)
+            p.wait(timeout=5)
         except Exception:
-            self.p.kill()
+            p.kill()
         self.f.flush()
         self.f.seek(0)
         sm, mx, reasons = [], [], set()
@@ -292,7 +330,7 @@ class ClockSampler:
 class Ctx:
     """Process-wide plumbing of the GPU arm: device, NCCL group, device-side timing (max over ranks)."""
 
-    def __init__(self):
+    def __init__(self, dump: bool = False):
         import torch
         import torch.distributed as dist
         self.torch, self.dist = torch, dist
@@ -313,6 +351,13 @@ class Ctx:
         self.lib = _lib.load()
         self.peak, self.peak_how, self.sm_mhz = peaks()
         self.num_sms = int(torch.cuda.get_device_properties(self.dev).multi_processor_count)
+        self.dump = dump and self.rank == 0
+        self.dumps = {}
+
+    def keep_outputs(self, prefix: str, arrays: dict):
+        """--dump-outputs: keep host copies of what the timed path's last step handed its caller (rank 0)."""
+        if self.dump:
+            self.dumps.update(dump_arrays(prefix, arrays))
 
     def sync_all(self):
         self.torch.cuda.synchronize()
@@ -492,16 +537,21 @@ def run_rpn(ctx, args) -> dict:
         for lg, rg in sets:
             pipe2.capture(lg, rg)
 
+        ticket = [None]
+
         def step_pipe(i):
             lg, rg = sets[i % N_ROTATE]
-            pipe2.submit(lg, rg)
+            ticket[0] = pipe2.submit(lg, rg)
 
         for i in range(max(args.warmup, 3)):
             step_pipe(i)
         pipe2.drain()
         ms = ctx.timed(step_pipe, args.steps, tail=pipe2.drain)
+        last = pipe2.result(ticket[0])
     else:
         ms = ms_one
+        last = (plan.rois, plan.count)
+    ctx.keep_outputs("rpn", {"rois": last[0], "count": last[1]})
     launches = launches_per_step * args.steps
     value = world * B * args.steps / (ms * 1e-3)
 
@@ -542,7 +592,7 @@ def run_rpn(ctx, args) -> dict:
         _, cnt = pipe.result(t)
         sink[0] += int(cnt[0])
 
-    e2e_steps = max(3, min(args.steps, 30))
+    e2e_steps = args.steps
     for i in range(3):
         e2e_serial(i)
     ms_e2e_serial = ctx.median_ms(e2e_serial, e2e_steps, runs=3)
@@ -767,7 +817,7 @@ def run_predict(ctx, args, which: str) -> dict:
     h, d, plan, fhw, n = _predict_setup(ctx, hw, B, R, NC, 9100 if voc else 9000, NR)
     ids = torch.arange(ctx.rank * B, (ctx.rank + 1) * B, dtype=torch.int64, device=ctx.dev)
     keep = {}
-    steps = max(5, min(args.steps, 50))
+    steps = args.steps
     gather = (not voc) and ctx.world > 1
 
     def step(i, gather=gather):
@@ -853,6 +903,13 @@ def run_predict(ctx, args, which: str) -> dict:
                     i_last = ((steps - 1 - j) // depth) * depth + j
                     verified = bool(verified) and verify_predict(mg[j][i_last % NR][1], d["feats"][i_last % NR], B - 1, R, NC, fhw)
             value = ctx.world * B * steps / (ms_multi * 1e-3)
+    # the outputs of the last timed step: in flight, else graph replay, else eager (the same input set in each form)
+    last = (mg[(steps - 1) % depth][(steps - 1) % NR][1] if ms_multi else
+            graphs[(steps - 1) % NR][1] if graphs else keep["out"])
+    arrays = {k: last[k] for k in ("rois", "cnt", "pooled", "prob", "boxes", "packed", "pc")}
+    if gather and last is not keep["out"]:   # the graphs hold this rank's detections; the caller receives the gathered ones
+        arrays["packed"], arrays["pc"] = keep["g"][0], keep["g"][1]
+    ctx.keep_outputs(which, arrays)
 
     # ---- end to end, strict form: EVERY input of the step from pinned host memory (head outputs, feature map, FC head
     #      outputs), the packed detections read back on the host, every step, serialised (latency form)
@@ -897,7 +954,7 @@ def run_predict(ctx, args, which: str) -> dict:
 
     for i in range(3):
         e2e_host(i); e2e_resident(i)
-    e_steps = max(5, min(steps, 20))
+    e_steps = steps
     ms_e2e = ctx.median_ms(e2e_host, e_steps, runs=3)
     ms_e2r = ctx.median_ms(e2e_resident, e_steps, runs=3)
     # the same with `depth` batches in flight: the detections of step i - depth are consumed on the host while steps
@@ -1006,7 +1063,7 @@ def run_train(ctx, args) -> dict:
     torch.manual_seed(3000 + rank)
     gen = targets.DeviceGenerator(dev) if args.sampling == "device" else None    # torch's mt19937 stream on the device
     stats = {}
-    steps = max(5, min(args.steps, 30))
+    steps = args.steps
 
     def step(i, gt=gt, lab=lab):
         # device sampling: 6 kernels, no host synchronisation; host sampling: 4 kernels + ONE D2H of counts
@@ -1069,6 +1126,7 @@ def run_train(ctx, args) -> dict:
         ms = ctx.timed(step_multi, steps, tail=fl.drain)
         torch.cuda.synchronize()
     out, gin, rois5, arg, t, r_last = stats["last"]
+    ctx.keep_outputs("train", dict(t, rois5=rois5, pooled=out, argmax=arg, grad_features=gin))
 
     verified = None
     if rank == 0:   # image 0 of the last step: RoIPool forward (max + argmax) bit-exact, backward within 1e-5 of max|grad|
@@ -1107,7 +1165,7 @@ def run_train(ctx, args) -> dict:
 
     for i in range(3):
         e2e(i)
-    e_steps = max(5, min(steps, 20))
+    e_steps = steps
     ms_e2e = ctx.median_ms(e2e, e_steps, runs=3)
     # the same with `depth` batches in flight (graph replays): H2D of the ground truth into the slot's tensors, both graphs,
     # D2H of the sampled class targets, the host consuming the result of step i - depth
@@ -1193,6 +1251,7 @@ def run_joint(ctx, args) -> dict:
     torch.manual_seed(4000 + rank)
     gen = targets.DeviceGenerator(dev)
     batches = [fh_.make_batch(B, hw, G, dev, seed=10 * rank + i) for i in range(3)]
+    kept = {}
 
     def step(i):
         x, gt, lab = batches[i % 3]
@@ -1200,6 +1259,7 @@ def run_joint(ctx, args) -> dict:
         loss = net(x, gt, lab, gen)
         loss[:, 0].mean().backward()
         opt.step()
+        kept["loss"] = loss
         return loss
 
     for i in range(max(args.warmup, 3)):
@@ -1207,6 +1267,7 @@ def run_joint(ctx, args) -> dict:
     l0 = ctx._lib.launch_count()
     ms = ctx.timed(step, args.steps)
     launches = ctx._lib.launch_count() - l0
+    ctx.keep_outputs("joint", {"loss": kept["loss"]})
     model.timer.enabled = True
     for i in range(4):
         step(i)
@@ -1234,7 +1295,7 @@ def _as_line(ctx, args, res: dict) -> dict:
 
 
 def run_ours(args):
-    ctx = Ctx()
+    ctx = Ctx(dump=args.dump_outputs is not None)
     sampler = ClockSampler(ctx.local) if ctx.rank == 0 else None
     threads = os.cpu_count() or 1
     want_cpu = ctx.rank == 0 and ctx.world == 1 and not args.no_cpu
@@ -1264,8 +1325,10 @@ def run_ours(args):
     if sampler is not None:
         line["clocks"] = sampler.stop()
     if ctx.rank == 0:
-        print(json.dumps(line))
+        print(json.dumps(line), flush=True)
     ctx.close()
+    if ctx.dump:   # after the result line: an oversized dump must not cost the measurement
+        write_outputs(ctx.dumps, args.dump_outputs)
 
 
 def main():
@@ -1285,7 +1348,13 @@ def main():
     ap.add_argument("--workload", default="all", choices=["all", "rpn", "voc1", "train", "infer", "joint"],
                     help="all = configs[1] headline + sub_results for configs[0], [2], [3] (the driver's line); rpn = configs[1] "
                          "only; voc1 = configs[0]; train = configs[2]; infer = configs[3]; joint = configs[4]")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's outputs of every workload run to DIR/<workload>_<output>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -143,7 +143,7 @@ def multiscale():
         full = np.zeros(out.shape, np.float32); full[order] = out.detach().numpy()
         gfull = np.zeros(out.shape, np.float32); gfull[order] = go.numpy()
         g[f"{tag}_out"] = full                          # rows in the order of rois5
-        g[f"{tag}_grad_out"] = gfull
+        g["grad_out"] = gfull                           # the same seeded gradient for both tags: stored once
         for i, f in enumerate(x.values()):
             g[f"{tag}_gin{i}"] = f.grad.numpy().copy()
         scales = pool.scales

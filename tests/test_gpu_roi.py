@@ -4,7 +4,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import golden
+from conftest import golden, sha
 from faster_rcnn_pytorch_b200 import ops, synth
 
 pytestmark = pytest.mark.gpu
@@ -85,22 +85,31 @@ def test_roi_pool_full_size_vs_oracle(oracle, B, C, fh, fw, K):
     assert arg_na is None and torch.equal(out_na, out)
 
 
-@pytest.mark.parametrize("K,B,want_argmax", [(3000, 2, True), (6000, 3, True), (1500, 1, False)])
+LONG_ROI_SHAPE = (24, 37, 62)                                             # C, fh, fw
+LONG_ROI_CASES = [(3000, 2, True), (6000, 3, True), (1500, 1, False)]     # K, B, want_argmax
+
+
+@pytest.mark.parametrize("K,B,want_argmax", LONG_ROI_CASES)
 def test_roi_pool_forward_long_roi_lists(K, B, want_argmax):
     """more rois than one scan round of the forward kernel holds (2688) and more rois of one image than one list round
-    (448), images interleaved, a few masked rows -- max and argmax bit-equal to torchvision's CUDA kernel"""
-    import torchvision  # noqa: F401  (registers torch.ops.torchvision)
-    C, fh, fw = 24, 37, 62
+    (448), images interleaved, a few masked rows -- max and argmax bit-equal to torchvision's RoIPool (sha256 of both
+    arrays and their values at sampled positions, made with torchvision 0.26's CPU kernel by
+    tests/golden/make_golden_roi_long.py)"""
+    g = golden("roi_long")
+    key = f"{K}_{B}"
+    C, fh, fw = LONG_ROI_SHAPE
     feat = dev(synth.features(710, B, C, fh, fw))
     rois5 = _mixed_rois(711, K, fh, fw, B, small_frac=0.2)
     keep = rois5[:, 0] >= 0
-    r = dev(rois5)
-    out, arg = ops.roi_pool_forward(feat, r, want_argmax=want_argmax)
-    tv_out, tv_arg = torch.ops.torchvision.roi_pool(feat, dev(rois5[keep]), 1.0, 7, 7)
+    out, arg = ops.roi_pool_forward(feat, dev(rois5), want_argmax=want_argmax)
     k = torch.from_numpy(keep).to(DEV)
-    assert torch.equal(out[k], tv_out)
+    got = {"out": out[k].cpu().numpy()}
     if want_argmax:
-        assert torch.equal(arg[k], tv_arg.to(arg.dtype))
+        got["argmax"] = arg[k].cpu().numpy()
+    for name, a in got.items():
+        assert a.shape == tuple(g[f"{key}_shape"]), name
+        assert np.array_equal(a.reshape(-1)[g[f"{key}_idx"]], g[f"{key}_{name}_sample"]), name
+        assert np.array_equal(sha(a), g[f"{key}_{name}_sha"]), name
 
 
 @pytest.mark.parametrize("B,C,fh,fw,K,scale,sr,aligned", [(2, 256, 50, 84, 200, 1.0, 2, False), (1, 256, 25, 42, 100, 0.5, 2, True),
@@ -243,7 +252,7 @@ def test_multiscale_roi_align_goldens(tag, shapes, channels_last):
                                            return_levels=True)
     assert np.array_equal(levels.cpu().numpy(), g[f"{tag}_levels"])
     np.testing.assert_allclose(out.detach().cpu().numpy(), g[f"{tag}_out"], rtol=RTOL, atol=ATOL)
-    out.backward(dev(g[f"{tag}_grad_out"]))
+    out.backward(dev(g["grad_out"]))
     for i, f in enumerate(feats):
         close_accum(f.grad.cpu().numpy(), g[f"{tag}_gin{i}"])
 

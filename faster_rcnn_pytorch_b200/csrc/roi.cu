@@ -350,14 +350,17 @@ __global__ void __launch_bounds__(kAlignStreamThreads)
 // ---------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------
-// 7x7 fast paths (roi_fast.cu): 0 = launched, 1 = shape outside the fast path, 2 = use the direct atomic kernel, < 0 = error
-int roi_fwd_fast(bool align, const float* feat, const float* rois, int K, int B, int C, int H, int W, int PH, int PW,
-                 float scale, int sampling, int aligned, int nhwc, float* out, int32_t* argmax, frr_stream_t stream);
-int roi_align_bwd_fast(const float* grad_out, const float* rois, int K, int B, int C, int H, int W, int PH, int PW,
-                       float scale, int sampling, int aligned, int nhwc, float* grad_in, frr_stream_t stream);
-// colour-class RoIPool backward (roi_pool_bwd.cu): 0 = launched, 1 = outside that path, < 0 = error
-int roi_pool_bwd_color(const float* grad_out, const int32_t* argmax, const float* rois, int K, int B, int C, int H, int W,
-                       int PH, int PW, float scale, int nhwc, float* grad_in, int force_tail, frr_stream_t stream);
+// 7x7 fast paths (roi_fast.cu, roi_pool_bwd.cu): *_pick fills the choice (false = shape outside the fast path),
+// *_launch runs it (0 = launched, < 0 = error)
+bool roi_fwd_fast_pick(bool align, int B, int C, int H, int W, int PH, int PW, int sampling, RoiPick* pk);
+int roi_fwd_fast_launch(const RoiPick& pk, const float* feat, const float* rois, int K, int B, int C, int H, int W,
+                        float scale, int aligned, int nhwc, float* out, int32_t* argmax, frr_stream_t stream);
+bool roi_align_bwd_fast_pick(int B, int C, int H, int W, int PH, int PW, int sampling, RoiPick* pk);
+int roi_align_bwd_fast_launch(const RoiPick& pk, const float* grad_out, const float* rois, int K, int B, int C, int H, int W,
+                              float scale, int aligned, int nhwc, float* grad_in, frr_stream_t stream);
+bool roi_pool_bwd_fast_pick(int K, int H, int W, int PH, int PW, bool ptrs_aligned, bool force_tail, RoiPick* pk);
+int roi_pool_bwd_fast_launch(const RoiPick& pk, const float* grad_out, const int32_t* argmax, const float* rois, int K, int B,
+                             int C, int H, int W, float scale, int nhwc, float* grad_in, frr_stream_t stream);
 
 // developer knob (A/B measurements only): FRR_ROI_POOL_BWD=tail sends every roi through the streaming atomic kernel
 static int pool_bwd_force_tail() {
@@ -386,31 +389,56 @@ static int pick_cb(int B, int C, int HW) {
     return best;  // 0 -> does not fit at all
 }
 
+// The kernel an RoI entry point runs (host only, launches nothing): shared by the launchers below and frr_roi_variant.
+// op: 0 roi_pool fwd, 1 roi_pool bwd, 2 roi_align fwd, 3 roi_align bwd.  ptrs_aligned: grad_out and argmax are 4-byte
+// aligned (the colour-class RoIPool backward copies them word by word with cp.async).
+static int roi_pick(int op, int K, int B, int C, int H, int W, int PH, int PW, int sampling, bool ptrs_aligned, RoiPick* pk) {
+    FRR_CHECK_ARG(op >= 0 && op <= 3, "roi variant: op %d not in 0..3", op);
+    FRR_CHECK_ARG(K >= 0 && B > 0 && C > 0 && H > 0 && W > 0 && PH > 0 && PW > 0 && B <= 65535, "roi %s: bad sizes",
+                  (op & 1) ? "backward" : "forward");
+    const bool align = op >= 2, bwd = (op & 1) != 0;
+    const int HW = H * W;
+    if (!bwd) {
+        if (K == 0) { *pk = RoiPick{kRoiNone, 0, 0, 0, 0}; return FRR_OK; }
+        if (roi_fwd_fast_pick(align, B, C, H, W, PH, PW, sampling, pk)) return FRR_OK;
+    } else if (K > 0) {
+        if (align ? roi_align_bwd_fast_pick(B, C, H, W, PH, PW, sampling, pk)
+                  : roi_pool_bwd_fast_pick(K, H, W, PH, PW, ptrs_aligned, pool_bwd_force_tail() != 0, pk))
+            return FRR_OK;
+    }
+    const int cb = pick_cb(B, C, HW);
+    if (cb > 0) *pk = RoiPick{bwd ? kBwdPlanes : kFwdPlanes, cb, 1, 0, roi_smem_bytes(cb, HW)};
+    else *pk = RoiPick{(bwd && K == 0) ? kRoiNone : bwd ? kBwdDirect : kFwdDirect, 0, 1, 0, 0};
+    return FRR_OK;
+}
+
+static int direct_blocks(size_t total) {
+    return (int)((total + 255) / 256 < (size_t)num_sms() * 16 ? (total + 255) / 256 : (size_t)num_sms() * 16);
+}
+
 template <bool kAlign>
 static int roi_forward(const float* feat, const float* rois, int K, int B, int C, int H, int W, int PH, int PW, float scale,
                        int sampling, int aligned, int nhwc, float* out, int32_t* argmax, frr_stream_t stream) {
     FRR_CHECK_ARG(K == 0 || (feat && out && rois), "roi forward: null pointer");
-    FRR_CHECK_ARG(K >= 0 && B > 0 && C > 0 && H > 0 && W > 0 && PH > 0 && PW > 0 && B <= 65535, "roi forward: bad sizes");
-    if (K == 0) return FRR_OK;
+    RoiPick pk;
     {
-        const int rc = roi_fwd_fast(kAlign, feat, rois, K, B, C, H, W, PH, PW, scale, sampling, aligned, nhwc, out, argmax, stream);
-        if (rc <= 0) return rc;
+        const int rc = roi_pick(kAlign ? 2 : 0, K, B, C, H, W, PH, PW, sampling, true, &pk);
+        if (rc) return rc;
     }
+    if (pk.kernel == kRoiNone) return FRR_OK;
+    if (pk.kernel == kPoolFwdFlat || pk.kernel == kAlignFwdFast)
+        return roi_fwd_fast_launch(pk, feat, rois, K, B, C, H, W, scale, aligned, nhwc, out, kAlign ? nullptr : argmax, stream);
     cudaStream_t st = (cudaStream_t)stream;
-    const int HW = H * W;
-    const int cb = pick_cb(B, C, HW);
-    if (cb > 0) {
-        const size_t smem = roi_smem_bytes(cb, HW);
+    if (pk.kernel == kFwdPlanes) {
         auto kern = roi_fwd_planes_kernel<kAlign>;
         FRR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        dim3 grid((C + cb - 1) / cb, B);
-        kern<<<grid, kRoiThreads, smem, st>>>(feat, rois, K, C, H, W, cb, PH, PW, scale, sampling, aligned, nhwc, out,
-                                              argmax);
+        dim3 grid((C + pk.cb - 1) / pk.cb, B);
+        kern<<<grid, kRoiThreads, pk.smem, st>>>(feat, rois, K, C, H, W, pk.cb, PH, PW, scale, sampling, aligned, nhwc, out,
+                                                 argmax);
     } else {
         const size_t total = (size_t)K * C * PH * PW;
-        const int blocks = (int)((total + 255) / 256 < (size_t)num_sms() * 16 ? (total + 255) / 256 : (size_t)num_sms() * 16);
-        roi_fwd_direct_kernel<kAlign><<<blocks, 256, 0, st>>>(feat, rois, total, B, C, H, W, PH, PW, scale, sampling, aligned,
-                                                              nhwc, out, argmax);
+        roi_fwd_direct_kernel<kAlign><<<direct_blocks(total), 256, 0, st>>>(feat, rois, total, B, C, H, W, PH, PW, scale,
+                                                                            sampling, aligned, nhwc, out, argmax);
     }
     count_launch();
     FRR_CHECK_LAUNCH("roi forward kernel");
@@ -423,46 +451,45 @@ static int roi_backward(const float* grad_out, const int32_t* argmax, const floa
                         frr_stream_t stream) {
     FRR_CHECK_ARG(grad_in && (K == 0 || (grad_out && rois)), "roi backward: null pointer");
     FRR_CHECK_ARG(kAlign || K == 0 || argmax, "roi_pool backward: argmax is required");
-    FRR_CHECK_ARG(K >= 0 && B > 0 && C > 0 && H > 0 && W > 0 && PH > 0 && PW > 0 && B <= 65535, "roi backward: bad sizes");
-    bool direct = false;
-    if (K > 0) {
-        int rc = 1;
-        if (kAlign) {
-            rc = roi_align_bwd_fast(grad_out, rois, K, B, C, H, W, PH, PW, scale, sampling, aligned, nhwc, grad_in, stream);
-        } else {
-            rc = roi_pool_bwd_color(grad_out, argmax, rois, K, B, C, H, W, PH, PW, scale, nhwc, grad_in, pool_bwd_force_tail(), stream);
-        }
-        if (rc <= 0) return rc;
-        direct = rc == 2;  // the fast path asks for the global-atomic kernel
+    const bool ptrs_aligned =
+        !(reinterpret_cast<uintptr_t>(grad_out) & 3u) && !(reinterpret_cast<uintptr_t>(argmax) & 3u);
+    RoiPick pk;
+    {
+        const int rc = roi_pick(kAlign ? 3 : 1, K, B, C, H, W, PH, PW, sampling, ptrs_aligned, &pk);
+        if (rc) return rc;
     }
     cudaStream_t st = (cudaStream_t)stream;
     const int HW = H * W;
-    if (kAlign && direct) {  // (rc == 2 is only returned for 7x7 bins with sampling_ratio 2)
-        FRR_CUDA(cudaMemsetAsync(grad_in, 0, (size_t)B * C * HW * sizeof(float), st));
-        roi_align_bwd_stream_kernel<<<K, kAlignStreamThreads, 0, st>>>(grad_out, rois, B, C, H, W, scale, aligned, nhwc, grad_in);
-        count_launch();
-        FRR_CHECK_LAUNCH("roi_align_bwd_stream_kernel");
-        return FRR_OK;
-    }
-    const int cb = direct ? 0 : pick_cb(B, C, HW);
-    if (cb > 0) {
-        const size_t smem = roi_smem_bytes(cb, HW);
-        auto kern = roi_bwd_planes_kernel<kAlign>;
-        FRR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        dim3 grid((C + cb - 1) / cb, B);
-        kern<<<grid, kRoiThreads, smem, st>>>(grad_out, argmax, rois, K, C, H, W, cb, PH, PW, scale, sampling, aligned, nhwc,
-                                              grad_in);
-        count_launch();
-    } else {
-        FRR_CUDA(cudaMemsetAsync(grad_in, 0, (size_t)B * C * HW * sizeof(float), st));
-        if (K > 0) {
-            const size_t total = (size_t)K * C * PH * PW;
-            const int blocks =
-                (int)((total + 255) / 256 < (size_t)num_sms() * 16 ? (total + 255) / 256 : (size_t)num_sms() * 16);
-            roi_bwd_direct_kernel<kAlign><<<blocks, 256, 0, st>>>(grad_out, argmax, rois, total, B, C, H, W, PH, PW, scale,
-                                                                  sampling, aligned, nhwc, grad_in);
+    switch (pk.kernel) {
+        case kPoolBwdColorTail:
+        case kPoolBwdTail:
+            return roi_pool_bwd_fast_launch(pk, grad_out, argmax, rois, K, B, C, H, W, scale, nhwc, grad_in, stream);
+        case kAlignBwdFast:
+            return roi_align_bwd_fast_launch(pk, grad_out, rois, K, B, C, H, W, scale, aligned, nhwc, grad_in, stream);
+        case kAlignBwdStream:
+            FRR_CUDA(cudaMemsetAsync(grad_in, 0, (size_t)B * C * HW * sizeof(float), st));
+            roi_align_bwd_stream_kernel<<<K, kAlignStreamThreads, 0, st>>>(grad_out, rois, B, C, H, W, scale, aligned, nhwc,
+                                                                           grad_in);
             count_launch();
+            FRR_CHECK_LAUNCH("roi_align_bwd_stream_kernel");
+            return FRR_OK;
+        case kBwdPlanes: {
+            auto kern = roi_bwd_planes_kernel<kAlign>;
+            FRR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+            dim3 grid((C + pk.cb - 1) / pk.cb, B);
+            kern<<<grid, kRoiThreads, pk.smem, st>>>(grad_out, argmax, rois, K, C, H, W, pk.cb, PH, PW, scale, sampling, aligned,
+                                                     nhwc, grad_in);
+            count_launch();
+            break;
         }
+        default:  // kBwdDirect, or kRoiNone (no rois): the zeroed gradient
+            FRR_CUDA(cudaMemsetAsync(grad_in, 0, (size_t)B * C * HW * sizeof(float), st));
+            if (pk.kernel == kBwdDirect) {
+                const size_t total = (size_t)K * C * PH * PW;
+                roi_bwd_direct_kernel<kAlign><<<direct_blocks(total), 256, 0, st>>>(grad_out, argmax, rois, total, B, C, H, W, PH,
+                                                                                    PW, scale, sampling, aligned, nhwc, grad_in);
+                count_launch();
+            }
     }
     FRR_CHECK_LAUNCH("roi backward kernel");
     return FRR_OK;
@@ -557,6 +584,21 @@ int frr_roi_align_bwd(const float* grad_out, const float* rois, int K, int B, in
                       frr_stream_t stream) {
     return frr::roi_backward<true>(grad_out, nullptr, rois, K, B, C, H, W, PH, PW, spatial_scale, sampling_ratio, aligned,
                                    channels_last, grad_in, stream);
+}
+
+int frr_roi_variant(int op, int K, int B, int C, int H, int W, int PH, int PW, int sampling_ratio, int want_argmax,
+                    int32_t* out4) {
+    using namespace frr;
+    FRR_CHECK_ARG(out4 != nullptr, "frr_roi_variant: null output");
+    (void)want_argmax;  // selects the kArg instantiation of the same kernel, never another kernel
+    RoiPick pk;
+    const int rc = roi_pick(op, K, B, C, H, W, PH, PW, sampling_ratio, true, &pk);
+    if (rc) return rc;
+    out4[0] = pk.kernel;
+    out4[1] = pk.cb;
+    out4[2] = pk.nz;
+    out4[3] = (int32_t)pk.smem;
+    return FRR_OK;
 }
 
 }  // extern "C"

@@ -11,6 +11,30 @@ constexpr int kRoiThreads = 512;
 constexpr int kRoiTile = 256;  // rois staged per pass
 
 // ---------------------------------------------------------------------------------------------
+// host dispatch: which kernel an RoI entry point runs (ids as reported by frr_roi_variant)
+// ---------------------------------------------------------------------------------------------
+enum RoiKernel {
+    kRoiNone = -1,          // nothing is launched (forward without rois; backward without rois on planes too large for smem)
+    kPoolFwdFlat = 0,       // roi_pool_fwd_flat_kernel<cb, argmax>
+    kAlignFwdFast = 1,      // roi_align_fwd_fast_kernel<cb>
+    kFwdPlanes = 2,         // roi_fwd_planes_kernel<align>
+    kFwdDirect = 3,         // roi_fwd_direct_kernel<align>
+    kPoolBwdColorTail = 4,  // roi_pool_bwd_color_kernel<8> + roi_pool_bwd_tail_kernel (small rois)
+    kPoolBwdTail = 5,       // roi_pool_bwd_tail_kernel for every roi
+    kAlignBwdFast = 6,      // roi_align_bwd_fast_kernel<cb>
+    kAlignBwdStream = 7,    // roi_align_bwd_stream_kernel
+    kBwdPlanes = 8,         // roi_bwd_planes_kernel<align>
+    kBwdDirect = 9,         // roi_bwd_direct_kernel<align>
+};
+struct RoiPick {
+    int kernel;   // RoiKernel
+    int cb;       // channels per CTA (0: the kernel walks output elements or rois)
+    int nz;       // CTAs per (image, channel group)
+    int rp;       // roi_align_fwd_fast_kernel: rois per pass
+    size_t smem;  // dynamic shared memory bytes
+};
+
+// ---------------------------------------------------------------------------------------------
 // TMA 1-D bulk copy helpers (global -> shared with mbarrier completion; shared -> global)
 // ---------------------------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }

@@ -4,7 +4,7 @@
 // A CTA owns CB channel planes of ONE image; every feature element is read from HBM once and every output
 // element written once (HBM traffic = the algorithmic bytes), for NCHW and channels_last inputs alike.
 //
-// Forward (CB = 16, 8 or 4): the features are staged in shared memory PIXEL-MAJOR ([pixel][CB], chunk-rotated so that the
+// Forward (CB = 8 or 4): the features are staged in shared memory PIXEL-MAJOR ([pixel][CB], chunk-rotated so that the
 //   8 lanes of a quarter-warp hit 8 different bank groups unless their pixels agree mod 8): a thread owns one bin and
 //   ALL CB channels, so CB/4 LDS.128 feed CB running maxima and every loop / bounds / index instruction is shared by
 //   CB channels (one channel per thread cost 131 warp instructions per bin and channel, this layout ~25).  The
@@ -530,6 +530,10 @@ __global__ void __launch_bounds__(kFlatThreads, (CB <= 8) ? 2 : 1)
                                 FRR_UPD(vb[k].z, 4 * k + 2, idx + 1); FRR_UPD(vb[k].w, 4 * k + 3, idx + 1);
 #undef FRR_UPD
                             } else {
+                                // fmaxf orders -0.0 below +0.0: a window whose maximum is zero and that holds both
+                                // signs stores +0.0 where torchvision (first strict maximum) may store -0.0 -- the only
+                                // difference from the argmax path.  A strict compare here (setp + predicated move)
+                                // costs 10 % of the inference workload on a B200 (27.7k -> 25.0k images/s)
                                 best[4 * k + 0] = fmaxf(best[4 * k + 0], fmaxf(va[k].x, vb[k].x));
                                 best[4 * k + 1] = fmaxf(best[4 * k + 1], fmaxf(va[k].y, vb[k].y));
                                 best[4 * k + 2] = fmaxf(best[4 * k + 2], fmaxf(va[k].z, vb[k].z));
@@ -717,14 +721,12 @@ static size_t align_fwd_smem(int CB, int HW, int rp) {
 static size_t fwd_budget(int CB) { return CB <= 8 ? (kSmemLimit - 2048) / 2 : kSmemLimit; }
 
 template <int CB>
-static int launch_align_fwd(const float* feat, const float* rois, int K, int B, int C, int H, int W, float scale, int aligned,
-                            int nhwc, float* out, cudaStream_t st) {
+static int launch_align_fwd(const RoiPick& pk, const float* feat, const float* rois, int K, int B, int C, int H, int W,
+                            float scale, int aligned, int nhwc, float* out, cudaStream_t st) {
     auto kern = roi_align_fwd_fast_kernel<CB>;
-    int rp = align_fwd_rp(CB, H * W, fwd_budget(CB));
-    if (rp == 0) rp = align_fwd_rp(CB, H * W, kSmemLimit);
     FRR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimit));
-    kern<<<dim3((C + CB - 1) / CB, B), kFastFwdThreads, align_fwd_smem(CB, H * W, rp), st>>>(feat, rois, K, C, H, W, rp, scale,
-                                                                                              aligned, nhwc, out);
+    kern<<<dim3((C + CB - 1) / CB, B), kFastFwdThreads, pk.smem, st>>>(feat, rois, K, C, H, W, pk.rp, scale, aligned, nhwc,
+                                                                        out);
     return FRR_OK;
 }
 
@@ -732,55 +734,65 @@ static size_t flat_smem(int CB, int HW) {
     return kHdrBytes + ((kFlatGeoCap * 56 + 127) & ~(size_t)127) + (size_t)CB * HW * 4;
 }
 template <bool kArg, int CB>
-static int launch_flat(const float* feat, const float* rois, int K, int B, int C, int H, int W, float scale, int nhwc,
-                       float* out, int32_t* argmax, cudaStream_t st) {
+static int launch_flat(const RoiPick& pk, const float* feat, const float* rois, int K, int B, int C, int H, int W, float scale,
+                       int nhwc, float* out, int32_t* argmax, cudaStream_t st) {
     auto kern = roi_pool_fwd_flat_kernel<CB, kArg>;
     FRR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimit));
-    // fewer CTAs than resident slots (two per SM): split the rois of an image over 2 or 4 CTAs with the same planes
-    const long ctas = (long)B * ((C + CB - 1) / CB), slots = 2L * num_sms();
-    const int nz = (CB <= 8 && ctas * 4 <= slots) ? 4 : (CB <= 8 && ctas * 2 <= slots) ? 2 : 1;
-    kern<<<dim3((C + CB - 1) / CB, B, nz), kFlatThreads, flat_smem(CB, H * W), st>>>(feat, rois, K, C, H, W, scale, nhwc, out,
-                                                                                      argmax);
+    kern<<<dim3((C + CB - 1) / CB, B, pk.nz), kFlatThreads, pk.smem, st>>>(feat, rois, K, C, H, W, scale, nhwc, out, argmax);
     return FRR_OK;
 }
 
-int roi_fwd_fast(bool align, const float* feat, const float* rois, int K, int B, int C, int H, int W, int PH, int PW,
-                 float scale, int sampling, int aligned, int nhwc, float* out, int32_t* argmax, frr_stream_t stream) {
-    if (PH != 7 || PW != 7 || (align && sampling != 2) || H > 32767 || W > 32767) return 1;
-    const bool arg = !align && argmax != nullptr;
+// 7x7 forward fast paths: false = shape outside them (the caller takes the generic kernels)
+bool roi_fwd_fast_pick(bool align, int B, int C, int H, int W, int PH, int PW, int sampling, RoiPick* pk) {
+    if (PH != 7 || PW != 7 || (align && sampling != 2) || H > 32767 || W > 32767) return false;
     const int HW = H * W;
-    cudaStream_t st = (cudaStream_t)stream;
-    int rc;
     if (!align) {
-        // CB = 8 (else 4) when two CTAs fit an SM, else the largest of {16, 8, 4} that fits at all
+        // CB = 8 (else 4) when two CTAs fit an SM, else 8 or 4 at one CTA per SM (16 planes would need HW <= 3326, where
+        // 4 planes already fit twice)
         int cbk = 0;
         if (flat_smem(8, HW) <= fwd_budget(8)) cbk = 8;
         else if (flat_smem(4, HW) <= fwd_budget(4)) cbk = 4;
         // a single image (or a thin batch) with 8 channels per CTA leaves SMs without a CTA (1 x 512 / 8 = 64 CTAs on 148
         // SMs): 4 channels per CTA then
         if (cbk == 8 && (long)B * ((C + 7) / 8) < (long)num_sms()) cbk = 4;
-        for (int t = 16; t >= 4 && cbk == 0; t >>= 1)
+        for (int t = 8; t >= 4 && cbk == 0; t >>= 1)
             if (flat_smem(t, HW) <= kSmemLimit) cbk = t;
-        if (cbk == 0) return 1;
+        if (cbk == 0) return false;
+        // fewer CTAs than resident slots (two per SM): split the rois of an image over 2 or 4 CTAs with the same planes
+        const long ctas = (long)B * ((C + cbk - 1) / cbk), slots = 2L * num_sms();
+        const int nz = ctas * 4 <= slots ? 4 : ctas * 2 <= slots ? 2 : 1;
+        *pk = RoiPick{kPoolFwdFlat, cbk, nz, 0, flat_smem(cbk, HW)};
+        return true;
+    }
+    // 8 (else 4) channels at two CTAs per SM, else at one (16 would need HW <= 3042, where 4 already fit twice)
+    int cbk = 0, rp = 0;
+    for (int t = 8; t >= 4 && cbk == 0; t >>= 1)
+        if ((rp = align_fwd_rp(t, HW, fwd_budget(t))) > 0) cbk = t;
+    for (int t = 8; t >= 4 && cbk == 0; t >>= 1)
+        if ((rp = align_fwd_rp(t, HW, kSmemLimit)) > 0) cbk = t;
+    if (cbk == 0) return false;
+    *pk = RoiPick{kAlignFwdFast, cbk, 1, rp, align_fwd_smem(cbk, HW, rp)};
+    return true;
+}
+
+int roi_fwd_fast_launch(const RoiPick& pk, const float* feat, const float* rois, int K, int B, int C, int H, int W,
+                        float scale, int aligned, int nhwc, float* out, int32_t* argmax, frr_stream_t stream) {
+    cudaStream_t st = (cudaStream_t)stream;
+    int rc;
+    if (pk.kernel == kPoolFwdFlat) {
+        const bool arg = argmax != nullptr;
 #define FRR_FLAT(CBK)                                                                                   \
-    (arg ? launch_flat<true, CBK>(feat, rois, K, B, C, H, W, scale, nhwc, out, argmax, st)              \
-         : launch_flat<false, CBK>(feat, rois, K, B, C, H, W, scale, nhwc, out, argmax, st))
-        rc = cbk == 16 ? FRR_FLAT(16) : cbk == 8 ? FRR_FLAT(8) : FRR_FLAT(4);
+    (arg ? launch_flat<true, CBK>(pk, feat, rois, K, B, C, H, W, scale, nhwc, out, argmax, st)          \
+         : launch_flat<false, CBK>(pk, feat, rois, K, B, C, H, W, scale, nhwc, out, argmax, st))
+        rc = pk.cb == 8 ? FRR_FLAT(8) : FRR_FLAT(4);
 #undef FRR_FLAT
         if (rc) return rc;
         count_launch();
         FRR_CHECK_LAUNCH("roi_pool_fwd_flat_kernel");
         return FRR_OK;
     }
-    int cbk = 0;
-    for (int t = 8; t >= 4 && cbk == 0; t >>= 1)
-        if (align_fwd_rp(t, HW, fwd_budget(t)) > 0) cbk = t;
-    for (int t = 16; t >= 4 && cbk == 0; t >>= 1)
-        if (align_fwd_rp(t, HW, kSmemLimit) > 0) cbk = t;
-    if (cbk == 0) return 1;
-    rc = cbk == 16 ? launch_align_fwd<16>(feat, rois, K, B, C, H, W, scale, aligned, nhwc, out, st)
-         : cbk == 8 ? launch_align_fwd<8>(feat, rois, K, B, C, H, W, scale, aligned, nhwc, out, st)
-                    : launch_align_fwd<4>(feat, rois, K, B, C, H, W, scale, aligned, nhwc, out, st);
+    rc = pk.cb == 8 ? launch_align_fwd<8>(pk, feat, rois, K, B, C, H, W, scale, aligned, nhwc, out, st)
+                    : launch_align_fwd<4>(pk, feat, rois, K, B, C, H, W, scale, aligned, nhwc, out, st);
     if (rc) return rc;
     count_launch();
     FRR_CHECK_LAUNCH("roi_align_fwd_fast_kernel");
@@ -792,18 +804,19 @@ static size_t align_bwd_smem(int CB, int HW) {
 }
 
 template <int CB>
-static int launch_align_bwd(const float* go, const float* rois, int K, int B, int C, int H, int W, float scale, int aligned,
-                            int nhwc, float* gin, cudaStream_t st) {
+static int launch_align_bwd(const RoiPick& pk, const float* go, const float* rois, int K, int B, int C, int H, int W,
+                            float scale, int aligned, int nhwc, float* gin, cudaStream_t st) {
     auto kern = roi_align_bwd_fast_kernel<CB>;
     FRR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimit));
-    kern<<<dim3((C + CB - 1) / CB, B), CB * 32, align_bwd_smem(CB, H * W), st>>>(go, rois, K, C, H, W, scale, aligned, nhwc, gin);
+    kern<<<dim3((C + CB - 1) / CB, B), CB * 32, pk.smem, st>>>(go, rois, K, C, H, W, scale, aligned, nhwc, gin);
     return FRR_OK;
 }
 
-int roi_align_bwd_fast(const float* grad_out, const float* rois, int K, int B, int C, int H, int W, int PH, int PW,
-                       float scale, int sampling, int aligned, int nhwc, float* grad_in, frr_stream_t stream) {
+// 7x7 RoIAlign backward (sampling_ratio 2): the separable plane kernel or the streaming atomic kernel (roi.cu);
+// false = shape outside both (the caller takes the generic kernels)
+bool roi_align_bwd_fast_pick(int B, int C, int H, int W, int PH, int PW, int sampling, RoiPick* pk) {
     // every roi may touch at most kAbCols pixel columns: guaranteed when the map is no wider than that
-    if (PH != 7 || PW != 7 || sampling != 2 || W > kAbCols) return 1;
+    if (PH != 7 || PW != 7 || sampling != 2 || W > kAbCols) return false;
     const int HW = H * W;
     int cbk = 0;
     for (int t = 16; t >= 4; t >>= 1) {
@@ -811,14 +824,20 @@ int roi_align_bwd_fast(const float* grad_out, const float* rois, int K, int B, i
         cbk = t;
         if ((long)B * ((C + t - 1) / t) >= (long)num_sms()) break;
     }
-    if (cbk == 0) return 1;
+    if (cbk == 0) return false;
     // when 16 planes do not fit (maps above ~3400 pixels: 50 x 83) this kernel is left with 8 warps per SM and is latency
-    // bound (2.7 ms on the config-4 shape): the caller takes the streaming atomic kernel (1.9-2.3 ms)
-    if (align_bwd_smem(16, HW) > kSmemLimit) return 2;
+    // bound (2.7 ms on the config-4 shape): the streaming atomic kernel instead (1.9-2.3 ms)
+    if (align_bwd_smem(16, HW) > kSmemLimit) *pk = RoiPick{kAlignBwdStream, 0, 1, 0, 0};
+    else *pk = RoiPick{kAlignBwdFast, cbk, 1, 0, align_bwd_smem(cbk, HW)};
+    return true;
+}
+
+int roi_align_bwd_fast_launch(const RoiPick& pk, const float* grad_out, const float* rois, int K, int B, int C, int H, int W,
+                              float scale, int aligned, int nhwc, float* grad_in, frr_stream_t stream) {
     cudaStream_t st = (cudaStream_t)stream;
-    const int rc = cbk == 16 ? launch_align_bwd<16>(grad_out, rois, K, B, C, H, W, scale, aligned, nhwc, grad_in, st)
-                 : cbk == 8  ? launch_align_bwd<8>(grad_out, rois, K, B, C, H, W, scale, aligned, nhwc, grad_in, st)
-                             : launch_align_bwd<4>(grad_out, rois, K, B, C, H, W, scale, aligned, nhwc, grad_in, st);
+    const int rc = pk.cb == 16 ? launch_align_bwd<16>(pk, grad_out, rois, K, B, C, H, W, scale, aligned, nhwc, grad_in, st)
+                 : pk.cb == 8  ? launch_align_bwd<8>(pk, grad_out, rois, K, B, C, H, W, scale, aligned, nhwc, grad_in, st)
+                               : launch_align_bwd<4>(pk, grad_out, rois, K, B, C, H, W, scale, aligned, nhwc, grad_in, st);
     if (rc) return rc;
     count_launch();
     FRR_CHECK_LAUNCH("roi_align_bwd_fast_kernel");

@@ -423,35 +423,42 @@ static size_t pool_bwd_color_smem(int CB, int HW) {
 }
 
 template <int CB>
-static int launch_pool_bwd_color(const float* go, const int32_t* argmax, const float* rois, int K, int B, int C, int H, int W,
-                                 float scale, int nhwc, float* gin, cudaStream_t st) {
+static int launch_pool_bwd_color(const RoiPick& pk, const float* go, const int32_t* argmax, const float* rois, int K, int B,
+                                 int C, int H, int W, float scale, int nhwc, float* gin, cudaStream_t st) {
     auto kern = roi_pool_bwd_color_kernel<CB>;
     FRR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPbSmemLimit));
-    kern<<<dim3((C + CB - 1) / CB, B), CB * 16, pool_bwd_color_smem(CB, H * W), st>>>(go, argmax, rois, K, C, H, W, scale, nhwc,
-                                                                                        gin);
+    kern<<<dim3((C + CB - 1) / CB, B), CB * 16, pk.smem, st>>>(go, argmax, rois, K, C, H, W, scale, nhwc, gin);
     return FRR_OK;
 }
 
-// 0 = launched, 1 = outside this path (caller falls back), < 0 = error
-int roi_pool_bwd_color(const float* grad_out, const int32_t* argmax, const float* rois, int K, int B, int C, int H, int W,
-                       int PH, int PW, float scale, int nhwc, float* grad_in, int force_tail, frr_stream_t stream) {
-    if (PH != 7 || PW != 7 || K > kPbIdMask) return 1;
-    if ((reinterpret_cast<uintptr_t>(grad_out) & 3u) || (reinterpret_cast<uintptr_t>(argmax) & 3u)) return 1;
+// 7x7 RoIPool backward: colour classes + tail, or the tail kernel for every roi (force_tail: FRR_ROI_POOL_BWD=tail).
+// false = outside this path (the caller takes the generic kernels)
+bool roi_pool_bwd_fast_pick(int K, int H, int W, int PH, int PW, bool ptrs_aligned, bool force_tail, RoiPick* pk) {
+    if (PH != 7 || PW != 7 || K > kPbIdMask || !ptrs_aligned) return false;
     const int HW = H * W;
-    cudaStream_t st = (cudaStream_t)stream;
     // Two co-resident CTAs of 8 planes (one zeroes / scans / stores while the other accumulates) when they fit: the
     // 37 x 62 map of a 600 x 1000 image.  Larger maps (50 x 83 of an 800 x 1333 image: 4 accumulating warps per SM)
     // are faster with every roi through the streaming atomic kernel (measured 216-300 us against 287-330 us, torchvision
     // 320-341 us).
-    int cbk = 2 * (pool_bwd_color_smem(8, HW) + 1024) <= kPbSmemLimit ? 8 : 0;
-    if (cbk == 0 || force_tail) {
+    if (2 * (pool_bwd_color_smem(8, HW) + 1024) <= kPbSmemLimit && !force_tail)
+        *pk = RoiPick{kPoolBwdColorTail, 8, 1, 0, pool_bwd_color_smem(8, HW)};
+    else
+        *pk = RoiPick{kPoolBwdTail, 0, 1, 0, 0};
+    return true;
+}
+
+int roi_pool_bwd_fast_launch(const RoiPick& pk, const float* grad_out, const int32_t* argmax, const float* rois, int K, int B,
+                             int C, int H, int W, float scale, int nhwc, float* grad_in, frr_stream_t stream) {
+    const int HW = H * W;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (pk.kernel == kPoolBwdTail) {
         FRR_CUDA(cudaMemsetAsync(grad_in, 0, (size_t)B * C * HW * sizeof(float), st));
         roi_pool_bwd_tail_kernel<<<K, 256, 0, st>>>(grad_out, argmax, rois, B, C, H, W, scale, nhwc, 1, grad_in);
         count_launch();
         FRR_CHECK_LAUNCH("roi_pool_bwd_tail_kernel");
         return FRR_OK;
     }
-    const int rc = launch_pool_bwd_color<8>(grad_out, argmax, rois, K, B, C, H, W, scale, nhwc, grad_in, st);
+    const int rc = launch_pool_bwd_color<8>(pk, grad_out, argmax, rois, K, B, C, H, W, scale, nhwc, grad_in, st);
     if (rc) return rc;
     count_launch();
     FRR_CHECK_LAUNCH("roi_pool_bwd_color_kernel");

@@ -183,6 +183,29 @@ def nms_variant(B: int, n: int, iou_threshold: float, max_keep: int | None = Non
     return dict(cluster_size=out[0], threads=out[1], variant=NMS_VARIANTS[out[2]], smem=out[3])
 
 
+ROI_OPS = {"roi_pool_fwd": 0, "roi_pool_bwd": 1, "roi_align_fwd": 2, "roi_align_bwd": 3}
+ROI_KERNELS = {-1: "none", 0: "pool_fwd_flat", 1: "align_fwd_fast", 2: "fwd_planes", 3: "fwd_direct",
+               4: "pool_bwd_color_tail", 5: "pool_bwd_tail", 6: "align_bwd_fast", 7: "align_bwd_stream", 8: "bwd_planes",
+               9: "bwd_direct"}
+
+
+def roi_variant(op: str, K: int, B: int, C: int, H: int, W: int, output_size=(7, 7), sampling_ratio: int = 2,
+                want_argmax: bool = True, device=None) -> dict:
+    """Kernel the RoI entry point ``op`` (a key of ROI_OPS) picks for this problem (host query, launches nothing).
+    Without a CUDA device the choice is made for 148 SMs."""
+    import ctypes
+    out = (ctypes.c_int32 * 4)()
+    args = (ROI_OPS[op], int(K), int(B), int(C), int(H), int(W), int(output_size[0]), int(output_size[1]),
+            int(sampling_ratio), int(bool(want_argmax)), out)
+    lib = _lib.load()
+    if torch.cuda.is_available():
+        with torch.cuda.device(device if device is not None else torch.cuda.current_device()):
+            _lib.check(lib.frr_roi_variant(*args), "frr_roi_variant")
+    else:
+        _lib.check(lib.frr_roi_variant(*args), "frr_roi_variant")
+    return dict(kernel=ROI_KERNELS[out[0]], cb=out[1], nz=out[2], smem=out[3])
+
+
 # ------------------------------------------------------------------------------------------------
 # RoIPool / RoIAlign (R1-R4): raw kernels + autograd functions
 # ------------------------------------------------------------------------------------------------

@@ -180,6 +180,8 @@ int frr_rpn_proposals_opt(const float* reg, const float* cls, int cls_is_logits,
  *        rois [K,5] = (batch index, x1,y1,x2,y2) fp32; out/argmax [K,C,PH,PW] contiguous
  *        (argmax int32 = h*W+w, -1 for empty bins; may be NULL in inference).
  *        Forward max/argmax bit-exact vs torchvision CPU; backward within 1e-5 (fp32 sum order).
+ *        Exception: with argmax == NULL, a 7x7 bin whose maximum is zero may hold +0.0 where torchvision
+ *        (first strict maximum) holds -0.0; the values compare equal and every other bit matches.
  * ------------------------------------------------------------------------------------- */
 /* R1 glue -- models/model.py:104-110 (roi * [fw,fh,fw,fh]) + TV ops/_utils.py:18-25 (list of per-image rois ->
  * Tensor[K,5] with the batch index): rois [B,R,4] normalised (e.g. the output of frr_rpn_proposals), count [B] or
@@ -215,6 +217,17 @@ int frr_roi_align_bwd(const float* grad_out, const float* rois, int K, int B, in
  * launches fill one [K,C,PH,PW] output without gathers or host synchronisation.  L = k_max - k_min + 1. */
 int frr_fpn_level_rois(const float* rois5, int K, int k_min, int k_max, int canonical_level, float canonical_scale, int L,
                        int32_t* levels, float* rois_per_level, frr_stream_t stream);
+
+/* Which kernel the RoI entry points pick (host only, launches nothing; tests assert through it that the kernel they mean
+ * to exercise is the one that runs).  op: 0 frr_roi_pool_fwd, 1 frr_roi_pool_bwd, 2 frr_roi_align_fwd,
+ * 3 frr_roi_align_bwd; want_argmax: the forward's argmax != NULL (same kernel either way).  Assumes 4-byte aligned
+ * grad_out / argmax and reads FRR_ROI_POOL_BWD like the launchers.  out4 = (kernel id, channels per CTA (0: the kernel
+ * walks output elements or rois), CTAs per (image, channel group), dynamic shared memory bytes).  Kernel ids:
+ * -1 nothing launched (no rois), 0 RoIPool forward flat, 1 RoIAlign forward fast, 2 forward planes, 3 forward direct,
+ * 4 RoIPool backward colour classes + tail, 5 RoIPool backward tail only, 6 RoIAlign backward fast,
+ * 7 RoIAlign backward stream, 8 backward planes, 9 backward direct. */
+int frr_roi_variant(int op, int K, int B, int C, int H, int W, int PH, int PW, int sampling_ratio, int want_argmax,
+                    int32_t* out4);
 
 /* Developer hook: per-phase clock64() cycles of CTA (0,0) of the 7x7 fast kernels, accumulated since the last call
  * (16 slots, see roi_fast.cu); copies to host_out16 and clears.  Synchronises the device. */

@@ -32,12 +32,10 @@ SIGNATURES = {
     "frr_rpn_decode": (_i, [_p, _p, _i, _p, _p, _i, _i, _i, _i, _f, _p, _p, _p, _i, _i, _p]),
     "frr_topk_desc": (_i, [_p, _p, _p, _i, _i, _i, _p, _p, _p, _p, _p, _p]),
     "frr_topk_desc_opt": (_i, [_p, _p, _p, _i, _i, _i, _p, _p, _p, _p, _p, _i, _p]),
-    "frr_topk_desc_profile": (_i, [_p, _p, _p, _i, _i, _i, _p, _p, _p, _p, _p, _p, _p]),
     "frr_nms_sorted": (_i, [_p, _p, _i, _i, _d, _i, _p, _p, _p, _i, _p]),
     "frr_rpn_proposals_workspace_bytes": (C.c_size_t, [_i, _i, _i, _i]),
     "frr_rpn_proposals": (_i, [_p, _p, _i, _p, _p, _i, _i, _i, _i, _f, _i, _i, _i, _i, _d, _p, _p, _p, C.c_size_t, _p]),
     "frr_rpn_proposals_opt": (_i, [_p, _p, _i, _p, _p, _i, _i, _i, _i, _f, _i, _i, _i, _i, _d, _p, _p, _p, C.c_size_t, _i, _p]),
-    "frr_nms_bucket_tune": (_i, [_i, _i, _i, _i]),
     "frr_nms_variant": (_i, [_i, _i, _d, _i, _i, _i, _i, _p]),
     "frr_rpn_proposals_workspace_layout": (_i, [_i, _i, _i, _i, _p]),
     "frr_nms_sorted_indirect": (_i, [_p, _i, _p, _p, _i, _i, _d, _i, _p, _p, _p, _i, _i, _p]),
@@ -47,7 +45,6 @@ SIGNATURES = {
     "frr_roi_align_fwd": (_i, [_p, _p, _i, _i, _i, _i, _i, _i, _i, _f, _i, _i, _i, _p, _p]),
     "frr_roi_align_bwd": (_i, [_p, _p, _i, _i, _i, _i, _i, _i, _i, _f, _i, _i, _i, _p, _p]),
     "frr_roi_variant": (_i, [_i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p]),
-    "frr_roi_debug_cycles": (_i, [_p]),
     "frr_fpn_level_rois": (_i, [_p, _i, _i, _i, _i, _f, _i, _p, _p, _p]),
     "frr_region_loss": (_i, [_p, _p, _p, _p, _i, _i, _p, _p, _p, _p, _i, _i, _i, _f, _f, _p, _p, _p, _p, _p, _p]),
     "frr_sample_targets": (_i, [_p, _p, _i, _i, _i, _i, _i, _p, _i, _p, _p, _p, _p, _p, _i, _p, _p, _i, _p]),
@@ -59,7 +56,7 @@ SIGNATURES = {
     "frr_pack_detections": (_i, [_p, _p, _p, _p, _i, _i, _i, _p, _i, _p, _p, _p]),
     "frr_class_nms_workspace_bytes": (C.c_size_t, [_i, _i, _i]),
     "frr_class_nms": (_i, [_p, _p, _p, _i, _i, _i, _f, _d, _i, _p, _p, _p, _p, _p, C.c_size_t, _p]),
-    "frr_nms_sorted_tuned": (_i, [_p, _p, _i, _i, _d, _i, _p, _p, _p, _i, _i, _p, _i, _p]),
+    "frr_nms_sorted_tuned": (_i, [_p, _p, _i, _i, _d, _i, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _p]),
 }
 
 
@@ -94,7 +91,7 @@ def load():
             fn = getattr(lib, name)
             fn.restype = res
             fn.argtypes = args
-        if lib.frr_abi_version() != 1:
+        if lib.frr_abi_version() != 2:
             raise FrrError("libfrr.so ABI version mismatch")
         _lib = lib
     return _lib

@@ -60,14 +60,11 @@ __device__ __forceinline__ bool bar_or(int id, int n, bool pred) {
     return r != 0;
 }
 
-enum { DBG_CHUNKS = 0, DBG_LOAD, DBG_P1, DBG_SYNC, DBG_P2, DBG_P3, DBG_P4, DBG_P5, DBG_SURV, DBG_ITERS, DBG_N };
-
 template <int kThreads, bool kFast, bool kUnit>
 __global__ void __launch_bounds__(kThreads)
     nms_keeplist_kernel(const float4* __restrict__ boxes, const int32_t* __restrict__ counts, int n, int max_keep,
                         int slice_cap, NmsThr thr, int32_t* __restrict__ keep, int32_t* __restrict__ keep_count,
-                        float4* __restrict__ out_boxes, long long* __restrict__ dbg,
-                        const int32_t* __restrict__ gather_idx, int src_n) {
+                        float4* __restrict__ out_boxes, const int32_t* __restrict__ gather_idx, int src_n) {
     static_assert(kThreads >= kChunk && kThreads % kGroup == 0, "bad thread count");
     constexpr int kWarps = kThreads / 32;
     constexpr int kParts = kThreads / kGroup;  // interleaved parts of the kept slice
@@ -93,22 +90,12 @@ __global__ void __launch_bounds__(kThreads)
     auto cand = [&](int i) -> float4 { return gi ? ib[gi[i]] : ib[i]; };
     int32_t* ikeep = keep + (size_t)img * max_keep;
     float4* iout = out_boxes ? out_boxes + (size_t)img * max_keep : nullptr;
-    const bool prof = (dbg != nullptr) && blockIdx.x == 0 && tid == 0;
-    long long t0 = 0;
-#define FRR_TICK(slot)                  \
-    if (prof) {                         \
-        const long long t1 = clock64(); \
-        dbg[slot] += t1 - t0;           \
-        t0 = t1;                        \
-    }
-
     int nk = 0;  // kept so far (identical in every CTA of the cluster)
     int par = 0;
     float4 nbx = make_float4(0.f, 0.f, 0.f, 0.f);  // prefetched candidate of the next chunk (first kChunk threads)
     if (tid < kChunk && tid < cnt) nbx = cand(tid);
     if (tid < 2 * kChunkWords) (&sm->acc[0][0])[tid] = 0u;
     for (int base = 0; base < cnt && nk < max_keep; base += kChunk, par ^= 1) {
-        if (prof) { t0 = clock64(); dbg[DBG_CHUNKS] += 1; }
         // ---- phase 0: stage the chunk's candidates in shared memory, prefetch the next chunk ----------
         if (tid < kChunk) {
             sm->cbox[tid] = nbx;
@@ -117,7 +104,6 @@ __global__ void __launch_bounds__(kThreads)
             if (nx < cnt) nbx = cand(nx);
         }
         __syncthreads();
-        FRR_TICK(DBG_LOAD);
 
         const int ns = (nk - rank + S - 1) / S;  // kept ordinals o with o % S == rank
         // ---- phase 1: 4 candidates per thread vs this CTA's slice of the kept list ----------------------
@@ -179,9 +165,7 @@ __global__ void __launch_bounds__(kThreads)
             unsigned int* dst = cluster.map_shared_rank(&sm->supp[par][rank][wd], dstr);
             *dst = sm->acc[par][wd];
         }
-        FRR_TICK(DBG_P1);
         cluster.sync();
-        FRR_TICK(DBG_SYNC);
 
         // ---- phase 2: combine the S words per 32 candidates, compact survivors (first kChunk threads) ---
         bool alive = false;
@@ -220,8 +204,6 @@ __global__ void __launch_bounds__(kThreads)
             }
         }
         __syncthreads();
-        FRR_TICK(DBG_P2);
-        if (prof) dbg[DBG_SURV] += s;
 
         // ---- phase 3: predecessor masks among survivors.  3a: warp item = (row, 32-column word), screen only (two
         //      words per trip for ILP); 3b: the few set bits are refined with the exact test, one (row, word) entry
@@ -263,7 +245,6 @@ __global__ void __launch_bounds__(kThreads)
             }
         }
         __syncthreads();
-        FRR_TICK(DBG_P3);
 
         // ---- phase 4: parallel fix-point over the survivors (first kChunk threads, named barrier 1).
         //      survivor i is kept once every predecessor that suppresses it is removed; removed as soon
@@ -294,14 +275,12 @@ __global__ void __launch_bounds__(kThreads)
                     sm->removed_w[cur ^ 1][warp] = rm;
                 }
                 cur ^= 1;
-                if (prof) dbg[DBG_ITERS] += 1;
                 if (!bar_or(1, kChunk, state == 0)) break;
             }
             fin = cur;
         }
         // every thread needs the final buffer index: it is uniform over the first kChunk threads
         fin = __syncthreads_or(fin);
-        FRR_TICK(DBG_P4);
 
         // ---- phase 5: append kept survivors --------------------------------------------------------------
         {
@@ -332,9 +311,7 @@ __global__ void __launch_bounds__(kThreads)
             nk = min(nk + ktot, max_keep);
         }
         __syncthreads();
-        FRR_TICK(DBG_P5);
     }
-#undef FRR_TICK
 
     if (rank == 0) {
         for (int o = nk + tid; o < max_keep; o += kThreads) {
@@ -402,7 +379,7 @@ static int nms_pick(int B, int n, double iou_thr, int max_keep, int cluster_size
 
 int nms_launch(const float* boxes, const int32_t* counts, int B, int n, double iou_thr, int max_keep,
                       int32_t* keep, int32_t* keep_count, float* out_boxes, int cluster_size, int threads,
-                      long long* dbg, int unit_boxes, frr_stream_t stream, const int32_t* gather_idx, int src_n) {
+                      const NmsTune& tune, int unit_boxes, frr_stream_t stream, const int32_t* gather_idx, int src_n) {
     FRR_CHECK_ARG(keep && keep_count, "frr_nms_sorted: null output");
     FRR_CHECK_ARG(n == 0 || (boxes && aligned16(boxes)), "frr_nms_sorted: boxes must be non-null, 16-byte aligned");
     FRR_CHECK_ARG(out_boxes == nullptr || aligned16(out_boxes), "frr_nms_sorted: out_boxes must be 16-byte aligned");
@@ -413,15 +390,15 @@ int nms_launch(const float* boxes, const int32_t* counts, int B, int n, double i
     }
     if (B == 0) return FRR_OK;
     if (pk.bucketed)
-        return nms_bucket_launch(boxes, counts, B, n, pk.thr, max_keep, keep, keep_count, out_boxes, pk.S, pk.threads, dbg,
+        return nms_bucket_launch(boxes, counts, B, n, pk.thr, max_keep, keep, keep_count, out_boxes, pk.S, pk.threads, tune,
                                  stream, gather_idx, src_n);
     const int S = pk.S, slice_cap = pk.slice_cap;
     threads = pk.threads;
     const size_t smem = pk.smem, limit = 227 * 1024;
     const NmsThr thr = pk.thr;
 
-    using kern_t = void (*)(const float4*, const int32_t*, int, int, int, NmsThr, int32_t*, int32_t*, float4*, long long*,
-                            const int32_t*, int);
+    using kern_t = void (*)(const float4*, const int32_t*, int, int, int, NmsThr, int32_t*, int32_t*, float4*, const int32_t*,
+                            int);
     kern_t kern = nullptr;
 #define FRR_NMS_PICK(F, U)                                                                      \
     (threads < kChunk * 2 ? nms_keeplist_kernel<kChunk, F, U>                                            \
@@ -446,7 +423,7 @@ int nms_launch(const float* boxes, const int32_t* counts, int B, int n, double i
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     FRR_CUDA(cudaLaunchKernelEx(&cfg, kern, (const float4*)boxes, counts, n, max_keep, slice_cap, thr, keep, keep_count,
-                                (float4*)out_boxes, dbg, gather_idx, src_n));
+                                (float4*)out_boxes, gather_idx, src_n));
     count_launch();
     FRR_CHECK_LAUNCH("nms_keeplist_kernel");
     return FRR_OK;
@@ -457,15 +434,23 @@ int nms_launch(const float* boxes, const int32_t* counts, int B, int n, double i
 extern "C" int frr_nms_sorted(const float* boxes, const int32_t* counts, int B, int n, double iou_thr, int max_keep,
                               int32_t* keep, int32_t* keep_count, float* out_boxes, int cluster_size,
                               frr_stream_t stream) {
-    return frr::nms_launch(boxes, counts, B, n, iou_thr, max_keep, keep, keep_count, out_boxes, cluster_size, 0, nullptr,
+    return frr::nms_launch(boxes, counts, B, n, iou_thr, max_keep, keep, keep_count, out_boxes, cluster_size, 0, frr::NmsTune{},
                            0, stream, nullptr, 0);
 }
 
 extern "C" int frr_nms_sorted_tuned(const float* boxes, const int32_t* counts, int B, int n, double iou_thr, int max_keep,
                                     int32_t* keep, int32_t* keep_count, float* out_boxes, int cluster_size, int threads,
-                                    int64_t* dbg_cycles, int unit_boxes, frr_stream_t stream) {
+                                    int first_chunk, int max_chunk, int lanes_screen, int lanes_pairs, int unit_boxes,
+                                    frr_stream_t stream) {
+    using frr::kBkChunk;
+    auto chunk_ok = [](int v) { return v == 0 || (v >= 256 && v <= kBkChunk); };
+    auto lanes_ok = [](int v) { return v == 0 || (v >= 1 && v <= 32 && (v & (v - 1)) == 0); };
+    FRR_CHECK_ARG(chunk_ok(first_chunk) && chunk_ok(max_chunk),
+                  "frr_nms_sorted_tuned: chunk sizes must be 0 or lie in [256, %d]", kBkChunk);
+    FRR_CHECK_ARG(lanes_ok(lanes_screen) && lanes_ok(lanes_pairs),
+                  "frr_nms_sorted_tuned: lanes per candidate must be 0 or a power of two <= 32");
     return frr::nms_launch(boxes, counts, B, n, iou_thr, max_keep, keep, keep_count, out_boxes, cluster_size, threads,
-                           (long long*)dbg_cycles, unit_boxes, stream, nullptr, 0);
+                           frr::NmsTune{first_chunk, max_chunk, lanes_screen, lanes_pairs}, unit_boxes, stream, nullptr, 0);
 }
 
 // Which kernel variant / launch geometry frr_nms_sorted* picks for a problem (host only, launches nothing):
@@ -490,6 +475,6 @@ extern "C" int frr_nms_sorted_indirect(const float* boxes_src, int src_n, const 
                                        int n, double iou_thr, int max_keep, int32_t* keep, int32_t* keep_count,
                                        float* out_boxes, int cluster_size, int unit_boxes, frr_stream_t stream) {
     FRR_CHECK_ARG(order != nullptr && src_n >= 0, "frr_nms_sorted_indirect: order must be given");
-    return frr::nms_launch(boxes_src, counts, B, n, iou_thr, max_keep, keep, keep_count, out_boxes, cluster_size, 0, nullptr,
+    return frr::nms_launch(boxes_src, counts, B, n, iou_thr, max_keep, keep, keep_count, out_boxes, cluster_size, 0, frr::NmsTune{},
                            unit_boxes, stream, order, src_n);
 }

@@ -26,24 +26,17 @@
 // pairs that provably cannot suppress.  tests/nms_model.py restates this algorithm on the CPU.
 #include <cooperative_groups.h>
 
-#include <atomic>
-
 #include "nms_common.cuh"
 
 namespace cg = cooperative_groups;
 
 namespace frr {
 
-constexpr int kBkChunk = 2048;     // most candidates per chunk (shared-memory arrays are sized for it)
 constexpr int kBkListCap = 2048;   // kept-list capacity (max_keep <= 2047)
 constexpr int kBkEdgeCap = 8192;   // edges per chunk over the whole cluster (each CTA owns kBkEdgeCap / S)
 constexpr int kBkBins = 3;         // x bins of a walk whose bounds are prefetched (more: tail loop)
 constexpr int kBkUpBins = 2;       // same for the upward walk (bins above the own one)
 constexpr int kBkHits = 4;         // screen hits a thread parks per walk before it falls back to the slow walk
-
-// lanes_screen 0 = automatic: 2 lanes per candidate when an image has 1-2 CTAs (batched launches: 146 vs 153 us with one
-// CTA per image, tools/nms_s1_sweep.py), 4 in the large clusters of the single-image form (81 vs 85 us)
-static std::atomic<int> g_bk_kc0{1024}, g_bk_kcmax{2048}, g_bk_nsub1{0}, g_bk_nsub2{4};
 
 struct BkSmem {
     unsigned int lhist[kKeyCap];  // kept list: key histogram, then scatter cursors
@@ -65,11 +58,6 @@ struct BkSmem {
     unsigned char pend[kBkChunk];
     unsigned char ovf[kBkChunk];
     unsigned int hitbuf[1024 * 4];  // per-thread ring of screen hits (phase H)
-};
-
-enum {
-    BK_CHUNKS = 0, BK_LOAD, BK_SCAN, BK_SCATTER, BK_SCREEN, BK_SYNC1, BK_SURV_SORT, BK_PRED, BK_SYNC2, BK_FIX, BK_APPEND,
-    BK_ROUNDS, BK_SURVIVORS, BK_EDGES, BK_VISITED, BK_OVF
 };
 
 // One warp: in-place exclusive scan of hist[0 .. kKeyCap) (kKeyPer consecutive entries per lane), optionally also
@@ -254,8 +242,7 @@ template <int kThreads>
 __global__ void __launch_bounds__(kThreads)
     nms_bucket_kernel(const float4* __restrict__ boxes, const int32_t* __restrict__ counts, int n, int max_keep, NmsThr thr,
                       int32_t* __restrict__ keep, int32_t* __restrict__ keep_count, float4* __restrict__ out_boxes,
-                      long long* __restrict__ dbg, const int32_t* __restrict__ gather_idx, int src_n, int kc0, int kc_max, int nsub1,
-                      int nsub2) {
+                      const int32_t* __restrict__ gather_idx, int src_n, int kc0, int kc_max, int nsub1, int nsub2) {
     cg::cluster_group cluster = cg::this_cluster();
     const int S = (int)cluster.num_blocks();
     const int rank = (int)cluster.block_rank();
@@ -278,15 +265,6 @@ __global__ void __launch_bounds__(kThreads)
     float4* iout = out_boxes ? out_boxes + (size_t)img * max_keep : nullptr;
     const int ecap = kBkEdgeCap / S;
 
-    const bool prof = (dbg != nullptr) && blockIdx.x == 0 && tid == 0;
-    long long t0 = 0;
-#define BK_TICK(slot)                   \
-    if (prof) {                         \
-        const long long t1 = clock64(); \
-        dbg[slot] += t1 - t0;           \
-        t0 = t1;                        \
-    }
-
     for (int e = tid; e < kKeyCap; e += kThreads) {
         sm->lhist[e] = 0u;
         sm->chist[e] = 0u;
@@ -308,7 +286,6 @@ __global__ void __launch_bounds__(kThreads)
     int kc = kc0;
     for (int base = 0; base < cnt && nk < max_keep; par ^= 1) {
         const int m = min(kc, cnt - base);
-        if (prof) { t0 = clock64(); dbg[BK_CHUNKS] += 1; dbg[BK_VISITED] += m; }
         unsigned char* st = sm->cstate[par];
         // ---- A: stage the chunk (screening areas, keys), histograms of the list keys and of the own candidates' keys
         for (int i = tid; i < m; i += kThreads) {
@@ -324,12 +301,10 @@ __global__ void __launch_bounds__(kThreads)
         }
         for (int k = tid; k < nk; k += kThreads) atomicAdd(&sm->lhist[bk_key(bbox[cur][k], barea[cur][k])], 1u);
         __syncthreads();
-        BK_TICK(BK_LOAD);
         // ---- B: exclusive scans (warp 0: list, warp 1: own candidates)
         if (warp == 0) bk_scan_keys(sm->lhist, sm->lstart, lane);
         else if (warp == 1) bk_scan_keys(sm->chist, nullptr, lane);
         __syncthreads();
-        BK_TICK(BK_SCAN);
         // ---- C: scatter the list into the other buffer, the own candidates into cord
         for (int k = tid; k < nk; k += kThreads) {
             const float4 b = bbox[cur][k];
@@ -342,7 +317,6 @@ __global__ void __launch_bounds__(kThreads)
             if (i % S == rank) sm->cord[atomicAdd(&sm->chist[sm->ckey[i]], 1u)] = (unsigned short)i;
         cur ^= 1;
         __syncthreads();
-        BK_TICK(BK_SCATTER);
         const float4* lb = bbox[cur];
         const float* la = barea[cur];
         // ---- D: screen the own candidates against the admissible part of the kept list: nsub1 lanes per candidate,
@@ -378,9 +352,7 @@ __global__ void __launch_bounds__(kThreads)
                 }
             }
         }
-        BK_TICK(BK_SCREEN);
         cluster_sync();
-        BK_TICK(BK_SYNC1);
         // ---- E: histogram of the survivors' keys; reset what the next chunk's phases A-D accumulate into
         for (int i = tid; i < kBkChunk; i += kThreads) sm->cstate[par ^ 1][i] = 0;
         for (int e = tid; e < kKeyCap; e += kThreads) {
@@ -415,8 +387,6 @@ __global__ void __launch_bounds__(kThreads)
             sm->sidx[p] = (unsigned short)i;
         }
         __syncthreads();
-        BK_TICK(BK_SURV_SORT);
-        if (prof) dbg[BK_SURVIVORS] += ns;
         // ---- H: suppression pairs among the survivors, every pair from its lower bucketed position (nsub2 lanes per
         //      survivor, dealt like phase D)
         {
@@ -475,12 +445,9 @@ __global__ void __launch_bounds__(kThreads)
             }
             if (tid < S) *cluster.map_shared_rank(&sm->ecount[rank], tid) = (unsigned int)ne;
         }
-        BK_TICK(BK_PRED);
         cluster_sync();
-        BK_TICK(BK_SYNC2);
         // ---- I: fix-point (every CTA on all survivors and all edges)
         for (;;) {
-            if (prof) dbg[BK_ROUNDS] += 1;
             {   // a thread works on one region: regions fill evenly (positions are dealt round-robin)
                 const int r = tid % S;
                 const int ne = (int)sm->ecount[r];
@@ -531,9 +498,6 @@ __global__ void __launch_bounds__(kThreads)
             }
             if (!__syncthreads_or(any)) break;
         }
-        BK_TICK(BK_FIX);
-        if (prof)
-            for (int r = 0; r < S; ++r) dbg[BK_EDGES] += sm->ecount[r];
         // ---- J: append the kept survivors in score order
         int kept_chunk;
         {
@@ -578,9 +542,7 @@ __global__ void __launch_bounds__(kThreads)
             kc = (int)min((long long)kc_max, max(256LL, next));
         }
         __syncthreads();
-        BK_TICK(BK_APPEND);
     }
-#undef BK_TICK
 
     if (rank == 0) {
         for (int o = nk + tid; o < max_keep; o += kThreads) {
@@ -601,24 +563,27 @@ size_t nms_bucket_smem_bytes() {
 }
 
 int nms_bucket_launch(const float* boxes, const int32_t* counts, int B, int n, const NmsThr& thr, int max_keep, int32_t* keep,
-                      int32_t* keep_count, float* out_boxes, int S, int threads, long long* dbg, frr_stream_t stream,
+                      int32_t* keep_count, float* out_boxes, int S, int threads, const NmsTune& tune, frr_stream_t stream,
                       const int32_t* gather_idx, int src_n) {
-    using kern_t = void (*)(const float4*, const int32_t*, int, int, NmsThr, int32_t*, int32_t*, float4*, long long*,
-                            const int32_t*, int, int, int, int, int);
+    using kern_t = void (*)(const float4*, const int32_t*, int, int, NmsThr, int32_t*, int32_t*, float4*, const int32_t*,
+                            int, int, int, int, int);
     kern_t kern = threads <= 256 ? nms_bucket_kernel<256> : threads == 512 ? nms_bucket_kernel<512> : nms_bucket_kernel<1024>;
     if (threads < 256) threads = 256;
     const size_t smem = nms_bucket_smem_bytes();
     FRR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     if (S > 8) FRR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
-    // first chunk: small when few boxes are wanted (test mode: 300), at most kc0
-    int kc_max = g_bk_kcmax.load(std::memory_order_relaxed);
-    int kc0 = g_bk_kc0.load(std::memory_order_relaxed);
-    kc_max = kc_max < 256 ? 256 : (kc_max > kBkChunk ? kBkChunk : (kc_max & ~255));
+    // chunk sizes (frr_nms_sorted_tuned has checked them to lie in [256, kBkChunk]): the first chunk is small when few
+    // boxes are wanted (test mode: 300), at most first_chunk (automatic: 1024)
+    const int kc_max = tune.max_chunk ? tune.max_chunk & ~255 : kBkChunk;
     int want = ((max_keep + max_keep / 2) + 255) & ~255;
     if (want < 256) want = 256;
-    kc0 = kc0 < 256 ? 256 : (kc0 & ~255);
+    int kc0 = tune.first_chunk ? tune.first_chunk & ~255 : 1024;
     if (kc0 > want) kc0 = want;
     if (kc0 > kc_max) kc0 = kc_max;
+    // lanes per candidate, automatic: 2 in the screen when an image has 1-2 CTAs (batched launches: 146 vs 153 us with
+    // one CTA per image, tools/nms_s1_sweep.py), 4 in the large clusters of the single-image form (81 vs 85 us)
+    const int nsub1 = tune.lanes_screen ? tune.lanes_screen : (S <= 2 ? 2 : 4);
+    const int nsub2 = tune.lanes_pairs ? tune.lanes_pairs : 4;
 
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)(B * S), 1, 1);
@@ -633,29 +598,10 @@ int nms_bucket_launch(const float* boxes, const int32_t* counts, int B, int n, c
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     FRR_CUDA(cudaLaunchKernelEx(&cfg, kern, (const float4*)boxes, counts, n, max_keep, thr, keep, keep_count,
-                                (float4*)out_boxes, dbg, gather_idx, src_n, kc0, kc_max,
-                                g_bk_nsub1.load(std::memory_order_relaxed) ? g_bk_nsub1.load(std::memory_order_relaxed)
-                                                                           : (S <= 2 ? 2 : 4),
-                                g_bk_nsub2.load(std::memory_order_relaxed)));
+                                (float4*)out_boxes, gather_idx, src_n, kc0, kc_max, nsub1, nsub2));
     count_launch();
     FRR_CHECK_LAUNCH("nms_bucket_kernel");
     return FRR_OK;
 }
 
 }  // namespace frr
-
-// Developer knob (profiling tools): sizes of the first chunk and of the largest chunk of the bucketed kernel
-// (multiples of 256, <= 2048) and the lanes per candidate in the screen / pair phases (1, 2, 4, ... 32; 0 keeps the
-// current value).  Process-wide; results never depend on them.
-extern "C" int frr_nms_bucket_tune(int first_chunk, int max_chunk, int lanes_screen, int lanes_pairs) {
-    FRR_CHECK_ARG(first_chunk >= 256 && max_chunk >= 256 && first_chunk <= frr::kBkChunk && max_chunk <= frr::kBkChunk,
-                  "frr_nms_bucket_tune: chunk sizes must lie in [256, %d]", frr::kBkChunk);
-    auto pow2 = [](int v) { return v >= 1 && v <= 32 && (v & (v - 1)) == 0; };
-    FRR_CHECK_ARG((lanes_screen == 0 || pow2(lanes_screen)) && (lanes_pairs == 0 || pow2(lanes_pairs)),
-                  "frr_nms_bucket_tune: lanes per candidate must be a power of two <= 32");
-    frr::g_bk_kc0.store(first_chunk);
-    frr::g_bk_kcmax.store(max_chunk);
-    frr::g_bk_nsub1.store(lanes_screen);  // (0: back to automatic)
-    if (lanes_pairs) frr::g_bk_nsub2.store(lanes_pairs);
-    return FRR_OK;
-}

@@ -9,13 +9,10 @@
 //       2. the cluster keep-list NMS kernel of nms.cu over the B*(C-1) sorted lists at IoU 0.3
 //          (double-threshold compare: IoU == 0.3f is suppressed, as torchvision's CPU kernel);
 //       3. one CTA per image: class-major compaction into [B, cap, 4] boxes / labels (l-1) / scores.
-#include "frr_common.cuh"
+#include "nms_common.cuh"
 
 namespace frr {
 
-int nms_launch(const float* boxes, const int32_t* counts, int B, int n, double iou_thr, int max_keep, int32_t* keep,
-               int32_t* keep_count, float* out_boxes, int cluster_size, int threads, long long* dbg, int unit_boxes,
-               frr_stream_t stream, const int32_t* gather_idx = nullptr, int src_n = 0);
 
 // ------------------------------------------------------------------------------------------------ D1
 // one warp per roi row
@@ -255,7 +252,7 @@ int frr_class_nms(const float* prob, const float* boxes, const int32_t* roi_coun
         count_launch();
         FRR_CHECK_LAUNCH("class_sort_kernel");
         int rc = nms_launch((const float*)sboxes, counts, (int)P, R, iou_thr, R, keep, keep_count, (float*)kboxes, 1, 256,
-                            nullptr, 0, stream);
+                            NmsTune{}, 0, stream);
         if (rc) return rc;
     } else {
         FRR_CUDA(cudaMemsetAsync(keep_count, 0, P * 4, st));

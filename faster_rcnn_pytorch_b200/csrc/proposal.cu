@@ -1,16 +1,13 @@
 // RegionProposal.forward for a batch in ONE C-ABI call (models/model.py:17-58): decode + clip + min-size
 // -> top-k -> NMS -> first post_nms_top_k boxes.  Three kernel launches on the caller's stream, every
 // intermediate lives in the caller-provided workspace; no allocation, no synchronisation, graph-capturable.
-#include "frr_common.cuh"
+#include "nms_common.cuh"
 
 namespace frr {
 
 int topk_desc_impl(const float* scores, const uint8_t* valid, const float* boxes, int B, int N, int k, float* out_scores,
                    int32_t* out_idx, int32_t* out_cidx, float* out_boxes, int32_t* out_count, int cluster_hint,
                    frr_stream_t stream);
-int nms_launch(const float* boxes, const int32_t* counts, int B, int n, double iou_thr, int max_keep, int32_t* keep,
-               int32_t* keep_count, float* out_boxes, int cluster_size, int threads, long long* dbg, int unit_boxes,
-               frr_stream_t stream, const int32_t* gather_idx = nullptr, int src_n = 0);
 
 struct ProposalWs {
     size_t boxes, scores, valid, top_idx, top_count, keep, total;
@@ -104,7 +101,7 @@ int frr_rpn_proposals_opt(const float* reg, const float* cls, int cls_is_logits,
                         nms_cluster_size == 1 ? 1 : 0, stream);
     if (rc) return rc;
     // the decoded boxes are clamped to [0,1] (models/model.py:34): unit-range screening
-    return nms_launch(boxes, top_count, B, k, iou_thr, post_nms_top_k, keep, roi_count, rois, nms_cluster_size, 0, nullptr, 1,
+    return nms_launch(boxes, top_count, B, k, iou_thr, post_nms_top_k, keep, roi_count, rois, nms_cluster_size, 0, NmsTune{}, 1,
                       stream, top_idx, N);
 }
 

@@ -14,9 +14,6 @@
 //
 // Numerics: RoIPool max/argmax bit-exact (first strict maximum in h-then-w order, -FLT_MAX start,
 // empty bin -> 0/-1); RoIAlign sums w1*v1+w2*v2+w3*v3+w4*v4 left to right without FMA contraction.
-#include <stdlib.h>
-#include <string.h>
-
 #include "roi_common.cuh"
 
 namespace frr {
@@ -358,18 +355,9 @@ int roi_fwd_fast_launch(const RoiPick& pk, const float* feat, const float* rois,
 bool roi_align_bwd_fast_pick(int B, int C, int H, int W, int PH, int PW, int sampling, RoiPick* pk);
 int roi_align_bwd_fast_launch(const RoiPick& pk, const float* grad_out, const float* rois, int K, int B, int C, int H, int W,
                               float scale, int aligned, int nhwc, float* grad_in, frr_stream_t stream);
-bool roi_pool_bwd_fast_pick(int K, int H, int W, int PH, int PW, bool ptrs_aligned, bool force_tail, RoiPick* pk);
+bool roi_pool_bwd_fast_pick(int K, int H, int W, int PH, int PW, bool ptrs_aligned, RoiPick* pk);
 int roi_pool_bwd_fast_launch(const RoiPick& pk, const float* grad_out, const int32_t* argmax, const float* rois, int K, int B,
                              int C, int H, int W, float scale, int nhwc, float* grad_in, frr_stream_t stream);
-
-// developer knob (A/B measurements only): FRR_ROI_POOL_BWD=tail sends every roi through the streaming atomic kernel
-static int pool_bwd_force_tail() {
-    static const int v = [] {
-        const char* e = getenv("FRR_ROI_POOL_BWD");
-        return (e && !strcmp(e, "tail")) ? 1 : 0;
-    }();
-    return v;
-}
 
 static size_t roi_smem_bytes(int CB, int HW) {
     return ((sizeof(RoiSmemHdr) + 127) & ~(size_t)127) + (size_t)CB * HW * sizeof(float);
@@ -403,7 +391,7 @@ static int roi_pick(int op, int K, int B, int C, int H, int W, int PH, int PW, i
         if (roi_fwd_fast_pick(align, B, C, H, W, PH, PW, sampling, pk)) return FRR_OK;
     } else if (K > 0) {
         if (align ? roi_align_bwd_fast_pick(B, C, H, W, PH, PW, sampling, pk)
-                  : roi_pool_bwd_fast_pick(K, H, W, PH, PW, ptrs_aligned, pool_bwd_force_tail() != 0, pk))
+                  : roi_pool_bwd_fast_pick(K, H, W, PH, PW, ptrs_aligned, pk))
             return FRR_OK;
     }
     const int cb = pick_cb(B, C, HW);

@@ -26,15 +26,6 @@ namespace frr {
 constexpr int kFastFwdThreads = 448;
 constexpr int kIdCap = 512;  // rois scanned per tile (one per thread, blockDim <= 512)
 
-// developer instrumentation: clock64() cycles of CTA (0,0) per phase, accumulated over launches
-__device__ long long g_roi_dbg[16];
-#define ROI_TICK(slot)                          \
-    if (prof) {                                 \
-        const long long t1_ = clock64();        \
-        g_roi_dbg[slot] += t1_ - t0_;           \
-        t0_ = t1_;                              \
-    }
-
 struct FastHdr {
     int cnt[16];
     int id[kIdCap];
@@ -277,10 +268,7 @@ __global__ void __launch_bounds__(kFastFwdThreads, (CB <= 8) ? 2 : 1)
     const int b = blockIdx.y, c0 = blockIdx.x * CB;
     const int HW = H * W;
     const int cb = min(CB, C - c0);
-    const bool prof = (blockIdx.x == 0 && blockIdx.y == 0 && tid == 0);
-    long long t0_ = clock64();
     load_pixels<CB, false>(px, feat, b, c0, C, HW, nhwc != 0);
-    ROI_TICK(0);
 
     // thread -> (roi slot rs, bin): the 49 bins of a roi sit in consecutive lanes
     const int rs = tid / 49;
@@ -293,7 +281,6 @@ __global__ void __launch_bounds__(kFastFwdThreads, (CB <= 8) ? 2 : 1)
 
     for (int tile = 0; tile < K; tile += kFastFwdThreads) {
         const int ns = stage_ids(rois, K, tile, b, hd);
-        ROI_TICK(1);
         for (int p0 = 0; p0 < ns; p0 += RP) {
             const int nr = min(RP, ns - p0);
             // ---- 14 y-sample and 14 x-sample records per roi, once per roi ---------------------------------
@@ -304,7 +291,6 @@ __global__ void __launch_bounds__(kFastFwdThreads, (CB <= 8) ? 2 : 1)
                                   : align_rec(sample_x(gm, (j - 14) >> 1, (j - 14) & 1), W);
             }
             __syncthreads();
-            ROI_TICK(2);
             if (worker) {
 #pragma unroll 1
                 for (int s = rs; s < nr; s += RS) {
@@ -342,7 +328,6 @@ __global__ void __launch_bounds__(kFastFwdThreads, (CB <= 8) ? 2 : 1)
                 }
             }
             __syncthreads();
-            ROI_TICK(3);
             // ---- copy-out: the cb*49 values of a roi are contiguous in the output -> coalesced 16-byte stores;
             //      warp w takes rois w, w + 14, ...: no index divisions
             {
@@ -358,10 +343,8 @@ __global__ void __launch_bounds__(kFastFwdThreads, (CB <= 8) ? 2 : 1)
                 }
             }
             __syncthreads();  // the staging tile and the sample records are rewritten next
-            ROI_TICK(4);
         }
     }
-    ROI_TICK(5);
 }
 
 // NCHW planes -> the planar staging layout ([chunk][pixel] of float4 = 4 channels) with 4-byte cp.async: no registers
@@ -416,13 +399,10 @@ __global__ void __launch_bounds__(kFlatThreads, (CB <= 8) ? 2 : 1)
     const int b = blockIdx.y, c0 = blockIdx.x * CB;
     const int HW = H * W;
     const int cb = min(CB, C - c0);
-    const bool prof = (blockIdx.x == 0 && blockIdx.y == 0 && tid == 0);
-    long long t0_ = clock64();
     if (nhwc)
         load_pixels<CB, true>(px, feat, b, c0, C, HW, true);
     else
         load_planes_async<CB>(px, feat, b, c0, C, HW);  // lands behind the roi scan and the bin geometry
-    ROI_TICK(0);
 
     constexpr int kScanPer = 6;  // 448 x 6 = 2688 rois per scan round
     for (int k0 = 0; k0 < K; k0 += kScanPer * kFlatThreads) {
@@ -445,7 +425,6 @@ __global__ void __launch_bounds__(kFlatThreads, (CB <= 8) ? 2 : 1)
             ns = mine;
             if (ns <= 0) continue;  // block-uniform
         }
-        ROI_TICK(1);
         for (int g0 = 0; g0 < ns; g0 += kFlatGeoCap) {
             const int ng = min(kFlatGeoCap, ns - g0);
             // one thread per (roi, dimension): the rounded roi once, then the 7 window starts and 7 window ends
@@ -466,7 +445,6 @@ __global__ void __launch_bounds__(kFlatThreads, (CB <= 8) ? 2 : 1)
             if (tid == 0) hd->cnt[15] = 0;  // slice counter of this group
             cp_async_wait_all();    // this thread's share of the planes (first group only; nothing pending afterwards)
             __syncthreads();
-            ROI_TICK(2);
             // With argmax (training): the (roi, bin) sequence of the group -- rois in descending window size -- is cut into
             // slices of 32 consecutive bins and the warps take the next slice from a shared counter as they finish (largest
             // first: the warps of a CTA end within one small slice of each other; fixed shares of ~9 rois per warp left them
@@ -553,14 +531,11 @@ __global__ void __launch_bounds__(kFlatThreads, (CB <= 8) ? 2 : 1)
                         if (c < cb) __stcs(argmax + o + c * 49, bidx[c]);
                 }
             }
-            ROI_TICK(3);
             __syncthreads();  // the boundaries (and, after the last group, the id list) are rewritten next
-            ROI_TICK(4);
         }
     }
     }
     cp_async_wait_all();  // (a CTA without rois leaves with nothing in flight)
-    ROI_TICK(5);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -845,23 +820,3 @@ int roi_align_bwd_fast_launch(const RoiPick& pk, const float* grad_out, const fl
 }
 
 }  // namespace frr
-
-// Developer hook: copies the 16 phase counters (cycles of CTA (0,0): forward 0 plane load, 1 roi scan, 2 geometry +
-// buffer wait, 3 compute, 4 store issue, 5 drain; backward 8 zero, 9 roi scan, 10 accumulate, 11 tile syncs,
-// 12 plane store) to the host and clears them.  Synchronises the device.
-namespace frr { void pool_bwd_debug_fetch(long long* host_out8); }
-extern "C" int frr_roi_debug_cycles(int64_t* host_out16) {
-    FRR_CHECK_ARG(host_out16 != nullptr, "frr_roi_debug_cycles: null pointer");
-    long long z[16] = {0};
-    FRR_CUDA(cudaMemcpyFromSymbol(host_out16, frr::g_roi_dbg, sizeof(z)));
-    FRR_CUDA(cudaMemcpyToSymbol(frr::g_roi_dbg, z, sizeof(z)));
-    // slots 8-15 when the colour-class RoIPool backward ran (roi_pool_bwd.cu): 8 wait full, 9 ring loads + adds, 10 release,
-    // 11 producer wait empty, 12 producer issue, 13 roi scan, 14 zero, 15 store
-    long long pb[8];
-    frr::pool_bwd_debug_fetch(pb);
-    bool any = false;
-    for (int i = 0; i < 8; ++i) any = any || pb[i] != 0;
-    if (any)
-        for (int i = 0; i < 8; ++i) host_out16[8 + i] = pb[i];
-    return FRR_OK;
-}

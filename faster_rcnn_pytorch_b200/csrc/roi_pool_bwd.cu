@@ -29,7 +29,6 @@
 // The contract on argmax is torchvision's: it comes from the forward call on the same rois and map shape (an index
 // outside [0, H*W) is ignored instead of written out of bounds).
 #include <stddef.h>
-#include <stdlib.h>
 
 #include "roi_common.cuh"
 
@@ -54,16 +53,6 @@ __host__ __device__ constexpr int ring_pos(int half, int bin) {
     const int i = (ph >> 1) * ((pw & 1) ? 3 : 4) + (pw >> 1);
     return (half * 16 + i) * 4 + q;
 }
-
-// developer instrumentation: clock64() cycles of CTA (0,0) warp 0, accumulated over launches (0 accumulate loop, 5 roi
-// scan, 6 zero, 7 store); read through frr_roi_debug_cycles (slots 8-15)
-__device__ long long g_pb_dbg[8];
-#define PB_TICK(slot)                           \
-    if (prof) {                                 \
-        const long long t1_ = clock64();        \
-        acc_[slot] += t1_ - t0_;                \
-        t0_ = t1_;                              \
-    }
 
 // shared memory through 32-bit shared-window addresses (no generic -> shared conversion inside the loops); volatile +
 // "memory": the read-modify-write steps of a warp stay in program order
@@ -221,9 +210,6 @@ __global__ void __launch_bounds__(CB * 16)
     const int HW = H * W;
     const int cb = min(CB, C - c0);
 
-    const bool prof = blockIdx.x == 0 && blockIdx.y == 0 && tid == 0;
-    long long t0_ = clock64();
-    long long acc_[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     {
         float4* p4 = reinterpret_cast<float4*>(planes);
         const int n4 = CB * HW / 4;
@@ -232,7 +218,6 @@ __global__ void __launch_bounds__(CB * 16)
         // argmax positions of bins that do not exist (classes with fewer than 16 bins) stay -1 for good
         for (int i = tid; i < kWarps * D * (kPbSlotBytes / 4); i += blockDim.x) ring[i] = -1;
     }
-    PB_TICK(6);
 
     // the shared-window base, converted once inside a volatile asm (the compiler would otherwise rematerialise the
     // conversion -- an S2R -- inside the loop)
@@ -269,7 +254,6 @@ __global__ void __launch_bounds__(CB * 16)
     for (int k0 = 0; k0 < K; k0 += kPbIdCap) {
         // (the barriers of the scan also order the initialisation above)
         const int n = collect_rois<kPbIdCap / (CB * 16)>(rois, K, k0, b, scale, hd);
-        PB_TICK(5);
         if (npl > 0 && n > 0) {
             // copies of roi r into the ring slot at byte offset `so` (always commits a group; past the end of the list
             // nothing is read)
@@ -337,16 +321,9 @@ __global__ void __launch_bounds__(CB * 16)
             }
             cp_async_wait<0>();
         }
-        PB_TICK(0);
         __syncthreads();  // the id list is rewritten by the next round
     }
     store_planes(planes, grad_in, b, c0, cb, C, HW, nhwc != 0);
-    PB_TICK(7);
-    if (prof) {
-#pragma unroll
-        for (int i = 0; i < 8; ++i)
-            if (acc_[i]) atomicAdd(reinterpret_cast<unsigned long long*>(&g_pb_dbg[i]), (unsigned long long)acc_[i]);
-    }
 }
 
 // The rois the plane kernel skipped (pb_small): one CTA per roi, which leaves at once unless the roi is small; a small
@@ -411,12 +388,6 @@ __global__ void __launch_bounds__(256)
     }
 }
 
-void pool_bwd_debug_fetch(long long* host_out8) {
-    long long z[8] = {0};
-    cudaMemcpyFromSymbol(host_out8, g_pb_dbg, sizeof(z));
-    cudaMemcpyToSymbol(g_pb_dbg, z, sizeof(z));
-}
-
 static const size_t kPbSmemLimit = 227 * 1024;
 static size_t pool_bwd_color_smem(int CB, int HW) {
     return kPbHdrBytes + (size_t)(CB / 2) * kPbDepth * kPbSlotBytes + (size_t)CB * HW * 4;
@@ -431,16 +402,16 @@ static int launch_pool_bwd_color(const RoiPick& pk, const float* go, const int32
     return FRR_OK;
 }
 
-// 7x7 RoIPool backward: colour classes + tail, or the tail kernel for every roi (force_tail: FRR_ROI_POOL_BWD=tail).
+// 7x7 RoIPool backward: colour classes + tail, or the tail kernel for every roi.
 // false = outside this path (the caller takes the generic kernels)
-bool roi_pool_bwd_fast_pick(int K, int H, int W, int PH, int PW, bool ptrs_aligned, bool force_tail, RoiPick* pk) {
+bool roi_pool_bwd_fast_pick(int K, int H, int W, int PH, int PW, bool ptrs_aligned, RoiPick* pk) {
     if (PH != 7 || PW != 7 || K > kPbIdMask || !ptrs_aligned) return false;
     const int HW = H * W;
     // Two co-resident CTAs of 8 planes (one zeroes / scans / stores while the other accumulates) when they fit: the
     // 37 x 62 map of a 600 x 1000 image.  Larger maps (50 x 83 of an 800 x 1333 image: 4 accumulating warps per SM)
     // are faster with every roi through the streaming atomic kernel (measured 216-300 us against 287-330 us, torchvision
     // 320-341 us).
-    if (2 * (pool_bwd_color_smem(8, HW) + 1024) <= kPbSmemLimit && !force_tail)
+    if (2 * (pool_bwd_color_smem(8, HW) + 1024) <= kPbSmemLimit)
         *pk = RoiPick{kPoolBwdColorTail, 8, 1, 0, pool_bwd_color_smem(8, HW)};
     else
         *pk = RoiPick{kPoolBwdTail, 0, 1, 0, 0};

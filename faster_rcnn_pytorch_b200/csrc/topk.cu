@@ -223,26 +223,13 @@ static size_t topk_smem_bytes(int nchunks, int P) {
 
 int topk_radix_launch(const float* scores, const uint8_t* valid, const float* boxes, int B, int N, int k,
                       float* out_scores, int32_t* out_idx, int32_t* out_cidx, float* out_boxes, int32_t* out_count,
-                      long long* dbg, frr_stream_t stream, int cluster_hint);
+                      frr_stream_t stream, int cluster_hint);
 
 int topk_desc_impl(const float* scores, const uint8_t* valid, const float* boxes, int B, int N, int k, float* out_scores,
                    int32_t* out_idx, int32_t* out_cidx, float* out_boxes, int32_t* out_count, int cluster_hint,
                    frr_stream_t stream);
 
 }  // namespace frr
-
-// Profiling variant: dbg = int64[16] accumulating clock64() cycles of CTA 0 per phase: [0..4] radix kernel (load+validity,
-// select, compaction, sort, write-out; only when image 0 was handed over), [8..13] bucket kernel (load + min/max,
-// histogram, scan, scatter, bucket sorts, write-out).  Returns FRR_E_UNSUPPORTED outside the fast path.
-extern "C" int frr_topk_desc_profile(const float* scores, const uint8_t* valid, const float* boxes, int B, int N, int k,
-                                     float* out_scores, int32_t* out_idx, int32_t* out_cidx, float* out_boxes,
-                                     int32_t* out_count, int64_t* dbg_cycles, frr_stream_t stream) {
-    using namespace frr;
-    FRR_CHECK_ARG(scores && out_idx && out_count && dbg_cycles && B > 0 && N > 0 && k > 0, "frr_topk_desc_profile: bad arguments");
-    const int rc = topk_radix_launch(scores, valid, boxes, B, N, k, out_scores, out_idx, out_cidx, out_boxes, out_count,
-                                     (long long*)dbg_cycles, stream, 1);
-    return rc == 1 ? FRR_E_UNSUPPORTED : rc;
-}
 
 extern "C" int frr_topk_desc(const float* scores, const uint8_t* valid, const float* boxes, int B, int N, int k,
                              float* out_scores, int32_t* out_idx, int32_t* out_cidx, float* out_boxes,
@@ -271,7 +258,7 @@ int frr::topk_desc_impl(const float* scores, const uint8_t* valid, const float* 
     FRR_CHECK_ARG(k <= 16384, "frr_topk_desc: k=%d exceeds the in-smem sort capacity 16384", k);
     {   // fast path: shared-memory radix sort (topk_radix.cu); shapes outside it take the bitonic kernel below
         const int rc = topk_radix_launch(scores, valid, boxes, B, N, k, out_scores, out_idx, out_cidx, out_boxes, out_count,
-                                         nullptr, stream, cluster_hint);
+                                         stream, cluster_hint);
         if (rc <= 0) return rc;
     }
     int P = 32;

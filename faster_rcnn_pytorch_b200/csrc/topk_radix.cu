@@ -1,6 +1,7 @@
 // P4 (fast path): pre-NMS top-k, sorted descending, ties lower-index-first (models/model.py:44-49).
 // Two algorithms in one launch: topk_bucket_kernel (below, the default) and the radix path described here, which it falls
-// into for inputs that do not bucket and which also runs alone when the bucket kernel's shared memory does not fit.
+// into for inputs that do not bucket.  The bucket kernel's shared memory fits for every shape the fast path takes
+// (static_assert at bucket_smem), so the radix path never runs as a kernel of its own.
 //
 // Radix path: one CTA (1024 threads) per image, everything after the first read of the scores stays in shared memory:
 //   0. validity words (ballot) + the order-preserving uint32 keys of all N scores staged in shared memory;
@@ -15,7 +16,6 @@
 // Compared with the bitonic version (105 compare-exchange stages with a barrier each, contended histogram
 // atomics) this is ~10x fewer shared-memory wavefronts and barriers.  HBM bytes: 5N in, 40k out per image.
 #include <cooperative_groups.h>
-#include <stdlib.h>
 
 #include "frr_common.cuh"
 
@@ -41,7 +41,7 @@ struct RsLayout {
     int db;  // digit bits of the sort passes (5 when the 2^db x 1024 u16 counters fit, else 4)
 };
 
-__host__ __device__ static inline size_t up16(size_t x) { return (x + 15) & ~(size_t)15; }
+__host__ __device__ constexpr size_t up16(size_t x) { return (x + 15) & ~(size_t)15; }
 
 static RsLayout rs_layout(int N, int kcap, int nchunks, bool want_stage, int db) {
     RsLayout L;
@@ -77,24 +77,15 @@ __device__ __forceinline__ unsigned int match_digit8(unsigned int d, bool act) {
     return m;
 }
 
-// The whole radix top-k of image blockIdx.x in the CTA's dynamic shared memory: the body of topk_radix_kernel, and the
-// path topk_bucket_kernel falls into for inputs that do not bucket.
+// The whole radix top-k of image blockIdx.x (or img) in the CTA's dynamic shared memory: the path the bucket kernels fall
+// into for inputs that do not bucket.
 template <bool kStaged>
 __device__ __forceinline__ void topk_radix_body(unsigned char* smem, const float* __restrict__ scores,
                                                 const uint8_t* __restrict__ valid, const float4* __restrict__ boxes, int N,
                                                 int k, int kcap, int nchunks, const RsLayout& L,
                                                 float* __restrict__ out_scores, int32_t* __restrict__ out_idx,
                                                 int32_t* __restrict__ out_cidx, float4* __restrict__ out_boxes,
-                                                int32_t* __restrict__ out_count, long long* __restrict__ dbg,
-                                                int img = -1) {
-    const bool prof = (dbg != nullptr) && blockIdx.x == 0 && threadIdx.x == 0;
-    long long t0 = prof ? clock64() : 0;
-#define RS_TICK(slot)                   \
-    if (prof) {                         \
-        const long long t1 = clock64(); \
-        dbg[slot] += t1 - t0;           \
-        t0 = t1;                        \
-    }
+                                                int32_t* __restrict__ out_count, int img = -1) {
     RsHdr* hd = reinterpret_cast<RsHdr*>(smem);
     unsigned int* vbits = reinterpret_cast<unsigned int*>(smem + L.vbits);
     unsigned int* gpre = reinterpret_cast<unsigned int*>(smem + L.gpre);
@@ -151,7 +142,6 @@ __device__ __forceinline__ void topk_radix_body(unsigned char* smem, const float
         if (tid == 0) hd->nvalid = run;
     }
     __syncthreads();
-    RS_TICK(0);
     const int keff = min(k, (int)hd->nvalid);
     if (tid == 0) {
         out_count[b] = keff;
@@ -237,7 +227,6 @@ __device__ __forceinline__ void topk_radix_body(unsigned char* smem, const float
         __syncthreads();  // the list (keyA) is dead from here on
         const unsigned int T = prefix;
         const unsigned int take_ties = hd->remaining;
-        RS_TICK(1);
 
         // ---- 2. order-preserving compaction ---------------------------------------------------------------
         for (int c = warp; c < nchunks; c += kRsWarps) {
@@ -277,7 +266,6 @@ __device__ __forceinline__ void topk_radix_body(unsigned char* smem, const float
         }
         __syncthreads();
 
-        RS_TICK(2);
         // ---- 3. stable LSD radix sort of keyA/idxA[0..keff) --------------------------------------------------
         // Thread t owns the `ipt` consecutive pairs [t*ipt, (t+1)*ipt) (ipt odd: conflict-free strided LDS) and a PRIVATE
         // u16 counter per digit, cnt[d][t]: counting and ranking are plain LDS / STS (no ballots, no atomics; the
@@ -363,7 +351,6 @@ __device__ __forceinline__ void topk_radix_body(unsigned char* smem, const float
             for (int i = tid; i < keff; i += kRsThreads) { keyA[i] = srcK[i]; idxA[i] = srcI[i]; }
             __syncthreads();
         }
-        RS_TICK(3);
     }
 
     // ---- 4. write-out (4 independent gathers in flight per thread) ------------------------------------------
@@ -396,19 +383,6 @@ __device__ __forceinline__ void topk_radix_body(unsigned char* smem, const float
         }
     }
     __syncthreads();
-    RS_TICK(4);
-#undef RS_TICK
-}
-
-template <bool kStaged>
-__global__ void __launch_bounds__(kRsThreads, 1)
-    topk_radix_kernel(const float* __restrict__ scores, const uint8_t* __restrict__ valid,
-                      const float4* __restrict__ boxes, int N, int k, int kcap, int nchunks, RsLayout L,
-                      float* __restrict__ out_scores, int32_t* __restrict__ out_idx, int32_t* __restrict__ out_cidx,
-                      float4* __restrict__ out_boxes, int32_t* __restrict__ out_count, long long* __restrict__ dbg) {
-    extern __shared__ __align__(16) unsigned char smem[];
-    topk_radix_body<kStaged>(smem, scores, valid, boxes, N, k, kcap, nchunks, L, out_scores, out_idx, out_cidx, out_boxes,
-                             out_count, dbg);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -420,7 +394,7 @@ __global__ void __launch_bounds__(kRsThreads, 1)
 //   bucket ranges (unordered, atomic cursors) and every bucket is insertion-sorted by one thread on the EXACT total
 //   order (ordered key descending, index ascending) -- the same order the radix kernel produces, so ties and the cut
 //   inside b* are bit-identical.  Inputs that do not bucket well (non-finite range, a bucket of > kBucketMax, more than
-//   `cap` stored pairs: e.g. all scores equal) are handed to the radix kernel through out_count = -1.
+//   `cap` stored pairs: e.g. all scores equal) are redone on the radix path in the same CTA.
 constexpr int kBuckets = 8192;
 constexpr int kBucketMax = 192;
 constexpr int kBucketSlack = 1024;  // pairs stored beyond k (the rest of bucket b*)
@@ -437,17 +411,8 @@ __global__ void __launch_bounds__(kRsThreads, 1)
     topk_bucket_kernel(const float* __restrict__ scores, const uint8_t* __restrict__ valid,
                        const float4* __restrict__ boxes, int N, int k, int cap, int nchunks,
                        float* __restrict__ out_scores, int32_t* __restrict__ out_idx, int32_t* __restrict__ out_cidx,
-                       float4* __restrict__ out_boxes, int32_t* __restrict__ out_count, long long* __restrict__ dbg,
-                       RsLayout L, int kcap) {
+                       float4* __restrict__ out_boxes, int32_t* __restrict__ out_count, RsLayout L, int kcap) {
     extern __shared__ __align__(16) unsigned char smem[];
-    const bool prof = (dbg != nullptr) && blockIdx.x == 0 && threadIdx.x == 0;
-    long long t0 = prof ? clock64() : 0;
-#define BK_TICK(slot)                   \
-    if (prof) {                         \
-        const long long t1 = clock64(); \
-        dbg[slot] += t1 - t0;           \
-        t0 = t1;                        \
-    }
     BkHdr* hd = reinterpret_cast<BkHdr*>(smem);
     size_t o = up16(sizeof(BkHdr));
     unsigned int* vbits = reinterpret_cast<unsigned int*>(smem + o); o += 4 * (size_t)nchunks;
@@ -527,7 +492,6 @@ __global__ void __launch_bounds__(kRsThreads, 1)
         if (tid == 0) hd->nvalid = run;
     }
     __syncthreads();
-    BK_TICK(0);
     const int keff = min(k, (int)hd->nvalid);
     const float smax = hd->smax;
     const float scale = (float)kBuckets / (smax - hd->smin);
@@ -542,7 +506,6 @@ __global__ void __launch_bounds__(kRsThreads, 1)
             if ((vbits[c] >> lane) & 1u) atomicAdd(&hist[bucket_of(score_at(i))], 1u);
         }
         __syncthreads();
-        BK_TICK(1);
         // ---- 2. bucket starts, the bucket b* of the k-th largest score, the largest bucket up to b* ----------
         {
             constexpr int kPerT = kBuckets / kRsThreads;
@@ -576,13 +539,12 @@ __global__ void __launch_bounds__(kRsThreads, 1)
             handover = hd->bad != 0u;
         }
     }
-    BK_TICK(2);
     if (handover) {  // block-uniform: the radix path redoes this image from scratch in the same shared memory
         __syncthreads();
         if (L.staged) topk_radix_body<true>(smem, scores, valid, boxes, N, k, kcap, nchunks, L, out_scores, out_idx, out_cidx,
-                                            out_boxes, out_count, dbg ? dbg - 8 : nullptr);
+                                            out_boxes, out_count);
         else topk_radix_body<false>(smem, scores, valid, boxes, N, k, kcap, nchunks, L, out_scores, out_idx, out_cidx,
-                                    out_boxes, out_count, dbg ? dbg - 8 : nullptr);
+                                    out_boxes, out_count);
         return;
     }
     if (tid == 0) out_count[b] = keff;
@@ -602,8 +564,6 @@ __global__ void __launch_bounds__(kRsThreads, 1)
             }
         }
         __syncthreads();
-        BK_TICK(3);
-        BK_TICK(4);
         // ---- 4. rank and write: every stored pair counts the pairs of ITS bucket that precede it in the exact total order
         //         (ordered key descending, index ascending); start[bucket] + that count is its final rank, and it goes
         //         straight to the output row -- no sorted copy in shared memory, no separate write-out pass.  One thread
@@ -649,8 +609,6 @@ __global__ void __launch_bounds__(kRsThreads, 1)
         if (out_boxes) out_boxes[oo] = make_float4(0.f, 0.f, 0.f, 0.f);
     }
     __syncthreads();
-    BK_TICK(5);
-#undef BK_TICK
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -870,9 +828,9 @@ __global__ void __launch_bounds__(kRsThreads, 1)
         cluster.sync();
         if (rank != 0) return;
         if (L.staged) topk_radix_body<true>(smem, scores, valid, boxes, N, k, kcap, nchunks, L, out_scores, out_idx, out_cidx,
-                                            out_boxes, out_count, nullptr, b);
+                                            out_boxes, out_count, b);
         else topk_radix_body<false>(smem, scores, valid, boxes, N, k, kcap, nchunks, L, out_scores, out_idx, out_cidx,
-                                    out_boxes, out_count, nullptr, b);
+                                    out_boxes, out_count, b);
         return;
     }
     if (rank == 0 && tid == 0) out_count[b] = keff;
@@ -958,7 +916,7 @@ __global__ void __launch_bounds__(kRsThreads, 1)
     cluster.sync();  // nobody leaves while a peer may still read its shared memory
 }
 
-static size_t bucket_smem(int N, int cap, int nchunks, bool staged) {
+constexpr size_t bucket_smem(int N, int cap, int nchunks, bool staged) {
     size_t o = up16(sizeof(BkHdr));
     o = up16(o + 8 * (size_t)nchunks);
     o = up16(o + 4 * (size_t)kBuckets);
@@ -966,13 +924,18 @@ static size_t bucket_smem(int N, int cap, int nchunks, bool staged) {
     o = up16(o + (staged ? 4 * (size_t)N : 0));
     return up16(o + 6 * (size_t)cap);
 }
+constexpr size_t kSmemLimit = 227 * 1024;
+// The largest shape topk_radix_launch takes (N 65536, k 16384) fits the bucket kernel unstaged, so every shape that has a
+// radix layout runs the bucket kernel, with the radix path as its hand-over.
+static_assert(bucket_smem(65536, 16384 + kBucketSlack, 65536 / 32, false) <= kSmemLimit,
+              "the bucket kernel must fit every shape of the fast path");
 
 // Returns FRR_OK when the launch was done, 1 when the shape is outside the fast path (caller falls back).
 int topk_radix_launch(const float* scores, const uint8_t* valid, const float* boxes, int B, int N, int k,
                       float* out_scores, int32_t* out_idx, int32_t* out_cidx, float* out_boxes, int32_t* out_count,
-                      long long* dbg, frr_stream_t stream, int cluster_hint) {
+                      frr_stream_t stream, int cluster_hint) {
     if (N > 65536 || k > 16384) return 1;
-    const size_t limit = 227 * 1024;
+    const size_t limit = kSmemLimit;
     const int kcap = (k + 31) & ~31;
     const int nchunks = (N + 31) / 32;
     RsLayout L = rs_layout(N, kcap, nchunks, true, 5);
@@ -980,22 +943,15 @@ int topk_radix_launch(const float* scores, const uint8_t* valid, const float* bo
     if (L.total > limit) L = rs_layout(N, kcap, nchunks, false, 5);
     if (L.total > limit) L = rs_layout(N, kcap, nchunks, false, 4);
     if (L.total > limit) return 1;
-    // bucket kernel (with the radix path compiled in as its hand-over) when its shared memory fits, else the radix
-    // kernel alone
+    // bucket kernel, with the radix path compiled in as its hand-over
     const int cap = kcap + kBucketSlack;
     const bool bstaged = bucket_smem(N, cap, nchunks, true) <= limit;
     const size_t bsm = bucket_smem(N, cap, nchunks, bstaged);
     // CTAs per image: small batches (B * S <= SMs) spread an image over a cluster; cluster_hint = 1 keeps one CTA per
-    // image (the least SM time: several batches in flight), the profiling entry (dbg) too
-    int S = 1;
-    if (bsm <= limit && cluster_hint != 1 && dbg == nullptr) {
-        const int nsm = num_sms();
-        // two CTAs per image when they fit: 26-27 us against 29-39 us; more do not pay (measured: 4 CTAs equal 2, 8 CTAs
-        // take 37-44 us -- five cluster barriers and an S-fold histogram merge against ~25 us of divisible work)
-        S = (long)B * 2 <= nsm ? 2 : 1;
-        static const int smax_dbg = getenv("FRR_TOPK_SMAX") ? atoi(getenv("FRR_TOPK_SMAX")) : 2;  // developer knob (tools/topk_latency.py)
-        if (smax_dbg != 2) S = (long)B * smax_dbg <= nsm ? smax_dbg : S;
-    }
+    // image (the least SM time: several batches in flight).  Two CTAs per image when they fit: 26-27 us against 29-39 us;
+    // more do not pay (measured: 4 CTAs equal 2, 8 CTAs take 37-44 us -- five cluster barriers and an S-fold histogram
+    // merge against ~25 us of divisible work)
+    const int S = cluster_hint != 1 && (long)B * 2 <= num_sms() ? 2 : 1;
     if (S > 1) {
         BkcLayout Lc = bkc_layout(cap, nchunks, S, true);
         const bool cstaged = Lc.total <= limit;
@@ -1022,22 +978,13 @@ int topk_radix_launch(const float* scores, const uint8_t* valid, const float* bo
             return FRR_OK;
         }
     }
-    if (bsm <= limit) {
-        auto bkern = bstaged ? topk_bucket_kernel<true> : topk_bucket_kernel<false>;
-        FRR_CUDA(cudaFuncSetAttribute(bkern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
-        bkern<<<B, kRsThreads, bsm > L.total ? bsm : L.total, (cudaStream_t)stream>>>(
-            scores, valid, (const float4*)boxes, N, k, cap, nchunks, out_scores, out_idx, out_cidx, (float4*)out_boxes,
-            out_count, dbg ? dbg + 8 : nullptr, L, kcap);
-        count_launch();
-        FRR_CHECK_LAUNCH("topk_bucket_kernel");
-        return FRR_OK;
-    }
-    auto kern = L.staged ? topk_radix_kernel<true> : topk_radix_kernel<false>;
-    FRR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
-    kern<<<B, kRsThreads, L.total, (cudaStream_t)stream>>>(scores, valid, (const float4*)boxes, N, k, kcap, nchunks, L,
-                                                            out_scores, out_idx, out_cidx, (float4*)out_boxes, out_count, dbg);
+    auto bkern = bstaged ? topk_bucket_kernel<true> : topk_bucket_kernel<false>;
+    FRR_CUDA(cudaFuncSetAttribute(bkern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    bkern<<<B, kRsThreads, bsm > L.total ? bsm : L.total, (cudaStream_t)stream>>>(
+        scores, valid, (const float4*)boxes, N, k, cap, nchunks, out_scores, out_idx, out_cidx, (float4*)out_boxes,
+        out_count, L, kcap);
     count_launch();
-    FRR_CHECK_LAUNCH("topk_radix_kernel");
+    FRR_CHECK_LAUNCH("topk_bucket_kernel");
     return FRR_OK;
 }
 

@@ -145,10 +145,13 @@ def topk_desc(scores, k: int, valid=None, boxes=None, want_cidx: bool = False, c
 
 
 def nms_sorted(boxes, iou_threshold: float, max_keep: int | None = None, counts=None, gather: bool = True,
-               cluster_size: int = 0, threads: int = 0, dbg=None, unit_boxes: bool = False):
+               cluster_size: int = 0, threads: int = 0, unit_boxes: bool = False, first_chunk: int = 0,
+               max_chunk: int = 0, lanes_screen: int = 0, lanes_pairs: int = 0):
     """N1 on score-sorted boxes [B,n,4].  Returns keep int32 [B,max_keep] (-1 padded), count int32 [B],
     rois [B,max_keep,4] (zero padded) or None.  ``unit_boxes``: the caller guarantees coordinates in [0,1]
-    (enables a cheaper, result-identical screening test)."""
+    (enables a cheaper, result-identical screening test).  ``first_chunk``, ``max_chunk``, ``lanes_screen``,
+    ``lanes_pairs``: settings of the bucketed variant, 0 = automatic (frr_nms_sorted_tuned); results do not
+    depend on them."""
     lib = _lib.load()
     boxes = _req(boxes, "boxes")
     if boxes.dim() != 3 or boxes.shape[-1] != 4:
@@ -164,7 +167,8 @@ def nms_sorted(boxes, iou_threshold: float, max_keep: int | None = None, counts=
         rois = torch.empty((B, mk, 4), dtype=torch.float32, device=dev) if gather else None
         _lib.check(lib.frr_nms_sorted_tuned(boxes.data_ptr(), _ptr(counts), B, n, float(iou_threshold), mk,
                                             keep.data_ptr(), cnt.data_ptr(), _ptr(rois), int(cluster_size), int(threads),
-                                            _ptr(dbg), int(bool(unit_boxes)), _stream()), "frr_nms_sorted")
+                                            int(first_chunk), int(max_chunk), int(lanes_screen), int(lanes_pairs),
+                                            int(bool(unit_boxes)), _stream()), "frr_nms_sorted")
     return keep, cnt, rois
 
 

@@ -30,7 +30,7 @@ extern "C" {
 #pragma GCC visibility push(default)
 #endif
 
-#define FRR_ABI_VERSION 1
+#define FRR_ABI_VERSION 2
 
 #define FRR_OK 0
 #define FRR_E_INVALID (-1)   /* bad argument (shape, alignment, range)        */
@@ -98,12 +98,6 @@ int frr_topk_desc_opt(const float* scores /* [B,N] */, const uint8_t* valid /* [
                   float* out_scores /* [B,k] or NULL */, int32_t* out_idx /* [B,k] */,
                   int32_t* out_cidx /* [B,k] or NULL */, float* out_boxes /* [B,k,4] or NULL */,
                   int32_t* out_count /* [B] */, int ctas_per_image, frr_stream_t stream);
-/* Profiling variant: dbg_cycles = int64[16] accumulating clock64() cycles of CTA 0 per phase: [0..4] radix kernel
- * (load+validity, select, compaction, sort, write-out; only when image 0 was handed over), [8..13] bucket kernel
- * (load + min/max, histogram, scan, scatter, -, rank + write-out). */
-int frr_topk_desc_profile(const float* scores, const uint8_t* valid, const float* boxes, int B, int N, int k,
-                          float* out_scores, int32_t* out_idx, int32_t* out_cidx, float* out_boxes,
-                          int32_t* out_count, int64_t* dbg_cycles, frr_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------
  * N1  greedy NMS on score-sorted boxes -- torchvision.ops.nms at models/model.py:53-55
@@ -116,14 +110,16 @@ int frr_nms_sorted(const float* boxes /* [B,n,4] */, const int32_t* counts /* [B
                    int n, double iou_thr, int max_keep, int32_t* keep /* [B,max_keep] */,
                    int32_t* keep_count /* [B] */, float* out_boxes /* [B,max_keep,4] or NULL */,
                    int cluster_size, frr_stream_t stream);
-/* Same, with tuning / profiling knobs: threads per CTA (0 = auto, 256, 512 or 1024); dbg_cycles = NULL
- * or int64[16] accumulating per-phase clock64() cycles of CTA 0 (slots: chunks, load, phase1, cluster
- * sync, phase2..5, survivors, fix-point rounds); unit_boxes != 0 = the caller guarantees every coordinate
- * lies in [0,1] (true for the clamped RPN / detection boxes of models/model.py:34,378), which enables a
- * cheaper screening test; results are identical.                                                    */
+/* Same, with tuning knobs: threads per CTA (0 = auto, 256, 512 or 1024); the settings of the bucketed variant (3 in
+ * frr_nms_variant), each 0 = automatic: first_chunk / max_chunk = candidates in the first / the largest chunk
+ * (multiples of 256 in [256, 2048]; automatic 1024 / 2048), lanes_screen / lanes_pairs = lanes per candidate of its
+ * screen / pair phases (powers of two <= 32; automatic: lanes_screen 2 with 1-2 CTAs per image, else 4; lanes_pairs 4);
+ * unit_boxes != 0 = the caller guarantees every coordinate lies in [0,1] (true for the clamped RPN / detection boxes of
+ * models/model.py:34,378), which enables a cheaper screening test.  Results are identical for every setting.         */
 int frr_nms_sorted_tuned(const float* boxes, const int32_t* counts, int B, int n, double iou_thr, int max_keep,
                          int32_t* keep, int32_t* keep_count, float* out_boxes, int cluster_size, int threads,
-                         int64_t* dbg_cycles, int unit_boxes, frr_stream_t stream);
+                         int first_chunk, int max_chunk, int lanes_screen, int lanes_pairs, int unit_boxes,
+                         frr_stream_t stream);
 
 /* Which kernel variant and launch geometry the NMS entry points pick for a problem (host only, launches nothing;
  * tests and bench.py assert through it that the variant they mean to exercise is the one that runs):
@@ -131,12 +127,6 @@ int frr_nms_sorted_tuned(const float* boxes, const int32_t* counts, int B, int n
  * 2 screened + unit range, 3 unit range + area-class / x-bin bucketed lists), out4[3] = dynamic shared memory.   */
 int frr_nms_variant(int B, int n, double iou_thr, int max_keep, int cluster_size, int threads, int unit_boxes,
                     int32_t* out4);
-
-/* Developer knob for the profiling tools: sizes of the first and of the largest chunk of the bucketed variant
- * (multiples of 256 in [256, 2048]) and the lanes per candidate of its screen / pair phases (powers of two <= 32;
- * lanes_screen 0 = automatic: 2 with 1-2 CTAs per image, else 4; lanes_pairs 0 = unchanged).  Process-wide; results
- * never depend on them. */
-int frr_nms_bucket_tune(int first_chunk, int max_chunk, int lanes_screen, int lanes_pairs);
 
 /* Same, with the score order given as indices into an unsorted array: candidate i of image b is
  * boxes_src[b][order[b][i]] (boxes_src [B,src_n,4]; order int32 [B,n] = out_idx of frr_topk_desc).  Only the
@@ -221,17 +211,13 @@ int frr_fpn_level_rois(const float* rois5, int K, int k_min, int k_max, int cano
 /* Which kernel the RoI entry points pick (host only, launches nothing; tests assert through it that the kernel they mean
  * to exercise is the one that runs).  op: 0 frr_roi_pool_fwd, 1 frr_roi_pool_bwd, 2 frr_roi_align_fwd,
  * 3 frr_roi_align_bwd; want_argmax: the forward's argmax != NULL (same kernel either way).  Assumes 4-byte aligned
- * grad_out / argmax and reads FRR_ROI_POOL_BWD like the launchers.  out4 = (kernel id, channels per CTA (0: the kernel
- * walks output elements or rois), CTAs per (image, channel group), dynamic shared memory bytes).  Kernel ids:
+ * grad_out / argmax.  out4 = (kernel id, channels per CTA (0: the kernel walks output elements or rois), CTAs per
+ * (image, channel group), dynamic shared memory bytes).  Kernel ids:
  * -1 nothing launched (no rois), 0 RoIPool forward flat, 1 RoIAlign forward fast, 2 forward planes, 3 forward direct,
  * 4 RoIPool backward colour classes + tail, 5 RoIPool backward tail only, 6 RoIAlign backward fast,
  * 7 RoIAlign backward stream, 8 backward planes, 9 backward direct. */
 int frr_roi_variant(int op, int K, int B, int C, int H, int W, int PH, int PW, int sampling_ratio, int want_argmax,
                     int32_t* out4);
-
-/* Developer hook: per-phase clock64() cycles of CTA (0,0) of the 7x7 fast kernels, accumulated since the last call
- * (16 slots, see roi_fast.cu); copies to host_out16 and clears.  Synchronises the device. */
-int frr_roi_debug_cycles(int64_t* host_out16);
 
 /* ---------------------------------------------------------------------------------------
  * T1  RPN target maker -- RPNTargetMaker.forward, models/model.py:186-266 (IoU: utils/util.py:66-102).

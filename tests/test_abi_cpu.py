@@ -1,6 +1,7 @@
 """CPU-side checks of the drop-in boundary: libfrr.so loads without a GPU and exports exactly the
 entry points include/frr.h declares; the product refuses CPU tensors (no fallback)."""
 import ctypes
+import subprocess
 
 import numpy as np
 import pytest
@@ -9,7 +10,7 @@ import torch
 from faster_rcnn_pytorch_b200 import _lib, ops
 
 
-def test_library_builds_loads_and_exports_every_declared_symbol():
+def test_library_builds_loads_and_exports_every_declared_symbol_at_abi_version_2():
     from faster_rcnn_pytorch_b200 import build
     build.build()
     lib = _lib.load()
@@ -19,7 +20,22 @@ def test_library_builds_loads_and_exports_every_declared_symbol():
         assert hasattr(lib, n), n
         assert n in _lib.SIGNATURES, f"{n} declared in frr.h but not bound in _lib.SIGNATURES"
     assert set(_lib.SIGNATURES) == set(names)
-    assert lib.frr_abi_version() == 1
+    assert lib.frr_abi_version() == 2
+
+
+def test_library_reads_no_environment_variables():
+    """Kernel and launch choices depend on the arguments and the device only, never on the process environment."""
+    _lib.load()
+    undefined = subprocess.run(["nm", "-D", "--undefined-only", _lib.LIB_PATH], check=True, capture_output=True,
+                               text=True).stdout
+    assert "getenv" not in undefined
+
+
+@pytest.mark.parametrize("tune", [(128, 0, 0, 0), (0, 4096, 0, 0), (0, 0, 3, 0), (0, 0, 0, 64), (0, 0, -2, 0)])
+def test_nms_tuning_settings_are_range_checked(tune):
+    lib = _lib.load()
+    rc = lib.frr_nms_sorted_tuned(None, None, 1, 0, 0.7, 0, None, None, None, 0, 0, *tune, 1, None)
+    assert rc == -1 and b"frr_nms_sorted_tuned" in lib.frr_last_error()
 
 
 def test_anchor_base_host_matches_oracle(oracle):

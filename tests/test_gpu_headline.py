@@ -195,16 +195,11 @@ def test_bucketed_nms_walk_ends_by_count_with_a_partial_last_chunk(oracle):
 
 
 @pytest.mark.parametrize("first,largest,lanes", [(256, 256, 1), (256, 2048, 32), (2048, 2048, 2), (512, 1024, 8)])
-def test_bucketed_nms_result_does_not_depend_on_chunk_sizes(oracle, first, largest, lanes):
-    from faster_rcnn_pytorch_b200 import _lib
-    lib = _lib.load()
-    try:
-        _lib.check(lib.frr_nms_bucket_tune(first, largest, lanes, lanes), "frr_nms_bucket_tune")
-        for name in ("rpn_like", "dense_duplicates", "staircase"):
-            b = nms_cases.make(name, 5, 7000)
-            want = oracle.nms(b, -np.arange(len(b), dtype=np.float32), 0.7)[:2000]
-            for cs in (1, 2, 8):
-                got = _run_nms(b, 0.7, 2000, cluster_size=cs, unit_boxes=True)
-                assert np.array_equal(got, want), (name, cs)
-    finally:
-        _lib.check(lib.frr_nms_bucket_tune(1024, 2048, 4, 4), "frr_nms_bucket_tune")
+def test_bucketed_nms_result_does_not_depend_on_per_call_chunk_sizes(oracle, first, largest, lanes):
+    tune = dict(first_chunk=first, max_chunk=largest, lanes_screen=lanes, lanes_pairs=lanes)
+    for name in ("rpn_like", "dense_duplicates", "staircase"):
+        b = nms_cases.make(name, 5, 7000)
+        want = oracle.nms(b, -np.arange(len(b), dtype=np.float32), 0.7)[:2000]
+        for cs in (1, 2, 8):
+            got = _run_nms(b, 0.7, 2000, cluster_size=cs, unit_boxes=True, **tune)
+            assert np.array_equal(got, want), (name, cs)

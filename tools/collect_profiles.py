@@ -10,7 +10,7 @@ def run(*cmd):
     return subprocess.run(cmd, capture_output=True, text=True).stdout
 
 
-for name in (f"{R}_bench_launches.csv", f"{R}_stage_profile.log", f"{R}_nms_phases.log", f"{R}_topk_phases.log",
+for name in (f"{R}_bench_launches.csv", f"{R}_stage_profile.log", f"{R}_nms_phases.log",
              f"{R}_msroialign.log", f"{R}_roi_bwd_probe.log"):
     if os.path.exists(os.path.join(G, name)):
         shutil.copy(os.path.join(G, name), os.path.join(P, name))

@@ -1,4 +1,4 @@
-"""Developer tool: NMS kernel timing + per-phase cycle breakdown on the config-2 workload (GPU box)."""
+"""Developer tool: bucketed NMS kernel timing over its per-call settings on the config-2 workload (GPU box)."""
 import sys, os, json
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -13,42 +13,31 @@ sc = torch.from_numpy(np.stack([x[2] for x in ins])).to(dev)
 boxes, scores, valid = ops.rpn_decode(reg, sc, image_hw=HW)
 top = ops.topk_desc(scores, 12000, valid=valid, boxes=boxes)
 tb, tc = top["boxes"], top["count"]
-# slots of nms_bucket_kernel (csrc/nms_bucket.cu, enum BK_*): cycles of CTA 0 per phase, then counters
-names = ["chunks", "load", "scan", "scatter", "screen", "sync1", "surv_sort", "pred", "sync2", "fix", "append",
-         "rounds", "survivors", "edges", "visited", "ovf"]
-from faster_rcnn_pytorch_b200 import _lib
-lib = _lib.load()
 
 
-def run(bx, cnt, S, threads, reps=20, dbg=False):
-    d = torch.zeros(16, dtype=torch.int64, device=dev) if dbg else None
+def run(bx, cnt, S, threads, tune, reps=20):
     for _ in range(3):
-        ops.nms_sorted(bx, 0.7, max_keep=2000, counts=cnt, cluster_size=S, threads=threads, unit_boxes=True)
+        ops.nms_sorted(bx, 0.7, max_keep=2000, counts=cnt, cluster_size=S, threads=threads, unit_boxes=True, **tune)
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(reps):
-        ops.nms_sorted(bx, 0.7, max_keep=2000, counts=cnt, cluster_size=S, threads=threads, unit_boxes=True)
+        ops.nms_sorted(bx, 0.7, max_keep=2000, counts=cnt, cluster_size=S, threads=threads, unit_boxes=True, **tune)
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / reps
-    out = {"B": bx.shape[0], "S": S, "threads": threads, "us": round(ms * 1e3, 1)}
-    if dbg:
-        keep, c, _ = ops.nms_sorted(bx, 0.7, max_keep=2000, counts=cnt, cluster_size=S, threads=threads, dbg=d, unit_boxes=True)
-        torch.cuda.synchronize()
-        out.update({k: int(v) for k, v in zip(names, d.cpu().tolist())})
-        out["kept"] = int(c[0])
-        out["last_keep_pos"] = int(keep[0, int(c[0]) - 1])
+    keep, c, _ = ops.nms_sorted(bx, 0.7, max_keep=2000, counts=cnt, cluster_size=S, threads=threads, unit_boxes=True, **tune)
+    out = {"B": bx.shape[0], "S": S, "threads": threads, "us": round(ms * 1e3, 1), "kept": int(c[0]),
+           "last_keep_pos": int(keep[0, int(c[0]) - 1])}
     print(json.dumps(out), flush=True)
 
 
 one, onec = tb[:1].contiguous(), tc[:1].contiguous()
 for first, largest, n1, n2 in ((512, 2048, 4, 4), (512, 2048, 8, 8), (512, 2048, 2, 2), (512, 2048, 1, 1), (512, 2048, 8, 4),
                                (512, 2048, 16, 8), (1024, 2048, 4, 4), (256, 2048, 4, 4), (512, 1536, 4, 4), (768, 2048, 4, 4)):
-    _lib.check(lib.frr_nms_bucket_tune(first, largest, n1, n2), "tune")
-    print(json.dumps({"first_chunk": first, "largest_chunk": largest, "lanes_screen": n1, "lanes_pairs": n2}), flush=True)
+    tune = dict(first_chunk=first, max_chunk=largest, lanes_screen=n1, lanes_pairs=n2)
+    print(json.dumps(tune), flush=True)
     for threads, S in ((1024, 2), (1024, 1), (1024, 4)):
-        run(tb, tc, S, threads, dbg=True)
+        run(tb, tc, S, threads, tune)
     for threads, S in ((1024, 16), (512, 16), (1024, 8)):
-        run(one, onec, S, threads, reps=50, dbg=True)
-_lib.check(lib.frr_nms_bucket_tune(1024, 2048, 0, 4), "tune")
+        run(one, onec, S, threads, tune, reps=50)

@@ -9,9 +9,8 @@ python bench.py > $O/${R}_bench_all.json 2> $O/${R}_bench_all.err || exit 1
 python bench.py --impl reference --steps 2 --warmup 1 > $O/${R}_bench_reference.json 2> $O/${R}_bench_reference.err
 python tools/stage_profile.py > $O/${R}_stage_profile.log 2>&1
 python tools/nms_profile.py > $O/${R}_nms_phases.log 2>&1
-python tools/topk_profile.py > $O/${R}_topk_phases.log 2>&1
 python tools/msroialign_profile.py > $O/${R}_msroialign.log 2>&1
-{ python tools/roi_bwd_probe.py; python tools/roi_bwd_probe.py cfg4; FRR_ROI_POOL_BWD=tail python tools/roi_bwd_probe.py; } > $O/${R}_roi_bwd_probe.log 2>&1
+{ python tools/roi_bwd_probe.py; python tools/roi_bwd_probe.py cfg4; } > $O/${R}_roi_bwd_probe.log 2>&1
 ncu --metrics gpu__time_duration.sum --clock-control none -c 400 --csv --log-file $O/${R}_bench_launches.csv \
     python bench.py --workload rpn --steps 3 --warmup 3 --no-cpu > $O/ncu1.log 2>&1
 # (the launch geometry of the timed path: one NMS CTA per image, as region.ProposalPipeline runs it)

@@ -5,7 +5,7 @@ import numpy as np, torch, torchvision
 from faster_rcnn_pytorch_b200 import ops, synth
 dev = torch.device("cuda:0")
 B, C, fh, fw, per = (8, 512, 50, 83, 300) if "cfg4" in sys.argv else (16, 512, 37, 62, 128)
-print("variant", os.environ.get("FRR_ROI_POOL_BWD", "default"), "shape", (B, C, fh, fw, per), flush=True)
+print("shape", (B, C, fh, fw, per), flush=True)
 K = B * per
 feat = torch.from_numpy(synth.features(1, B, C, fh, fw)).to(dev)
 go = torch.randn((K, C, 7, 7), device=dev)

@@ -1,5 +1,5 @@
 """Developer tool: RoIPool forward (with argmax) on the config-3 shape, synthetic and RPN-made rois, L2 flushed between
-launches.  Prints microseconds per launch (variants are chosen through environment knobs of the library)."""
+launches.  Prints microseconds per launch."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -22,7 +22,6 @@ def timeit(fn, reps=20):
     return tot / reps * 1e3
 
 
-print("knobs", {k: v for k, v in os.environ.items() if k.startswith("FRR_")}, flush=True)
 for tag, B, C, fh, fw, per in (("cfg3", 16, 512, 37, 62, 128), ("cfg4", 8, 512, 50, 83, 300)):
     feat = torch.from_numpy(synth.features(1, B, C, fh, fw)).to(dev)
     syn = torch.from_numpy(np.concatenate([np.concatenate([np.full((per, 1), b, np.float32), synth.random_rois(10 + b, per, fh, fw, 1)[:, 1:]], 1) for b in range(B)])).to(dev)

@@ -1,5 +1,4 @@
-"""Developer tool: times roi_pool_forward (with / without argmax) at the config-3 shape on RPN-sized and small rois,
-and prints the per-phase cycles of CTA (0,0)."""
+"""Developer tool: times roi_pool_forward (with / without argmax) at the config-3 shape on RPN-sized and small rois."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -32,16 +31,6 @@ print(
       "small-rois us", round(t(lambda i: ops.roi_pool_forward(feats[i % 3], small)), 1),
       "noarg us", round(t(lambda i: ops.roi_pool_forward(feats[i % 3], rois5, want_argmax=False)), 1),
       "checksum", float(out0[0].double().sum()), int(out0[1].long().sum()))
-import ctypes
-from faster_rcnn_pytorch_b200 import _lib
-lib = _lib.load()
-buf = (ctypes.c_int64 * 16)()
-lib.frr_roi_debug_cycles(buf)
-F = {0: "load", 1: "roiscan", 2: "geom", 3: "compute", 4: "copyout", 5: "tail"}
-for tag, r in (("rpn", rois5), ("small", small)):
-    ops.roi_pool_forward(feats[0], r); torch.cuda.synchronize()
-    lib.frr_roi_debug_cycles(buf)
-    print("phases", tag, {n: int(buf[i]) for i, n in F.items()})
 wh = (rois5[:, 3] - rois5[:, 1]), (rois5[:, 4] - rois5[:, 2])
 print("rpn roi w/h mean", float(wh[0].mean()), float(wh[1].mean()), "max", float(wh[0].max()), float(wh[1].max()))
 wh = (small[:, 3] - small[:, 1]), (small[:, 4] - small[:, 2])

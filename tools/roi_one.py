@@ -30,17 +30,3 @@ for _ in range(2):
     ga = ops.roi_align_backward(go, rois, feat.shape, sampling_ratio=2)
 torch.cuda.synchronize()
 print("ok")
-import ctypes
-from faster_rcnn_pytorch_b200 import _lib
-lib = _lib.load()
-buf = (ctypes.c_int64 * 16)()
-lib.frr_roi_debug_cycles(buf)
-def phases(tag, fn, names):
-    fn(); torch.cuda.synchronize()
-    lib.frr_roi_debug_cycles(buf)
-    print(tag, {n: int(buf[i]) for i, n in names.items()})
-F = {0: "load", 1: "roiscan", 2: "geom+bufwait", 3: "compute", 4: "store_issue", 5: "drain"}
-Bk = {8: "accumulate_loop", 13: "roiscan", 14: "init", 15: "planestore"}
-phases("pool_fwd", lambda: ops.roi_pool_forward(feat, rois), F)
-phases("pool_bwd", lambda: ops.roi_pool_backward(go, arg, rois, feat.shape), Bk)
-phases("align_fwd", lambda: ops.roi_align_forward(feat, rois, sampling_ratio=2), F)

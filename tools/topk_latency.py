@@ -1,5 +1,4 @@
-"""Developer tool: device time of frr_topk_desc (graph replay of 20 calls) at batch 1 / 8 / 64 for the three proposal shapes;
-FRR_TOPK_SMAX caps the CTAs per image (experiment knob)."""
+"""Developer tool: device time of frr_topk_desc (graph replay of 20 calls) at batch 1 / 8 / 64 for the three proposal shapes."""
 import os, sys
 sys.path.insert(0, os.getcwd())
 import numpy as np, torch
@@ -25,4 +24,4 @@ for HW, k in (((608, 1008), 12000), ((600, 1000), 6000), ((800, 1333), 6000)):
         g.replay(); torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(); g.replay(); e1.record(); torch.cuda.synchronize()
-        print(f"SMAX={os.environ.get('FRR_TOPK_SMAX','8')} HW={HW} k={k} B={B}: {e0.elapsed_time(e1)/20*1e3:.1f} us", flush=True)
+        print(f"HW={HW} k={k} B={B}: {e0.elapsed_time(e1)/20*1e3:.1f} us", flush=True)

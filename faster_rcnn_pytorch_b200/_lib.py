@@ -44,6 +44,8 @@ SIGNATURES = {
     "frr_roi_pool_bwd": (_i, [_p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _f, _i, _p, _p]),
     "frr_roi_align_fwd": (_i, [_p, _p, _i, _i, _i, _i, _i, _i, _i, _f, _i, _i, _i, _p, _p]),
     "frr_roi_align_bwd": (_i, [_p, _p, _i, _i, _i, _i, _i, _i, _i, _f, _i, _i, _i, _p, _p]),
+    "frr_roi_pool_bwd_deterministic": (_i, [_p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _f, _i, _p, _p]),
+    "frr_roi_align_bwd_deterministic": (_i, [_p, _p, _i, _i, _i, _i, _i, _i, _i, _f, _i, _i, _i, _p, _p]),
     "frr_roi_variant": (_i, [_i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p]),
     "frr_fpn_level_rois": (_i, [_p, _i, _i, _i, _i, _f, _i, _p, _p, _p]),
     "frr_region_loss": (_i, [_p, _p, _p, _p, _i, _i, _p, _p, _p, _p, _i, _i, _i, _f, _f, _p, _p, _p, _p, _p, _p]),

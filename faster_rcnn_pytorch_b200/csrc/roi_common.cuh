@@ -69,6 +69,14 @@ __device__ __forceinline__ void bulk_commit_wait() {
 }
 __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
+// 4-byte cp.async global -> shared (src_bytes 0: zero fill, nothing is read) and its group bookkeeping
+__device__ __forceinline__ void cp_async4_zfill(uint32_t dst, const void* src, uint32_t src_bytes) {
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 4, %2;" ::"r"(dst), "l"(src), "r"(src_bytes) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int N>
+__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
+
 // Load CB planes of image b into smem planes[CB][HW].  NCHW: contiguous chunk (TMA when 16-B aligned),
 // NHWC: gather CB consecutive channels per pixel.
 __device__ __forceinline__ void load_planes(float* planes, const float* __restrict__ feat, int b, int c0, int CB, int C,

@@ -70,9 +70,6 @@ __device__ __forceinline__ void sts_f32(uint32_t a, float v) { asm volatile("st.
 __device__ __forceinline__ void cp_async4(uint32_t dst, const void* src) {
     asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dst), "l"(src) : "memory");
 }
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
 // Smallest s in 2..7 such that the (unclipped) windows of bins p and p + s never overlap: floor((p+s)*b) >= ceil((p+1)*b)
 // for all p, evaluated with the forward's own fp32 arithmetic.  r >= 6 gives 2; 7 puts every bin of the dimension into
@@ -182,9 +179,6 @@ __device__ __forceinline__ void rmw_load(float& t, int a, uint32_t hw, uint32_t 
 }
 __device__ __forceinline__ void rmw_store(float v, int a, uint32_t hw, uint32_t addr) {
     asm volatile("{\n\t.reg .pred p;\n\tsetp.lt.u32 p, %1, %2;\n\t@p st.shared.f32 [%3], %0;\n\t}" ::"f"(v), "r"(a), "r"(hw), "r"(addr) : "memory");
-}
-__device__ __forceinline__ void cp_async4_zfill(uint32_t dst, const void* src, uint32_t src_bytes) {
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 4, %2;" ::"r"(dst), "l"(src), "r"(src_bytes) : "memory");
 }
 
 struct PbVals {  // the four colour-class values of one lane for one roi

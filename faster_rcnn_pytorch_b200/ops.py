@@ -274,8 +274,16 @@ def roi_pool_forward(feat, rois5, output_size=(7, 7), spatial_scale: float = 1.0
     return out, arg
 
 
-def roi_pool_backward(grad_out, argmax, rois5, feat_shape, spatial_scale: float = 1.0, channels_last: bool = False):
+def _deterministic(flag):
+    return torch.are_deterministic_algorithms_enabled() if flag is None else bool(flag)
+
+
+def roi_pool_backward(grad_out, argmax, rois5, feat_shape, spatial_scale: float = 1.0, channels_last: bool = False,
+                      deterministic: bool | None = None):
+    """``deterministic``: True runs the kernel whose gradient is bit-exact with torchvision's CPU backward and the same
+    on every run; None (default) follows ``torch.use_deterministic_algorithms``."""
     lib = _lib.load()
+    fn = lib.frr_roi_pool_bwd_deterministic if _deterministic(deterministic) else lib.frr_roi_pool_bwd
     grad_out = _req(grad_out, "grad_out")
     argmax = _req(argmax, "argmax", torch.int32)
     rois5 = _req(rois5, "rois")
@@ -284,9 +292,8 @@ def roi_pool_backward(grad_out, argmax, rois5, feat_shape, spatial_scale: float 
     with torch.cuda.device(grad_out.device):
         gin = torch.empty((B, C, H, W), dtype=torch.float32, device=grad_out.device,
                           memory_format=torch.channels_last if channels_last else torch.contiguous_format)
-        _lib.check(lib.frr_roi_pool_bwd(grad_out.data_ptr(), argmax.data_ptr(), rois5.data_ptr(), K, B, C, H, W, PH, PW,
-                                        float(spatial_scale), int(channels_last), gin.data_ptr(), _stream()),
-                   "frr_roi_pool_bwd")
+        _lib.check(fn(grad_out.data_ptr(), argmax.data_ptr(), rois5.data_ptr(), K, B, C, H, W, PH, PW, float(spatial_scale),
+                      int(channels_last), gin.data_ptr(), _stream()), fn.__name__)
     return gin
 
 
@@ -313,8 +320,10 @@ def roi_align_forward(feat, rois5, output_size=(7, 7), spatial_scale: float = 1.
 
 
 def roi_align_backward(grad_out, rois5, feat_shape, spatial_scale: float = 1.0, sampling_ratio: int = 2,
-                       aligned: bool = False, channels_last: bool = False):
+                       aligned: bool = False, channels_last: bool = False, deterministic: bool | None = None):
+    """``deterministic``: as for ``roi_pool_backward``."""
     lib = _lib.load()
+    fn = lib.frr_roi_align_bwd_deterministic if _deterministic(deterministic) else lib.frr_roi_align_bwd
     grad_out = _req(grad_out, "grad_out")
     rois5 = _req(rois5, "rois")
     B, C, H, W = feat_shape
@@ -322,9 +331,8 @@ def roi_align_backward(grad_out, rois5, feat_shape, spatial_scale: float = 1.0, 
     with torch.cuda.device(grad_out.device):
         gin = torch.empty((B, C, H, W), dtype=torch.float32, device=grad_out.device,
                           memory_format=torch.channels_last if channels_last else torch.contiguous_format)
-        _lib.check(lib.frr_roi_align_bwd(grad_out.data_ptr(), rois5.data_ptr(), K, B, C, H, W, PH, PW, float(spatial_scale),
-                                         int(sampling_ratio), int(aligned), int(channels_last), gin.data_ptr(), _stream()),
-                   "frr_roi_align_bwd")
+        _lib.check(fn(grad_out.data_ptr(), rois5.data_ptr(), K, B, C, H, W, PH, PW, float(spatial_scale),
+                      int(sampling_ratio), int(aligned), int(channels_last), gin.data_ptr(), _stream()), fn.__name__)
     return gin
 
 

@@ -332,7 +332,9 @@ class InferPlan:
 class TrainPlan:
     """The training-side region stage for a fixed batch shape (models/model.py:310-335): both target makers with the
     reference's sampling replayed on the device (no host synchronisation), RoIPool forward of the sampled rois and its
-    backward.  ``targets_and_pool`` / ``pool_backward`` can be recorded into CUDA graphs with ``capture_*``."""
+    backward.  ``targets_and_pool`` / ``pool_backward`` can be recorded into CUDA graphs with ``capture_*``.
+    ``pool_backward`` follows ``torch.use_deterministic_algorithms`` when it runs; a captured graph keeps the backward
+    kernel chosen at capture time, whatever the flag is when the graph is replayed."""
 
     def __init__(self, B: int, image_hw, device, generator=None, stride: int = 16):
         from . import targets

@@ -169,7 +169,8 @@ int frr_rpn_proposals_opt(const float* reg, const float* cls, int cls_is_logits,
  *        feat [B,C,H,W] fp32, NCHW (channels_last=0) or NHWC memory (channels_last=1);
  *        rois [K,5] = (batch index, x1,y1,x2,y2) fp32; out/argmax [K,C,PH,PW] contiguous
  *        (argmax int32 = h*W+w, -1 for empty bins; may be NULL in inference).
- *        Forward max/argmax bit-exact vs torchvision CPU; backward within 1e-5 (fp32 sum order).
+ *        Forward max/argmax bit-exact vs torchvision CPU; backward within 1e-5 (fp32 sum order), or bit-exact through
+ *        frr_roi_pool_bwd_deterministic below.
  *        Exception: with argmax == NULL, a 7x7 bin whose maximum is zero may hold +0.0 where torchvision
  *        (first strict maximum) holds -0.0; the values compare equal and every other bit matches.
  * ------------------------------------------------------------------------------------- */
@@ -199,6 +200,29 @@ int frr_roi_align_fwd(const float* feat, const float* rois, int K, int B, int C,
 int frr_roi_align_bwd(const float* grad_out, const float* rois, int K, int B, int C, int H, int W, int PH, int PW,
                       float spatial_scale, int sampling_ratio, int aligned, int channels_last, float* grad_in,
                       frr_stream_t stream);
+
+/* Deterministic backward, bit-exact with torchvision's CPU kernels (torchvision::_roi_pool_backward /
+ * _roi_align_backward on CPU): the same arguments as frr_roi_pool_bwd / frr_roi_align_bwd, for callers that need the
+ * same gradient bits on every run (torch.use_deterministic_algorithms).
+ * grad_in[b,c,p] is the fp32 sum, starting at +0.0, of the following terms, added in this order.  Only rois with
+ * 0 <= (int)rois[k,0] < B count, taken in ascending k.
+ *  - RoIPool: for each k, then ph, then pw (row-major): grad_out[k,c,ph,pw] if argmax[k,c,ph,pw] == p and p lies inside
+ *    that bin's clipped window.  The forward only produces argmax values of that kind; a value that is -1, out of range
+ *    or outside the window contributes nothing.
+ *  - RoIAlign: for each k, then ph, pw, iy, ix, then tap 1, 2, 3, 4 of a valid sample: (go * w_t) / count whenever tap
+ *    t lands on p (torchvision's bilinear_interpolate_gradient arithmetic).  At the last row or column the snapped taps
+ *    land on the same pixel and are added separately, in tap order.  The division is IEEE round-to-nearest (exact for
+ *    counts below 2^27 samples per bin).
+ * The result is a pure function of the inputs: the same on any stream, inside or outside a CUDA graph, whatever else
+ * runs; no atomic touches a value.  NaN / Inf in grad_out reach the same elements as in the CPU loop.  grad_in is fully
+ * written (no pre-zeroing needed), NCHW or channels_last like the entry points above.  grad_out / argmax must be
+ * 4-byte aligned; PH and PW up to about 70 (a one-channel ring of four rois must fit shared memory). */
+int frr_roi_pool_bwd_deterministic(const float* grad_out, const int32_t* argmax, const float* rois, int K, int B, int C,
+                                   int H, int W, int PH, int PW, float spatial_scale, int channels_last, float* grad_in,
+                                   frr_stream_t stream);
+int frr_roi_align_bwd_deterministic(const float* grad_out, const float* rois, int K, int B, int C, int H, int W, int PH,
+                                    int PW, float spatial_scale, int sampling_ratio, int aligned, int channels_last,
+                                    float* grad_in, frr_stream_t stream);
 
 /* MultiScaleRoIAlign level assignment -- TV ops/poolers.py LevelMapper as used by models/new_model.py:127,143:
  * level = clamp(floor(canonical_level + log2(sqrt(area)/canonical_scale) + 1e-6), k_min, k_max) - k_min, rois in image

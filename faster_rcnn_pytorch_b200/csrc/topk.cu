@@ -1,5 +1,5 @@
 // P4 (general path): pre-NMS top-k of the RPN objectness scores, sorted descending (models/model.py:44-49).
-// The fast path for N <= 65536 is the shared-memory radix sort of topk_radix.cu; this kernel covers larger N.
+// The fast path for N <= 65536 is the shared-memory bucket top-k of topk_radix.cu; this kernel covers larger N.
 //
 // One CTA (1024 threads) per image:
 //   1. MSB-first radix select (4 x 8-bit digits) over order-preserving uint32 keys finds the
@@ -256,7 +256,7 @@ int frr::topk_desc_impl(const float* scores, const uint8_t* valid, const float* 
                   "frr_topk_desc: boxes must be given and 16-byte aligned when out_boxes is requested");
     if (B == 0 || k == 0) return FRR_OK;
     FRR_CHECK_ARG(k <= 16384, "frr_topk_desc: k=%d exceeds the in-smem sort capacity 16384", k);
-    {   // fast path: shared-memory radix sort (topk_radix.cu); shapes outside it take the bitonic kernel below
+    {   // fast path: shared-memory bucket top-k (topk_radix.cu); shapes outside it take the bitonic kernel below
         const int rc = topk_radix_launch(scores, valid, boxes, B, N, k, out_scores, out_idx, out_cidx, out_boxes, out_count,
                                          stream, cluster_hint);
         if (rc <= 0) return rc;

@@ -1,7 +1,7 @@
 // P4 (fast path): pre-NMS top-k, sorted descending, ties lower-index-first (models/model.py:44-49).
-// Two algorithms in one launch: topk_bucket_kernel (below, the default) and the radix path described here, which it falls
-// into for inputs that do not bucket.  The bucket kernel's shared memory fits for every shape the fast path takes
-// (static_assert at bucket_smem), so the radix path never runs as a kernel of its own.
+// Two algorithms in one launch: topk_bucket_kernel (below, the default: one or two CTAs per image) and the radix path
+// described here, which it falls into for inputs that do not bucket.  The bucket kernel's shared memory fits for every
+// shape the fast path takes (static_assert after bkc_layout), so the radix path never runs as a kernel of its own.
 //
 // Radix path: one CTA (1024 threads) per image, everything after the first read of the scores stays in shared memory:
 //   0. validity words (ballot) + the order-preserving uint32 keys of all N scores staged in shared memory;
@@ -391,235 +391,22 @@ __device__ __forceinline__ void topk_radix_body(unsigned char* smem, const float
 //   (float arithmetic is monotone under rounding, so a higher score never lands in a later bucket; RPN scores are
 //   sigmoid outputs, nearly uniform in value, ~2.6 per bucket).  A shared-memory histogram + one block scan give the
 //   bucket b* in which the k-th largest score lies; the (key, index) pairs of buckets <= b* are scattered to their
-//   bucket ranges (unordered, atomic cursors) and every bucket is insertion-sorted by one thread on the EXACT total
-//   order (ordered key descending, index ascending) -- the same order the radix kernel produces, so ties and the cut
-//   inside b* are bit-identical.  Inputs that do not bucket well (non-finite range, a bucket of > kBucketMax, more than
-//   `cap` stored pairs: e.g. all scores equal) are redone on the radix path in the same CTA.
+//   bucket ranges (unordered, atomic cursors) and every pair is ranked inside its bucket on the EXACT total order
+//   (ordered key descending, index ascending) -- the same order the radix path produces, so ties and the cut inside b*
+//   are bit-identical.  Inputs that do not bucket well (non-finite range, a bucket of > kBucketMax, more than `cap`
+//   stored pairs: e.g. all scores equal) are redone on the radix path by CTA 0 of the image alone.
+//
+// An image runs on a thread-block CLUSTER of S = 1 or 2 CTAs (small batches: one CTA per image leaves most SMs idle -- a
+// single image ran on ONE SM).  CTA r of the S CTAs owns a contiguous range of the 32-anchor chunks: it loads / stages /
+// histograms its own scores; the S histograms are merged through distributed shared memory (every CTA reads the peers'
+// counts and derives the same bucket starts, plus how many pairs the lower-ranked CTAs put in every bucket: its first
+// scatter cursors); pairs are scattered straight into the shared memory of the CTA that OWNS their bucket (buckets are
+// dealt to the CTAs by their start position, whole buckets only), which ranks them and writes its contiguous piece of
+// the output row.  Same buckets, same exact total order for every S: identical results.
 constexpr int kBuckets = 8192;
 constexpr int kBucketMax = 192;
 constexpr int kBucketSlack = 1024;  // pairs stored beyond k (the rest of bucket b*)
 
-struct BkHdr {
-    unsigned int warp_tmp[kRsWarps];
-    unsigned int red[kRsWarps];
-    unsigned int nvalid, bstar, stored, bad;
-    float smin, smax;
-};
-
-template <bool kStaged>  // scores staged in shared memory (N up to ~27 k) or re-read from global / L2 in the two passes
-__global__ void __launch_bounds__(kRsThreads, 1)
-    topk_bucket_kernel(const float* __restrict__ scores, const uint8_t* __restrict__ valid,
-                       const float4* __restrict__ boxes, int N, int k, int cap, int nchunks,
-                       float* __restrict__ out_scores, int32_t* __restrict__ out_idx, int32_t* __restrict__ out_cidx,
-                       float4* __restrict__ out_boxes, int32_t* __restrict__ out_count, RsLayout L, int kcap) {
-    extern __shared__ __align__(16) unsigned char smem[];
-    BkHdr* hd = reinterpret_cast<BkHdr*>(smem);
-    size_t o = up16(sizeof(BkHdr));
-    unsigned int* vbits = reinterpret_cast<unsigned int*>(smem + o); o += 4 * (size_t)nchunks;
-    unsigned int* vpre = reinterpret_cast<unsigned int*>(smem + o);  o = up16(o + 4 * (size_t)nchunks);
-    unsigned int* hist = reinterpret_cast<unsigned int*>(smem + o);  o += 4 * (size_t)kBuckets;
-    unsigned short* start = reinterpret_cast<unsigned short*>(smem + o); o = up16(o + 2 * (size_t)(kBuckets + 1));
-    float* sval = reinterpret_cast<float*>(smem + o);                o = up16(o + (kStaged ? 4 * (size_t)N : 0));
-    unsigned int* keyA = reinterpret_cast<unsigned int*>(smem + o);  o += 4 * (size_t)cap;
-    unsigned short* idxA = reinterpret_cast<unsigned short*>(smem + o);
-
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int b = blockIdx.x;
-    const float* sc = scores + (size_t)b * N;
-    const uint8_t* va = valid ? valid + (size_t)b * N : nullptr;
-
-    // ---- 0. validity words, staged scores, min / max of the valid scores, zeroed histogram ---------------
-    float lmin = 3.0e38f, lmax = -3.0e38f;
-    bool lbad = false;
-    constexpr int kLd = 4;  // chunks per trip: 8 independent loads in flight per thread (16 measured slower)
-    for (int c0 = warp; c0 < nchunks; c0 += kLd * kRsWarps) {
-        uint8_t v4[kLd];
-        float s4[kLd];
-#pragma unroll
-        for (int j = 0; j < kLd; ++j) {
-            const int i = (c0 + j * kRsWarps) * 32 + lane;
-            v4[j] = (i < N && va) ? va[i] : (uint8_t)1;
-            s4[j] = (i < N) ? sc[i] : 0.f;
-        }
-#pragma unroll
-        for (int j = 0; j < kLd; ++j) {
-            const int c = c0 + j * kRsWarps;
-            const int i = c * 32 + lane;
-            const bool ok = (i < N) && (v4[j] != 0);
-            const unsigned int w = __ballot_sync(0xffffffffu, ok);
-            if (c < nchunks) {
-                if (lane == 0) vbits[c] = w;
-                if (kStaged && i < N) sval[i] = s4[j];
-                if (ok) {
-                    lbad |= !(fabsf(s4[j]) <= 3.0e38f);  // NaN / inf: no monotone float bucket map
-                    lmin = fminf(lmin, s4[j]);
-                    lmax = fmaxf(lmax, s4[j]);
-                }
-            }
-        }
-    }
-    for (int i = tid; i < kBuckets; i += kRsThreads) hist[i] = 0u;
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) {
-        lmin = fminf(lmin, __shfl_xor_sync(0xffffffffu, lmin, off));
-        lmax = fmaxf(lmax, __shfl_xor_sync(0xffffffffu, lmax, off));
-    }
-    const bool wbad = __any_sync(0xffffffffu, lbad);
-    if (lane == 0) { hd->warp_tmp[warp] = __float_as_uint(lmin); hd->red[warp] = __float_as_uint(lmax); }
-    if (tid == 0) hd->bad = 0u;
-    __syncthreads();
-    if (wbad && lane == 0) hd->bad = 1u;
-    if (warp == 0) {
-        float a = __uint_as_float(hd->warp_tmp[lane]), z = __uint_as_float(hd->red[lane]);
-#pragma unroll
-        for (int off = 16; off > 0; off >>= 1) {
-            a = fminf(a, __shfl_xor_sync(0xffffffffu, a, off));
-            z = fmaxf(z, __shfl_xor_sync(0xffffffffu, z, off));
-        }
-        if (lane == 0) { hd->smin = a; hd->smax = z; }
-    }
-    __syncthreads();
-    {   // exclusive prefix of the valid counts per chunk (compacted indices) and the number of valid scores
-        unsigned int run = 0;
-        for (int base = 0; base < nchunks; base += kRsThreads) {
-            const int c = base + tid;
-            const unsigned int v = (c < nchunks) ? __popc(vbits[c]) : 0u;
-            unsigned int tot;
-            const unsigned int ex = block_exclusive_scan(v, hd->warp_tmp, &tot);
-            if (c < nchunks) vpre[c] = run + ex;
-            run += tot;
-        }
-        if (tid == 0) hd->nvalid = run;
-    }
-    __syncthreads();
-    const int keff = min(k, (int)hd->nvalid);
-    const float smax = hd->smax;
-    const float scale = (float)kBuckets / (smax - hd->smin);
-    bool handover = hd->bad != 0u || (keff > 0 && !(scale <= 3.0e38f));  // empty range (all equal) or overflow
-    auto bucket_of = [&](float s) { return min(kBuckets - 1, (int)((smax - s) * scale)); };
-    auto score_at = [&](int i) -> float { return kStaged ? sval[i] : sc[i]; };
-
-    if (keff > 0 && !handover) {
-        // ---- 1. histogram of the valid scores ------------------------------------------------------------
-        for (int c = warp; c < nchunks; c += kRsWarps) {
-            const int i = c * 32 + lane;
-            if ((vbits[c] >> lane) & 1u) atomicAdd(&hist[bucket_of(score_at(i))], 1u);
-        }
-        __syncthreads();
-        // ---- 2. bucket starts, the bucket b* of the k-th largest score, the largest bucket up to b* ----------
-        {
-            constexpr int kPerT = kBuckets / kRsThreads;
-            unsigned int h4[kPerT], t4 = 0;
-#pragma unroll
-            for (int q = 0; q < kPerT; ++q) { h4[q] = hist[kPerT * tid + q]; t4 += h4[q]; }
-            unsigned int tot;
-            unsigned int run = block_exclusive_scan(t4, hd->warp_tmp, &tot);
-            unsigned int big = 0;
-#pragma unroll
-            for (int q = 0; q < kPerT; ++q) {
-                // only the buckets up to b* are ever looked at: positions beyond 65535 (N > 65535 never gets here) are moot
-                start[kPerT * tid + q] = (unsigned short)min(run, 65535u);
-                if (run < (unsigned int)keff) {
-                    big = max(big, h4[q]);
-                    if (run + h4[q] >= (unsigned int)keff) { hd->bstar = kPerT * tid + q; hd->stored = run + h4[q]; }
-                }
-                run += h4[q];
-            }
-            if (tid == kRsThreads - 1) start[kBuckets] = (unsigned short)min(run, 65535u);
-            big = __reduce_max_sync(0xffffffffu, big);
-            __syncthreads();
-            if (lane == 0) hd->red[warp] = big;
-            __syncthreads();
-            if (warp == 0) {
-                big = __reduce_max_sync(0xffffffffu, hd->red[lane]);
-                if (lane == 0 && (big > kBucketMax || hd->stored > (unsigned int)cap)) hd->bad = 1u;
-            }
-            for (int i = tid; i < kBuckets; i += kRsThreads) hist[i] = 0u;  // now the scatter cursors
-            __syncthreads();
-            handover = hd->bad != 0u;
-        }
-    }
-    if (handover) {  // block-uniform: the radix path redoes this image from scratch in the same shared memory
-        __syncthreads();
-        if (L.staged) topk_radix_body<true>(smem, scores, valid, boxes, N, k, kcap, nchunks, L, out_scores, out_idx, out_cidx,
-                                            out_boxes, out_count);
-        else topk_radix_body<false>(smem, scores, valid, boxes, N, k, kcap, nchunks, L, out_scores, out_idx, out_cidx,
-                                    out_boxes, out_count);
-        return;
-    }
-    if (tid == 0) out_count[b] = keff;
-    if (keff > 0) {
-        const int bstar = (int)hd->bstar;
-        // ---- 3. scatter the pairs of buckets <= b* into their ranges (unordered inside a bucket) --------------
-        for (int c = warp; c < nchunks; c += kRsWarps) {
-            const int i = c * 32 + lane;
-            if ((vbits[c] >> lane) & 1u) {
-                const float sv = score_at(i);
-                const int bk = bucket_of(sv);
-                if (bk <= bstar) {
-                    const unsigned int pos = start[bk] + atomicAdd(&hist[bk], 1u);
-                    keyA[pos] = float_to_ordered(sv);
-                    idxA[pos] = (unsigned short)i;
-                }
-            }
-        }
-        __syncthreads();
-        // ---- 4. rank and write: every stored pair counts the pairs of ITS bucket that precede it in the exact total order
-        //         (ordered key descending, index ascending); start[bucket] + that count is its final rank, and it goes
-        //         straight to the output row -- no sorted copy in shared memory, no separate write-out pass.  One thread
-        //         per pair: ~2.6 pairs per bucket, so the loops are a few iterations long and every lane is busy (a
-        //         thread sorting whole buckets left the warp waiting for its largest bucket: 19 k of 59 k cycles).
-        const int stored = (int)hd->stored;
-        // the scatter cursors are dead: their 32 KB stage the output row (u16 anchor index per rank), so that the global
-        // writes of the index row are coalesced instead of one sector per pair (12 000 scattered 4-byte stores)
-        unsigned short* orow = reinterpret_cast<unsigned short*>(hist);
-        const bool stage_row = (size_t)keff * 2 <= 4 * (size_t)kBuckets;
-        for (int p2 = tid; p2 < stored; p2 += kRsThreads) {
-            const unsigned int ku = keyA[p2];
-            const unsigned int ki = idxA[p2];
-            const int bk = bucket_of(ordered_to_float(ku));
-            const int s0 = (int)start[bk], s1 = (int)start[bk + 1];
-            int rank = s0;
-            for (int a = s0; a < s1; ++a) {
-                const unsigned int ka = keyA[a];
-                rank += (ka > ku || (ka == ku && (unsigned int)idxA[a] < ki)) ? 1 : 0;
-            }
-            if (rank < keff) {
-                const size_t oo = (size_t)b * k + rank;
-                const int i = (int)ki;
-                if (stage_row) orow[rank] = (unsigned short)ki;
-                else out_idx[oo] = i;
-                if (out_scores) out_scores[oo] = ordered_to_float(ku);
-                if (out_cidx) out_cidx[oo] = (int)(vpre[i >> 5] + __popc(vbits[i >> 5] & ((1u << (i & 31)) - 1u)));
-                if (out_boxes) out_boxes[oo] = boxes[(size_t)b * N + i];
-            }
-        }
-        if (stage_row) {
-            __syncthreads();
-            int32_t* orow_g = out_idx + (size_t)b * k;
-            for (int j2 = tid; j2 < keff; j2 += kRsThreads) orow_g[j2] = (int32_t)orow[j2];
-        }
-    }
-    // ---- 5. padding past the count ----------------------------------------------------------------------
-    for (int j2 = keff + tid; j2 < k; j2 += kRsThreads) {
-        const size_t oo = (size_t)b * k + j2;
-        out_idx[oo] = -1;
-        if (out_scores) out_scores[oo] = __uint_as_float(0xff800000u);  // -inf
-        if (out_cidx) out_cidx[oo] = -1;
-        if (out_boxes) out_boxes[oo] = make_float4(0.f, 0.f, 0.f, 0.f);
-    }
-    __syncthreads();
-}
-
-// ------------------------------------------------------------------------------------------------
-// Bucket top-k over a thread-block CLUSTER per image (small batches: one CTA per image leaves most SMs idle -- a single
-// image ran on ONE SM).  CTA r of the S CTAs owns a contiguous range of the 32-anchor chunks: it loads / stages /
-// histograms its own scores; the S histograms are merged through distributed shared memory (every CTA reads the peers'
-// counts and derives the same bucket starts, plus the offset of its own pairs inside every bucket); pairs are scattered
-// straight into the shared memory of the CTA that OWNS their bucket (buckets are dealt to the CTAs by their start
-// position, whole buckets only), which ranks them and writes its contiguous piece of the output row.  Same buckets, same
-// exact total order (key descending, index ascending) as the one-CTA kernel: identical results; inputs that do not bucket
-// are redone by CTA 0 alone on the radix path.
 struct BkXch {
     float mn, mx;
     unsigned int nvalid, bad;
@@ -635,19 +422,20 @@ struct BkcHdr {
 };
 
 struct BkcLayout {
-    size_t vbits, vpre, hist, start, off, sval, keyA, idxA, total;
+    size_t vbits, vpre, hist, start, sval, keyA, idxA, total;
     int cper, capS;
 };
-static BkcLayout bkc_layout(int cap, int nchunks, int S, bool staged) {
-    BkcLayout L;
+constexpr BkcLayout bkc_layout(int cap, int nchunks, int S, bool staged) {
+    BkcLayout L{};
     L.cper = (nchunks + S - 1) / S;
-    L.capS = (cap + S - 1) / S + 256;
+    // pairs a CTA may own: a single CTA owns all `stored <= cap`; with S > 1 an owner may take up to one bucket
+    // (<= kBucketMax pairs) beyond cap / S
+    L.capS = S == 1 ? cap : (cap + S - 1) / S + 256;
     size_t o = up16(sizeof(BkcHdr));
     L.vbits = o; o += 4 * (size_t)L.cper;
     L.vpre = o;  o = up16(o + 4 * (size_t)L.cper);
     L.hist = o;  o += 4 * (size_t)kBuckets;
     L.start = o; o = up16(o + 2 * (size_t)(kBuckets + 1));
-    L.off = o;   o = up16(o + 2 * (size_t)kBuckets);
     L.sval = o;  o = up16(o + (staged ? 4 * 32 * (size_t)L.cper : 0));
     L.keyA = o;  o += 4 * (size_t)L.capS;
     L.idxA = o;  o = up16(o + 2 * (size_t)L.capS);
@@ -655,24 +443,29 @@ static BkcLayout bkc_layout(int cap, int nchunks, int S, bool staged) {
     return L;
 }
 
-template <bool kStaged>
+// kStaged: scores staged in shared memory, or re-read from global / L2 in the two passes.  kCluster: launched with S > 1;
+// without it (S = 1) the cluster barriers and distributed-shared-memory mappings below are plain CTA barriers and shared
+// accesses -- a cluster barrier carries a memory fence and an L1 invalidate, and a mapped access is a generic one, which
+// cost one CTA per image 22-32 % of its time (tools/topk_latency.py, B200 at 1000 W)
+template <bool kStaged, bool kCluster>
 __global__ void __launch_bounds__(kRsThreads, 1)
-    topk_bucket_cluster_kernel(const float* __restrict__ scores, const uint8_t* __restrict__ valid,
-                               const float4* __restrict__ boxes, int N, int k, int cap, int nchunks,
-                               float* __restrict__ out_scores, int32_t* __restrict__ out_idx, int32_t* __restrict__ out_cidx,
-                               float4* __restrict__ out_boxes, int32_t* __restrict__ out_count, RsLayout L, int kcap,
-                               BkcLayout Lc) {
+    topk_bucket_kernel(const float* __restrict__ scores, const uint8_t* __restrict__ valid,
+                       const float4* __restrict__ boxes, int N, int k, int cap, int nchunks,
+                       float* __restrict__ out_scores, int32_t* __restrict__ out_idx, int32_t* __restrict__ out_cidx,
+                       float4* __restrict__ out_boxes, int32_t* __restrict__ out_count, RsLayout L, int kcap,
+                       BkcLayout Lc) {
     namespace cg = cooperative_groups;
     extern __shared__ __align__(16) unsigned char smem[];
     cg::cluster_group cluster = cg::this_cluster();
-    const int S = (int)cluster.num_blocks(), rank = (int)cluster.block_rank();
+    const int S = kCluster ? (int)cluster.num_blocks() : 1, rank = kCluster ? (int)cluster.block_rank() : 0;
+    auto csync = [&] { if (kCluster) cluster.sync(); else __syncthreads(); };
+    auto peer = [&](auto* p, int r) { return kCluster ? cluster.map_shared_rank(p, r) : p; };
     const int b = (int)blockIdx.x / S;
     BkcHdr* hd = reinterpret_cast<BkcHdr*>(smem);
     unsigned int* vbits = reinterpret_cast<unsigned int*>(smem + Lc.vbits);
     unsigned int* vpre = reinterpret_cast<unsigned int*>(smem + Lc.vpre);
     unsigned int* hist = reinterpret_cast<unsigned int*>(smem + Lc.hist);
     unsigned short* start = reinterpret_cast<unsigned short*>(smem + Lc.start);
-    unsigned short* off = reinterpret_cast<unsigned short*>(smem + Lc.off);
     float* sval = reinterpret_cast<float*>(smem + Lc.sval);
     unsigned int* keyA = reinterpret_cast<unsigned int*>(smem + Lc.keyA);
     unsigned short* idxA = reinterpret_cast<unsigned short*>(smem + Lc.idxA);
@@ -753,11 +546,11 @@ __global__ void __launch_bounds__(kRsThreads, 1)
             if (lane < S) {  // this CTA's summary into every CTA's exchange array
                 BkXch x;
                 x.mn = a; x.mx = z; x.nvalid = nvalid_local; x.bad = hd->bad;
-                *cluster.map_shared_rank(&hd->xch[rank], lane) = x;
+                *peer(&hd->xch[rank], lane) = x;
             }
         }
     }
-    cluster.sync();
+    csync();
     float smin = 3.0e38f, smax = -3.0e38f;
     unsigned int nvalid = 0, anybad = 0;
     for (int r = 0; r < S; ++r) {
@@ -779,15 +572,16 @@ __global__ void __launch_bounds__(kRsThreads, 1)
             const int i = c * 32 + lane;
             if ((vbits[c - c_lo] >> lane) & 1u) atomicAdd(&hist[bucket_of(score_at(i))], 1u);
         }
-        cluster.sync();  // every CTA's counts are complete
-        // ---- 2. merged counts -> bucket starts (same in every CTA), offset of the own pairs inside every bucket ------
+        csync();  // every CTA's counts are complete
+        // ---- 2. merged counts -> bucket starts (same in every CTA), pairs of the lower-ranked CTAs in every bucket ----
+        constexpr int kPerT = kBuckets / kRsThreads;
+        unsigned int o4[kPerT];
         {
-            constexpr int kPerT = kBuckets / kRsThreads;
-            unsigned int h4[kPerT], o4[kPerT], t4 = 0;
+            unsigned int h4[kPerT], t4 = 0;
 #pragma unroll
             for (int q = 0; q < kPerT; ++q) { h4[q] = 0; o4[q] = 0; }
             for (int r = 0; r < S; ++r) {
-                const uint4* ph = reinterpret_cast<const uint4*>(cluster.map_shared_rank(hist, r) + kPerT * tid);
+                const uint4* ph = reinterpret_cast<const uint4*>(peer(hist, r) + kPerT * tid);
 #pragma unroll
                 for (int q4 = 0; q4 < kPerT / 4; ++q4) {
                     const uint4 v = ph[q4];
@@ -796,7 +590,7 @@ __global__ void __launch_bounds__(kRsThreads, 1)
                 }
             }
 #pragma unroll
-            for (int q = 0; q < kPerT; ++q) { t4 += h4[q]; off[kPerT * tid + q] = (unsigned short)min(o4[q], 65535u); }
+            for (int q = 0; q < kPerT; ++q) t4 += h4[q];
             unsigned int tot;
             unsigned int run = block_exclusive_scan(t4, hd->warp_tmp, &tot);
             unsigned int big = 0;
@@ -822,10 +616,14 @@ __global__ void __launch_bounds__(kRsThreads, 1)
             __syncthreads();
             handover = hd->bad != 0u;
         }
-        cluster.sync();  // every CTA has read the counts: they become the scatter cursors
+        csync();  // every CTA has read the counts: they become the scatter cursors, past the lower ranks' pairs
+        uint4* cur = reinterpret_cast<uint4*>(hist + kPerT * tid);
+#pragma unroll
+        for (int q4 = 0; q4 < kPerT / 4; ++q4)
+            cur[q4] = make_uint4(o4[4 * q4 + 0], o4[4 * q4 + 1], o4[4 * q4 + 2], o4[4 * q4 + 3]);
     }
     if (handover) {  // cluster-uniform: CTA 0 redoes the image alone on the radix path
-        cluster.sync();
+        csync();
         if (rank != 0) return;
         if (L.staged) topk_radix_body<true>(smem, scores, valid, boxes, N, k, kcap, nchunks, L, out_scores, out_idx, out_cidx,
                                             out_boxes, out_count, b);
@@ -844,7 +642,6 @@ __global__ void __launch_bounds__(kRsThreads, 1)
             const unsigned int o = owner_of(start[bk]);
             if (bk == 0 || owner_of(start[bk - 1]) != o) hd->obase[o] = start[bk];
         }
-        for (int i = tid; i < kBuckets; i += kRsThreads) hist[i] = 0u;
         __syncthreads();
         // ---- 3. scatter the own pairs of buckets <= b* into their owners' arrays ------------------------------------
         for (int c = c_lo + warp; c < c_hi; c += kRsWarps) {
@@ -854,22 +651,28 @@ __global__ void __launch_bounds__(kRsThreads, 1)
                 const int bk = bucket_of(sv);
                 if (bk <= bstar) {
                     const unsigned int s0 = start[bk];
-                    const unsigned int pos = s0 + off[bk] + atomicAdd(&hist[bk], 1u);
+                    const unsigned int pos = s0 + atomicAdd(&hist[bk], 1u);
                     const unsigned int o = owner_of(s0);
                     const unsigned int li = pos - hd->obase[o];
-                    cluster.map_shared_rank(keyA, o)[li] = float_to_ordered(sv);
-                    cluster.map_shared_rank(idxA, o)[li] = (unsigned short)i;
+                    peer(keyA, o)[li] = float_to_ordered(sv);
+                    peer(idxA, o)[li] = (unsigned short)i;
                 }
             }
         }
-        cluster.sync();
-        // ---- 4. rank the own range and write its piece of the output row ---------------------------------------------
+        csync();
+        // ---- 4. rank the own range and write its piece of the output row: every stored pair counts the pairs of ITS
+        //         bucket that precede it in the exact total order (ordered key descending, index ascending); start[bucket]
+        //         + that count is its final rank -- no sorted copy in shared memory, no separate write-out pass.  One
+        //         thread per pair: ~2.6 pairs per bucket, so the loops are a few iterations long and every lane is busy (a
+        //         thread sorting whole buckets left the warp waiting for its largest bucket: 19 k of 59 k cycles).
         const unsigned int my0 = hd->obase[rank];
         unsigned int my1 = stored;
         for (int o = rank + 1; o < S; ++o)
             if (hd->obase[o] != 0xffffffffu) { my1 = hd->obase[o]; break; }
         const int cnt = my0 == 0xffffffffu ? 0 : (int)(my1 - my0);
-        unsigned short* orow = reinterpret_cast<unsigned short*>(hist);  // cursors are dead: staged output piece
+        // the scatter cursors are dead: their 32 KB stage the output piece (u16 anchor index per rank, keff <= 16384), so
+        // that the global writes of the index row are coalesced instead of one sector per pair
+        unsigned short* orow = reinterpret_cast<unsigned short*>(hist);
         __syncthreads();
         for (int p2 = tid; p2 < cnt; p2 += kRsThreads) {
             const unsigned int ku = keyA[p2];
@@ -889,8 +692,8 @@ __global__ void __launch_bounds__(kRsThreads, 1)
                 if (out_scores) out_scores[oo] = ordered_to_float(ku);
                 if (out_cidx) {
                     const int hc = i >> 5, hr = min(S - 1, hc / Lc.cper);   // the anchor's home CTA holds its validity words
-                    const unsigned int hb = cluster.map_shared_rank(vbits, hr)[hc - hr * Lc.cper];
-                    const unsigned int hp = cluster.map_shared_rank(vpre, hr)[hc - hr * Lc.cper];
+                    const unsigned int hb = peer(vbits, hr)[hc - hr * Lc.cper];
+                    const unsigned int hp = peer(vpre, hr)[hc - hr * Lc.cper];
                     unsigned int base_r = 0;
                     for (int q = 0; q < hr; ++q) base_r += hd->xch[q].nvalid;
                     out_cidx[oo] = (int)(base_r + hp + __popc(hb & ((1u << (i & 31)) - 1u)));
@@ -913,21 +716,14 @@ __global__ void __launch_bounds__(kRsThreads, 1)
         if (out_cidx) out_cidx[oo] = -1;
         if (out_boxes) out_boxes[oo] = make_float4(0.f, 0.f, 0.f, 0.f);
     }
-    cluster.sync();  // nobody leaves while a peer may still read its shared memory
+    csync();  // nobody leaves while a peer may still read its shared memory
 }
 
-constexpr size_t bucket_smem(int N, int cap, int nchunks, bool staged) {
-    size_t o = up16(sizeof(BkHdr));
-    o = up16(o + 8 * (size_t)nchunks);
-    o = up16(o + 4 * (size_t)kBuckets);
-    o = up16(o + 2 * (size_t)(kBuckets + 1));
-    o = up16(o + (staged ? 4 * (size_t)N : 0));
-    return up16(o + 6 * (size_t)cap);
-}
 constexpr size_t kSmemLimit = 227 * 1024;
-// The largest shape topk_radix_launch takes (N 65536, k 16384) fits the bucket kernel unstaged, so every shape that has a
-// radix layout runs the bucket kernel, with the radix path as its hand-over.
-static_assert(bucket_smem(65536, 16384 + kBucketSlack, 65536 / 32, false) <= kSmemLimit,
+// The largest shape topk_radix_launch takes (N 65536, k 16384) fits the bucket kernel unstaged at one CTA per image (two
+// CTAs per image need less), so every shape that has a radix layout runs the bucket kernel, with the radix path as its
+// hand-over.
+static_assert(bkc_layout(16384 + kBucketSlack, 65536 / 32, 1, false).total <= kSmemLimit,
               "the bucket kernel must fit every shape of the fast path");
 
 // Returns FRR_OK when the launch was done, 1 when the shape is outside the fast path (caller falls back).
@@ -945,44 +741,31 @@ int topk_radix_launch(const float* scores, const uint8_t* valid, const float* bo
     if (L.total > limit) return 1;
     // bucket kernel, with the radix path compiled in as its hand-over
     const int cap = kcap + kBucketSlack;
-    const bool bstaged = bucket_smem(N, cap, nchunks, true) <= limit;
-    const size_t bsm = bucket_smem(N, cap, nchunks, bstaged);
     // CTAs per image: small batches (B * S <= SMs) spread an image over a cluster; cluster_hint = 1 keeps one CTA per
     // image (the least SM time: several batches in flight).  Two CTAs per image when they fit: 26-27 us against 29-39 us;
     // more do not pay (measured: 4 CTAs equal 2, 8 CTAs take 37-44 us -- five cluster barriers and an S-fold histogram
     // merge against ~25 us of divisible work)
     const int S = cluster_hint != 1 && (long)B * 2 <= num_sms() ? 2 : 1;
-    if (S > 1) {
-        BkcLayout Lc = bkc_layout(cap, nchunks, S, true);
-        const bool cstaged = Lc.total <= limit;
-        if (!cstaged) Lc = bkc_layout(cap, nchunks, S, false);
-        if (Lc.total <= limit) {
-            auto ckern = cstaged ? topk_bucket_cluster_kernel<true> : topk_bucket_cluster_kernel<false>;
-            FRR_CUDA(cudaFuncSetAttribute(ckern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
-            cudaLaunchConfig_t cfg = {};
-            cfg.gridDim = dim3((unsigned)(B * S), 1, 1);
-            cfg.blockDim = dim3((unsigned)kRsThreads, 1, 1);
-            cfg.dynamicSmemBytes = Lc.total > L.total ? Lc.total : L.total;
-            cfg.stream = (cudaStream_t)stream;
-            cudaLaunchAttribute attr[1];
-            attr[0].id = cudaLaunchAttributeClusterDimension;
-            attr[0].val.clusterDim.x = (unsigned)S;
-            attr[0].val.clusterDim.y = 1;
-            attr[0].val.clusterDim.z = 1;
-            cfg.attrs = attr;
-            cfg.numAttrs = 1;
-            FRR_CUDA(cudaLaunchKernelEx(&cfg, ckern, scores, valid, (const float4*)boxes, N, k, cap, nchunks, out_scores, out_idx,
-                                        out_cidx, (float4*)out_boxes, out_count, L, kcap, Lc));
-            count_launch();
-            FRR_CHECK_LAUNCH("topk_bucket_cluster_kernel");
-            return FRR_OK;
-        }
-    }
-    auto bkern = bstaged ? topk_bucket_kernel<true> : topk_bucket_kernel<false>;
-    FRR_CUDA(cudaFuncSetAttribute(bkern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
-    bkern<<<B, kRsThreads, bsm > L.total ? bsm : L.total, (cudaStream_t)stream>>>(
-        scores, valid, (const float4*)boxes, N, k, cap, nchunks, out_scores, out_idx, out_cidx, (float4*)out_boxes,
-        out_count, L, kcap);
+    BkcLayout Lc = bkc_layout(cap, nchunks, S, true);
+    const bool staged = Lc.total <= limit;
+    if (!staged) Lc = bkc_layout(cap, nchunks, S, false);
+    auto kern = S > 1 ? (staged ? topk_bucket_kernel<true, true> : topk_bucket_kernel<false, true>)
+                      : (staged ? topk_bucket_kernel<true, false> : topk_bucket_kernel<false, false>);
+    FRR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)(B * S), 1, 1);
+    cfg.blockDim = dim3((unsigned)kRsThreads, 1, 1);
+    cfg.dynamicSmemBytes = Lc.total > L.total ? Lc.total : L.total;
+    cfg.stream = (cudaStream_t)stream;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = (unsigned)S;
+    attr[0].val.clusterDim.y = 1;
+    attr[0].val.clusterDim.z = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = S > 1 ? 1 : 0;  // one CTA per image: a plain launch
+    FRR_CUDA(cudaLaunchKernelEx(&cfg, kern, scores, valid, (const float4*)boxes, N, k, cap, nchunks, out_scores, out_idx,
+                                out_cidx, (float4*)out_boxes, out_count, L, kcap, Lc));
     count_launch();
     FRR_CHECK_LAUNCH("topk_bucket_kernel");
     return FRR_OK;

@@ -408,9 +408,9 @@ def test_topk_more_than_65536_anchors_takes_the_general_kernel(oracle):
 
 
 def test_topk_bucket_kernel_hands_over_badly_bucketing_inputs(oracle):
-    """The bucket top-k (one histogram pass + per-bucket sorts) hands images whose scores do not bucket well to the radix
-    kernel (out_count = -1 between the two launches): all scores equal (empty range), one value repeated far beyond the
-    bucket capacity, infinities.  Mixed in one batch with a well-behaved image; every row must equal the oracle's
+    """The bucket top-k (one histogram pass + per-bucket ranking) hands images whose scores do not bucket well to the radix
+    path, which CTA 0 of the image runs in the same launch: all scores equal (empty range), one value repeated far beyond
+    the bucket capacity, infinities.  Mixed in one batch with a well-behaved image; every row must equal the oracle's
     order (descending, ties lower index first)."""
     rs = np.random.RandomState(77)
     N, k = 9000, 5000
@@ -460,9 +460,9 @@ def test_proposal_plan_is_cuda_graph_capturable(oracle):
 
 @pytest.mark.parametrize("B,N,k", [(1, 21546, 12000), (3, 20646, 6000), (2, 37350, 6000), (5, 3000, 4000)])
 def test_topk_cluster_kernel_equals_one_cta_kernel(B, N, k):
-    """topk_bucket_cluster_kernel (two CTAs per image, histograms merged through distributed shared memory) against the
-    one-CTA kernel: every output identical -- random scores with an invalid mask, heavy ties (quantised scores), all scores
-    equal (handed to the radix path by CTA 0 alone), and a batch with empty images."""
+    """topk_bucket_kernel on a two-CTA cluster per image (histograms merged through distributed shared memory) against
+    one CTA per image: every output identical -- random scores with an invalid mask, heavy ties (quantised scores), all
+    scores equal (handed to the radix path by CTA 0 alone), and a batch with empty images."""
     rs = np.random.RandomState(77)
     cases = {
         "random": rs.rand(B, N).astype(np.float32),

@@ -2,7 +2,7 @@
 // [0,1] (models/model.py:34): greedy NMS in LARGE chunks with every pair test restricted to admissible buckets.
 //
 // One thread-block cluster per image; every CTA holds the WHOLE kept list in shared memory, the candidates of a chunk
-// (up to 2048, in score order) are dealt round-robin to the CTAs.  Per chunk:
+// (up to 2048 at 1024 threads, 1024 below, in score order) are dealt round-robin to the CTAs.  Per chunk:
 //   A-C  the kept list is re-bucketed (counting sort by key = (area class, x bin), see nms_common.cuh) and every CTA
 //        orders its own candidates by key, so the lanes of a warp walk ranges of similar length;
 //   D    screen: a candidate walks only the kept boxes whose keys are admissible for it -- IoU >= thr needs an area
@@ -33,31 +33,41 @@ namespace cg = cooperative_groups;
 namespace frr {
 
 constexpr int kBkListCap = 2048;   // kept-list capacity (max_keep <= 2047)
-constexpr int kBkEdgeCap = 8192;   // edges per chunk over the whole cluster (each CTA owns kBkEdgeCap / S)
 constexpr int kBkBins = 3;         // x bins of a walk whose bounds are prefetched (more: tail loop)
 constexpr int kBkUpBins = 2;       // same for the upward walk (bins above the own one)
 constexpr int kBkHits = 4;         // screen hits a thread parks per walk before it falls back to the slow walk
 
+// Largest chunk of a CTA of `threads` threads.  Below 1024 threads the chunk arrays are sized for 1024 candidates, which
+// brings the layout of the 512-thread form under half an SM's shared memory: two CTAs (two images) share an SM and
+// one's barrier-bound phases overlap the other's pair tests.  Results never depend on the chunk size.
+__host__ __device__ constexpr int bk_chunk_cap(int threads) { return threads >= 1024 ? kBkChunk : kBkChunk / 2; }
+
+template <int kThreads>
 struct BkSmem {
-    unsigned int lhist[kKeyCap];  // kept list: key histogram, then scatter cursors
+    static constexpr int kCap = bk_chunk_cap(kThreads);
+    static constexpr int kEdgeCap = 2 * kCap;  // edges per chunk over the whole cluster (each CTA owns kEdgeCap / S)
+    float4 lbox[kBkListCap];  // kept list: bucketed by key in phase C, new keeps appended in score order in phase J
+    float la[kBkListCap];     // its c2-scaled screening areas
+    float4 sbox[kCap];        // the chunk's survivors, bucketed (phase G)
+    float ssa[kCap];
+    float4 cbox[kCap];  // the chunk's candidates, score order
+    float csa[kCap];    // c2-scaled screening areas (NaN = always take the exact path)
+    unsigned int lhist[kKeyCap];  // kept list: key histogram, then scatter cursors; from phase E on the same for the survivors
     unsigned int chist[kKeyCap];  // this CTA's candidates
-    unsigned int shist[kKeyCap];  // the chunk's survivors
     unsigned short lstart[kKeyCap];  // first list position of key s; [kKeys + 1] = list length
     unsigned short sstart[kKeyCap];  // same for the bucketed survivors
-    unsigned int edges[kBkEdgeCap];  // (later << 16) | earlier, chunk-local positions; region r belongs to CTA r
+    unsigned int edges[kEdgeCap];    // (later << 16) | earlier, chunk-local positions; region r belongs to CTA r
     unsigned int ecount[kMaxCluster];
     unsigned int ecursor;
     unsigned int work[2];  // dynamic dealing of the items of phases D and H
     unsigned int warp_tmp[32];
-    float4 cbox[kBkChunk];  // the chunk's candidates, score order
-    float csa[kBkChunk];    // c2-scaled screening areas (NaN = always take the exact path)
-    unsigned short ckey[kBkChunk];
-    unsigned short cord[kBkChunk];  // this CTA's candidates ordered by key
-    unsigned short sidx[kBkChunk];  // bucketed survivor -> chunk position
-    unsigned char cstate[2][kBkChunk];  // [chunk parity]: 0 undecided, 1 kept, 2 removed
-    unsigned char pend[kBkChunk];
-    unsigned char ovf[kBkChunk];
-    unsigned int hitbuf[1024 * 4];  // per-thread ring of screen hits (phase H)
+    unsigned short ckey[kCap];
+    unsigned short cord[kCap];  // this CTA's candidates ordered by key
+    unsigned short sidx[kCap];  // bucketed survivor -> chunk position
+    unsigned short hitbuf[kThreads * kBkHits];  // per-thread ring of screen hits (phase H): bucketed survivor positions
+    unsigned char cstate[2][kCap];  // [chunk parity]: 0 undecided, 1 kept, 2 removed
+    unsigned char pend[kCap];
+    unsigned char ovf[kCap];
 };
 
 // One warp: in-place exclusive scan of hist[0 .. kKeyCap) (kKeyPer consecutive entries per lane), optionally also
@@ -225,7 +235,8 @@ __device__ __noinline__ void bk_walk_up_slow(const unsigned short* __restrict__ 
 // A confirmed suppression pair of the chunk: the later box (chunk position i) has the earlier one (j) as predecessor.
 // Appended to this CTA's edge region (mirrored into the other CTAs after the phase); if the region is full the later
 // box is flagged and decides from a walk of its own in the fix-point.
-__device__ __forceinline__ void bk_push_edge(BkSmem* sm, int i, int j, int rank, int ecap) {
+template <class Smem>
+__device__ __forceinline__ void bk_push_edge(Smem* sm, int i, int j, int rank, int ecap) {
     const unsigned int e = atomicAdd(&sm->ecursor, 1u);
     if (e < (unsigned int)ecap) sm->edges[rank * ecap + e] = ((unsigned int)i << 16) | (unsigned int)j;
     else sm->ovf[i] = 1;
@@ -239,7 +250,7 @@ __device__ __forceinline__ int bk_grab(unsigned int* cursor, int per_warp, int l
 }
 
 template <int kThreads>
-__global__ void __launch_bounds__(kThreads)
+__global__ void __launch_bounds__(kThreads, kThreads <= 512 ? 2 : 1)
     nms_bucket_kernel(const float4* __restrict__ boxes, const int32_t* __restrict__ counts, int n, int max_keep, NmsThr thr,
                       int32_t* __restrict__ keep, int32_t* __restrict__ keep_count, float4* __restrict__ out_boxes,
                       const int32_t* __restrict__ gather_idx, int src_n, int kc0, int kc_max, int nsub1, int nsub2) {
@@ -249,28 +260,25 @@ __global__ void __launch_bounds__(kThreads)
     const int img = blockIdx.x / S;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
 
+    using Smem = BkSmem<kThreads>;
+    constexpr int kCap = Smem::kCap;
+    constexpr int kRegList = kBkListCap - kCap;     // phase C: list entries held in registers ...
+    constexpr int kListPer = kRegList / kThreads;   // ... per thread
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    BkSmem* sm = reinterpret_cast<BkSmem*>(smem_raw);
-    float4* bbox[2];
-    float* barea[2];
-    bbox[0] = reinterpret_cast<float4*>(smem_raw + ((sizeof(BkSmem) + 15) & ~(size_t)15));
-    bbox[1] = bbox[0] + kBkListCap;
-    barea[0] = reinterpret_cast<float*>(bbox[1] + kBkListCap);
-    barea[1] = barea[0] + kBkListCap;
+    Smem* sm = reinterpret_cast<Smem*>(smem_raw);
 
     const int cnt = counts ? min(counts[img], n) : n;
     const float4* ib = boxes + (size_t)img * (gather_idx ? src_n : n);
     const int32_t* gi = gather_idx ? gather_idx + (size_t)img * n : nullptr;
     int32_t* ikeep = keep + (size_t)img * max_keep;
     float4* iout = out_boxes ? out_boxes + (size_t)img * max_keep : nullptr;
-    const int ecap = kBkEdgeCap / S;
+    const int ecap = Smem::kEdgeCap / S;
 
     for (int e = tid; e < kKeyCap; e += kThreads) {
         sm->lhist[e] = 0u;
         sm->chist[e] = 0u;
-        sm->shist[e] = 0u;
     }
-    for (int i = tid; i < kBkChunk; i += kThreads) sm->cstate[0][i] = 0;
+    for (int i = tid; i < kCap; i += kThreads) sm->cstate[0][i] = 0;
     if (tid == 0) {
         sm->ecursor = 0u;
         sm->work[0] = 0u;
@@ -281,15 +289,25 @@ __global__ void __launch_bounds__(kThreads)
     cluster_sync();  // every CTA's shared memory is initialised before a peer writes into it
 
     int nk = 0;   // kept so far (identical in every CTA of the cluster)
-    int cur = 0;  // buffer that holds the kept list
     int par = 0;  // chunk parity (cstate double buffer)
     int kc = kc0;
     for (int base = 0; base < cnt && nk < max_keep; par ^= 1) {
         const int m = min(kc, cnt - base);
         unsigned char* st = sm->cstate[par];
         // ---- A: stage the chunk (screening areas, keys), histograms of the list keys and of the own candidates' keys
-        for (int i = tid; i < m; i += kThreads) {
-            const float4 b = gi ? ib[gi[base + i]] : ib[base + i];
+        //      (a thread's gather indices are all loaded before the first box: one memory latency, not two per box)
+        constexpr int kPerA = kCap / kThreads;
+        int src[kPerA];
+#pragma unroll
+        for (int q = 0; q < kPerA; ++q) {
+            const int i = tid + q * kThreads;
+            src[q] = i < m ? (gi ? gi[base + i] : base + i) : 0;
+        }
+#pragma unroll
+        for (int q = 0; q < kPerA; ++q) {
+            const int i = tid + q * kThreads;
+            if (i >= m) break;
+            const float4 b = ib[src[q]];
             const float sa = screen_area(b, thr.c2);
             const int key = bk_key(b, sa);
             sm->cbox[i] = b;
@@ -299,29 +317,59 @@ __global__ void __launch_bounds__(kThreads)
             sm->ovf[i] = 0;
             if (i % S == rank) atomicAdd(&sm->chist[key], 1u);
         }
-        for (int k = tid; k < nk; k += kThreads) atomicAdd(&sm->lhist[bk_key(bbox[cur][k], barea[cur][k])], 1u);
+        for (int k = tid; k < nk; k += kThreads) atomicAdd(&sm->lhist[bk_key(sm->lbox[k], sm->la[k])], 1u);
         __syncthreads();
         // ---- B: exclusive scans (warp 0: list, warp 1: own candidates)
         if (warp == 0) bk_scan_keys(sm->lhist, sm->lstart, lane);
         else if (warp == 1) bk_scan_keys(sm->chist, nullptr, lane);
         __syncthreads();
-        // ---- C: scatter the list into the other buffer, the own candidates into cord
-        for (int k = tid; k < nk; k += kThreads) {
-            const float4 b = bbox[cur][k];
-            const float a = barea[cur][k];
-            const unsigned int pos = atomicAdd(&sm->lhist[bk_key(b, a)], 1u);
-            bbox[cur ^ 1][pos] = b;
-            barea[cur ^ 1][pos] = a;
+        // ---- C: scatter the list in place (order inside a bucket does not matter to any decision), the own
+        //      candidates into cord.  Every entry is read before any is written: list entries below kRegList wait in
+        //      registers (their screening area is recomputed, it is screen_area() of the box), the others in the
+        //      survivors' arrays, which are free until phase G.
+        {
+            float4 lb_r[kListPer > 0 ? kListPer : 1];
+            unsigned int pos[kListPer > 0 ? (kListPer + 1) / 2 : 1];  // two 16-bit list positions per register
+#pragma unroll
+            for (int q = 0; q < kListPer; ++q) {
+                const int k = tid + q * kThreads;
+                if (k < nk) {
+                    lb_r[q] = sm->lbox[k];
+                    const unsigned int p = atomicAdd(&sm->lhist[bk_key(lb_r[q], sm->la[k])], 1u);
+                    pos[q / 2] = (q & 1) ? (pos[q / 2] | (p << 16)) : p;
+                }
+            }
+            for (int k = kRegList + tid; k < nk; k += kThreads) {
+                const float4 b = sm->lbox[k];
+                const float a = sm->la[k];
+                sm->sidx[k - kRegList] = (unsigned short)atomicAdd(&sm->lhist[bk_key(b, a)], 1u);
+                sm->sbox[k - kRegList] = b;
+                sm->ssa[k - kRegList] = a;
+            }
+            for (int i = tid; i < m; i += kThreads)
+                if (i % S == rank) sm->cord[atomicAdd(&sm->chist[sm->ckey[i]], 1u)] = (unsigned short)i;
+            __syncthreads();
+#pragma unroll
+            for (int q = 0; q < kListPer; ++q) {
+                if (tid + q * kThreads < nk) {
+                    const unsigned int p = (pos[q / 2] >> (16 * (q & 1))) & 0xffffu;
+                    sm->lbox[p] = lb_r[q];
+                    sm->la[p] = screen_area(lb_r[q], thr.c2);
+                }
+            }
+            for (int k = kRegList + tid; k < nk; k += kThreads) {
+                const int p = sm->sidx[k - kRegList];
+                sm->lbox[p] = sm->sbox[k - kRegList];
+                sm->la[p] = sm->ssa[k - kRegList];
+            }
         }
-        for (int i = tid; i < m; i += kThreads)
-            if (i % S == rank) sm->cord[atomicAdd(&sm->chist[sm->ckey[i]], 1u)] = (unsigned short)i;
-        cur ^= 1;
         __syncthreads();
-        const float4* lb = bbox[cur];
-        const float* la = barea[cur];
+        const float4* lb = sm->lbox;
+        const float* la = sm->la;
         // ---- D: screen the own candidates against the admissible part of the kept list: nsub1 lanes per candidate,
         //      a warp takes 32 / nsub1 candidates (adjacent in key order: walks of similar length) at a time
         const int n_own = (m - rank + S - 1) / S;
+        for (int e = tid; e < kKeyCap; e += kThreads) sm->lhist[e] = 0u;  // the survivors' histogram of phase E
         if (nk > 0) {
             const int per_warp = 32 / nsub1, sub = lane % nsub1;
             for (;;) {
@@ -354,25 +402,23 @@ __global__ void __launch_bounds__(kThreads)
         }
         cluster_sync();
         // ---- E: histogram of the survivors' keys; reset what the next chunk's phases A-D accumulate into
-        for (int i = tid; i < kBkChunk; i += kThreads) sm->cstate[par ^ 1][i] = 0;
-        for (int e = tid; e < kKeyCap; e += kThreads) {
-            sm->lhist[e] = 0u;
-            sm->chist[e] = 0u;
-        }
+        unsigned int* shist = sm->lhist;  // the list's cursors are done with (zeroed in phase D)
+        for (int i = tid; i < kCap; i += kThreads) sm->cstate[par ^ 1][i] = 0;
+        for (int e = tid; e < kKeyCap; e += kThreads) sm->chist[e] = 0u;
         for (int i = tid; i < m; i += kThreads)
-            if (st[i] == 0) atomicAdd(&sm->shist[sm->ckey[i]], 1u);
+            if (st[i] == 0) atomicAdd(&shist[sm->ckey[i]], 1u);
         __syncthreads();
         // ---- F: scan
-        if (warp == 0) bk_scan_keys(sm->shist, sm->sstart, lane);
+        if (warp == 0) bk_scan_keys(shist, sm->sstart, lane);
         __syncthreads();
-        // ---- G: bucket the survivors into the free list buffer, ordered by (key, chunk position): an unordered
-        //      scatter of the positions, then every entry ranks itself inside its bucket -- the array is the same in
-        //      every CTA of the cluster, which phase H relies on to deal the pairs out
-        float4* sb = bbox[cur ^ 1];
-        float* sa_ = barea[cur ^ 1];
+        // ---- G: bucket the survivors, ordered by (key, chunk position): an unordered scatter of the positions, then
+        //      every entry ranks itself inside its bucket -- the array is the same in every CTA of the cluster, which
+        //      phase H relies on to deal the pairs out
+        float4* sb = sm->sbox;
+        float* sa_ = sm->ssa;
         unsigned short* tmp = sm->cord;  // the own-candidate order is not needed any more
         for (int i = tid; i < m; i += kThreads)
-            if (st[i] == 0) tmp[atomicAdd(&sm->shist[sm->ckey[i]], 1u)] = (unsigned short)i;
+            if (st[i] == 0) tmp[atomicAdd(&shist[sm->ckey[i]], 1u)] = (unsigned short)i;
         __syncthreads();
         const int ns = sm->sstart[kKeys + 1];
         for (int t = tid; t < ns; t += kThreads) {
@@ -392,7 +438,7 @@ __global__ void __launch_bounds__(kThreads)
         {
             const int ns_own = (ns - rank + S - 1) / S;
             const int per_warp = 32 / nsub2, sub = lane % nsub2;
-            unsigned int* hb = sm->hitbuf + tid * kBkHits;
+            unsigned short* hb = sm->hitbuf + tid * kBkHits;
             for (;;) {
                 const int q = bk_grab(&sm->work[1], per_warp, lane) + lane / nsub2;
                 if (q - lane / nsub2 >= ns_own) break;
@@ -404,14 +450,14 @@ __global__ void __launch_bounds__(kThreads)
                 int nh = 0;
                 bk_walk_up(sm->sstart, p, sm->ckey[i], cbx, ca, thr, sub, nsub2, [&](int k) {
                     if (suppress_screen<true>(sb[k], sa_[k], cbx, ca)) {
-                        hb[nh & (kBkHits - 1)] = (unsigned int)k;
+                        hb[nh & (kBkHits - 1)] = (unsigned short)k;
                         ++nh;
                     }
                 });
                 if (nh > kBkHits) {  // more screen hits than the ring holds: walk the share again, confirming as they come
                     const float up = thr.up;
                     const unsigned short* sidx = sm->sidx;
-                    BkSmem* smp = sm;
+                    Smem* smp = sm;
                     bk_walk_up_slow(sm->sstart, p, sm->ckey[i], cbx, ca, thr, sub, nsub2, [=](int k) {
                         if (suppress_screen<true>(sb[k], sa_[k], cbx, ca) && suppress_exact(sb[k], cbx, up)) {
                             const int j = sidx[k];
@@ -501,7 +547,7 @@ __global__ void __launch_bounds__(kThreads)
         // ---- J: append the kept survivors in score order
         int kept_chunk;
         {
-            constexpr int kPer = kBkChunk / kThreads;  // consecutive candidates per thread
+            constexpr int kPer = kCap / kThreads;  // consecutive candidates per thread
             const int i0 = tid * kPer;
             unsigned int c = 0;
 #pragma unroll
@@ -514,8 +560,8 @@ __global__ void __launch_bounds__(kThreads)
                 if (i < m && st[i] == 1) {
                     if (o < max_keep) {
                         const float4 kb = sm->cbox[i];
-                        bbox[cur][o] = kb;
-                        barea[cur][o] = sm->csa[i];
+                        sm->lbox[o] = kb;
+                        sm->la[o] = sm->csa[i];
                         if (rank == 0) {
                             ikeep[o] = base + i;
                             if (iout) iout[o] = kb;
@@ -527,7 +573,7 @@ __global__ void __launch_bounds__(kThreads)
             kept_chunk = (int)total;
             nk = min(nk + kept_chunk, max_keep);
         }
-        for (int e = tid; e < kKeyCap; e += kThreads) sm->shist[e] = 0u;
+        for (int e = tid; e < kKeyCap; e += kThreads) shist[e] = 0u;
         if (tid == 0) {
             sm->ecursor = 0u;
             sm->work[0] = 0u;
@@ -558,9 +604,11 @@ bool nms_bucket_eligible(int n, int max_keep, const NmsThr& thr, int unit_boxes)
     return thr.fast && unit_boxes && kcap < kBkListCap && n >= 1;
 }
 
-size_t nms_bucket_smem_bytes() {
-    return ((sizeof(BkSmem) + 15) & ~(size_t)15) + (size_t)2 * kBkListCap * (sizeof(float4) + sizeof(float));
+size_t nms_bucket_smem_bytes(int threads) {
+    return threads <= 256 ? sizeof(BkSmem<256>) : threads == 512 ? sizeof(BkSmem<512>) : sizeof(BkSmem<1024>);
 }
+// two CTAs of the throughput form per SM: 228 KB of shared memory per SM, 1 KB of it reserved per CTA
+static_assert(sizeof(BkSmem<512>) <= 115712, "the 512-thread layout must fit twice per SM");
 
 int nms_bucket_launch(const float* boxes, const int32_t* counts, int B, int n, const NmsThr& thr, int max_keep, int32_t* keep,
                       int32_t* keep_count, float* out_boxes, int S, int threads, const NmsTune& tune, frr_stream_t stream,
@@ -569,12 +617,16 @@ int nms_bucket_launch(const float* boxes, const int32_t* counts, int B, int n, c
                             int, int, int, int, int);
     kern_t kern = threads <= 256 ? nms_bucket_kernel<256> : threads == 512 ? nms_bucket_kernel<512> : nms_bucket_kernel<1024>;
     if (threads < 256) threads = 256;
-    const size_t smem = nms_bucket_smem_bytes();
+    const size_t smem = nms_bucket_smem_bytes(threads);
     FRR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    // (otherwise the driver may pick an L1 / shared split that holds one CTA of the 512-thread form per SM)
+    FRR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     if (S > 8) FRR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
-    // chunk sizes (frr_nms_sorted_tuned has checked them to lie in [256, kBkChunk]): the first chunk is small when few
-    // boxes are wanted (test mode: 300), at most first_chunk (automatic: 1024)
-    const int kc_max = tune.max_chunk ? tune.max_chunk & ~255 : kBkChunk;
+    // chunk sizes (frr_nms_sorted_tuned has checked them to lie in [256, kBkChunk]; clamped to what the thread count's
+    // layout holds): the first chunk is small when few boxes are wanted (test mode: 300), at most first_chunk
+    // (automatic: 1024)
+    const int cap = bk_chunk_cap(threads);
+    const int kc_max = tune.max_chunk ? min(tune.max_chunk & ~255, cap) : cap;
     int want = ((max_keep + max_keep / 2) + 255) & ~255;
     if (want < 256) want = 256;
     int kc0 = tune.first_chunk ? tune.first_chunk & ~255 : 1024;

@@ -8,11 +8,12 @@
 namespace frr {
 
 constexpr int kMaxCluster = 16;
-constexpr int kBkChunk = 2048;  // most candidates per chunk of the bucketed kernel (its shared-memory arrays are sized for it)
+constexpr int kBkChunk = 2048;  // most candidates per chunk of the bucketed kernel (1024 below 1024 threads: bk_chunk_cap)
 
 // Per-call settings of the bucketed kernel (frr_nms_sorted_tuned); 0 = automatic.  Results never depend on them.
 struct NmsTune {
-    int first_chunk, max_chunk;      // candidates in the first / the largest chunk: multiples of 256 in [256, kBkChunk]
+    int first_chunk, max_chunk;      // candidates in the first / the largest chunk: multiples of 256 in [256, kBkChunk],
+                                     // clamped to the chunk capacity of the launch's thread count
     int lanes_screen, lanes_pairs;   // lanes per candidate of the screen / pair phases: powers of two <= 32
 };
 
@@ -112,7 +113,7 @@ int nms_launch(const float* boxes, const int32_t* counts, int B, int n, double i
 
 // nms_bucket.cu: eligibility + launch of the bucketed kernel (unit-range boxes, screenable threshold, kept list <= 2047)
 bool nms_bucket_eligible(int n, int max_keep, const NmsThr& thr, int unit_boxes);
-size_t nms_bucket_smem_bytes();
+size_t nms_bucket_smem_bytes(int threads);  // dynamic shared memory of a launch with `threads` threads per CTA
 int nms_bucket_launch(const float* boxes, const int32_t* counts, int B, int n, const NmsThr& thr, int max_keep, int32_t* keep,
                       int32_t* keep_count, float* out_boxes, int S, int threads, const NmsTune& tune, frr_stream_t stream,
                       const int32_t* gather_idx, int src_n);

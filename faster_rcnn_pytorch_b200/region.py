@@ -146,9 +146,10 @@ class ProposalPlan:
 class ProposalPipeline:
     """Throughput mode for DEVICE-resident head outputs: ``depth`` independent plans, each on its own stream, so
     that consecutive batches overlap on the GPU.  The top-k and NMS kernels run one CTA per image (NMS with
-    ``nms_cluster_size=1``: 146 us per image-CTA instead of 121 us for a 2-CTA cluster, but 9.4 k instead of 15.5 k
+    ``nms_cluster_size=1``: 144 us per image-CTA instead of 108 us for a 2-CTA cluster, but 9.2 k instead of 13.8 k
     SM-microseconds per 64 images); the 84 SMs they leave idle at 64 images are filled by the neighbouring batches'
-    kernels.  Measured at 64 images of 21 546 anchors: 413 k images/s one batch at a time, 654 k / 708 k with 3 / 4 in flight.
+    kernels.  Measured at 64 images of 21 546 anchors (B200, 1965 MHz, 1000 W): 456 k images/s one batch at a time,
+    772-777 k with 4 in flight.
 
     ``submit(cls, reg)`` orders the plan's stream after the caller's current stream (the producer of cls / reg),
     issues one ``frr_rpn_proposals`` call (or replays the graph captured for these tensors) and returns a ticket;

@@ -1,0 +1,37 @@
+// Developer tool: resident CTAs per SM of every bucketed NMS kernel at the shared memory its launches use
+// (cudaOccupancyMaxActiveBlocksPerMultiprocessor).  Built and run by tools/nms_two_per_sm.py; one JSON line per kernel.
+#include <cstdarg>
+#include <cstdio>
+
+#include "nms_bucket.cu"
+
+namespace frr {
+std::atomic<uint64_t> g_launches{0};
+void set_error(const char* fmt, ...) {
+    va_list ap;
+    va_start(ap, fmt);
+    vfprintf(stderr, fmt, ap);
+    va_end(ap);
+    fputc('\n', stderr);
+}
+}  // namespace frr
+
+template <int kThreads>
+static int report() {
+    auto kern = frr::nms_bucket_kernel<kThreads>;
+    const size_t smem = frr::nms_bucket_smem_bytes(kThreads);
+    FRR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    FRR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    cudaFuncAttributes fa;
+    FRR_CUDA(cudaFuncGetAttributes(&fa, kern));
+    int blocks = 0;
+    FRR_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, kern, kThreads, smem));
+    printf("{\"kernel\": \"nms_bucket_kernel<%d>\", \"dynamic_smem\": %zu, \"registers\": %d, \"local_bytes\": %zu, "
+           "\"ctas_per_sm\": %d}\n", kThreads, smem, fa.numRegs, fa.localSizeBytes, blocks);
+    return 0;
+}
+
+int main() {
+    if (report<256>() || report<512>() || report<1024>()) return 1;
+    return 0;
+}

@@ -59,6 +59,16 @@ SIGNATURES = {
     "frr_class_nms_workspace_bytes": (C.c_size_t, [_i, _i, _i]),
     "frr_class_nms": (_i, [_p, _p, _p, _i, _i, _i, _f, _d, _i, _p, _p, _p, _p, _p, C.c_size_t, _p]),
     "frr_nms_sorted_tuned": (_i, [_p, _p, _i, _i, _d, _i, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _p]),
+    # mixed-size batches: per-image sizes image_hw [B,2] on the device
+    "frr_rpn_decode_sized": (_i, [_p, _p, _i, _p, _i, _p, _i, _i, _i, _f, _p, _p, _p, _i, _i, _p]),
+    "frr_rpn_proposals_sized": (_i, [_p, _p, _i, _p, _i, _p, _i, _i, _i, _f, _i, _i, _i, _i, _d, _p, _p, _p, C.c_size_t, _i,
+                                     _p]),
+    "frr_rois5_sized": (_i, [_p, _p, _i, _i, _p, _i, _i, _i, _p, _p]),
+    "frr_roi_pool_fwd_sized": (_i, [_p, _p, _i, _i, _i, _i, _i, _i, _i, _f, _i, _p, _i, _p, _p, _p]),
+    "frr_roi_pool_bwd_deterministic_sized": (_i, [_p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _f, _i, _p, _i, _p, _p]),
+    "frr_rpn_targets_assign_sized": (_i, [_p, _p, _i, _i, _p, _i, _p, _i, _i, _i, _i, _f, _f, _f, _i, _i, _p, _p, _p, _p, _p,
+                                          _p, _p]),
+    "frr_rpn_targets_finalize_sized": (_i, [_p, _i, _i, _p, _i, _p, _i, _i, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p, _p]),
 }
 
 

@@ -59,6 +59,31 @@ __global__ void __launch_bounds__(256) anchors_pyramid_kernel(float4* __restrict
     out[i] = r;
 }
 
+// One image's box, score and validity from its regression t and logits l (l.y alone: a score) and the anchor in centre
+// form, for the mixed-size decode.  The same operations, in the same order, as the body of rpn_decode_kernel below (which
+// keeps them inline: moving them into this function changes that kernel's register allocation).
+template <bool kLogits>
+__device__ __forceinline__ void decode_one(const float4& t, const float2& l, float acx, float acy, float aw, float ah,
+                                           float min_size, float4* boxes, float* scores, uint8_t* valid, size_t g) {
+    float s = l.y;
+    if (kLogits) s = __frcp_rn(__fadd_rn(1.0f, expf(__fsub_rn(l.x, l.y))));
+    // decode: c = t_xy * a_wh + a_c ; wh/2 = exp(t_wh) * a_wh / 2 ; cxcy_to_xy ; clamp(0,1)
+    const float cx = __fadd_rn(__fmul_rn(t.x, aw), acx), cy = __fadd_rn(__fmul_rn(t.y, ah), acy);
+    const float hw = __fmul_rn(__fmul_rn(expf(t.z), aw), 0.5f);
+    const float hh = __fmul_rn(__fmul_rn(expf(t.w), ah), 0.5f);
+    const float r0 = __fsub_rn(cx, hw), r1 = __fsub_rn(cy, hh), r2 = __fadd_rn(cx, hw), r3 = __fadd_rn(cy, hh);
+    float4 bx;
+    bx.x = __saturatef(r0);
+    bx.y = __saturatef(r1);
+    bx.z = __saturatef(r2);
+    bx.w = __saturatef(r3);
+    const bool finite = (r0 == r0) && (r1 == r1) && (r2 == r2) && (r3 == r3);
+    const bool ok = finite && (__fsub_rn(bx.w, bx.y) >= min_size) && (__fsub_rn(bx.z, bx.x) >= min_size);
+    st_stream(boxes + g, bx);
+    scores[g] = s;
+    valid[g] = ok ? 1 : 0;
+}
+
 // One thread per anchor and kImgs images (grid.y = image group): the anchor (4 IEEE divisions) and its
 // centre form are built once and reused for every image of the group; the 2*kImgs loads of a thread are
 // issued back to back (memory-level parallelism) before any arithmetic.
@@ -122,6 +147,57 @@ __global__ void __launch_bounds__(256)
             st_stream(boxes + g, bx);
             scores[g] = s;
             valid[g] = ok ? 1 : 0;
+        }
+    }
+}
+
+// The same for a batch padded to grid_h x grid_w cells (N = grid_h * grid_w * A): only the cell shift is shared by the
+// images of a group; every image divides the anchor by its own (W_b, H_b), exactly as frr_rpn_decode does for that image
+// alone, and cells outside its own grid get box 0, score 0, valid 0 whatever the head outputs hold there.
+template <bool kLogits, int kImgs>
+__global__ void __launch_bounds__(256)
+    rpn_decode_sized_kernel(const float4* __restrict__ reg, const float* __restrict__ cls, AnchorTable tab, int B, int N,
+                            int grid_h, int grid_w, int stride, const int32_t* __restrict__ image_hw, float min_size,
+                            float4* __restrict__ boxes, float* __restrict__ scores, uint8_t* __restrict__ valid) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= N) return;
+    const int b0 = blockIdx.y * kImgs;
+
+    float4 t[kImgs];
+    float2 l[kImgs];
+#pragma unroll
+    for (int j = 0; j < kImgs; ++j) {
+        if (b0 + j < B) {
+            const size_t g = (size_t)(b0 + j) * N + i;
+            t[j] = ld_stream(reg + g);
+            if (kLogits) l[j] = __ldg(reinterpret_cast<const float2*>(cls) + g);
+            else l[j].y = __ldg(cls + g);
+        }
+    }
+
+    const int cell = i / tab.A, a = i - cell * tab.A;
+    const int y = cell / grid_w, x = cell - y * grid_w;
+    const float sx = (float)x * (float)stride, sy = (float)y * (float)stride;  // exact: small integers
+    const float bx1 = __fadd_rn(tab.v[4 * a + 0], sx), by1 = __fadd_rn(tab.v[4 * a + 1], sy);
+    const float bx2 = __fadd_rn(tab.v[4 * a + 2], sx), by2 = __fadd_rn(tab.v[4 * a + 3], sy);
+
+#pragma unroll
+    for (int j = 0; j < kImgs; ++j) {
+        if (b0 + j < B) {
+            const size_t g = (size_t)(b0 + j) * N + i;
+            const int2 ext = image_cells(image_hw, b0 + j, stride, grid_h, grid_w);
+            if (y < ext.x && x < ext.y) {
+                const int2 hw = __ldg(reinterpret_cast<const int2*>(image_hw) + b0 + j);
+                const float W = (float)hw.y, H = (float)hw.x;
+                const float4 an = make_float4(__fdiv_rn(bx1, W), __fdiv_rn(by1, H), __fdiv_rn(bx2, W), __fdiv_rn(by2, H));
+                const float acx = __fmul_rn(__fadd_rn(an.z, an.x), 0.5f), acy = __fmul_rn(__fadd_rn(an.w, an.y), 0.5f);
+                const float aw = __fsub_rn(an.z, an.x), ah = __fsub_rn(an.w, an.y);
+                decode_one<kLogits>(t[j], l[j], acx, acy, aw, ah, min_size, boxes, scores, valid, g);
+            } else {  // padding cell of this image
+                st_stream(boxes + g, make_float4(0.f, 0.f, 0.f, 0.f));
+                scores[g] = 0.f;
+                valid[g] = 0;
+            }
         }
     }
 }
@@ -221,6 +297,38 @@ int frr_rpn_decode(const float* reg, const float* cls, int cls_is_logits, const 
 #undef LAUNCH
     count_launch();
     FRR_CHECK_LAUNCH("rpn_decode_kernel");
+    return FRR_OK;
+}
+
+int frr_rpn_decode_sized(const float* reg, const float* cls, int cls_is_logits, const float* base_table_host, int A,
+                         const int32_t* image_hw, int grid_h, int grid_w, int stride, float min_size, float* boxes,
+                         float* scores, uint8_t* valid, int B, int N, frr_stream_t stream) {
+    using namespace frr;
+    FRR_CHECK_ARG(reg && cls && boxes && scores && valid && image_hw, "frr_rpn_decode_sized: null pointer");
+    FRR_CHECK_ARG(B >= 0 && N >= 0 && B <= 65535, "frr_rpn_decode_sized: bad B=%d N=%d", B, N);
+    FRR_CHECK_ARG(aligned16(reg) && aligned16(boxes), "frr_rpn_decode_sized: reg/boxes must be 16-byte aligned");
+    FRR_CHECK_ARG((reinterpret_cast<uintptr_t>(cls) & 7u) == 0 && aligned8(image_hw),
+                  "frr_rpn_decode_sized: cls and image_hw must be 8-byte aligned");
+    FRR_CHECK_ARG(grid_h >= 0 && grid_w >= 0 && stride > 0, "frr_rpn_decode_sized: bad grid %dx%d / stride %d", grid_h,
+                  grid_w, stride);
+    AnchorTable tab;
+    int rc = fill_anchor_table(&tab, base_table_host, A, stride);
+    if (rc) return rc;
+    FRR_CHECK_ARG((long long)grid_h * grid_w * tab.A == N, "frr_rpn_decode_sized: N=%d does not match a %dx%d grid x A=%d",
+                  N, grid_h, grid_w, tab.A);
+    if (B == 0 || N == 0) return FRR_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+#define LAUNCH(L, I)                                                                                                   \
+    rpn_decode_sized_kernel<L, I><<<dim3((N + 255) / 256, (B + I - 1) / I), 256, 0, st>>>(                           \
+        (const float4*)reg, cls, tab, B, N, grid_h, grid_w, stride, image_hw, min_size, (float4*)boxes, scores, valid)
+    if (cls_is_logits) {
+        if (B >= 4) LAUNCH(true, 4); else LAUNCH(true, 1);
+    } else {
+        if (B >= 4) LAUNCH(false, 4); else LAUNCH(false, 1);
+    }
+#undef LAUNCH
+    count_launch();
+    FRR_CHECK_LAUNCH("rpn_decode_sized_kernel");
     return FRR_OK;
 }
 

@@ -112,4 +112,15 @@ struct AnchorTable {
 
 int fill_anchor_table(AnchorTable* t, const float* base_table_host, int A, int stride);
 
+// Mixed-size batches (the *_sized entry points): image b of a batch padded to a grid of grid_h x grid_w cells has
+// image_hw[b] = (H_b, W_b) pixels and covers cells y < H_b / stride, x < W_b / stride.  The sizes live in device memory,
+// where the host cannot check them, so the extent is clamped to [0, grid] here: an out-of-range size never reads or
+// writes outside the padded grid, and an image with an empty extent has no cells.  image_hw must be 8-byte aligned.
+__device__ __forceinline__ int2 image_cells(const int32_t* __restrict__ image_hw, int b, int stride, int grid_h,
+                                            int grid_w) {
+    const int2 hw = __ldg(reinterpret_cast<const int2*>(image_hw) + b);
+    return make_int2(min(max(hw.x / stride, 0), grid_h), min(max(hw.y / stride, 0), grid_w));
+}
+inline bool aligned8(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 7u) == 0; }
+
 }  // namespace frr

@@ -48,16 +48,19 @@ struct RoiSmemHdr {
 // ---------------------------------------------------------------------------------------------
 // forward (planes in shared memory)
 // ---------------------------------------------------------------------------------------------
-template <bool kAlign>
-__global__ void __launch_bounds__(kRoiThreads)
-    roi_fwd_planes_kernel(const float* __restrict__ feat, const float* __restrict__ rois, int K, int C, int H, int W,
-                          int CB, int PH, int PW, float scale, int sampling, int aligned, int nhwc,
-                          float* __restrict__ out, int32_t* __restrict__ argmax) {
+// kSized: RoIPool windows are clipped to image b's own extent (image_cells) instead of the padded H x W map
+template <bool kAlign, bool kSized>
+__device__ __forceinline__ void roi_fwd_planes_body(const float* __restrict__ feat, const float* __restrict__ rois, int K,
+                                                    int C, int H, int W, int CB, int PH, int PW, float scale, int sampling,
+                                                    int aligned, int nhwc, float* __restrict__ out,
+                                                    int32_t* __restrict__ argmax, const int32_t* __restrict__ image_hw,
+                                                    int stride) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     RoiSmemHdr* hd = reinterpret_cast<RoiSmemHdr*>(smem_raw);
     float* planes = reinterpret_cast<float*>(smem_raw + ((sizeof(RoiSmemHdr) + 127) & ~(size_t)127));
     const int b = blockIdx.y, c0 = blockIdx.x * CB;
     const int HW = H * W, bins = PH * PW;
+    const int2 ext = kSized ? image_cells(image_hw, b, stride, H, W) : make_int2(H, W);
     const int cb = min(CB, C - c0);
     load_planes(planes, feat, b, c0, cb, C, HW, nhwc != 0, &hd->bar);
 
@@ -74,7 +77,7 @@ __global__ void __launch_bounds__(kRoiThreads)
             if (!kAlign) {
                 const PoolGeom g = pool_geom(hd->roi + 5 * slot, scale);
                 int hs, he, ws, we;
-                pool_window(g, ph, pw, PH, PW, H, W, hs, he, ws, we);
+                pool_window(g, ph, pw, PH, PW, ext.x, ext.y, hs, he, ws, we);
                 const bool empty = (he <= hs) || (we <= ws);
                 float best = empty ? 0.f : -FLT_MAX;
                 int bi = -1;
@@ -106,6 +109,20 @@ __global__ void __launch_bounds__(kRoiThreads)
         }
         __syncthreads();
     }
+}
+template <bool kAlign>
+__global__ void __launch_bounds__(kRoiThreads)
+    roi_fwd_planes_kernel(const float* __restrict__ feat, const float* __restrict__ rois, int K, int C, int H, int W,
+                          int CB, int PH, int PW, float scale, int sampling, int aligned, int nhwc,
+                          float* __restrict__ out, int32_t* __restrict__ argmax) {
+    roi_fwd_planes_body<kAlign, false>(feat, rois, K, C, H, W, CB, PH, PW, scale, sampling, aligned, nhwc, out, argmax,
+                                       nullptr, 0);
+}
+__global__ void __launch_bounds__(kRoiThreads)
+    roi_pool_fwd_planes_sized_kernel(const float* __restrict__ feat, const float* __restrict__ rois, int K, int C, int H,
+                                     int W, int CB, int PH, int PW, float scale, int nhwc, float* __restrict__ out,
+                                     int32_t* __restrict__ argmax, const int32_t* __restrict__ image_hw, int stride) {
+    roi_fwd_planes_body<false, true>(feat, rois, K, C, H, W, CB, PH, PW, scale, 0, 0, nhwc, out, argmax, image_hw, stride);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -164,11 +181,12 @@ __global__ void __launch_bounds__(kRoiThreads)
 // ---------------------------------------------------------------------------------------------
 // direct global-memory kernels for planes too large for shared memory (NCHW or NHWC)
 // ---------------------------------------------------------------------------------------------
-template <bool kAlign>
-__global__ void __launch_bounds__(256)
-    roi_fwd_direct_kernel(const float* __restrict__ feat, const float* __restrict__ rois, size_t total, int B, int C, int H, int W,
-                          int PH, int PW, float scale, int sampling, int aligned, int nhwc, float* __restrict__ out,
-                          int32_t* __restrict__ argmax) {
+template <bool kAlign, bool kSized>
+__device__ __forceinline__ void roi_fwd_direct_body(const float* __restrict__ feat, const float* __restrict__ rois,
+                                                    size_t total, int B, int C, int H, int W, int PH, int PW, float scale,
+                                                    int sampling, int aligned, int nhwc, float* __restrict__ out,
+                                                    int32_t* __restrict__ argmax, const int32_t* __restrict__ image_hw,
+                                                    int stride) {
     const int bins = PH * PW;
     for (size_t o = (size_t)blockIdx.x * blockDim.x + threadIdx.x; o < total; o += (size_t)gridDim.x * blockDim.x) {
         const int bin = (int)(o % bins);
@@ -184,8 +202,9 @@ __global__ void __launch_bounds__(256)
         const size_t ps = nhwc ? (size_t)C : 1;  // pixel stride
         if (!kAlign) {
             const PoolGeom g = pool_geom(r, scale);
+            const int2 ext = kSized ? image_cells(image_hw, b, stride, H, W) : make_int2(H, W);
             int hs, he, ws, we;
-            pool_window(g, ph, pw, PH, PW, H, W, hs, he, ws, we);
+            pool_window(g, ph, pw, PH, PW, ext.x, ext.y, hs, he, ws, we);
             const bool empty = (he <= hs) || (we <= ws);
             float best = empty ? 0.f : -FLT_MAX;
             int bi = -1;
@@ -216,6 +235,20 @@ __global__ void __launch_bounds__(256)
             out[o] = __fdiv_rn(acc, g.count);
         }
     }
+}
+template <bool kAlign>
+__global__ void __launch_bounds__(256)
+    roi_fwd_direct_kernel(const float* __restrict__ feat, const float* __restrict__ rois, size_t total, int B, int C, int H, int W,
+                          int PH, int PW, float scale, int sampling, int aligned, int nhwc, float* __restrict__ out,
+                          int32_t* __restrict__ argmax) {
+    roi_fwd_direct_body<kAlign, false>(feat, rois, total, B, C, H, W, PH, PW, scale, sampling, aligned, nhwc, out, argmax,
+                                       nullptr, 0);
+}
+__global__ void __launch_bounds__(256)
+    roi_pool_fwd_direct_sized_kernel(const float* __restrict__ feat, const float* __restrict__ rois, size_t total, int B,
+                                     int C, int H, int W, int PH, int PW, float scale, int nhwc, float* __restrict__ out,
+                                     int32_t* __restrict__ argmax, const int32_t* __restrict__ image_hw, int stride) {
+    roi_fwd_direct_body<false, true>(feat, rois, total, B, C, H, W, PH, PW, scale, 0, 0, nhwc, out, argmax, image_hw, stride);
 }
 
 template <bool kAlign>
@@ -351,7 +384,8 @@ __global__ void __launch_bounds__(kAlignStreamThreads)
 // *_launch runs it (0 = launched, < 0 = error)
 bool roi_fwd_fast_pick(bool align, int B, int C, int H, int W, int PH, int PW, int sampling, RoiPick* pk);
 int roi_fwd_fast_launch(const RoiPick& pk, const float* feat, const float* rois, int K, int B, int C, int H, int W,
-                        float scale, int aligned, int nhwc, float* out, int32_t* argmax, frr_stream_t stream);
+                        float scale, int aligned, int nhwc, float* out, int32_t* argmax, const int32_t* image_hw, int stride,
+                        frr_stream_t stream);
 bool roi_align_bwd_fast_pick(int B, int C, int H, int W, int PH, int PW, int sampling, RoiPick* pk);
 int roi_align_bwd_fast_launch(const RoiPick& pk, const float* grad_out, const float* rois, int K, int B, int C, int H, int W,
                               float scale, int aligned, int nhwc, float* grad_in, frr_stream_t stream);
@@ -404,9 +438,11 @@ static int direct_blocks(size_t total) {
     return (int)((total + 255) / 256 < (size_t)num_sms() * 16 ? (total + 255) / 256 : (size_t)num_sms() * 16);
 }
 
+// image_hw != nullptr (RoIPool only): windows clipped to each image's extent, image_cells(image_hw, b, stride, H, W)
 template <bool kAlign>
 static int roi_forward(const float* feat, const float* rois, int K, int B, int C, int H, int W, int PH, int PW, float scale,
-                       int sampling, int aligned, int nhwc, float* out, int32_t* argmax, frr_stream_t stream) {
+                       int sampling, int aligned, int nhwc, float* out, int32_t* argmax, frr_stream_t stream,
+                       const int32_t* image_hw = nullptr, int stride = 0) {
     FRR_CHECK_ARG(K == 0 || (feat && out && rois), "roi forward: null pointer");
     RoiPick pk;
     {
@@ -415,9 +451,21 @@ static int roi_forward(const float* feat, const float* rois, int K, int B, int C
     }
     if (pk.kernel == kRoiNone) return FRR_OK;
     if (pk.kernel == kPoolFwdFlat || pk.kernel == kAlignFwdFast)
-        return roi_fwd_fast_launch(pk, feat, rois, K, B, C, H, W, scale, aligned, nhwc, out, kAlign ? nullptr : argmax, stream);
+        return roi_fwd_fast_launch(pk, feat, rois, K, B, C, H, W, scale, aligned, nhwc, out, kAlign ? nullptr : argmax,
+                                   image_hw, stride, stream);
     cudaStream_t st = (cudaStream_t)stream;
-    if (pk.kernel == kFwdPlanes) {
+    if (!kAlign && image_hw) {
+        if (pk.kernel == kFwdPlanes) {
+            auto kern = roi_pool_fwd_planes_sized_kernel;
+            FRR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+            kern<<<dim3((C + pk.cb - 1) / pk.cb, B), kRoiThreads, pk.smem, st>>>(feat, rois, K, C, H, W, pk.cb, PH, PW, scale,
+                                                                                 nhwc, out, argmax, image_hw, stride);
+        } else {
+            const size_t total = (size_t)K * C * PH * PW;
+            roi_pool_fwd_direct_sized_kernel<<<direct_blocks(total), 256, 0, st>>>(feat, rois, total, B, C, H, W, PH, PW, scale,
+                                                                                  nhwc, out, argmax, image_hw, stride);
+        }
+    } else if (pk.kernel == kFwdPlanes) {
         auto kern = roi_fwd_planes_kernel<kAlign>;
         FRR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
         dim3 grid((C + pk.cb - 1) / pk.cb, B);
@@ -523,9 +571,42 @@ __global__ void __launch_bounds__(256)
     o[4] = __fmul_rn(v.w, fh);
 }
 
+// The same for a padded batch: image b is scaled by its own grid (fw_b, fh_b) = image_cells(...); the rows of an image
+// whose extent is empty are masked like padding rows.
+__global__ void __launch_bounds__(256)
+    rois5_sized_kernel(const float4* __restrict__ rois, const int32_t* __restrict__ count, int B, int R,
+                       const int32_t* __restrict__ image_hw, int stride, int grid_h, int grid_w, float* __restrict__ out) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= B * R) return;
+    const int b = k / R, r = k - b * R;
+    const int2 ext = image_cells(image_hw, b, stride, grid_h, grid_w);
+    const float fw = (float)ext.y, fh = (float)ext.x;
+    const float4 v = rois[k];
+    float* o = out + 5 * (size_t)k;
+    o[0] = (ext.x > 0 && ext.y > 0 && (count == nullptr || r < count[b])) ? (float)b : -1.0f;
+    o[1] = __fmul_rn(v.x, fw);
+    o[2] = __fmul_rn(v.y, fh);
+    o[3] = __fmul_rn(v.z, fw);
+    o[4] = __fmul_rn(v.w, fh);
+}
+
 }  // namespace frr
 
 extern "C" {
+
+int frr_rois5_sized(const float* rois, const int32_t* count, int B, int R, const int32_t* image_hw, int stride, int grid_h,
+                    int grid_w, float* rois5, frr_stream_t stream) {
+    using namespace frr;
+    FRR_CHECK_ARG(B >= 0 && R >= 0 && stride > 0 && grid_h >= 0 && grid_w >= 0, "frr_rois5_sized: bad sizes");
+    if (B == 0 || R == 0) return FRR_OK;
+    FRR_CHECK_ARG(rois && rois5 && image_hw && aligned16(rois) && aligned8(image_hw),
+                  "frr_rois5_sized: rois (16-byte aligned), image_hw (8-byte aligned) and rois5 must be non-null");
+    rois5_sized_kernel<<<(B * R + 255) / 256, 256, 0, (cudaStream_t)stream>>>((const float4*)rois, count, B, R, image_hw,
+                                                                              stride, grid_h, grid_w, rois5);
+    count_launch();
+    FRR_CHECK_LAUNCH("rois5_sized_kernel");
+    return FRR_OK;
+}
 
 int frr_rois5(const float* rois, const int32_t* count, int B, int R, float fw, float fh, float* rois5, frr_stream_t stream) {
     using namespace frr;
@@ -555,6 +636,15 @@ int frr_fpn_level_rois(const float* rois5, int K, int k_min, int k_max, int cano
 int frr_roi_pool_fwd(const float* feat, const float* rois, int K, int B, int C, int H, int W, int PH, int PW,
                      float spatial_scale, int channels_last, float* out, int32_t* argmax, frr_stream_t stream) {
     return frr::roi_forward<false>(feat, rois, K, B, C, H, W, PH, PW, spatial_scale, 0, 0, channels_last, out, argmax, stream);
+}
+int frr_roi_pool_fwd_sized(const float* feat, const float* rois, int K, int B, int C, int H, int W, int PH, int PW,
+                           float spatial_scale, int channels_last, const int32_t* image_hw, int stride, float* out,
+                           int32_t* argmax, frr_stream_t stream) {
+    using namespace frr;
+    FRR_CHECK_ARG(image_hw && aligned8(image_hw) && stride > 0,
+                  "frr_roi_pool_fwd_sized: image_hw must be non-null and 8-byte aligned, stride > 0");
+    return roi_forward<false>(feat, rois, K, B, C, H, W, PH, PW, spatial_scale, 0, 0, channels_last, out, argmax, stream,
+                              image_hw, stride);
 }
 int frr_roi_pool_bwd(const float* grad_out, const int32_t* argmax, const float* rois, int K, int B, int C, int H, int W,
                      int PH, int PW, float spatial_scale, int channels_last, float* grad_in, frr_stream_t stream) {

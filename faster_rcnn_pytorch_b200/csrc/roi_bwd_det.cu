@@ -126,11 +126,13 @@ __device__ __forceinline__ float det_div(float t, double c, double inv) {
 }
 
 // kCG: channels per CTA = channel sums per thread, 16 unless a ring of 16-channel slots does not fit shared memory
-template <bool kAlign, int kCG>
-__global__ void __launch_bounds__(kDetThreads)
-    roi_bwd_det_kernel(const float* __restrict__ grad_out, const int32_t* __restrict__ argmax,
-                       const float* __restrict__ rois, int K, int C, int H, int W, int PH, int PW, float scale,
-                       int sampling, int aligned, int nhwc, int TW, int tiles_w, float* __restrict__ grad_in) {
+// kSized (RoIPool only): the bin windows are clipped to image b's own extent (image_cells), as in the sized forward
+template <bool kAlign, int kCG, bool kSized>
+__device__ __forceinline__ void roi_bwd_det_body(const float* __restrict__ grad_out, const int32_t* __restrict__ argmax,
+                                                 const float* __restrict__ rois, int K, int C, int H, int W, int PH, int PW,
+                                                 float scale, int sampling, int aligned, int nhwc, int TW, int tiles_w,
+                                                 float* __restrict__ grad_in, const int32_t* __restrict__ image_hw,
+                                                 int stride) {
     constexpr int CG = kCG;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     DetHdr* hd = reinterpret_cast<DetHdr*>(smem_raw);
@@ -147,6 +149,7 @@ __global__ void __launch_bounds__(kDetThreads)
     const bool mine = h < H && w < W;
     const int bins = PH * PW, rows = cg * bins;
     const bool al = aligned != 0;
+    const int2 ext = kSized ? image_cells(image_hw, b, stride, H, W) : make_int2(H, W);  // RoIPool window clip
 
     float acc[CG];
 #pragma unroll
@@ -163,7 +166,7 @@ __global__ void __launch_bounds__(kDetThreads)
             const float* r = rois + 5 * (size_t)k;
             if ((int)__ldg(r) != b) continue;
             int r0, r1, q0, q1;
-            det_footprint<kAlign>(r, scale, H, W, PH, PW, sampling, al, r0, r1, q0, q1);
+            det_footprint<kAlign>(r, scale, ext.x, ext.y, PH, PW, sampling, al, r0, r1, q0, q1);
             if (r0 <= r1 && q0 <= q1 && r0 <= ty1 && r1 >= ty0 && q0 <= tx1 && q1 >= tx0) keep |= 1u << j;
         }
         unsigned int n;
@@ -196,11 +199,11 @@ __global__ void __launch_bounds__(kDetThreads)
                     for (int i = tid; i < PH + PW; i += kDetThreads) {
                         int hs, he, ws, we;
                         if (i < PH) {
-                            pool_window(g, i, 0, PH, PW, H, W, hs, he, ws, we);
+                            pool_window(g, i, 0, PH, PW, ext.x, ext.y, hs, he, ws, we);
                             win[i] = hs;
                             win[PH + i] = he;
                         } else {
-                            pool_window(g, 0, i - PH, PH, PW, H, W, hs, he, ws, we);
+                            pool_window(g, 0, i - PH, PH, PW, ext.x, ext.y, hs, he, ws, we);
                             win[2 * PH + i - PH] = ws;
                             win[2 * PH + PW + i - PH] = we;
                         }
@@ -221,7 +224,7 @@ __global__ void __launch_bounds__(kDetThreads)
                         dr->big = ny > L.ycap || nx > L.xcap;
                     }
                 }
-                if (tid == 0) det_footprint<kAlign>(rr, scale, H, W, PH, PW, sampling, al, dr->r0, dr->r1, dr->q0, dr->q1);
+                if (tid == 0) det_footprint<kAlign>(rr, scale, ext.x, ext.y, PH, PW, sampling, al, dr->r0, dr->r1, dr->q0, dr->q1);
             }
             cp_async_commit();
         };
@@ -329,13 +332,30 @@ __global__ void __launch_bounds__(kDetThreads)
             if (c < cg) dst[(size_t)c * H * W] = acc[c];
     }
 }
+template <bool kAlign, int kCG>
+__global__ void __launch_bounds__(kDetThreads)
+    roi_bwd_det_kernel(const float* __restrict__ grad_out, const int32_t* __restrict__ argmax,
+                       const float* __restrict__ rois, int K, int C, int H, int W, int PH, int PW, float scale,
+                       int sampling, int aligned, int nhwc, int TW, int tiles_w, float* __restrict__ grad_in) {
+    roi_bwd_det_body<kAlign, kCG, false>(grad_out, argmax, rois, K, C, H, W, PH, PW, scale, sampling, aligned, nhwc, TW,
+                                         tiles_w, grad_in, nullptr, 0);
+}
+template <int kCG>
+__global__ void __launch_bounds__(kDetThreads)
+    roi_pool_bwd_det_sized_kernel(const float* __restrict__ grad_out, const int32_t* __restrict__ argmax,
+                                  const float* __restrict__ rois, int K, int C, int H, int W, int PH, int PW, float scale,
+                                  int nhwc, int TW, int tiles_w, float* __restrict__ grad_in,
+                                  const int32_t* __restrict__ image_hw, int stride) {
+    roi_bwd_det_body<false, kCG, true>(grad_out, argmax, rois, K, C, H, W, PH, PW, scale, 0, 0, nhwc, TW, tiles_w, grad_in,
+                                       image_hw, stride);
+}
 
 static const size_t kDetSmemLimit = 227 * 1024;
 
 template <bool kAlign>
 static int roi_backward_det(const float* grad_out, const int32_t* argmax, const float* rois, int K, int B, int C, int H,
                             int W, int PH, int PW, float scale, int sampling, int aligned, int nhwc, float* grad_in,
-                            frr_stream_t stream) {
+                            frr_stream_t stream, const int32_t* image_hw = nullptr, int stride = 0) {
     FRR_CHECK_ARG(K >= 0 && B > 0 && C > 0 && H > 0 && W > 0 && PH > 0 && PW > 0 && B <= 65535,
                   "roi deterministic backward: bad sizes");
     FRR_CHECK_ARG(grad_in && (K == 0 || (grad_out && rois && (kAlign || argmax))),
@@ -357,14 +377,24 @@ static int roi_backward_det(const float* grad_out, const int32_t* argmax, const 
     const int tiles_w = (W + TW - 1) / TW;
     const long tiles = (long)tiles_w * ((H + TH - 1) / TH);
     FRR_CHECK_ARG(tiles <= INT32_MAX, "roi deterministic backward: map too large");
-    auto kern = CG == 16 ? roi_bwd_det_kernel<kAlign, 16>
-              : CG == 8  ? roi_bwd_det_kernel<kAlign, 8>
-              : CG == 2  ? roi_bwd_det_kernel<kAlign, 2>
-                         : roi_bwd_det_kernel<kAlign, 1>;
-    FRR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kDetSmemLimit));
     const dim3 grid((unsigned)tiles, (unsigned)((C + CG - 1) / CG), (unsigned)B);
-    kern<<<grid, kDetThreads, smem, (cudaStream_t)stream>>>(grad_out, argmax, rois, K, C, H, W, PH, PW, scale, sampling,
-                                                            aligned, nhwc, TW, tiles_w, grad_in);
+    if (!kAlign && image_hw) {
+        auto kern = CG == 16 ? roi_pool_bwd_det_sized_kernel<16>
+                  : CG == 8  ? roi_pool_bwd_det_sized_kernel<8>
+                  : CG == 2  ? roi_pool_bwd_det_sized_kernel<2>
+                             : roi_pool_bwd_det_sized_kernel<1>;
+        FRR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kDetSmemLimit));
+        kern<<<grid, kDetThreads, smem, (cudaStream_t)stream>>>(grad_out, argmax, rois, K, C, H, W, PH, PW, scale, nhwc, TW,
+                                                                tiles_w, grad_in, image_hw, stride);
+    } else {
+        auto kern = CG == 16 ? roi_bwd_det_kernel<kAlign, 16>
+                  : CG == 8  ? roi_bwd_det_kernel<kAlign, 8>
+                  : CG == 2  ? roi_bwd_det_kernel<kAlign, 2>
+                             : roi_bwd_det_kernel<kAlign, 1>;
+        FRR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kDetSmemLimit));
+        kern<<<grid, kDetThreads, smem, (cudaStream_t)stream>>>(grad_out, argmax, rois, K, C, H, W, PH, PW, scale, sampling,
+                                                                aligned, nhwc, TW, tiles_w, grad_in);
+    }
     count_launch();
     FRR_CHECK_LAUNCH(kAlign ? "roi_bwd_det_kernel<align>" : "roi_bwd_det_kernel<pool>");
     return FRR_OK;
@@ -379,6 +409,15 @@ int frr_roi_pool_bwd_deterministic(const float* grad_out, const int32_t* argmax,
                                    frr_stream_t stream) {
     return frr::roi_backward_det<false>(grad_out, argmax, rois, K, B, C, H, W, PH, PW, spatial_scale, 0, 0, channels_last,
                                         grad_in, stream);
+}
+int frr_roi_pool_bwd_deterministic_sized(const float* grad_out, const int32_t* argmax, const float* rois, int K, int B,
+                                         int C, int H, int W, int PH, int PW, float spatial_scale, int channels_last,
+                                         const int32_t* image_hw, int stride, float* grad_in, frr_stream_t stream) {
+    using namespace frr;
+    FRR_CHECK_ARG(image_hw && aligned8(image_hw) && stride > 0,
+                  "frr_roi_pool_bwd_deterministic_sized: image_hw must be non-null and 8-byte aligned, stride > 0");
+    return roi_backward_det<false>(grad_out, argmax, rois, K, B, C, H, W, PH, PW, spatial_scale, 0, 0, channels_last,
+                                   grad_in, stream, image_hw, stride);
 }
 int frr_roi_align_bwd_deterministic(const float* grad_out, const float* rois, int K, int B, int C, int H, int W, int PH,
                                     int PW, float spatial_scale, int sampling_ratio, int aligned, int channels_last,

@@ -384,10 +384,12 @@ __device__ __forceinline__ void load_planes_async(float4* px, const float* __res
 constexpr int kFlatThreads = 448;
 constexpr int kFlatGeoCap = 252;  // rois whose bin boundaries are held at once (56 bytes each)
 
-template <int CB, bool kArg>
-__global__ void __launch_bounds__(kFlatThreads, (CB <= 8) ? 2 : 1)
-    roi_pool_fwd_flat_kernel(const float* __restrict__ feat, const float* __restrict__ rois, int K, int C, int H, int W,
-                             float scale, int nhwc, float* __restrict__ out, int32_t* __restrict__ argmax) {
+// kSized: the bin windows are clipped to image b's own extent (image_cells), not to the padded H x W map
+template <int CB, bool kArg, bool kSized>
+__device__ __forceinline__ void roi_pool_fwd_flat_body(const float* __restrict__ feat, const float* __restrict__ rois, int K,
+                                                       int C, int H, int W, float scale, int nhwc, float* __restrict__ out,
+                                                       int32_t* __restrict__ argmax, const int32_t* __restrict__ image_hw,
+                                                       int stride) {
     constexpr int NCH = CB / 4;
     constexpr int kWarps = kFlatThreads / 32;
     extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -399,6 +401,7 @@ __global__ void __launch_bounds__(kFlatThreads, (CB <= 8) ? 2 : 1)
     const int b = blockIdx.y, c0 = blockIdx.x * CB;
     const int HW = H * W;
     const int cb = min(CB, C - c0);
+    const int2 ext = kSized ? image_cells(image_hw, b, stride, H, W) : make_int2(H, W);
     if (nhwc)
         load_pixels<CB, true>(px, feat, b, c0, C, HW, true);
     else
@@ -431,7 +434,7 @@ __global__ void __launch_bounds__(kFlatThreads, (CB <= 8) ? 2 : 1)
             for (int t = tid; t < ng * 2; t += kFlatThreads) {
                 const int s = t >> 1, isw = t & 1;
                 const PoolGeom gm = pool_geom(rois + 5 * (size_t)hd->id[g0 + s], scale);
-                const int len = isw ? gm.rw : gm.rh, start = isw ? gm.sw : gm.sh, lim = isw ? W : H;
+                const int len = isw ? gm.rw : gm.rh, start = isw ? gm.sw : gm.sh, lim = isw ? ext.y : ext.x;
                 const float bsz = __fdiv_rn((float)len, 7.0f);
                 short* o = geo + s * 28 + isw * 14;
 #pragma unroll
@@ -536,6 +539,19 @@ __global__ void __launch_bounds__(kFlatThreads, (CB <= 8) ? 2 : 1)
     }
     }
     cp_async_wait_all();  // (a CTA without rois leaves with nothing in flight)
+}
+template <int CB, bool kArg>
+__global__ void __launch_bounds__(kFlatThreads, (CB <= 8) ? 2 : 1)
+    roi_pool_fwd_flat_kernel(const float* __restrict__ feat, const float* __restrict__ rois, int K, int C, int H, int W,
+                             float scale, int nhwc, float* __restrict__ out, int32_t* __restrict__ argmax) {
+    roi_pool_fwd_flat_body<CB, kArg, false>(feat, rois, K, C, H, W, scale, nhwc, out, argmax, nullptr, 0);
+}
+template <int CB, bool kArg>
+__global__ void __launch_bounds__(kFlatThreads, (CB <= 8) ? 2 : 1)
+    roi_pool_fwd_flat_sized_kernel(const float* __restrict__ feat, const float* __restrict__ rois, int K, int C, int H,
+                                   int W, float scale, int nhwc, float* __restrict__ out, int32_t* __restrict__ argmax,
+                                   const int32_t* __restrict__ image_hw, int stride) {
+    roi_pool_fwd_flat_body<CB, kArg, true>(feat, rois, K, C, H, W, scale, nhwc, out, argmax, image_hw, stride);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -710,10 +726,17 @@ static size_t flat_smem(int CB, int HW) {
 }
 template <bool kArg, int CB>
 static int launch_flat(const RoiPick& pk, const float* feat, const float* rois, int K, int B, int C, int H, int W, float scale,
-                       int nhwc, float* out, int32_t* argmax, cudaStream_t st) {
+                       int nhwc, float* out, int32_t* argmax, const int32_t* image_hw, int stride, cudaStream_t st) {
+    const dim3 grid((C + CB - 1) / CB, B, pk.nz);
+    if (image_hw) {
+        auto kern = roi_pool_fwd_flat_sized_kernel<CB, kArg>;
+        FRR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimit));
+        kern<<<grid, kFlatThreads, pk.smem, st>>>(feat, rois, K, C, H, W, scale, nhwc, out, argmax, image_hw, stride);
+        return FRR_OK;
+    }
     auto kern = roi_pool_fwd_flat_kernel<CB, kArg>;
     FRR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimit));
-    kern<<<dim3((C + CB - 1) / CB, B, pk.nz), kFlatThreads, pk.smem, st>>>(feat, rois, K, C, H, W, scale, nhwc, out, argmax);
+    kern<<<grid, kFlatThreads, pk.smem, st>>>(feat, rois, K, C, H, W, scale, nhwc, out, argmax);
     return FRR_OK;
 }
 
@@ -751,14 +774,15 @@ bool roi_fwd_fast_pick(bool align, int B, int C, int H, int W, int PH, int PW, i
 }
 
 int roi_fwd_fast_launch(const RoiPick& pk, const float* feat, const float* rois, int K, int B, int C, int H, int W,
-                        float scale, int aligned, int nhwc, float* out, int32_t* argmax, frr_stream_t stream) {
+                        float scale, int aligned, int nhwc, float* out, int32_t* argmax, const int32_t* image_hw, int stride,
+                        frr_stream_t stream) {
     cudaStream_t st = (cudaStream_t)stream;
     int rc;
     if (pk.kernel == kPoolFwdFlat) {
         const bool arg = argmax != nullptr;
 #define FRR_FLAT(CBK)                                                                                   \
-    (arg ? launch_flat<true, CBK>(pk, feat, rois, K, B, C, H, W, scale, nhwc, out, argmax, st)          \
-         : launch_flat<false, CBK>(pk, feat, rois, K, B, C, H, W, scale, nhwc, out, argmax, st))
+    (arg ? launch_flat<true, CBK>(pk, feat, rois, K, B, C, H, W, scale, nhwc, out, argmax, image_hw, stride, st)  \
+         : launch_flat<false, CBK>(pk, feat, rois, K, B, C, H, W, scale, nhwc, out, argmax, image_hw, stride, st))
         rc = pk.cb == 8 ? FRR_FLAT(8) : FRR_FLAT(4);
 #undef FRR_FLAT
         if (rc) return rc;

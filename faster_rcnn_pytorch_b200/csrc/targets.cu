@@ -63,6 +63,13 @@ __device__ __forceinline__ float4 anchor_at(const float4* __restrict__ anchors, 
     return r;
 }
 
+// anchor i of a padded batch (cell-major over a grid fw cells wide) lies inside the image extent ext = (fh, fw)
+__device__ __forceinline__ bool in_grid(const AnchorTable& tab, int i, int fw, int2 ext) {
+    const int cell = i / tab.A;
+    const int y = cell / fw, x = cell - y * fw;
+    return y < ext.x && x < ext.y;
+}
+
 struct TgtSmem {
     unsigned int warp_tmp[32];
     unsigned int total[2];
@@ -133,13 +140,17 @@ __device__ void ordered_lists(const int8_t* __restrict__ lab8, int n, int32_t* _
 // at 16 images per batch: 87 us for 165 k IoUs.)
 constexpr int kTgtMaxCluster = 8;
 
-__global__ void __launch_bounds__(kTgtThreads)
-    rpn_assign_kernel(const float4* __restrict__ gt, const int32_t* __restrict__ gt_count, int Gmax,
-                      const float4* __restrict__ anchors, AnchorTable tab, int N, int fw, float stride, float W, float H,
-                      float neg_thr, float pos_thr, float eps, int inside_only, int tie_inclusive,
-                      float* __restrict__ iou_max, int32_t* __restrict__ argmax,
-                      int8_t* __restrict__ lab8, int32_t* __restrict__ pos_list, int32_t* __restrict__ neg_list,
-                      int32_t* __restrict__ counts /* [B,2] */) {
+// kSized: a batch padded to grid_h x fw cells; image b's anchors are divided by its own (W_b, H_b) = image_hw[b] and the
+// cells outside its own grid are labelled like anchors outside the image (-2)
+template <bool kSized>
+__device__ __forceinline__ void rpn_assign_body(const float4* __restrict__ gt, const int32_t* __restrict__ gt_count, int Gmax,
+                                                const float4* __restrict__ anchors, AnchorTable tab, int N, int fw,
+                                                float stride, float W, float H, float neg_thr, float pos_thr, float eps,
+                                                int inside_only, int tie_inclusive, float* __restrict__ iou_max,
+                                                int32_t* __restrict__ argmax, int8_t* __restrict__ lab8,
+                                                int32_t* __restrict__ pos_list, int32_t* __restrict__ neg_list,
+                                                int32_t* __restrict__ counts /* [B,2] */,
+                                                const int32_t* __restrict__ image_hw, int grid_h) {
     namespace cg = cooperative_groups;
     cg::cluster_group cluster = cg::this_cluster();
     const int S = (int)cluster.num_blocks(), rank = (int)cluster.block_rank();
@@ -158,6 +169,13 @@ __global__ void __launch_bounds__(kTgtThreads)
 
     const int b = blockIdx.x / S, tid = threadIdx.x;
     const int i0 = min(rank * cpc * 32, N), i1 = min((rank + 1) * cpc * 32, N);  // this CTA's anchors
+    int2 ext = make_int2(0, 0);
+    if (kSized) {
+        ext = image_cells(image_hw, b, (int)stride, grid_h, fw);
+        const int2 hw = __ldg(reinterpret_cast<const int2*>(image_hw) + b);
+        H = (float)hw.x;
+        W = (float)hw.y;
+    }
     const int G = min(gt_count ? gt_count[b] : Gmax, Gmax);
     for (int g = tid; g < G; g += kTgtThreads) {
         const float4 v = gt[(size_t)b * Gmax + g];
@@ -174,7 +192,8 @@ __global__ void __launch_bounds__(kTgtThreads)
     // pass 1: row max / first argmax, per-GT best inside anchor (iou bits, then lowest index)
     for (int i = i0 + tid; i < i1; i += kTgtThreads) {
         const float4 a = anchor_at(anchors, tab, i, fw, stride, W, H);
-        const bool inside = !inside_only || ((a.x >= 0.f) && (a.y >= 0.f) && (a.z <= 1.f) && (a.w <= 1.f));
+        const bool inside = (!kSized || in_grid(tab, i, fw, ext)) &&
+                            (!inside_only || ((a.x >= 0.f) && (a.y >= 0.f) && (a.z <= 1.f) && (a.w <= 1.f)));
         float mx = 0.f;
         int arg = 0;
         int8_t l = -2;  // outside the image
@@ -259,16 +278,42 @@ __global__ void __launch_bounds__(kTgtThreads)
     ordered_write(lb + i0, i1 - i0, i0, pos_list + (size_t)b * N + base_a, neg_list + (size_t)b * N + base_b, cnt_a, cnt_b);
     if (rank == 0 && tid == 0) { counts[2 * b] = (int)tot_a; counts[2 * b + 1] = (int)tot_b; }
 }
-
 __global__ void __launch_bounds__(kTgtThreads)
-    rpn_finalize_kernel(const float4* __restrict__ gt, int Gmax, const float4* __restrict__ anchors, AnchorTable tab,
-                        int N, int fw, float stride, float W, float H, const int32_t* __restrict__ argmax,
-                        int8_t* __restrict__ lab8, const int32_t* __restrict__ pos_list,
-                        const int32_t* __restrict__ neg_list, const int32_t* __restrict__ disable /* positions */,
-                        const int32_t* __restrict__ disable_off /* [B,3]: start_pos, start_neg, end */,
-                        int64_t* __restrict__ labels, float4* __restrict__ reg) {
+    rpn_assign_kernel(const float4* __restrict__ gt, const int32_t* __restrict__ gt_count, int Gmax,
+                      const float4* __restrict__ anchors, AnchorTable tab, int N, int fw, float stride, float W, float H,
+                      float neg_thr, float pos_thr, float eps, int inside_only, int tie_inclusive,
+                      float* __restrict__ iou_max, int32_t* __restrict__ argmax,
+                      int8_t* __restrict__ lab8, int32_t* __restrict__ pos_list, int32_t* __restrict__ neg_list,
+                      int32_t* __restrict__ counts /* [B,2] */) {
+    rpn_assign_body<false>(gt, gt_count, Gmax, anchors, tab, N, fw, stride, W, H, neg_thr, pos_thr, eps, inside_only,
+                           tie_inclusive, iou_max, argmax, lab8, pos_list, neg_list, counts, nullptr, 0);
+}
+__global__ void __launch_bounds__(kTgtThreads)
+    rpn_assign_sized_kernel(const float4* __restrict__ gt, const int32_t* __restrict__ gt_count, int Gmax, AnchorTable tab,
+                            int N, int grid_h, int grid_w, float stride, const int32_t* __restrict__ image_hw, float neg_thr,
+                            float pos_thr, float eps, int inside_only, int tie_inclusive, float* __restrict__ iou_max,
+                            int32_t* __restrict__ argmax, int8_t* __restrict__ lab8, int32_t* __restrict__ pos_list,
+                            int32_t* __restrict__ neg_list, int32_t* __restrict__ counts /* [B,2] */) {
+    rpn_assign_body<true>(gt, gt_count, Gmax, nullptr, tab, N, grid_w, stride, 0.f, 0.f, neg_thr, pos_thr, eps, inside_only,
+                          tie_inclusive, iou_max, argmax, lab8, pos_list, neg_list, counts, image_hw, grid_h);
+}
+
+// kSized: image b's anchors divided by its own (W_b, H_b); its padding cells carry label -2 from the assign kernel
+template <bool kSized>
+__device__ __forceinline__ void rpn_finalize_body(const float4* __restrict__ gt, int Gmax, const float4* __restrict__ anchors,
+                                                  AnchorTable tab, int N, int fw, float stride, float W, float H,
+                                                  const int32_t* __restrict__ argmax, int8_t* __restrict__ lab8,
+                                                  const int32_t* __restrict__ pos_list, const int32_t* __restrict__ neg_list,
+                                                  const int32_t* __restrict__ disable, const int32_t* __restrict__ disable_off,
+                                                  int64_t* __restrict__ labels, float4* __restrict__ reg,
+                                                  const int32_t* __restrict__ image_hw) {
     // grid = (anchor slabs, images): every CTA finalises a contiguous slab of one image's anchors
     const int b = blockIdx.y, tid = threadIdx.x;
+    if (kSized) {
+        const int2 hw = __ldg(reinterpret_cast<const int2*>(image_hw) + b);
+        H = (float)hw.x;
+        W = (float)hw.y;
+    }
     const int per = (((N + (int)gridDim.x - 1) / (int)gridDim.x) + 31) & ~31;
     const int i0 = min((int)blockIdx.x * per, N), i1 = min(i0 + per, N);
     int8_t* lb = lab8 + (size_t)b * N;
@@ -292,6 +337,25 @@ __global__ void __launch_bounds__(kTgtThreads)
             reg[o] = encode_box(gt[(size_t)b * Gmax + argmax[o]], a);  // :253, for ALL inside anchors
         }
     }
+}
+__global__ void __launch_bounds__(kTgtThreads)
+    rpn_finalize_kernel(const float4* __restrict__ gt, int Gmax, const float4* __restrict__ anchors, AnchorTable tab,
+                        int N, int fw, float stride, float W, float H, const int32_t* __restrict__ argmax,
+                        int8_t* __restrict__ lab8, const int32_t* __restrict__ pos_list,
+                        const int32_t* __restrict__ neg_list, const int32_t* __restrict__ disable /* positions */,
+                        const int32_t* __restrict__ disable_off /* [B,3]: start_pos, start_neg, end */,
+                        int64_t* __restrict__ labels, float4* __restrict__ reg) {
+    rpn_finalize_body<false>(gt, Gmax, anchors, tab, N, fw, stride, W, H, argmax, lab8, pos_list, neg_list, disable,
+                             disable_off, labels, reg, nullptr);
+}
+__global__ void __launch_bounds__(kTgtThreads)
+    rpn_finalize_sized_kernel(const float4* __restrict__ gt, int Gmax, AnchorTable tab, int N, int grid_w, float stride,
+                              const int32_t* __restrict__ image_hw, const int32_t* __restrict__ argmax,
+                              int8_t* __restrict__ lab8, const int32_t* __restrict__ pos_list,
+                              const int32_t* __restrict__ neg_list, const int32_t* __restrict__ disable,
+                              const int32_t* __restrict__ disable_off, int64_t* __restrict__ labels, float4* __restrict__ reg) {
+    rpn_finalize_body<true>(gt, Gmax, nullptr, tab, N, grid_w, stride, 0.f, 0.f, argmax, lab8, pos_list, neg_list, disable,
+                            disable_off, labels, reg, image_hw);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -408,6 +472,49 @@ static int anchor_args(AnchorTable* tab, int* fw, const float* anchors, const fl
     return FRR_OK;
 }
 
+// anchors generated for a padded grid of grid_h x grid_w cells (the *_sized target entry points)
+static int sized_anchor_args(AnchorTable* tab, const float* base_table_host, int A, int grid_h, int grid_w, int stride, int N) {
+    FRR_CHECK_ARG(grid_h >= 0 && grid_w > 0 && stride > 0, "rpn targets: bad grid %dx%d / stride %d", grid_h, grid_w, stride);
+    int rc = fill_anchor_table(tab, base_table_host, A, stride);
+    if (rc) return rc;
+    FRR_CHECK_ARG((long long)grid_h * grid_w * tab->A == N, "rpn targets: N=%d does not match a %dx%d grid", N, grid_h,
+                  grid_w);
+    return FRR_OK;
+}
+
+// One cluster of S CTAs per image: one CTA per ~2048 anchors, at most 8, and no more CTAs than ~2 per SM for the batch
+template <typename... KArgs, typename... Args>
+static int launch_rpn_assign(void (*kern)(KArgs...), int B, int N, int Gmax, frr_stream_t stream, Args... args) {
+    int S = 1;
+    while (S < kTgtMaxCluster && N >= 2048 * (S * 2) && (long)B * (S * 2) <= 2L * num_sms()) S *= 2;
+    const size_t smem = rpn_assign_smem(Gmax, N, S);
+    FRR_CHECK_ARG(smem <= 227 * 1024, "frr_rpn_targets_assign: Gmax=%d N=%d needs %zu B shared memory", Gmax, N, smem);
+    FRR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)(B * S), 1, 1);
+    cfg.blockDim = dim3((unsigned)kTgtThreads, 1, 1);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = (cudaStream_t)stream;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = (unsigned)S;
+    attr[0].val.clusterDim.y = 1;
+    attr[0].val.clusterDim.z = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    FRR_CUDA(cudaLaunchKernelEx(&cfg, kern, args...));
+    count_launch();
+    FRR_CHECK_LAUNCH("rpn_assign_kernel");
+    return FRR_OK;
+}
+
+// finalize: ~2048 anchors per CTA, about two CTAs per SM for the batch at most
+static int finalize_slabs(int B, int N) {
+    int slabs = 1;
+    while (slabs < 16 && N >= 2048 * (slabs * 2) && (long)B * (slabs * 2) <= 2L * num_sms()) slabs *= 2;
+    return slabs;
+}
+
 }  // namespace frr
 
 extern "C" {
@@ -426,29 +533,50 @@ int frr_rpn_targets_assign(const float* gt, const int32_t* gt_count, int B, int 
     int rc = anchor_args(&tab, &fw, anchors, base_table_host, A, img_h, img_w, stride, N);
     if (rc) return rc;
     if (B == 0) return FRR_OK;
-    // cluster size: one CTA per ~2048 anchors, at most 8, and no more CTAs than ~2 per SM for the whole batch
-    int S = 1;
-    while (S < kTgtMaxCluster && N >= 2048 * (S * 2) && (long)B * (S * 2) <= 2L * num_sms()) S *= 2;
-    const size_t smem = rpn_assign_smem(Gmax, N, S);
-    FRR_CHECK_ARG(smem <= 227 * 1024, "frr_rpn_targets_assign: Gmax=%d N=%d needs %zu B shared memory", Gmax, N, smem);
-    FRR_CUDA(cudaFuncSetAttribute(rpn_assign_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)(B * S), 1, 1);
-    cfg.blockDim = dim3((unsigned)kTgtThreads, 1, 1);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = (cudaStream_t)stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = (unsigned)S;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    FRR_CUDA(cudaLaunchKernelEx(&cfg, rpn_assign_kernel, (const float4*)gt, gt_count, Gmax, (const float4*)anchors, tab, N, fw,
-                                (float)stride, (float)img_w, (float)img_h, neg_thr, pos_thr, iou_eps_, inside_only,
-                                tie_inclusive, iou_max, argmax, label8, pos_list, neg_list, counts));
+    return launch_rpn_assign(rpn_assign_kernel, B, N, Gmax, stream, (const float4*)gt, gt_count, Gmax, (const float4*)anchors,
+                             tab, N, fw, (float)stride, (float)img_w, (float)img_h, neg_thr, pos_thr, iou_eps_, inside_only,
+                             tie_inclusive, iou_max, argmax, label8, pos_list, neg_list, counts);
+}
+
+int frr_rpn_targets_assign_sized(const float* gt, const int32_t* gt_count, int B, int Gmax, const float* base_table_host,
+                                 int A, const int32_t* image_hw, int grid_h, int grid_w, int stride, int N, float neg_thr,
+                                 float pos_thr, float iou_eps_, int inside_only, int tie_inclusive, float* iou_max,
+                                 int32_t* argmax, int8_t* label8, int32_t* pos_list, int32_t* neg_list, int32_t* counts,
+                                 frr_stream_t stream) {
+    using namespace frr;
+    FRR_CHECK_ARG(gt && iou_max && argmax && label8 && pos_list && neg_list && counts && image_hw,
+                  "frr_rpn_targets_assign_sized: null pointer");
+    FRR_CHECK_ARG(B >= 0 && Gmax >= 1 && N >= 1, "frr_rpn_targets_assign_sized: bad sizes");
+    FRR_CHECK_ARG(aligned16(gt) && aligned8(image_hw), "frr_rpn_targets_assign_sized: gt / image_hw must be 16 / 8-byte aligned");
+    AnchorTable tab;
+    int rc = sized_anchor_args(&tab, base_table_host, A, grid_h, grid_w, stride, N);
+    if (rc) return rc;
+    if (B == 0) return FRR_OK;
+    return launch_rpn_assign(rpn_assign_sized_kernel, B, N, Gmax, stream, (const float4*)gt, gt_count, Gmax, tab, N, grid_h,
+                             grid_w, (float)stride, image_hw, neg_thr, pos_thr, iou_eps_, inside_only, tie_inclusive, iou_max,
+                             argmax, label8, pos_list, neg_list, counts);
+}
+
+int frr_rpn_targets_finalize_sized(const float* gt, int B, int Gmax, const float* base_table_host, int A,
+                                   const int32_t* image_hw, int grid_h, int grid_w, int stride, int N, const int32_t* argmax,
+                                   int8_t* label8, const int32_t* pos_list, const int32_t* neg_list, const int32_t* disable,
+                                   const int32_t* disable_off, int64_t* labels, float* reg, frr_stream_t stream) {
+    using namespace frr;
+    FRR_CHECK_ARG(gt && argmax && label8 && pos_list && neg_list && labels && reg && image_hw,
+                  "frr_rpn_targets_finalize_sized: null pointer");
+    FRR_CHECK_ARG((disable == nullptr) == (disable_off == nullptr), "frr_rpn_targets_finalize_sized: disable/disable_off mismatch");
+    FRR_CHECK_ARG(aligned16(gt) && aligned16(reg) && aligned8(image_hw),
+                  "frr_rpn_targets_finalize_sized: gt/reg must be 16-byte aligned, image_hw 8-byte aligned");
+    AnchorTable tab;
+    int rc = sized_anchor_args(&tab, base_table_host, A, grid_h, grid_w, stride, N);
+    if (rc) return rc;
+    if (B == 0) return FRR_OK;
+    FRR_CHECK_ARG(B <= 65535, "frr_rpn_targets_finalize_sized: B=%d exceeds the grid limit", B);
+    rpn_finalize_sized_kernel<<<dim3((unsigned)finalize_slabs(B, N), (unsigned)B), kTgtThreads, 0, (cudaStream_t)stream>>>(
+        (const float4*)gt, Gmax, tab, N, grid_w, (float)stride, image_hw, argmax, label8, pos_list, neg_list, disable,
+        disable_off, labels, (float4*)reg);
     count_launch();
-    FRR_CHECK_LAUNCH("rpn_assign_kernel");
+    FRR_CHECK_LAUNCH("rpn_finalize_sized_kernel");
     return FRR_OK;
 }
 
@@ -465,10 +593,8 @@ int frr_rpn_targets_finalize(const float* gt, int B, int Gmax, const float* anch
     int rc = anchor_args(&tab, &fw, anchors, base_table_host, A, img_h, img_w, stride, N);
     if (rc) return rc;
     if (B == 0) return FRR_OK;
-    int slabs = 1;  // ~2048 anchors per CTA, about two CTAs per SM for the batch at most
-    while (slabs < 16 && N >= 2048 * (slabs * 2) && (long)B * (slabs * 2) <= 2L * num_sms()) slabs *= 2;
     FRR_CHECK_ARG(B <= 65535, "frr_rpn_targets_finalize: B=%d exceeds the grid limit", B);
-    rpn_finalize_kernel<<<dim3((unsigned)slabs, (unsigned)B), kTgtThreads, 0, (cudaStream_t)stream>>>(
+    rpn_finalize_kernel<<<dim3((unsigned)finalize_slabs(B, N), (unsigned)B), kTgtThreads, 0, (cudaStream_t)stream>>>(
         (const float4*)gt, Gmax, (const float4*)anchors, tab, N, fw, (float)stride, (float)img_w, (float)img_h, argmax,
         label8, pos_list, neg_list, disable, disable_off, labels, (float4*)reg);
     count_launch();

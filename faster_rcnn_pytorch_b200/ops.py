@@ -87,9 +87,44 @@ def anchors_pyramid(feature_hws, image_hw, device, sizes=(32, 64, 128, 256, 512)
     return out
 
 
-def rpn_decode(reg, cls, image_hw=None, anchors=None, stride: int = 16, table=None, min_size: float = _MIN_SIZE):
+def is_sized(image_hw) -> bool:
+    """True when ``image_hw`` gives one (H, W) per image ([B,2]: a mixed-size batch) rather than one for the batch."""
+    if isinstance(image_hw, torch.Tensor):
+        return image_hw.dim() == 2
+    return image_hw is not None and np.ndim(image_hw) == 2
+
+
+def sized_hw(image_hw, B: int, grid_hw, stride: int, device) -> torch.Tensor:
+    """Per-image sizes of a mixed-size batch as the int32 [B,2] (H, W) device tensor the *_sized kernels read.
+
+    A CUDA tensor is used as it is (int32, [B,2]): its values are read by the kernels when they run, so one captured CUDA
+    graph serves every mix of sizes written into it, and the kernels clamp each image's grid (H // stride, W // stride) to
+    ``grid_hw``.  Host sizes (CPU tensor, numpy array, list of pairs) are checked here, where that costs nothing: every
+    image's grid must fit ``grid_hw``, else ValueError, and they are copied to ``device``."""
+    gh, gw = int(grid_hw[0]), int(grid_hw[1])
+    if isinstance(image_hw, torch.Tensor) and image_hw.is_cuda:
+        if image_hw.dtype != torch.int32 or tuple(image_hw.shape) != (B, 2):
+            raise ValueError(f"image_hw must be an int32 [{B},2] tensor of (H, W) per image")
+        dev = torch.device(device)
+        if dev.type != "cuda" or (dev.index is not None and image_hw.device.index != dev.index):
+            raise ValueError("image_hw must be on the device of the batch")
+        return image_hw.contiguous()
+    hw = np.asarray(image_hw.numpy() if isinstance(image_hw, torch.Tensor) else image_hw, dtype=np.int64)
+    if hw.shape != (B, 2):
+        raise ValueError(f"image_hw must be [{B},2] (H, W) per image, got shape {hw.shape}")
+    if (hw < 0).any() or (hw[:, 0] // stride > gh).any() or (hw[:, 1] // stride > gw).any():
+        raise ValueError(f"image_hw: every image's grid (H // {stride}, W // {stride}) must fit the padded grid {gh}x{gw}")
+    return torch.from_numpy(hw.astype(np.int32)).to(device)
+
+
+def rpn_decode(reg, cls, image_hw=None, anchors=None, stride: int = 16, table=None, min_size: float = _MIN_SIZE,
+               grid_hw=None):
     """Fused A2+P1+P2+P3.  reg [B,N,4]; cls [B,N,2] logits or [B,N] scores.
-    Returns boxes [B,N,4], scores [B,N], valid uint8 [B,N]."""
+    Returns boxes [B,N,4], scores [B,N], valid uint8 [B,N].
+
+    Mixed-size batch: ``image_hw`` [B,2] (one (H, W) per image, see ``sized_hw``) and ``grid_hw`` = the padded grid in
+    cells, N = grid_h * grid_w * A.  Each image is decoded exactly as alone at its own size; its padding cells get
+    box 0, score 0, valid 0."""
     lib = _lib.load()
     reg = _req(reg, "reg")
     cls = _req(cls, "cls")
@@ -100,6 +135,18 @@ def rpn_decode(reg, cls, image_hw=None, anchors=None, stride: int = 16, table=No
     if tuple(cls.shape) != ((B, N, 2) if logits else (B, N)):
         raise ValueError("cls must be [B,N,2] logits or [B,N] scores")
     keep, tptr, A = _table_arg(table)
+    if is_sized(image_hw):
+        if anchors is not None or grid_hw is None:
+            raise ValueError("rpn_decode: per-image sizes need grid_hw and generated anchors")
+        hw = sized_hw(image_hw, B, grid_hw, stride, reg.device)
+        with torch.cuda.device(reg.device):
+            boxes = torch.empty((B, N, 4), dtype=torch.float32, device=reg.device)
+            scores = torch.empty((B, N), dtype=torch.float32, device=reg.device)
+            valid = torch.empty((B, N), dtype=torch.uint8, device=reg.device)
+            _lib.check(lib.frr_rpn_decode_sized(reg.data_ptr(), cls.data_ptr(), int(logits), tptr, A, hw.data_ptr(),
+                                                int(grid_hw[0]), int(grid_hw[1]), stride, float(min_size), boxes.data_ptr(),
+                                                scores.data_ptr(), valid.data_ptr(), B, N, _stream()), "frr_rpn_decode_sized")
+        return boxes, scores, valid
     if anchors is not None:
         anchors = _req(anchors, "anchors")
         if tuple(anchors.shape) != (N, 4):
@@ -238,9 +285,11 @@ def convert_rois(rois, device=None) -> torch.Tensor:
     return rois
 
 
-def rois5(rois, count, feat_hw, out=None):
+def rois5(rois, count, feat_hw, out=None, image_hw=None, stride: int = 16):
     """models/model.py:104-110 for a batch: normalised rois [B,R,4] (+ int32 count [B] or None) -> [B*R,5] feature-map
-    rois with the batch index; rows past count[b] are masked (index -1).  One kernel, no host synchronisation."""
+    rois with the batch index; rows past count[b] are masked (index -1).  One kernel, no host synchronisation.
+    ``image_hw`` [B,2] (mixed-size batch, ``feat_hw`` = the padded grid): image b is scaled by its own grid
+    (W_b // stride, H_b // stride)."""
     lib = _lib.load()
     rois = _req(rois, "rois")
     if rois.dim() != 3 or rois.shape[-1] != 4:
@@ -251,12 +300,20 @@ def rois5(rois, count, feat_hw, out=None):
     with torch.cuda.device(rois.device):
         if out is None:
             out = torch.empty((B * R, 5), dtype=torch.float32, device=rois.device)
+        if image_hw is not None:
+            hw = sized_hw(image_hw, B, feat_hw, stride, rois.device)
+            _lib.check(lib.frr_rois5_sized(rois.data_ptr(), _ptr(count), B, R, hw.data_ptr(), int(stride), int(feat_hw[0]),
+                                           int(feat_hw[1]), out.data_ptr(), _stream()), "frr_rois5_sized")
+            return out
         _lib.check(lib.frr_rois5(rois.data_ptr(), _ptr(count), B, R, float(feat_hw[1]), float(feat_hw[0]), out.data_ptr(),
                                  _stream()), "frr_rois5")
     return out
 
 
-def roi_pool_forward(feat, rois5, output_size=(7, 7), spatial_scale: float = 1.0, want_argmax: bool = True):
+def roi_pool_forward(feat, rois5, output_size=(7, 7), spatial_scale: float = 1.0, want_argmax: bool = True,
+                     image_hw=None, stride: int = 16):
+    """``image_hw`` [B,2] (mixed-size batch padded to the map's H x W cells): every bin window of a roi of image b is
+    clipped to that image's own grid (H_b // stride, W_b // stride) -- stride 1 when ``image_hw`` holds feature extents."""
     lib = _lib.load()
     feat = _req(feat, "features") if feat.is_contiguous() else feat
     if not feat.is_cuda or feat.dtype != torch.float32:
@@ -269,6 +326,12 @@ def roi_pool_forward(feat, rois5, output_size=(7, 7), spatial_scale: float = 1.0
     with torch.cuda.device(feat.device):
         out = torch.empty((K, C, PH, PW), dtype=torch.float32, device=feat.device)
         arg = torch.empty((K, C, PH, PW), dtype=torch.int32, device=feat.device) if want_argmax else None
+        if image_hw is not None:
+            hw = sized_hw(image_hw, B, (H, W), stride, feat.device)
+            _lib.check(lib.frr_roi_pool_fwd_sized(feat.data_ptr(), rois5.data_ptr(), K, B, C, H, W, PH, PW,
+                                                  float(spatial_scale), cl, hw.data_ptr(), int(stride), out.data_ptr(),
+                                                  _ptr(arg), _stream()), "frr_roi_pool_fwd_sized")
+            return out, arg
         _lib.check(lib.frr_roi_pool_fwd(feat.data_ptr(), rois5.data_ptr(), K, B, C, H, W, PH, PW, float(spatial_scale), cl,
                                         out.data_ptr(), _ptr(arg), _stream()), "frr_roi_pool_fwd")
     return out, arg
@@ -279,11 +342,14 @@ def _deterministic(flag):
 
 
 def roi_pool_backward(grad_out, argmax, rois5, feat_shape, spatial_scale: float = 1.0, channels_last: bool = False,
-                      deterministic: bool | None = None):
+                      deterministic: bool | None = None, image_hw=None, stride: int = 16):
     """``deterministic``: True runs the kernel whose gradient is bit-exact with torchvision's CPU backward and the same
-    on every run; None (default) follows ``torch.use_deterministic_algorithms``."""
+    on every run; None (default) follows ``torch.use_deterministic_algorithms``.  ``image_hw``: the per-image sizes the
+    forward clipped with (mixed-size batch); the default backward follows argmax and needs none, the deterministic one
+    clips each bin window to the image's own grid.  The padding region of the gradient is zero either way."""
     lib = _lib.load()
-    fn = lib.frr_roi_pool_bwd_deterministic if _deterministic(deterministic) else lib.frr_roi_pool_bwd
+    det = _deterministic(deterministic)
+    fn = lib.frr_roi_pool_bwd_deterministic if det else lib.frr_roi_pool_bwd
     grad_out = _req(grad_out, "grad_out")
     argmax = _req(argmax, "argmax", torch.int32)
     rois5 = _req(rois5, "rois")
@@ -292,6 +358,13 @@ def roi_pool_backward(grad_out, argmax, rois5, feat_shape, spatial_scale: float 
     with torch.cuda.device(grad_out.device):
         gin = torch.empty((B, C, H, W), dtype=torch.float32, device=grad_out.device,
                           memory_format=torch.channels_last if channels_last else torch.contiguous_format)
+        if det and image_hw is not None:
+            hw = sized_hw(image_hw, B, (H, W), stride, grad_out.device)
+            _lib.check(lib.frr_roi_pool_bwd_deterministic_sized(grad_out.data_ptr(), argmax.data_ptr(), rois5.data_ptr(), K, B,
+                                                                C, H, W, PH, PW, float(spatial_scale), int(channels_last),
+                                                                hw.data_ptr(), int(stride), gin.data_ptr(), _stream()),
+                       "frr_roi_pool_bwd_deterministic_sized")
+            return gin
         _lib.check(fn(grad_out.data_ptr(), argmax.data_ptr(), rois5.data_ptr(), K, B, C, H, W, PH, PW, float(spatial_scale),
                       int(channels_last), gin.data_ptr(), _stream()), fn.__name__)
     return gin
@@ -338,18 +411,22 @@ def roi_align_backward(grad_out, rois5, feat_shape, spatial_scale: float = 1.0, 
 
 class _RoIPoolFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, feat, rois5, output_size, spatial_scale):
+    def forward(ctx, feat, rois5, output_size, spatial_scale, image_hw, stride):
         feat_l, cl = _feat_layout(feat)
-        out, arg = roi_pool_forward(feat_l, rois5, output_size, spatial_scale, want_argmax=True)
-        ctx.save_for_backward(rois5, arg)
-        ctx.meta = (tuple(feat.shape), float(spatial_scale), bool(cl))
+        if image_hw is not None:
+            image_hw = sized_hw(image_hw, feat.shape[0], feat.shape[2:], stride, feat.device)
+        out, arg = roi_pool_forward(feat_l, rois5, output_size, spatial_scale, want_argmax=True, image_hw=image_hw,
+                                    stride=stride)
+        ctx.save_for_backward(rois5, arg, image_hw)
+        ctx.meta = (tuple(feat.shape), float(spatial_scale), bool(cl), int(stride))
         return out
 
     @staticmethod
     def backward(ctx, grad_out):
-        rois5, arg = ctx.saved_tensors
-        shape, scale, cl = ctx.meta
-        return roi_pool_backward(grad_out.contiguous(), arg, rois5, shape, scale, cl), None, None, None
+        rois5, arg, image_hw = ctx.saved_tensors
+        shape, scale, cl, stride = ctx.meta
+        return (roi_pool_backward(grad_out.contiguous(), arg, rois5, shape, scale, cl, image_hw=image_hw, stride=stride),
+                None, None, None, None, None)
 
 
 class _RoIAlignFn(torch.autograd.Function):
@@ -368,12 +445,14 @@ class _RoIAlignFn(torch.autograd.Function):
         return roi_align_backward(grad_out.contiguous(), rois5, shape, scale, sr, al, cl), None, None, None, None, None
 
 
-def roi_pool(input, boxes, output_size, spatial_scale: float = 1.0):
-    """Drop-in for torchvision.ops.roi_pool (differentiable w.r.t. ``input``)."""
+def roi_pool(input, boxes, output_size, spatial_scale: float = 1.0, image_hw=None, stride: int = 16):
+    """Drop-in for torchvision.ops.roi_pool (differentiable w.r.t. ``input``).  ``image_hw`` [B,2]: a mixed-size batch
+    padded to the map's size; windows are clipped to each image's own grid (see ``roi_pool_forward``), in the forward
+    and in the deterministic backward."""
     if isinstance(output_size, int):
         output_size = (output_size, output_size)
     rois5 = convert_rois(boxes, input.device).to(torch.float32)
-    return _RoIPoolFn.apply(input, rois5.contiguous(), tuple(output_size), float(spatial_scale))
+    return _RoIPoolFn.apply(input, rois5.contiguous(), tuple(output_size), float(spatial_scale), image_hw, int(stride))
 
 
 def roi_align(input, boxes, output_size, spatial_scale: float = 1.0, sampling_ratio: int = -1, aligned: bool = False):
@@ -398,7 +477,9 @@ VARIANTS = {   # (iou_eps, inside_only, tie_inclusive): models/model.py vs model
 
 
 def rpn_targets_assign(gt, gt_count, N, image_hw=None, anchors=None, stride=16, table=None, neg_thr=0.3, pos_thr=0.7,
-                       variant: str = "vgg"):
+                       variant: str = "vgg", grid_hw=None):
+    """``image_hw`` [B,2] + ``grid_hw`` (mixed-size batch, N = grid_h * grid_w * A): each image's anchors and inside-image
+    test are its own, its padding cells are labelled like anchors outside the image."""
     lib = _lib.load()
     eps, inside_only, tie_inclusive = VARIANTS[variant]
     gt = _req(gt, "gt")
@@ -410,7 +491,13 @@ def rpn_targets_assign(gt, gt_count, N, image_hw=None, anchors=None, stride=16, 
     if gt_count is not None:
         gt_count = _req(gt_count, "gt_count", torch.int32)
     keep, tptr, A = _table_arg(table)
-    if anchors is not None:
+    hw = None
+    if is_sized(image_hw):
+        if anchors is not None or grid_hw is None:
+            raise ValueError("rpn_targets_assign: per-image sizes need grid_hw and generated anchors")
+        hw = sized_hw(image_hw, B, grid_hw, stride, gt.device)
+        H, W = int(grid_hw[0]), int(grid_hw[1])      # with hw set: the padded grid in cells
+    elif anchors is not None:
         anchors = _req(anchors, "anchors")
         H = W = 0
     else:
@@ -423,12 +510,16 @@ def rpn_targets_assign(gt, gt_count, N, image_hw=None, anchors=None, stride=16, 
                   pos_list=torch.empty((B, N), dtype=torch.int32, device=dev),
                   neg_list=torch.empty((B, N), dtype=torch.int32, device=dev),
                   counts=torch.empty((B, 2), dtype=torch.int32, device=dev))
-        _lib.check(lib.frr_rpn_targets_assign(gt.data_ptr(), _ptr(gt_count), B, G, _ptr(anchors), tptr, A, H, W, stride, N,
-                                              float(np.float32(neg_thr)), float(np.float32(pos_thr)), eps, inside_only,
-                                              tie_inclusive, ws["iou_max"].data_ptr(), ws["argmax"].data_ptr(), ws["label8"].data_ptr(),
-                                              ws["pos_list"].data_ptr(), ws["neg_list"].data_ptr(), ws["counts"].data_ptr(),
-                                              _stream()), "frr_rpn_targets_assign")
-    ws.update(gt=gt, anchors=anchors, geom=(H, W, stride, table, N))
+        outs = (ws["iou_max"].data_ptr(), ws["argmax"].data_ptr(), ws["label8"].data_ptr(), ws["pos_list"].data_ptr(),
+                ws["neg_list"].data_ptr(), ws["counts"].data_ptr(), _stream())
+        thr = (float(np.float32(neg_thr)), float(np.float32(pos_thr)), eps, inside_only, tie_inclusive)
+        if hw is not None:
+            _lib.check(lib.frr_rpn_targets_assign_sized(gt.data_ptr(), _ptr(gt_count), B, G, tptr, A, hw.data_ptr(), H, W,
+                                                        stride, N, *thr, *outs), "frr_rpn_targets_assign_sized")
+        else:
+            _lib.check(lib.frr_rpn_targets_assign(gt.data_ptr(), _ptr(gt_count), B, G, _ptr(anchors), tptr, A, H, W, stride, N,
+                                                  *thr, *outs), "frr_rpn_targets_assign")
+    ws.update(gt=gt, anchors=anchors, geom=(H, W, stride, table, N), image_hw=hw)
     return ws
 
 
@@ -442,10 +533,14 @@ def rpn_targets_finalize(ws, disable=None, disable_off=None):
     with torch.cuda.device(dev):
         labels = torch.empty((B, N), dtype=torch.int64, device=dev)
         reg = torch.empty((B, N, 4), dtype=torch.float32, device=dev)
-        _lib.check(lib.frr_rpn_targets_finalize(gt.data_ptr(), B, G, _ptr(anchors), tptr, A, H, W, stride, N,
-                                                ws["argmax"].data_ptr(), ws["label8"].data_ptr(), ws["pos_list"].data_ptr(),
-                                                ws["neg_list"].data_ptr(), _ptr(disable), _ptr(disable_off),
-                                                labels.data_ptr(), reg.data_ptr(), _stream()), "frr_rpn_targets_finalize")
+        rest = (ws["argmax"].data_ptr(), ws["label8"].data_ptr(), ws["pos_list"].data_ptr(), ws["neg_list"].data_ptr(),
+                _ptr(disable), _ptr(disable_off), labels.data_ptr(), reg.data_ptr(), _stream())
+        if ws.get("image_hw") is not None:
+            _lib.check(lib.frr_rpn_targets_finalize_sized(gt.data_ptr(), B, G, tptr, A, ws["image_hw"].data_ptr(), H, W,
+                                                          stride, N, *rest), "frr_rpn_targets_finalize_sized")
+        else:
+            _lib.check(lib.frr_rpn_targets_finalize(gt.data_ptr(), B, G, _ptr(anchors), tptr, A, H, W, stride, N, *rest),
+                       "frr_rpn_targets_finalize")
     return labels, reg
 
 

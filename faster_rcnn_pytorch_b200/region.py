@@ -41,14 +41,16 @@ def rpn_head_views(cls_map, reg_map):
 def rpn_proposals(cls, reg, image_hw=None, mode: str = "train", anchors=None, stride: int = 16, table=None,
                   pre_nms_top_k: int | None = None, post_nms_top_k: int | None = None,
                   nms_thresh: float = RPN_NMS_THRESH, cluster_size: int = 0, return_all: bool = False,
-                  min_size: float = ops._MIN_SIZE):
+                  min_size: float = ops._MIN_SIZE, grid_hw=None):
     """cls [B,N,2] logits (or [B,N] fg scores), reg [B,N,4] -> rois [B,post,4] (zero padded), count int32 [B].
-    ``min_size`` is the normalised side threshold (models/model.py:39: 1/1000; models/new_model.py:66: 10/1000)."""
+    ``min_size`` is the normalised side threshold (models/model.py:39: 1/1000; models/new_model.py:66: 10/1000).
+    Mixed-size batch: ``image_hw`` [B,2] per-image (H, W) and ``grid_hw`` the padded grid in cells (N = grid_h * grid_w
+    * A); every image's proposals are those it gets alone at its own size (top-k indices refer to the padded N)."""
     pre_k, post_k = PROPOSAL_MODES[mode]
     pre_k = pre_k if pre_nms_top_k is None else int(pre_nms_top_k)
     post_k = post_k if post_nms_top_k is None else int(post_nms_top_k)
     boxes, scores, valid = ops.rpn_decode(reg, cls, image_hw=image_hw, anchors=anchors, stride=stride, table=table,
-                                          min_size=min_size)
+                                          min_size=min_size, grid_hw=grid_hw)
     k = min(pre_k, boxes.shape[1])
     top = ops.topk_desc(scores, k, valid=valid, boxes=boxes, want_cidx=return_all)
     keep, count, rois = ops.nms_sorted(top["boxes"], nms_thresh, max_keep=post_k, counts=top["count"],
@@ -60,7 +62,11 @@ def rpn_proposals(cls, reg, image_hw=None, mode: str = "train", anchors=None, st
 
 class ProposalPlan:
     """Pre-planned proposal layer for a fixed (B, N) shape: workspace and outputs are allocated once;
-    ``run(cls, reg)`` is one ``frr_rpn_proposals`` call on the current stream (no allocation, no sync)."""
+    ``run(cls, reg)`` is one ``frr_rpn_proposals`` call on the current stream (no allocation, no sync).
+
+    Mixed-size batches: ``image_hw`` is then the padded (max) size of the batch and ``run(cls, reg, image_hw=sizes)``
+    takes the per-image sizes as an int32 [B,2] device tensor, read by the kernels when they run: a graph captured with
+    ``capture(cls, reg, sizes)`` serves every mix of sizes later written into ``sizes``."""
 
     def __init__(self, B: int, N: int, device, image_hw=None, anchors=None, mode: str = "train", stride: int = 16,
                  table=None, logits: bool = True, pre_nms_top_k=None, post_nms_top_k=None,
@@ -83,6 +89,7 @@ class ProposalPlan:
                 raise ValueError("image_hw is required when anchors are generated in-kernel")
             self.anchors = None
             self.H, self.W = int(image_hw[0]), int(image_hw[1])
+        self.grid_hw = (self.H // self.stride, self.W // self.stride)   # padded grid of a mixed-size batch
         with torch.cuda.device(self.device):
             self.ws_bytes = int(self.lib.frr_rpn_proposals_workspace_bytes(self.B, self.N, self.pre_k, self.post_k))
             self._ws = torch.empty((self.ws_bytes + 256,), dtype=torch.uint8, device=self.device)
@@ -90,9 +97,11 @@ class ProposalPlan:
             self.rois = torch.empty((self.B, self.post_k, 4), dtype=torch.float32, device=self.device)
             self.count = torch.empty((self.B,), dtype=torch.int32, device=self.device)
 
-    def run(self, cls, reg, rois=None, count=None):
+    def run(self, cls, reg, rois=None, count=None, image_hw=None):
         """cls [B,N,2] logits / [B,N] scores and reg [B,N,4]: CUDA fp32 contiguous.  Returns (rois, count) --
-        the plan's own output buffers unless ``rois`` / ``count`` are given (overwritten by the next run)."""
+        the plan's own output buffers unless ``rois`` / ``count`` are given (overwritten by the next run).
+        ``image_hw``: per-image sizes (see the class doc); host sizes are checked and copied, so pass a device tensor
+        where the call is captured into a graph."""
         if not (cls.is_cuda and reg.is_cuda and cls.dtype == torch.float32 and reg.dtype == torch.float32):
             raise ValueError("ProposalPlan.run: cls / reg must be CUDA fp32 tensors: the region stage has no CPU path")
         if tuple(reg.shape) != (self.B, self.N, 4) or not reg.is_contiguous() or not cls.is_contiguous() or \
@@ -100,6 +109,17 @@ class ProposalPlan:
             raise ValueError("ProposalPlan.run: shape mismatch with the plan")
         rois = self.rois if rois is None else rois
         count = self.count if count is None else count
+        if image_hw is not None:
+            if self.anchors is not None:
+                raise ValueError("ProposalPlan.run: per-image sizes need generated anchors (a plan built with image_hw)")
+            hw = ops.sized_hw(image_hw, self.B, self.grid_hw, self.stride, self.device)
+            _lib.check(self.lib.frr_rpn_proposals_sized(reg.data_ptr(), cls.data_ptr(), int(self.logits), self._tptr, self.A,
+                                                        hw.data_ptr(), self.grid_hw[0], self.grid_hw[1], self.stride,
+                                                        self.min_size, self.B, self.N, self.pre_k, self.post_k, self.thr,
+                                                        rois.data_ptr(), count.data_ptr(), self._ws_ptr, self.ws_bytes,
+                                                        self.nms_cluster_size, torch.cuda.current_stream().cuda_stream),
+                       "frr_rpn_proposals_sized")
+            return rois, count
         _lib.check(self.lib.frr_rpn_proposals_opt(reg.data_ptr(), cls.data_ptr(), int(self.logits), ops._ptr(self.anchors),
                                                   self._tptr, self.A, self.H, self.W, self.stride, self.min_size, self.B,
                                                   self.N, self.pre_k, self.post_k, self.thr, rois.data_ptr(),
@@ -130,16 +150,17 @@ class ProposalPlan:
                     top_count=view(off[4], B * 4, torch.int32, (B,)),
                     keep=view(off[5], B * self.post_k * 4, torch.int32, (B, self.post_k)))
 
-    def capture(self, cls, reg):
+    def capture(self, cls, reg, image_hw=None):
         """Capture one ``run(cls, reg)`` into a CUDA graph (the call neither allocates nor synchronises) and return the
         ``torch.cuda.CUDAGraph``; ``graph.replay()`` then re-runs the whole proposal layer on whatever ``cls`` / ``reg``
-        hold at that moment, writing ``self.rois`` / ``self.count``, for one graph launch instead of four kernel launches."""
-        self.run(cls, reg)                                    # warm-up outside the capture (function attributes, tables)
+        (and the device tensor ``image_hw``) hold at that moment, writing ``self.rois`` / ``self.count``, for one graph
+        launch instead of four kernel launches."""
+        self.run(cls, reg, image_hw=image_hw)                 # warm-up outside the capture (function attributes, tables)
         torch.cuda.synchronize(self.device)
         graph = torch.cuda.CUDAGraph()
         # thread_local: CUDA calls of other threads (e.g. NCCL's watchdog under torchrun) must not invalidate the capture
         with torch.cuda.graph(graph, capture_error_mode="thread_local"):
-            self.run(cls, reg)
+            self.run(cls, reg, image_hw=image_hw)
         return graph
 
 
@@ -165,26 +186,41 @@ class ProposalPipeline:
             self.streams = [torch.cuda.Stream(device=self.device) for _ in range(self.depth)]
         self._done = [torch.cuda.Event() for _ in range(self.depth)]
         self._graphs = {}
+        self._captured_sizes = []
         self._n = 0
 
-    def capture(self, cls, reg):
-        """Capture the call for these input tensors once per plan; ``submit`` on the same tensors then replays."""
+    def capture(self, cls, reg, image_hw=None):
+        """Capture the call for these input tensors once per plan; ``submit`` on the same tensors then replays.
+        ``image_hw``: per-image sizes of a mixed-size batch (see ``ProposalPlan``); the graphs read the device tensor at
+        every replay, so pass the int32 [B,2] device tensor that ``submit`` will get (host sizes are copied to a device
+        tensor the graphs keep, and are then fixed)."""
+        image_hw = self._sizes(image_hw)
+        if image_hw is not None:
+            self._captured_sizes.append(image_hw)
         for j, plan in enumerate(self.plans):
             with torch.cuda.stream(self.streams[j]):
-                self._graphs[(j, cls.data_ptr(), reg.data_ptr())] = plan.capture(cls, reg)
+                self._graphs[(j, cls.data_ptr(), reg.data_ptr(), ops._ptr(image_hw))] = plan.capture(cls, reg, image_hw)
         torch.cuda.synchronize(self.device)
 
-    def submit(self, cls, reg) -> int:
+    def _sizes(self, image_hw):
+        """per-image sizes as the device tensor the plans read (host sizes checked and copied on the current stream)"""
+        if image_hw is None:
+            return None
+        p = self.plans[0]
+        return ops.sized_hw(image_hw, p.B, p.grid_hw, p.stride, self.device)
+
+    def submit(self, cls, reg, image_hw=None) -> int:
+        image_hw = self._sizes(image_hw)
         t = self._n
         j = t % self.depth
         s = self.streams[j]
         s.wait_stream(torch.cuda.current_stream(self.device))
         with torch.cuda.stream(s):
-            g = self._graphs.get((j, cls.data_ptr(), reg.data_ptr()))
+            g = self._graphs.get((j, cls.data_ptr(), reg.data_ptr(), ops._ptr(image_hw)))
             if g is not None:
                 g.replay()
             else:
-                self.plans[j].run(cls, reg)
+                self.plans[j].run(cls, reg, image_hw=image_hw)
             self._done[j].record(s)
         self._n += 1
         return t
@@ -289,7 +325,11 @@ class InferPlan:
     ``detect(head_cls, head_reg)``  per-class decode (:369-378) -> per-class NMS (:382-402) -> packed detections
                                   [B,max_det,6] (x1,y1,x2,y2,score,label) + counts, the evaluation hand-off
 
-    Neither half synchronises with the host; ``capture_*`` record them into CUDA graphs (one graph launch per half)."""
+    Neither half synchronises with the host; ``capture_*`` record them into CUDA graphs (one graph launch per half).
+
+    Mixed-size batches: build the plan with the padded (max) ``image_hw`` and pass the per-image sizes to ``pool`` /
+    ``capture_pool`` as an int32 [B,2] device tensor: anchors, the roi scaling and the RoIPool window clip then use each
+    image's own size, and a captured graph reads the sizes at every replay."""
 
     def __init__(self, B: int, image_hw, num_classes: int, device, stride: int = 16, max_det: int = 100,
                  score_thres: float = 0.05, iou_thr: float = 0.3, mode: str = "test", logits: bool = True,
@@ -297,6 +337,7 @@ class InferPlan:
         from . import dist as fdist
         self._fdist = fdist
         self.B, self.hw, self.NC, self.device = int(B), (int(image_hw[0]), int(image_hw[1])), int(num_classes), torch.device(device)
+        self.stride = int(stride)
         self.fhw = (self.hw[0] // stride, self.hw[1] // stride)
         self.N = self.fhw[0] * self.fhw[1] * 9
         self.proposal = ProposalPlan(self.B, self.N, self.device, image_hw=self.hw, mode=mode, stride=stride, logits=logits,
@@ -306,10 +347,10 @@ class InferPlan:
         with torch.cuda.device(self.device):
             self.rois5 = torch.empty((self.B * self.R, 5), dtype=torch.float32, device=self.device)
 
-    def pool(self, feat, cls, reg, want_argmax: bool = False):
-        rois, cnt = self.proposal.run(cls, reg)
-        ops.rois5(rois, cnt, self.fhw, out=self.rois5)
-        pooled, arg = ops.roi_pool_forward(feat, self.rois5, want_argmax=want_argmax)
+    def pool(self, feat, cls, reg, want_argmax: bool = False, image_hw=None):
+        rois, cnt = self.proposal.run(cls, reg, image_hw=image_hw)
+        ops.rois5(rois, cnt, self.fhw, out=self.rois5, image_hw=image_hw, stride=self.stride)
+        pooled, arg = ops.roi_pool_forward(feat, self.rois5, want_argmax=want_argmax, image_hw=image_hw, stride=self.stride)
         return (pooled, rois, cnt, arg) if want_argmax else (pooled, rois, cnt)
 
     def detect(self, head_cls, head_reg, return_all: bool = False):
@@ -323,8 +364,8 @@ class InferPlan:
             return dict(packed=packed, count=pc, prob=prob, boxes=boxes, det=(db, dl, ds, dc))
         return packed, pc
 
-    def capture_pool(self, feat, cls, reg):
-        return _capture(lambda: self.pool(feat, cls, reg), self.device)
+    def capture_pool(self, feat, cls, reg, image_hw=None):
+        return _capture(lambda: self.pool(feat, cls, reg, image_hw=image_hw), self.device)
 
     def capture_detect(self, head_cls, head_reg):
         return _capture(lambda: self.detect(head_cls, head_reg), self.device)
@@ -335,33 +376,43 @@ class TrainPlan:
     reference's sampling replayed on the device (no host synchronisation), RoIPool forward of the sampled rois and its
     backward.  ``targets_and_pool`` / ``pool_backward`` can be recorded into CUDA graphs with ``capture_*``.
     ``pool_backward`` follows ``torch.use_deterministic_algorithms`` when it runs; a captured graph keeps the backward
-    kernel chosen at capture time, whatever the flag is when the graph is replayed."""
+    kernel chosen at capture time, whatever the flag is when the graph is replayed.
+
+    Mixed-size batches: build the plan with the padded (max) ``image_hw`` and pass the per-image sizes to
+    ``targets_and_pool`` / ``capture_targets_and_pool`` as an int32 [B,2] device tensor (read at every replay);
+    ``pool_backward`` uses the sizes of the last ``targets_and_pool``."""
 
     def __init__(self, B: int, image_hw, device, generator=None, stride: int = 16):
         from . import targets
         self._targets = targets
         self.B, self.hw, self.device = int(B), (int(image_hw[0]), int(image_hw[1])), torch.device(device)
+        self.stride = int(stride)
         self.fhw = (self.hw[0] // stride, self.hw[1] // stride)
         self.generator = generator if generator is not None else targets.DeviceGenerator(self.device)
         with torch.cuda.device(self.device):
             self.rois5 = torch.empty((self.B * targets.FRCNN_BATCH, 5), dtype=torch.float32, device=self.device)
         self.last = None
 
-    def targets_and_pool(self, feat, gt, gt_label, proposals, proposal_count, gt_count=None):
-        t = self._targets.make_targets(gt, gt_count, gt_label, proposals, proposal_count, image_hw=self.hw,
-                                       generator=self.generator)
-        ops.rois5(t["sample_rois"], t["n_samples"], self.fhw, out=self.rois5)
-        pooled, arg = ops.roi_pool_forward(feat, self.rois5)
+    def targets_and_pool(self, feat, gt, gt_label, proposals, proposal_count, gt_count=None, image_hw=None):
+        if image_hw is not None:
+            image_hw = ops.sized_hw(image_hw, self.B, self.fhw, self.stride, self.device)
+        t = self._targets.make_targets(gt, gt_count, gt_label, proposals, proposal_count,
+                                       image_hw=self.hw if image_hw is None else image_hw, generator=self.generator,
+                                       grid_hw=self.fhw)
+        ops.rois5(t["sample_rois"], t["n_samples"], self.fhw, out=self.rois5, image_hw=image_hw, stride=self.stride)
+        pooled, arg = ops.roi_pool_forward(feat, self.rois5, image_hw=image_hw, stride=self.stride)
         self.last = dict(targets=t, pooled=pooled, argmax=arg, feat_shape=tuple(feat.shape),
-                         channels_last=(not feat.is_contiguous()))
+                         channels_last=(not feat.is_contiguous()), image_hw=image_hw)
         return t, pooled
 
     def pool_backward(self, grad_out):
         s = self.last
-        return ops.roi_pool_backward(grad_out, s["argmax"], self.rois5, s["feat_shape"], channels_last=s["channels_last"])
+        return ops.roi_pool_backward(grad_out, s["argmax"], self.rois5, s["feat_shape"], channels_last=s["channels_last"],
+                                     image_hw=s["image_hw"], stride=self.stride)
 
-    def capture_targets_and_pool(self, feat, gt, gt_label, proposals, proposal_count):
-        return _capture(lambda: self.targets_and_pool(feat, gt, gt_label, proposals, proposal_count), self.device)
+    def capture_targets_and_pool(self, feat, gt, gt_label, proposals, proposal_count, image_hw=None):
+        return _capture(lambda: self.targets_and_pool(feat, gt, gt_label, proposals, proposal_count, image_hw=image_hw),
+                        self.device)
 
     def capture_pool_backward(self, grad_out):
         return _capture(lambda: self.pool_backward(grad_out), self.device)

@@ -120,13 +120,26 @@ def _upload_select(per_image, device, batch: int = FRCNN_BATCH):
     return torch.from_numpy(sel).to(device, non_blocking=True), torch.from_numpy(sel_n).to(device, non_blocking=True)
 
 
-def rpn_targets(gt, gt_count=None, image_hw=None, anchors=None, N=None, randperm=torch.randperm, generator=None, **kw):
+def _anchor_count(image_hw, anchors, grid_hw):
+    if anchors is not None:
+        return anchors.shape[0]
+    if ops.is_sized(image_hw):
+        if grid_hw is None:
+            raise ValueError("per-image sizes need grid_hw, the padded grid in cells")
+        return int(grid_hw[0]) * int(grid_hw[1]) * 9
+    return (image_hw[0] // 16) * (image_hw[1] // 16) * 9
+
+
+def rpn_targets(gt, gt_count=None, image_hw=None, anchors=None, N=None, randperm=torch.randperm, generator=None,
+                grid_hw=None, **kw):
     """Batched RPNTargetMaker: gt [B,Gmax,4] (+ gt_count) -> labels int64 [B,N], reg fp32 [B,N,4].
     ``variant="fpn"`` = models/new_model.py:299-349 (no inside filter, eps-free IoU, tie-inclusive low-quality match).
-    ``generator``: a ``DeviceGenerator`` -> sampling on the device, no host synchronisation."""
+    ``generator``: a ``DeviceGenerator`` -> sampling on the device, no host synchronisation.
+    Mixed-size batch: ``image_hw`` [B,2] per-image sizes and ``grid_hw`` the padded grid in cells; every image gets the
+    labels and draws it would get alone, its padding cells label -1 and a zero target."""
     if N is None:
-        N = anchors.shape[0] if anchors is not None else (image_hw[0] // 16) * (image_hw[1] // 16) * 9
-    ws = ops.rpn_targets_assign(gt, gt_count, N, image_hw=image_hw, anchors=anchors, **kw)
+        N = _anchor_count(image_hw, anchors, grid_hw)
+    ws = ops.rpn_targets_assign(gt, gt_count, N, image_hw=image_hw, anchors=anchors, grid_hw=grid_hw, **kw)
     if generator is not None:
         ops.sample_targets(generator.state, ws_rpn=ws, rpn_batch=RPN_BATCH, rpn_max_pos=RPN_MAX_POS)
         return ops.rpn_targets_finalize(ws)
@@ -154,13 +167,14 @@ def frcnn_targets(rois, roi_count, gt, gt_count, gt_label, randperm=torch.randpe
 
 
 def make_targets(gt, gt_count, gt_label, rois, roi_count, image_hw=None, anchors=None, N=None, randperm=torch.randperm,
-                 generator=None):
+                 generator=None, grid_hw=None):
     """Both target makers for a batch.  Permutations are drawn per image in the reference's order (RPN positives, RPN
     negatives, Fast R-CNN positives, Fast R-CNN negatives): on the host with a single synchronisation (default), or on
-    the device with none (``generator`` = a ``DeviceGenerator``; ``n_samples`` is then a device tensor)."""
+    the device with none (``generator`` = a ``DeviceGenerator``; ``n_samples`` is then a device tensor).
+    ``image_hw`` [B,2] + ``grid_hw``: a mixed-size batch, as in ``rpn_targets``."""
     if N is None:
-        N = anchors.shape[0] if anchors is not None else (image_hw[0] // 16) * (image_hw[1] // 16) * 9
-    ws_r = ops.rpn_targets_assign(gt, gt_count, N, image_hw=image_hw, anchors=anchors)
+        N = _anchor_count(image_hw, anchors, grid_hw)
+    ws_r = ops.rpn_targets_assign(gt, gt_count, N, image_hw=image_hw, anchors=anchors, grid_hw=grid_hw)
     ws_f = ops.frcnn_targets_assign(rois, roi_count, gt, gt_count)
     if generator is not None:
         sel, sel_n = ops.sample_targets(generator.state, ws_rpn=ws_r, ws_frcnn=ws_f, rpn_batch=RPN_BATCH,

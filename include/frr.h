@@ -79,6 +79,23 @@ int frr_rpn_decode(const float* reg /* [B,N,4] */, const float* cls /* [B,N,2] l
                    float* scores /* [B,N] */, uint8_t* valid /* [B,N] */, int B, int N,
                    frr_stream_t stream);
 
+/* Mixed-size batches -- the reference builds anchors from each image's own size (models/model.py:310-312,352-354) and
+ *     scales rois by each image's own feature grid (:104-110).  A batch of differently sized images is padded to one grid
+ *     of grid_h x grid_w cells (N = grid_h * grid_w * A anchors per image, cell-major / anchor-minor over the PADDED grid);
+ *     image_hw int32 [B,2] (device, 8-byte aligned) holds each image's (H_b, W_b) in pixels.  Image b covers the cells
+ *     y < fh_b = H_b / stride, x < fw_b = W_b / stride; the rest of the grid is padding.  Every *_sized entry point gives
+ *     image b exactly what its uniform form gives for image b alone at (H_b, W_b) on the cropped inputs, with indices
+ *     mapped by (y * grid_w + x) * A + a <-> (y * fw_b + x) * A + a.  The sizes are read on the device at run time (one
+ *     CUDA graph serves every mix of sizes that fits the grid), so the host cannot check them: fh_b / fw_b are clamped to
+ *     [0, grid_h] / [0, grid_w], and an image with an empty grid has no valid anchor, no proposal (count 0) and no rois.
+ * frr_rpn_decode_sized: anchors divided by each image's own (W_b, H_b) (the __fdiv_rn recipe of frr_rpn_decode);
+ *     padding cells get box 0, score 0, valid 0 whatever reg / cls hold there (NaN included).                        */
+int frr_rpn_decode_sized(const float* reg /* [B,N,4] */, const float* cls /* [B,N,2] logits or [B,N] scores */,
+                         int cls_is_logits, const float* base_table_host /* [A*4] or NULL */, int A,
+                         const int32_t* image_hw /* [B,2] device */, int grid_h, int grid_w, int stride, float min_size,
+                         float* boxes /* [B,N,4] */, float* scores /* [B,N] */, uint8_t* valid /* [B,N] */, int B, int N,
+                         frr_stream_t stream);
+
 /* ---------------------------------------------------------------------------------------
  * P4  pre-NMS top-k, sorted descending -- models/model.py:44-49.  One CTA per image, in shared
  *     memory: monotone bucketing of the scores + exact ranking inside the buckets (radix select + radix
@@ -162,6 +179,16 @@ int frr_rpn_proposals_opt(const float* reg, const float* cls, int cls_is_logits,
                           int N, int pre_nms_top_k, int post_nms_top_k, double iou_thr, float* rois, int32_t* roi_count,
                           void* workspace, size_t workspace_bytes, int nms_cluster_size, frr_stream_t stream);
 
+/* frr_rpn_proposals_opt for a mixed-size batch padded to grid_h x grid_w cells (see frr_rpn_decode_sized): the decode
+ * is the sized one, top-k and NMS are unchanged (padding cells are invalid; the row-major order of the padded grid keeps
+ * each image's relative anchor order, so ties break as for the image alone).  Workspace size and layout are those of
+ * frr_rpn_proposals_workspace_bytes / _layout for the padded N; the top-k order holds indices into the padded N.      */
+int frr_rpn_proposals_sized(const float* reg, const float* cls, int cls_is_logits, const float* base_table_host, int A,
+                            const int32_t* image_hw /* [B,2] device */, int grid_h, int grid_w, int stride, float min_size,
+                            int B, int N, int pre_nms_top_k, int post_nms_top_k, double iou_thr, float* rois,
+                            int32_t* roi_count, void* workspace, size_t workspace_bytes, int nms_cluster_size,
+                            frr_stream_t stream);
+
 /* ---------------------------------------------------------------------------------------
  * R1-R3  RoIPool -- torchvision.ops.RoIPool((7,7), 1.0) at models/model.py:97,113 and its autograd
  *        backward (train.py:36).  Schemas replaced: torchvision::roi_pool(input, rois, spatial_scale,
@@ -182,6 +209,20 @@ int frr_rois5(const float* rois, const int32_t* count, int B, int R, float fw, f
               frr_stream_t stream);
 int frr_roi_pool_fwd(const float* feat, const float* rois, int K, int B, int C, int H, int W, int PH, int PW,
                      float spatial_scale, int channels_last, float* out, int32_t* argmax, frr_stream_t stream);
+/* Mixed-size batches (see frr_rpn_decode_sized), features padded to H x W cells.  frr_rois5_sized scales image b's rois
+ * by its own grid (fw_b, fh_b) (models/model.py:104-110) and masks the rows of an image with an empty grid.
+ * frr_roi_pool_fwd_sized clips every bin window of a roi of image b to [0, fh_b) x [0, fw_b) instead of the padded map,
+ * as torchvision does on that image alone: a roi clamped to the image edge has round(x2 * fw_b) == fw_b and loses its
+ * last window column there, while the padded map holds padding values in that column.  argmax stays h * W + w, an index
+ * into the padded plane, and never points at padding.  fh_b = image_hw[b,0] / stride and fw_b = image_hw[b,1] / stride,
+ * clamped to [0, H] / [0, W] (stride 1: image_hw holds the feature extents themselves).  Same kernel choice as
+ * frr_roi_pool_fwd (frr_roi_variant).  frr_roi_pool_bwd needs no extent: it follows argmax, so the padding region of
+ * grad_in comes out zero. */
+int frr_rois5_sized(const float* rois, const int32_t* count, int B, int R, const int32_t* image_hw /* [B,2] device */,
+                    int stride, int grid_h, int grid_w, float* rois5, frr_stream_t stream);
+int frr_roi_pool_fwd_sized(const float* feat, const float* rois, int K, int B, int C, int H, int W, int PH, int PW,
+                           float spatial_scale, int channels_last, const int32_t* image_hw /* [B,2] device */, int stride,
+                           float* out, int32_t* argmax, frr_stream_t stream);
 /* grad_in [B,C,H,W] (same memory format as feat) is fully written (no pre-zeroing needed).  Rois of at least 6 feature
  * pixels per side are accumulated in shared memory in a fixed order (bit-reproducible); smaller rois, and every roi on maps
  * whose 8 planes do not fit twice per SM, are added with global fp32 atomics (same sums, order not fixed).  argmax must be
@@ -220,6 +261,12 @@ int frr_roi_align_bwd(const float* grad_out, const float* rois, int K, int B, in
 int frr_roi_pool_bwd_deterministic(const float* grad_out, const int32_t* argmax, const float* rois, int K, int B, int C,
                                    int H, int W, int PH, int PW, float spatial_scale, int channels_last, float* grad_in,
                                    frr_stream_t stream);
+/* The same for a mixed-size batch: "p lies inside that bin's clipped window" uses image b's extent, exactly as
+ * frr_roi_pool_fwd_sized clips (image_hw, stride as there); the padding region of grad_in is written as +0.0. */
+int frr_roi_pool_bwd_deterministic_sized(const float* grad_out, const int32_t* argmax, const float* rois, int K, int B,
+                                         int C, int H, int W, int PH, int PW, float spatial_scale, int channels_last,
+                                         const int32_t* image_hw /* [B,2] device */, int stride, float* grad_in,
+                                         frr_stream_t stream);
 int frr_roi_align_bwd_deterministic(const float* grad_out, const float* rois, int K, int B, int C, int H, int W, int PH,
                                     int PW, float spatial_scale, int sampling_ratio, int aligned, int channels_last,
                                     float* grad_in, frr_stream_t stream);
@@ -267,6 +314,21 @@ int frr_rpn_targets_finalize(const float* gt, int B, int Gmax, const float* anch
                              int A, int img_h, int img_w, int stride, int N, const int32_t* argmax, int8_t* label8,
                              const int32_t* pos_list, const int32_t* neg_list, const int32_t* disable,
                              const int32_t* disable_off, int64_t* labels, float* reg, frr_stream_t stream);
+/* The same for a mixed-size batch padded to grid_h x grid_w cells (see frr_rpn_decode_sized), anchors generated: image b's
+ * anchors are divided by its own (W_b, H_b) and the inside-image test is its own; its padding cells behave like anchors
+ * outside the image (label8 -2, then label -1 and a zero target).  pos_list / neg_list hold padded indices in the same
+ * order as the image's own lists, and counts are the image's own, so the host randperm path and frr_sample_targets draw
+ * the same numbers as for the image alone.  iou_max / argmax / label8 / lists / labels / reg are [B,N] of the padded N. */
+int frr_rpn_targets_assign_sized(const float* gt, const int32_t* gt_count, int B, int Gmax, const float* base_table_host,
+                                 int A, const int32_t* image_hw /* [B,2] device */, int grid_h, int grid_w, int stride, int N,
+                                 float neg_thr, float pos_thr, float iou_eps, int inside_only, int tie_inclusive,
+                                 float* iou_max, int32_t* argmax, int8_t* label8, int32_t* pos_list, int32_t* neg_list,
+                                 int32_t* counts, frr_stream_t stream);
+int frr_rpn_targets_finalize_sized(const float* gt, int B, int Gmax, const float* base_table_host, int A,
+                                   const int32_t* image_hw /* [B,2] device */, int grid_h, int grid_w, int stride, int N,
+                                   const int32_t* argmax, int8_t* label8, const int32_t* pos_list, const int32_t* neg_list,
+                                   const int32_t* disable, const int32_t* disable_off, int64_t* labels, float* reg,
+                                   frr_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------
  * T3  Fast R-CNN target maker -- FastRcnnTargetMaker.forward, models/model.py:127-179.

@@ -56,6 +56,8 @@ SIGNATURES = {
     "frr_frcnn_targets_finalize": (_i, [_p, _p, _i, _i, _p, _p, _i, _p, _p, _p, _p, _p, _i, _p, _i, _p, _p, _p, _p, _p]),
     "frr_decode_classwise": (_i, [_p, _p, _p, _i, _i, _p, _p, _p, _p]),
     "frr_pack_detections": (_i, [_p, _p, _p, _p, _i, _i, _i, _p, _i, _p, _p, _p]),
+    "frr_pack_detections_ranked_workspace_bytes": (C.c_size_t, [_i, _i, _i]),
+    "frr_pack_detections_ranked": (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _p, _i, _p, _p, _p, C.c_size_t, _p]),
     "frr_class_nms_workspace_bytes": (C.c_size_t, [_i, _i, _i]),
     "frr_class_nms": (_i, [_p, _p, _p, _i, _i, _i, _f, _d, _i, _p, _p, _p, _p, _p, C.c_size_t, _p]),
     "frr_nms_sorted_tuned": (_i, [_p, _p, _i, _i, _d, _i, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _p]),

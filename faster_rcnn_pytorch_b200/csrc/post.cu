@@ -9,10 +9,17 @@
 //       2. the cluster keep-list NMS kernel of nms.cu over the B*(C-1) sorted lists at IoU 0.3
 //          (double-threshold compare: IoU == 0.3f is suppressed, as torchvision's CPU kernel);
 //       3. one CTA per image: class-major compaction into [B, cap, 4] boxes / labels (l-1) / scores.
+//   frr_pack_detections        : the evaluation hand-off, the first max_det class-major rows of every image;
+//   frr_pack_detections_ranked : the same rows for the max_det highest-scoring detections (optionally at most
+//                                per_class_max per class first): an eligibility mask, the top-k of topk_radix.cu over
+//                                the masked scores, and a gather into the packed rows.
 #include "nms_common.cuh"
 
 namespace frr {
 
+int topk_desc_impl(const float* scores, const uint8_t* valid, const float* boxes, int B, int N, int k, float* out_scores,
+                   int32_t* out_idx, int32_t* out_cidx, float* out_boxes, int32_t* out_count, int cluster_hint,
+                   frr_stream_t stream);
 
 // ------------------------------------------------------------------------------------------------ D1
 // one warp per roi row
@@ -149,8 +156,22 @@ __global__ void __launch_bounds__(256)
 static size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
 
 // Evaluation hand-off (test.py:68-88 + evaluation/coco_eval.py:70-92,156-158): scale the normalised boxes to pixels,
-// optionally convert xyxy -> xywh, and pack the first max_det detections of every image into fixed-shape rows
-// (x, y, x2|w, y2|h, score, label) for ONE tensor all-gather instead of a pickled one.
+// optionally convert xyxy -> xywh, and pack detections into fixed-shape rows (x, y, x2|w, y2|h, score, label) for ONE
+// tensor all-gather instead of a pickled one.  Both packers write a row through this helper, so a detection gets the
+// same bits whichever selection picked it.
+__device__ __forceinline__ void pack_row(float* __restrict__ o, float4 bx, float score, int32_t label, float2 wh,
+                                         int xywh) {
+    const float x1 = __fmul_rn(bx.x, wh.x), y1 = __fmul_rn(bx.y, wh.y);
+    const float x2 = __fmul_rn(bx.z, wh.x), y2 = __fmul_rn(bx.w, wh.y);
+    o[0] = x1;
+    o[1] = y1;
+    o[2] = xywh ? __fsub_rn(x2, x1) : x2;
+    o[3] = xywh ? __fsub_rn(y2, y1) : y2;
+    o[4] = score;
+    o[5] = (float)label;
+}
+
+// The first max_det class-major rows of every image.
 __global__ void __launch_bounds__(128)
     pack_detections_kernel(const float4* __restrict__ det_boxes, const int32_t* __restrict__ det_labels,
                            const float* __restrict__ det_scores, const int32_t* __restrict__ det_count, int cap,
@@ -162,15 +183,46 @@ __global__ void __launch_bounds__(128)
     for (int j = threadIdx.x; j < max_det; j += blockDim.x) {
         float* o = out + ((size_t)b * max_det + j) * 6;
         if (j < n) {
-            const float4 bx = det_boxes[(size_t)b * cap + j];
-            const float x1 = __fmul_rn(bx.x, wh.x), y1 = __fmul_rn(bx.y, wh.y);
-            const float x2 = __fmul_rn(bx.z, wh.x), y2 = __fmul_rn(bx.w, wh.y);
-            o[0] = x1;
-            o[1] = y1;
-            o[2] = xywh ? __fsub_rn(x2, x1) : x2;
-            o[3] = xywh ? __fsub_rn(y2, y1) : y2;
-            o[4] = det_scores[(size_t)b * cap + j];
-            o[5] = (float)det_labels[(size_t)b * cap + j];
+            const size_t s = (size_t)b * cap + j;
+            pack_row(o, det_boxes[s], det_scores[s], det_labels[s], wh, xywh);
+        } else {
+#pragma unroll
+            for (int q = 0; q < 6; ++q) o[q] = 0.f;
+        }
+    }
+    if (threadIdx.x == 0) out_count[b] = n;
+}
+
+// Ranked selection, step 1: valid[b][j] = row j of image b takes part in the ranking.  It must be one of the image's
+// det_count[b] rows and, with per_class_max = m > 0, among the first m rows of its class.  The rows are class-major, so
+// row j is past its class's cap exactly when row j - m has the same label: no scan over the class is needed.
+__global__ void __launch_bounds__(256)
+    rank_eligible_kernel(const int32_t* __restrict__ det_labels, const int32_t* __restrict__ det_count, int cap,
+                         int per_class_max, uint8_t* __restrict__ valid) {
+    const int b = blockIdx.y;
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= cap) return;
+    const size_t o = (size_t)b * cap + j;
+    bool ok = j < det_count[b];
+    if (ok && per_class_max > 0 && j >= per_class_max) ok = det_labels[o - per_class_max] != det_labels[o];
+    valid[o] = ok ? 1 : 0;
+}
+
+// Ranked selection, step 3: packed row i of image b is detection order[b][i] (order [B,k] from the top-k, order_count
+// [B] rows valid; both NULL when nothing is ranked).
+__global__ void __launch_bounds__(128)
+    pack_ranked_kernel(const float4* __restrict__ det_boxes, const int32_t* __restrict__ det_labels,
+                       const float* __restrict__ det_scores, int cap, const int32_t* __restrict__ order,
+                       const int32_t* __restrict__ order_count, int k, int max_det, const float2* __restrict__ image_wh,
+                       int xywh, float* __restrict__ out, int32_t* __restrict__ out_count) {
+    const int b = blockIdx.x;
+    const int n = order_count ? min(order_count[b], max_det) : 0;
+    const float2 wh = image_wh ? image_wh[b] : make_float2(1.f, 1.f);
+    for (int i = threadIdx.x; i < max_det; i += blockDim.x) {
+        float* o = out + ((size_t)b * max_det + i) * 6;
+        if (i < n) {
+            const size_t s = (size_t)b * cap + order[(size_t)b * k + i];
+            pack_row(o, det_boxes[s], det_scores[s], det_labels[s], wh, xywh);
         } else {
 #pragma unroll
             for (int q = 0; q < 6; ++q) o[q] = 0.f;
@@ -212,6 +264,60 @@ int frr_pack_detections(const float* det_boxes, const int32_t* det_labels, const
                                                                 cap, max_det, (const float2*)image_wh, xywh, out, out_count);
     count_launch();
     FRR_CHECK_LAUNCH("pack_detections_kernel");
+    return FRR_OK;
+}
+
+// The top-k never needs more than the cap rows an image has.
+static int ranked_k(int cap, int max_det) { return cap < max_det ? cap : max_det; }
+
+size_t frr_pack_detections_ranked_workspace_bytes(int B, int cap, int max_det) {
+    using namespace frr;
+    if (B < 0 || cap < 0 || max_det < 1) return 0;
+    const size_t k = (size_t)ranked_k(cap, max_det);
+    return align256((size_t)B * cap) + align256((size_t)B * k * 4) + align256((size_t)B * 4);
+}
+
+int frr_pack_detections_ranked(const float* det_boxes, const int32_t* det_labels, const float* det_scores,
+                               const int32_t* det_count, int B, int cap, int max_det, int per_class_max,
+                               const float* image_wh, int xywh, float* out, int32_t* out_count, void* workspace,
+                               size_t workspace_bytes, frr_stream_t stream) {
+    using namespace frr;
+    FRR_CHECK_ARG(B >= 0 && B <= 65535 && cap >= 0 && max_det >= 1 && per_class_max >= 0,
+                  "frr_pack_detections_ranked: bad sizes");
+    const int k = ranked_k(cap, max_det);
+    FRR_CHECK_ARG(k <= 16384, "frr_pack_detections_ranked: min(max_det, cap) = %d exceeds the top-k capacity 16384", k);
+    if (B == 0) return FRR_OK;
+    FRR_CHECK_ARG(det_boxes && det_labels && det_scores && det_count && out && out_count && workspace,
+                  "frr_pack_detections_ranked: null pointer");
+    FRR_CHECK_ARG(aligned16(det_boxes) && (image_wh == nullptr || aligned8(image_wh)) &&
+                      (reinterpret_cast<uintptr_t>(workspace) & 255u) == 0,
+                  "frr_pack_detections_ranked: det_boxes must be 16-byte aligned, image_wh 8-byte aligned, workspace "
+                  "256-byte aligned");
+    const size_t need = frr_pack_detections_ranked_workspace_bytes(B, cap, max_det);
+    if (workspace_bytes < need) {
+        set_error("frr_pack_detections_ranked: workspace too small (%zu < %zu)", workspace_bytes, need);
+        return FRR_E_WORKSPACE;
+    }
+    char* w = (char*)workspace;
+    uint8_t* valid = (uint8_t*)w;     w += align256((size_t)B * cap);
+    int32_t* order = (int32_t*)w;     w += align256((size_t)B * k * 4);
+    int32_t* order_count = (int32_t*)w;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (k > 0) {
+        rank_eligible_kernel<<<dim3((unsigned)((cap + 255) / 256), (unsigned)B), 256, 0, st>>>(det_labels, det_count, cap,
+                                                                                            per_class_max, valid);
+        count_launch();
+        FRR_CHECK_LAUNCH("rank_eligible_kernel");
+        // score descending, lower class-major position first on equal scores
+        const int rc = topk_desc_impl(det_scores, valid, nullptr, B, cap, k, nullptr, order, nullptr, nullptr, order_count,
+                                      0, stream);
+        if (rc) return rc;
+    }
+    pack_ranked_kernel<<<B, 128, 0, st>>>((const float4*)det_boxes, det_labels, det_scores, cap, k > 0 ? order : nullptr,
+                                          k > 0 ? order_count : nullptr, k, max_det, (const float2*)image_wh, xywh, out,
+                                          out_count);
+    count_launch();
+    FRR_CHECK_LAUNCH("pack_ranked_kernel");
     return FRR_OK;
 }
 

@@ -27,13 +27,17 @@ def shard_range(n_items: int, rank: int | None = None, world_size: int | None = 
     return lo, lo + base + (1 if rank < extra else 0)
 
 
-def pack_detections(det_boxes, det_labels, det_scores, det_count, max_det: int, image_wh=None, xywh: bool = False):
+def pack_detections(det_boxes, det_labels, det_scores, det_count, max_det: int, image_wh=None, xywh: bool = False,
+                    rank: str = "class", per_class_max: int = 0, workspace=None):
     """[B,cap,4] boxes, [B,cap] int32 labels, [B,cap] scores, [B] counts (class-major order as produced by
-    ``ops.class_nms``) -> ([B,max_det,6] fp32 rows (x, y, x2|w, y2|h, score, label), [B] int32 counts): the first
-    ``max_det`` detections of every image, rows past the count zero; optional pixel scaling and xyxy -> xywh
-    (test.py:68-88, evaluation/coco_eval.py:156-158).  One ``frr_pack_detections`` kernel."""
+    ``ops.class_nms``) -> ([B,max_det,6] fp32 rows (x, y, x2|w, y2|h, score, label), [B] int32 counts): ``max_det``
+    detections of every image, rows past the count zero; optional pixel scaling and xyxy -> xywh
+    (test.py:68-88, evaluation/coco_eval.py:156-158).  ``rank="class"`` (one ``frr_pack_detections`` kernel) keeps the
+    first ``max_det`` in class order, ``rank="score"`` (``frr_pack_detections_ranked``) the highest-scoring ones, at
+    most ``per_class_max`` per class when that is > 0: see ``ops.pack_detections``."""
     from . import ops
-    return ops.pack_detections(det_boxes, det_labels, det_scores, det_count, max_det, image_wh=image_wh, xywh=xywh)
+    return ops.pack_detections(det_boxes, det_labels, det_scores, det_count, max_det, image_wh=image_wh, xywh=xywh,
+                               rank=rank, per_class_max=per_class_max, workspace=workspace)
 
 
 def gather_detections(packed, counts, image_ids, group=None, equal_batch: bool = False):

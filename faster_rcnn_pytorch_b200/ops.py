@@ -755,9 +755,34 @@ def class_nms(prob, boxes, num_classes: int, score_thres: float = 0.05, iou_thr:
     return db, dl, ds, dc
 
 
-def pack_detections(det_boxes, det_labels, det_scores, det_count, max_det: int, image_wh=None, xywh: bool = False):
+def check_rank(rank: str, per_class_max: int):
+    """Raises ValueError unless (rank, per_class_max) is a selection ``pack_detections`` offers."""
+    if rank not in ("class", "score"):
+        raise ValueError(f"pack_detections: rank must be 'class' or 'score', got {rank!r}")
+    if int(per_class_max) < 0 or (rank == "class" and int(per_class_max) != 0):
+        raise ValueError("pack_detections: per_class_max is a count >= 0 and applies to rank='score' only")
+
+
+def pack_ranked_workspace(B: int, cap: int, max_det: int, device) -> torch.Tensor:
+    """Workspace of ``pack_detections(..., rank="score")`` for ``[B,cap]`` detections and ``max_det`` rows: allocate it
+    once and pass it to every call (a captured CUDA graph then allocates nothing for the ranking)."""
+    nbytes = int(_lib.load().frr_pack_detections_ranked_workspace_bytes(int(B), int(cap), int(max_det)))
+    return torch.empty((nbytes + 256,), dtype=torch.uint8, device=device)
+
+
+def pack_detections(det_boxes, det_labels, det_scores, det_count, max_det: int, image_wh=None, xywh: bool = False,
+                    rank: str = "class", per_class_max: int = 0, workspace=None):
     """Evaluation hand-off (test.py:68-88, evaluation/coco_eval.py:156-158): [B,cap,4] / [B,cap] / [B,cap] / [B] ->
-    ([B,max_det,6] rows (x, y, x2|w, y2|h, score, label) scaled by ``image_wh [B,2]`` = (w, h), int32 counts [B])."""
+    ([B,max_det,6] rows (x, y, x2|w, y2|h, score, label) scaled by ``image_wh [B,2]`` = (w, h), int32 counts [B]).
+
+    Which ``max_det`` detections of an image become its rows (the input is ``class_nms``'s class-major output):
+    ``rank="class"`` keeps the first ``max_det`` in class order; ``rank="score"`` keeps the ``max_det`` highest scores
+    (ties: lower class-major position first), after dropping, with ``per_class_max > 0``, every detection past the
+    first ``per_class_max`` of its class.  ``rank="score", max_det=100`` is the torchvision / Detectron per-image cap;
+    ``per_class_max=100`` with a large ``max_det`` hands COCOeval (maxDets 100) every detection it can score.  The
+    ranking sees only the rows ``class_nms`` kept: leave its ``cap`` at the default ``R*(C-1)`` for a complete one.
+    ``workspace``: from ``pack_ranked_workspace`` (allocated here when None)."""
+    check_rank(rank, per_class_max)
     lib = _lib.load()
     det_boxes = _req(det_boxes, "det_boxes")
     det_labels = _req(det_labels, "det_labels", torch.int32)
@@ -770,9 +795,20 @@ def pack_detections(det_boxes, det_labels, det_scores, det_count, max_det: int, 
     with torch.cuda.device(dev):
         out = torch.empty((B, int(max_det), 6), dtype=torch.float32, device=dev)
         cnt = torch.empty((B,), dtype=torch.int32, device=dev)
-        _lib.check(lib.frr_pack_detections(det_boxes.data_ptr(), det_labels.data_ptr(), det_scores.data_ptr(),
-                                           det_count.data_ptr(), B, cap, int(max_det), _ptr(image_wh), int(bool(xywh)),
-                                           out.data_ptr(), cnt.data_ptr(), _stream()), "frr_pack_detections")
+        if rank == "class":
+            _lib.check(lib.frr_pack_detections(det_boxes.data_ptr(), det_labels.data_ptr(), det_scores.data_ptr(),
+                                               det_count.data_ptr(), B, cap, int(max_det), _ptr(image_wh), int(bool(xywh)),
+                                               out.data_ptr(), cnt.data_ptr(), _stream()), "frr_pack_detections")
+            return out, cnt
+        if workspace is None:
+            workspace = pack_ranked_workspace(B, cap, max_det, dev)
+        workspace = _req(workspace, "workspace", torch.uint8)
+        off = (-workspace.data_ptr()) % 256
+        _lib.check(lib.frr_pack_detections_ranked(det_boxes.data_ptr(), det_labels.data_ptr(), det_scores.data_ptr(),
+                                                  det_count.data_ptr(), B, cap, int(max_det), int(per_class_max),
+                                                  _ptr(image_wh), int(bool(xywh)), out.data_ptr(), cnt.data_ptr(),
+                                                  workspace.data_ptr() + off, max(workspace.numel() - off, 0), _stream()),
+                   "frr_pack_detections_ranked")
     return out, cnt
 
 

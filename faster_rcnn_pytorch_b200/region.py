@@ -329,11 +329,16 @@ class InferPlan:
 
     Mixed-size batches: build the plan with the padded (max) ``image_hw`` and pass the per-image sizes to ``pool`` /
     ``capture_pool`` as an int32 [B,2] device tensor: anchors, the roi scaling and the RoIPool window clip then use each
-    image's own size, and a captured graph reads the sizes at every replay."""
+    image's own size, and a captured graph reads the sizes at every replay.
+
+    ``rank`` / ``per_class_max`` choose which ``max_det`` detections of an image ``detect`` packs (see
+    ``ops.pack_detections``): ``"class"`` (default) the first in class order, ``"score"`` the highest-scoring, at most
+    ``per_class_max`` per class when that is > 0.  ``class_nms`` runs at its full capacity, so the ranking sees every
+    detection; the ranking's workspace is allocated here, once."""
 
     def __init__(self, B: int, image_hw, num_classes: int, device, stride: int = 16, max_det: int = 100,
                  score_thres: float = 0.05, iou_thr: float = 0.3, mode: str = "test", logits: bool = True,
-                 nms_cluster_size: int = 0):
+                 nms_cluster_size: int = 0, rank: str = "class", per_class_max: int = 0):
         from . import dist as fdist
         self._fdist = fdist
         self.B, self.hw, self.NC, self.device = int(B), (int(image_hw[0]), int(image_hw[1])), int(num_classes), torch.device(device)
@@ -344,8 +349,12 @@ class InferPlan:
                                      nms_cluster_size=nms_cluster_size)
         self.R = self.proposal.post_k
         self.max_det, self.score_thres, self.iou_thr = int(max_det), float(score_thres), float(iou_thr)
+        ops.check_rank(rank, per_class_max)
+        self.rank, self.per_class_max = rank, int(per_class_max)
         with torch.cuda.device(self.device):
             self.rois5 = torch.empty((self.B * self.R, 5), dtype=torch.float32, device=self.device)
+            self.rank_ws = (ops.pack_ranked_workspace(self.B, self.R * (self.NC - 1), self.max_det, self.device)
+                            if rank == "score" else None)
 
     def pool(self, feat, cls, reg, want_argmax: bool = False, image_hw=None):
         rois, cnt = self.proposal.run(cls, reg, image_hw=image_hw)
@@ -359,7 +368,8 @@ class InferPlan:
         prob, boxes = ops.decode_classwise(head_cls, head_reg, rois.reshape(-1, 4), NC)
         db, dl, ds, dc = ops.class_nms(prob.reshape(B, R, NC), boxes.reshape(B, R, 4 * NC), NC, score_thres=self.score_thres,
                                        iou_thr=self.iou_thr, roi_count=cnt)
-        packed, pc = self._fdist.pack_detections(db, dl, ds, dc, self.max_det)
+        packed, pc = self._fdist.pack_detections(db, dl, ds, dc, self.max_det, rank=self.rank,
+                                                 per_class_max=self.per_class_max, workspace=self.rank_ws)
         if return_all:
             return dict(packed=packed, count=pc, prob=prob, boxes=boxes, det=(db, dl, ds, dc))
         return packed, pc

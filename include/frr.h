@@ -409,6 +409,22 @@ int frr_pack_detections(const float* det_boxes /* [B,cap,4] */, const int32_t* d
                         const float* det_scores /* [B,cap] */, const int32_t* det_count /* [B] */, int B, int cap,
                         int max_det, const float* image_wh, int xywh, float* out /* [B,max_det,6] */,
                         int32_t* out_count /* [B] */, frr_stream_t stream);
+/* The same rows for each image's max_det HIGHEST-SCORING detections, the selection evaluators make (torchvision /
+ * Detectron keep the top 100 per image by score; COCOeval keeps the top maxDets per (image, category) by score),
+ * where frr_pack_detections keeps the first max_det in class order.  Of image b's det_count[b] class-major rows
+ * (frr_class_nms's output), per_class_max > 0 first drops every row at position >= per_class_max inside its class;
+ * the rest are ordered by score, descending, lower class-major position first on equal scores, and the first max_det
+ * are packed exactly as frr_pack_detections packs a row (same scaling, same xywh, zero padding past out_count[b]).
+ * Only the rows frr_class_nms kept are ranked: leave its cap at R*(C-1) for a complete ranking.
+ * min(max_det, cap) <= 16384, and the top-k's shared-memory limit on cap applies (cap <= 65536 always fits).
+ * Workspace from frr_pack_detections_ranked_workspace_bytes, 256-byte aligned.  Three launches: eligibility mask,
+ * the top-k of frr_topk_desc over the masked scores, gather into the packed rows. */
+size_t frr_pack_detections_ranked_workspace_bytes(int B, int cap, int max_det);
+int frr_pack_detections_ranked(const float* det_boxes /* [B,cap,4] */, const int32_t* det_labels /* [B,cap] */,
+                               const float* det_scores /* [B,cap] */, const int32_t* det_count /* [B] */, int B,
+                               int cap, int max_det, int per_class_max, const float* image_wh, int xywh,
+                               float* out /* [B,max_det,6] */, int32_t* out_count /* [B] */, void* workspace,
+                               size_t workspace_bytes, frr_stream_t stream);
 
 #ifdef __cplusplus
 #pragma GCC visibility pop

@@ -22,6 +22,9 @@ int topk_desc_impl(const float* scores, const uint8_t* valid, const float* boxes
                    frr_stream_t stream);
 
 // ------------------------------------------------------------------------------------------------ D1
+// torch's clamp(0, 1): NaN stays NaN (fmaxf alone would turn it into 0), every other value as fminf(fmaxf(.))
+__device__ __forceinline__ float clamp01(float v) { return v != v ? v : fminf(fmaxf(v, 0.f), 1.f); }
+
 // one warp per roi row
 __global__ void __launch_bounds__(256)
     decode_classwise_kernel(const float* __restrict__ cls, const float4* __restrict__ reg, const float4* __restrict__ rois,
@@ -50,10 +53,10 @@ __global__ void __launch_bounds__(256)
         const float w = __fmul_rn(expf(t.z), rw), h = __fmul_rn(expf(t.w), rh);
         const float hw = __fmul_rn(w, 0.5f), hh = __fmul_rn(h, 0.5f);
         float4 b;
-        b.x = fminf(fmaxf(__fsub_rn(cx, hw), 0.f), 1.f);
-        b.y = fminf(fmaxf(__fsub_rn(cy, hh), 0.f), 1.f);
-        b.z = fminf(fmaxf(__fadd_rn(cx, hw), 0.f), 1.f);
-        b.w = fminf(fmaxf(__fadd_rn(cy, hh), 0.f), 1.f);
+        b.x = clamp01(__fsub_rn(cx, hw));
+        b.y = clamp01(__fsub_rn(cy, hh));
+        b.z = clamp01(__fadd_rn(cx, hw));
+        b.w = clamp01(__fadd_rn(cy, hh));
         boxes[(size_t)row * C + c] = b;
     }
 }
@@ -257,7 +260,9 @@ int frr_pack_detections(const float* det_boxes, const int32_t* det_labels, const
     using namespace frr;
     FRR_CHECK_ARG(B >= 0 && cap >= 0 && max_det >= 1, "frr_pack_detections: bad sizes");
     if (B == 0) return FRR_OK;
-    FRR_CHECK_ARG(det_boxes && det_labels && det_scores && det_count && out && out_count, "frr_pack_detections: null pointer");
+    // with cap == 0 there are no rows to read (class_nms(cap=0) hands over empty, unallocated arrays)
+    FRR_CHECK_ARG((cap == 0 || (det_boxes && det_labels && det_scores)) && det_count && out && out_count,
+                  "frr_pack_detections: null pointer");
     FRR_CHECK_ARG(aligned16(det_boxes) && (image_wh == nullptr || (reinterpret_cast<uintptr_t>(image_wh) & 7u) == 0),
                   "frr_pack_detections: det_boxes must be 16-byte aligned, image_wh 8-byte aligned");
     pack_detections_kernel<<<B, 128, 0, (cudaStream_t)stream>>>((const float4*)det_boxes, det_labels, det_scores, det_count,
@@ -287,7 +292,7 @@ int frr_pack_detections_ranked(const float* det_boxes, const int32_t* det_labels
     const int k = ranked_k(cap, max_det);
     FRR_CHECK_ARG(k <= 16384, "frr_pack_detections_ranked: min(max_det, cap) = %d exceeds the top-k capacity 16384", k);
     if (B == 0) return FRR_OK;
-    FRR_CHECK_ARG(det_boxes && det_labels && det_scores && det_count && out && out_count && workspace,
+    FRR_CHECK_ARG((cap == 0 || (det_boxes && det_labels && det_scores)) && det_count && out && out_count && workspace,
                   "frr_pack_detections_ranked: null pointer");
     FRR_CHECK_ARG(aligned16(det_boxes) && (image_wh == nullptr || aligned8(image_wh)) &&
                       (reinterpret_cast<uintptr_t>(workspace) & 255u) == 0,
@@ -334,7 +339,9 @@ int frr_class_nms(const float* prob, const float* boxes, const int32_t* roi_coun
     FRR_CHECK_ARG(B >= 0 && R >= 0 && C >= 2 && cap >= 0, "frr_class_nms: bad sizes");
     FRR_CHECK_ARG(R <= 4096 && C <= 1024, "frr_class_nms: R <= 4096 and C <= 1024 supported");
     if (B == 0) return FRR_OK;
-    FRR_CHECK_ARG(prob && boxes && det_boxes && det_labels && det_scores && det_count && workspace, "frr_class_nms: null pointer");
+    // cap == 0 asks for the counts only: the detection arrays are empty and may be null
+    FRR_CHECK_ARG(prob && boxes && det_count && workspace && (cap == 0 || (det_boxes && det_labels && det_scores)),
+                  "frr_class_nms: null pointer");
     FRR_CHECK_ARG(aligned16(boxes) && aligned16(det_boxes) && (reinterpret_cast<uintptr_t>(workspace) & 255u) == 0,
                   "frr_class_nms: boxes must be 16-byte aligned, workspace 256-byte aligned");
     if (workspace_bytes < frr_class_nms_workspace_bytes(B, R, C)) {

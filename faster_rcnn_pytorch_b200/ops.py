@@ -636,51 +636,61 @@ def sample_targets(mt_state, ws_rpn=None, ws_frcnn=None, rpn_batch: int = 256, r
 RPN_BETA, FRCNN_BETA = float(np.float32(1 / 9)), 1.0      # losses/loss.py:21,47
 
 
+def region_loss_kernel(rpn_cls, rpn_reg, frc_cls, frc_reg, rpn_tcls, rpn_treg, frc_tcls, frc_treg, need):
+    """One ``frr_region_loss`` launch on arguments checked by ``region_loss_args``: returns loss [B,5] and, for each of
+    the four predictions with ``need[j]`` set, the gradient of its image's total for a unit upstream gradient (else
+    None)."""
+    lib = _lib.load()
+    have_rpn, have_frc = rpn_cls is not None, frc_cls is not None
+    ref = rpn_cls if have_rpn else frc_cls
+    dev = ref.device
+    B = ref.shape[0]
+    N = rpn_cls.shape[1] if have_rpn else 0
+    S, C = (frc_cls.shape[1], frc_cls.shape[2]) if have_frc else (0, 0)
+    CR = frc_reg.shape[2] if have_frc else 0
+    need = [have_rpn and need[0], have_rpn and need[1], have_frc and need[2], have_frc and need[3]]
+    with torch.cuda.device(dev):
+        loss = torch.empty((B, 5), dtype=torch.float32, device=dev)
+        grads = [torch.empty_like(t) if n else None for t, n in zip((rpn_cls, rpn_reg, frc_cls, frc_reg), need)]
+        _lib.check(lib.frr_region_loss(_ptr(rpn_cls), _ptr(rpn_reg), _ptr(rpn_tcls), _ptr(rpn_treg), B, N, _ptr(frc_cls),
+                                       _ptr(frc_reg), _ptr(frc_tcls), _ptr(frc_treg), S, C, CR, RPN_BETA, FRCNN_BETA,
+                                       loss.data_ptr(), _ptr(grads[0]), _ptr(grads[1]), _ptr(grads[2]), _ptr(grads[3]),
+                                       _stream()), "frr_region_loss")
+    return loss, grads
+
+
+def region_loss_scale(saved, g):
+    """Gradients of the four predictions for the upstream ``g`` [B,5] of (total, rpn_cls, rpn_reg, frcnn_cls,
+    frcnn_reg), from the unit gradients ``region_loss_kernel`` saved (None stays None)."""
+    out = []
+    for j, s in enumerate(saved):
+        if s is None:
+            out.append(None)
+            continue
+        up = (g[:, 0] + g[:, 1 + j]).reshape((-1,) + (1,) * (s.dim() - 1))
+        out.append(s * up)
+    return out
+
+
 class _RegionLossFn(torch.autograd.Function):
     """One kernel computes the four losses and, for a unit upstream gradient, their gradients w.r.t. the predictions;
     backward only scales the saved gradients by the upstream values."""
 
     @staticmethod
     def forward(ctx, rpn_cls, rpn_reg, frc_cls, frc_reg, rpn_tcls, rpn_treg, frc_tcls, frc_treg):
-        lib = _lib.load()
-        have_rpn, have_frc = rpn_cls is not None, frc_cls is not None
-        ref = rpn_cls if have_rpn else frc_cls
-        dev = ref.device
-        B = ref.shape[0]
-        N = rpn_cls.shape[1] if have_rpn else 0
-        S, C = (frc_cls.shape[1], frc_cls.shape[2]) if have_frc else (0, 0)
-        CR = frc_reg.shape[2] if have_frc else 0
-        need = [have_rpn and ctx.needs_input_grad[0], have_rpn and ctx.needs_input_grad[1],
-                have_frc and ctx.needs_input_grad[2], have_frc and ctx.needs_input_grad[3]]
-        with torch.cuda.device(dev):
-            loss = torch.empty((B, 5), dtype=torch.float32, device=dev)
-            grads = [torch.empty_like(t) if n else None for t, n in zip((rpn_cls, rpn_reg, frc_cls, frc_reg), need)]
-            _lib.check(lib.frr_region_loss(_ptr(rpn_cls), _ptr(rpn_reg), _ptr(rpn_tcls), _ptr(rpn_treg), B, N, _ptr(frc_cls),
-                                           _ptr(frc_reg), _ptr(frc_tcls), _ptr(frc_treg), S, C, CR, RPN_BETA, FRCNN_BETA,
-                                           loss.data_ptr(), _ptr(grads[0]), _ptr(grads[1]), _ptr(grads[2]), _ptr(grads[3]),
-                                           _stream()), "frr_region_loss")
-        ctx.grads = grads
+        loss, ctx.grads = region_loss_kernel(rpn_cls, rpn_reg, frc_cls, frc_reg, rpn_tcls, rpn_treg, frc_tcls, frc_treg,
+                                             ctx.needs_input_grad[:4])
         return loss
 
     @staticmethod
     def backward(ctx, g):            # g [B,5]: upstream of (total, rpn_cls, rpn_reg, frcnn_cls, frcnn_reg)
-        out = []
-        for j, saved in enumerate(ctx.grads):
-            if saved is None:
-                out.append(None)
-                continue
-            up = (g[:, 0] + g[:, 1 + j]).reshape((-1,) + (1,) * (saved.dim() - 1))
-            out.append(saved * up)
-        return tuple(out) + (None, None, None, None)
+        return tuple(region_loss_scale(ctx.grads, g)) + (None, None, None, None)
 
 
-def region_loss(rpn_cls=None, rpn_reg=None, rpn_target_cls=None, rpn_target_reg=None, frcnn_cls=None, frcnn_reg=None,
-                frcnn_target_cls=None, frcnn_target_reg=None):
-    """Batched FRCNNLoss (losses/loss.py:62-82): per image (total, rpn_cls, rpn_reg, frcnn_cls, frcnn_reg) -> [B,5],
-    differentiable w.r.t. the four prediction tensors.  rpn_cls [B,N,2], rpn_reg [B,N,4], rpn_target_cls int64 [B,N],
-    rpn_target_reg [B,N,4]; frcnn_cls [B,S,C], frcnn_reg [B,S,C,4] (or [B,S,C*4]: the head output, the class row is
-    gathered in the kernel, models/model.py:340-341) or [B,S,4] (already gathered), frcnn_target_cls int64 [B,S]
-    (negative = padding), frcnn_target_reg [B,S,4].  Either half may be omitted."""
+def region_loss_args(rpn_cls=None, rpn_reg=None, rpn_target_cls=None, rpn_target_reg=None, frcnn_cls=None, frcnn_reg=None,
+                     frcnn_target_cls=None, frcnn_target_reg=None):
+    """The checks of ``region_loss``: returns its tensors contiguous, frcnn_reg as [B,S,C|1,4], in the kernel's order
+    (rpn_cls, rpn_reg, frcnn_cls, frcnn_reg, rpn_target_cls, rpn_target_reg, frcnn_target_cls, frcnn_target_reg)."""
     if rpn_cls is None and frcnn_cls is None:
         raise ValueError("region_loss: nothing to compute")
     if rpn_cls is not None:
@@ -703,8 +713,18 @@ def region_loss(rpn_cls=None, rpn_reg=None, rpn_target_cls=None, rpn_target_reg=
             raise ValueError("region_loss: frcnn_reg must hold C or 1 rows of 4 per sample")
         if tuple(frcnn_target_cls.shape) != (B, S) or tuple(frcnn_target_reg.shape) != (B, S, 4):
             raise ValueError("region_loss: Fast R-CNN targets must be [B,S] and [B,S,4]")
-    return _RegionLossFn.apply(rpn_cls, rpn_reg, frcnn_cls, frcnn_reg, rpn_target_cls, rpn_target_reg, frcnn_target_cls,
-                               frcnn_target_reg)
+    return rpn_cls, rpn_reg, frcnn_cls, frcnn_reg, rpn_target_cls, rpn_target_reg, frcnn_target_cls, frcnn_target_reg
+
+
+def region_loss(rpn_cls=None, rpn_reg=None, rpn_target_cls=None, rpn_target_reg=None, frcnn_cls=None, frcnn_reg=None,
+                frcnn_target_cls=None, frcnn_target_reg=None):
+    """Batched FRCNNLoss (losses/loss.py:62-82): per image (total, rpn_cls, rpn_reg, frcnn_cls, frcnn_reg) -> [B,5],
+    differentiable w.r.t. the four prediction tensors.  rpn_cls [B,N,2], rpn_reg [B,N,4], rpn_target_cls int64 [B,N],
+    rpn_target_reg [B,N,4]; frcnn_cls [B,S,C], frcnn_reg [B,S,C,4] (or [B,S,C*4]: the head output, the class row is
+    gathered in the kernel, models/model.py:340-341) or [B,S,4] (already gathered), frcnn_target_cls int64 [B,S]
+    (negative = padding), frcnn_target_reg [B,S,4].  Either half may be omitted."""
+    return _RegionLossFn.apply(*region_loss_args(rpn_cls, rpn_reg, rpn_target_cls, rpn_target_reg, frcnn_cls, frcnn_reg,
+                                                 frcnn_target_cls, frcnn_target_reg))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -841,17 +861,32 @@ def fpn_level_rois(rois5, k_min: int, k_max: int, canonical_scale: float = 224.0
     return levels, per
 
 
+def multiscale_roi_align_forward(feats, rois5, output_size, sampling_ratio: int, scales, k_min: int, k_max: int,
+                                 canonical_scale: float = 224.0, canonical_level: int = 4):
+    """The kernels of ``multiscale_roi_align`` for given per-level ``scales`` (see ``infer_scales``): returns (out
+    [K,C,PH,PW], levels int32 [K], the per-level rois [L,K,5] the backward reads, channels_last flag per level)."""
+    K, C = rois5.shape[0], feats[0].shape[1]
+    levels, per = fpn_level_rois(rois5, k_min, k_max, canonical_scale, canonical_level)
+    out = torch.empty((K, C, output_size[0], output_size[1]), dtype=torch.float32, device=rois5.device)
+    lay = []
+    for l, f in enumerate(feats):
+        f_l, cl = _feat_layout(f)
+        lay.append(bool(cl))
+        roi_align_forward(f_l, per[l], output_size, scales[l], sampling_ratio, False, out=out)
+    return out, levels, per, lay
+
+
+def multiscale_roi_align_backward(grad_out, per, shapes, scales, sampling_ratio: int, lay):
+    """Feature gradients (one per level, [B,C,Hl,Wl], channels_last where ``lay[l]``) of ``multiscale_roi_align_forward``."""
+    go = grad_out.contiguous()
+    return [roi_align_backward(go, per[l], shapes[l], scales[l], sampling_ratio, False, lay[l]) for l in range(len(shapes))]
+
+
 class _MultiScaleRoIAlignFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, rois5, output_size, sampling_ratio, scales, k_min, k_max, canonical_scale, canonical_level, *feats):
-        K, C = rois5.shape[0], feats[0].shape[1]
-        levels, per = fpn_level_rois(rois5, k_min, k_max, canonical_scale, canonical_level)
-        out = torch.empty((K, C, output_size[0], output_size[1]), dtype=torch.float32, device=rois5.device)
-        lay = []
-        for l, f in enumerate(feats):
-            f_l, cl = _feat_layout(f)
-            lay.append(bool(cl))
-            roi_align_forward(f_l, per[l], output_size, scales[l], sampling_ratio, False, out=out)
+        out, levels, per, lay = multiscale_roi_align_forward(feats, rois5, output_size, sampling_ratio, scales, k_min, k_max,
+                                                             canonical_scale, canonical_level)
         ctx.save_for_backward(per)
         ctx.meta = ([tuple(f.shape) for f in feats], list(scales), int(sampling_ratio), lay)
         ctx.mark_non_differentiable(levels)
@@ -861,9 +896,7 @@ class _MultiScaleRoIAlignFn(torch.autograd.Function):
     def backward(ctx, grad_out, _grad_levels):
         (per,) = ctx.saved_tensors
         shapes, scales, sr, lay = ctx.meta
-        go = grad_out.contiguous()
-        grads = [roi_align_backward(go, per[l], shapes[l], scales[l], sr, False, lay[l]) for l in range(len(shapes))]
-        return (None,) * 8 + tuple(grads)
+        return (None,) * 8 + tuple(multiscale_roi_align_backward(grad_out, per, shapes, scales, sr, lay))
 
 
 def multiscale_roi_align(features, boxes, image_shapes, output_size=7, sampling_ratio: int = 2,

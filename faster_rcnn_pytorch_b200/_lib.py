@@ -30,28 +30,28 @@ SIGNATURES = {
     "frr_anchors_pyramid": (_i, [_p, _i, _p, _p, _i, _i, _i, _p]),
     "frr_anchors": (_i, [_p, _i, _i, _i, _p, _i, _p]),
     "frr_rpn_decode": (_i, [_p, _p, _i, _p, _p, _i, _i, _i, _i, _f, _p, _p, _p, _i, _i, _p]),
-    "frr_topk_desc": (_i, [_p, _p, _p, _i, _i, _i, _p, _p, _p, _p, _p, _p]),
     "frr_topk_desc_opt": (_i, [_p, _p, _p, _i, _i, _i, _p, _p, _p, _p, _p, _i, _p]),
-    "frr_nms_sorted": (_i, [_p, _p, _i, _i, _d, _i, _p, _p, _p, _i, _p]),
+    "frr_nms_sorted": (_i, [_p, _p, _i, _i, _d, _i, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _p]),
     "frr_rpn_proposals_workspace_bytes": (C.c_size_t, [_i, _i, _i, _i]),
-    "frr_rpn_proposals": (_i, [_p, _p, _i, _p, _p, _i, _i, _i, _i, _f, _i, _i, _i, _i, _d, _p, _p, _p, C.c_size_t, _p]),
-    "frr_rpn_proposals_opt": (_i, [_p, _p, _i, _p, _p, _i, _i, _i, _i, _f, _i, _i, _i, _i, _d, _p, _p, _p, C.c_size_t, _i, _p]),
+    "frr_rpn_proposals": (_i, [_p, _p, _i, _p, _p, _i, _i, _i, _p, _i, _f, _i, _i, _i, _i, _d, _p, _p, _p, C.c_size_t, _i,
+                               _p]),
     "frr_nms_variant": (_i, [_i, _i, _d, _i, _i, _i, _i, _p]),
     "frr_rpn_proposals_workspace_layout": (_i, [_i, _i, _i, _i, _p]),
     "frr_nms_sorted_indirect": (_i, [_p, _i, _p, _p, _i, _i, _d, _i, _p, _p, _p, _i, _i, _p]),
-    "frr_rois5": (_i, [_p, _p, _i, _i, _f, _f, _p, _p]),
-    "frr_roi_pool_fwd": (_i, [_p, _p, _i, _i, _i, _i, _i, _i, _i, _f, _i, _p, _p, _p]),
+    "frr_rois5": (_i, [_p, _p, _i, _i, _i, _i, _p, _i, _p, _p]),
+    "frr_roi_pool_fwd": (_i, [_p, _p, _i, _i, _i, _i, _i, _i, _i, _f, _i, _p, _i, _p, _p, _p]),
     "frr_roi_pool_bwd": (_i, [_p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _f, _i, _p, _p]),
     "frr_roi_align_fwd": (_i, [_p, _p, _i, _i, _i, _i, _i, _i, _i, _f, _i, _i, _i, _p, _p]),
     "frr_roi_align_bwd": (_i, [_p, _p, _i, _i, _i, _i, _i, _i, _i, _f, _i, _i, _i, _p, _p]),
-    "frr_roi_pool_bwd_deterministic": (_i, [_p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _f, _i, _p, _p]),
+    "frr_roi_pool_bwd_deterministic": (_i, [_p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _f, _i, _p, _i, _p, _p]),
     "frr_roi_align_bwd_deterministic": (_i, [_p, _p, _i, _i, _i, _i, _i, _i, _i, _f, _i, _i, _i, _p, _p]),
     "frr_roi_variant": (_i, [_i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p]),
     "frr_fpn_level_rois": (_i, [_p, _i, _i, _i, _i, _f, _i, _p, _p, _p]),
     "frr_region_loss": (_i, [_p, _p, _p, _p, _i, _i, _p, _p, _p, _p, _i, _i, _i, _f, _f, _p, _p, _p, _p, _p, _p]),
     "frr_sample_targets": (_i, [_p, _p, _i, _i, _i, _i, _i, _p, _i, _p, _p, _p, _p, _p, _i, _p, _p, _i, _p]),
-    "frr_rpn_targets_assign": (_i, [_p, _p, _i, _i, _p, _p, _i, _i, _i, _i, _i, _f, _f, _f, _i, _i, _p, _p, _p, _p, _p, _p, _p]),
-    "frr_rpn_targets_finalize": (_i, [_p, _i, _i, _p, _p, _i, _i, _i, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p, _p]),
+    "frr_rpn_targets_assign": (_i, [_p, _p, _i, _i, _p, _p, _i, _i, _i, _p, _i, _i, _f, _f, _f, _i, _i, _p, _p, _p, _p, _p, _p,
+                                    _p]),
+    "frr_rpn_targets_finalize": (_i, [_p, _i, _i, _p, _p, _i, _i, _i, _p, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p, _p]),
     "frr_frcnn_targets_assign": (_i, [_p, _p, _i, _i, _p, _p, _i, _f, _f, _p, _p, _p, _p, _p, _p, _p]),
     "frr_frcnn_targets_finalize": (_i, [_p, _p, _i, _i, _p, _p, _i, _p, _p, _p, _p, _p, _i, _p, _i, _p, _p, _p, _p, _p]),
     "frr_decode_classwise": (_i, [_p, _p, _p, _i, _i, _p, _p, _p, _p]),
@@ -60,17 +60,8 @@ SIGNATURES = {
     "frr_pack_detections_ranked": (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _p, _i, _p, _p, _p, C.c_size_t, _p]),
     "frr_class_nms_workspace_bytes": (C.c_size_t, [_i, _i, _i]),
     "frr_class_nms": (_i, [_p, _p, _p, _i, _i, _i, _f, _d, _i, _p, _p, _p, _p, _p, C.c_size_t, _p]),
-    "frr_nms_sorted_tuned": (_i, [_p, _p, _i, _i, _d, _i, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _p]),
-    # mixed-size batches: per-image sizes image_hw [B,2] on the device
+    # mixed-size batch: per-image sizes image_hw [B,2] on the device
     "frr_rpn_decode_sized": (_i, [_p, _p, _i, _p, _i, _p, _i, _i, _i, _f, _p, _p, _p, _i, _i, _p]),
-    "frr_rpn_proposals_sized": (_i, [_p, _p, _i, _p, _i, _p, _i, _i, _i, _f, _i, _i, _i, _i, _d, _p, _p, _p, C.c_size_t, _i,
-                                     _p]),
-    "frr_rois5_sized": (_i, [_p, _p, _i, _i, _p, _i, _i, _i, _p, _p]),
-    "frr_roi_pool_fwd_sized": (_i, [_p, _p, _i, _i, _i, _i, _i, _i, _i, _f, _i, _p, _i, _p, _p, _p]),
-    "frr_roi_pool_bwd_deterministic_sized": (_i, [_p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _f, _i, _p, _i, _p, _p]),
-    "frr_rpn_targets_assign_sized": (_i, [_p, _p, _i, _i, _p, _i, _p, _i, _i, _i, _i, _f, _f, _f, _i, _i, _p, _p, _p, _p, _p,
-                                          _p, _p]),
-    "frr_rpn_targets_finalize_sized": (_i, [_p, _i, _i, _p, _i, _p, _i, _i, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p, _p]),
 }
 
 
@@ -105,7 +96,7 @@ def load():
             fn = getattr(lib, name)
             fn.restype = res
             fn.argtypes = args
-        if lib.frr_abi_version() != 2:
+        if lib.frr_abi_version() != 3:
             raise FrrError("libfrr.so ABI version mismatch")
         _lib = lib
     return _lib

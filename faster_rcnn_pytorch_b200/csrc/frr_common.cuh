@@ -112,7 +112,7 @@ struct AnchorTable {
 
 int fill_anchor_table(AnchorTable* t, const float* base_table_host, int A, int stride);
 
-// Mixed-size batches (the *_sized entry points): image b of a batch padded to a grid of grid_h x grid_w cells has
+// Mixed-size batches (the entry points given image_hw): image b of a batch padded to a grid of grid_h x grid_w cells has
 // image_hw[b] = (H_b, W_b) pixels and covers cells y < H_b / stride, x < W_b / stride.  The sizes live in device memory,
 // where the host cannot check them, so the extent is clamped to [0, grid] here: an out-of-range size never reads or
 // writes outside the padded grid, and an image with an empty extent has no cells.  image_hw must be 8-byte aligned.

@@ -435,23 +435,16 @@ int nms_launch(const float* boxes, const int32_t* counts, int B, int n, double i
 }  // namespace frr
 
 extern "C" int frr_nms_sorted(const float* boxes, const int32_t* counts, int B, int n, double iou_thr, int max_keep,
-                              int32_t* keep, int32_t* keep_count, float* out_boxes, int cluster_size,
+                              int32_t* keep, int32_t* keep_count, float* out_boxes, int cluster_size, int threads,
+                              int first_chunk, int max_chunk, int lanes_screen, int lanes_pairs, int unit_boxes,
                               frr_stream_t stream) {
-    return frr::nms_launch(boxes, counts, B, n, iou_thr, max_keep, keep, keep_count, out_boxes, cluster_size, 0, frr::NmsTune{},
-                           0, stream, nullptr, 0);
-}
-
-extern "C" int frr_nms_sorted_tuned(const float* boxes, const int32_t* counts, int B, int n, double iou_thr, int max_keep,
-                                    int32_t* keep, int32_t* keep_count, float* out_boxes, int cluster_size, int threads,
-                                    int first_chunk, int max_chunk, int lanes_screen, int lanes_pairs, int unit_boxes,
-                                    frr_stream_t stream) {
     using frr::kBkChunk;
     auto chunk_ok = [](int v) { return v == 0 || (v >= 256 && v <= kBkChunk); };
     auto lanes_ok = [](int v) { return v == 0 || (v >= 1 && v <= 32 && (v & (v - 1)) == 0); };
     FRR_CHECK_ARG(chunk_ok(first_chunk) && chunk_ok(max_chunk),
-                  "frr_nms_sorted_tuned: chunk sizes must be 0 or lie in [256, %d]", kBkChunk);
+                  "frr_nms_sorted: chunk sizes must be 0 or lie in [256, %d]", kBkChunk);
     FRR_CHECK_ARG(lanes_ok(lanes_screen) && lanes_ok(lanes_pairs),
-                  "frr_nms_sorted_tuned: lanes per candidate must be 0 or a power of two <= 32");
+                  "frr_nms_sorted: lanes per candidate must be 0 or a power of two <= 32");
     return frr::nms_launch(boxes, counts, B, n, iou_thr, max_keep, keep, keep_count, out_boxes, cluster_size, threads,
                            frr::NmsTune{first_chunk, max_chunk, lanes_screen, lanes_pairs}, unit_boxes, stream, nullptr, 0);
 }
@@ -472,8 +465,8 @@ extern "C" int frr_nms_variant(int B, int n, double iou_thr, int max_keep, int c
     return FRR_OK;
 }
 
-// Same as frr_nms_sorted_tuned, but the score order is given as indices: candidate i of image b is
-// boxes_src[b][order[b][i]] (boxes_src [B,src_n,4], order int32 [B,n], e.g. the out_idx of frr_topk_desc).
+// Same as frr_nms_sorted, but the score order is given as indices: candidate i of image b is
+// boxes_src[b][order[b][i]] (boxes_src [B,src_n,4], order int32 [B,n], e.g. the out_idx of frr_topk_desc_opt).
 extern "C" int frr_nms_sorted_indirect(const float* boxes_src, int src_n, const int32_t* order, const int32_t* counts, int B,
                                        int n, double iou_thr, int max_keep, int32_t* keep, int32_t* keep_count,
                                        float* out_boxes, int cluster_size, int unit_boxes, frr_stream_t stream) {

@@ -622,7 +622,7 @@ int nms_bucket_launch(const float* boxes, const int32_t* counts, int B, int n, c
     // (otherwise the driver may pick an L1 / shared split that holds one CTA of the 512-thread form per SM)
     FRR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     if (S > 8) FRR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
-    // chunk sizes (frr_nms_sorted_tuned has checked them to lie in [256, kBkChunk]; clamped to what the thread count's
+    // chunk sizes (frr_nms_sorted has checked them to lie in [256, kBkChunk]; clamped to what the thread count's
     // layout holds): the first chunk is small when few boxes are wanted (test mode: 300), at most first_chunk
     // (automatic: 1024)
     const int cap = bk_chunk_cap(threads);

@@ -10,7 +10,7 @@ namespace frr {
 constexpr int kMaxCluster = 16;
 constexpr int kBkChunk = 2048;  // most candidates per chunk of the bucketed kernel (1024 below 1024 threads: bk_chunk_cap)
 
-// Per-call settings of the bucketed kernel (frr_nms_sorted_tuned); 0 = automatic.  Results never depend on them.
+// Per-call settings of the bucketed kernel (frr_nms_sorted); 0 = automatic.  Results never depend on them.
 struct NmsTune {
     int first_chunk, max_chunk;      // candidates in the first / the largest chunk: multiples of 256 in [256, kBkChunk],
                                      // clamped to the chunk capacity of the launch's thread count

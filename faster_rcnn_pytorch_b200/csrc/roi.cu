@@ -594,28 +594,23 @@ __global__ void __launch_bounds__(256)
 
 extern "C" {
 
-int frr_rois5_sized(const float* rois, const int32_t* count, int B, int R, const int32_t* image_hw, int stride, int grid_h,
-                    int grid_w, float* rois5, frr_stream_t stream) {
+int frr_rois5(const float* rois, const int32_t* count, int B, int R, int grid_h, int grid_w, const int32_t* image_hw,
+              int stride, float* rois5, frr_stream_t stream) {
     using namespace frr;
-    FRR_CHECK_ARG(B >= 0 && R >= 0 && stride > 0 && grid_h >= 0 && grid_w >= 0, "frr_rois5_sized: bad sizes");
+    FRR_CHECK_ARG(B >= 0 && R >= 0 && (image_hw == nullptr || (stride > 0 && grid_h >= 0 && grid_w >= 0)),
+                  "frr_rois5: bad sizes");
     if (B == 0 || R == 0) return FRR_OK;
-    FRR_CHECK_ARG(rois && rois5 && image_hw && aligned16(rois) && aligned8(image_hw),
-                  "frr_rois5_sized: rois (16-byte aligned), image_hw (8-byte aligned) and rois5 must be non-null");
-    rois5_sized_kernel<<<(B * R + 255) / 256, 256, 0, (cudaStream_t)stream>>>((const float4*)rois, count, B, R, image_hw,
-                                                                              stride, grid_h, grid_w, rois5);
+    FRR_CHECK_ARG(rois && rois5 && aligned16(rois) && (image_hw == nullptr || aligned8(image_hw)),
+                  "frr_rois5: rois (16-byte aligned), rois5 must be non-null, image_hw 8-byte aligned");
+    const int blocks = (B * R + 255) / 256;
+    if (image_hw)
+        rois5_sized_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>((const float4*)rois, count, B, R, image_hw, stride,
+                                                                     grid_h, grid_w, rois5);
+    else
+        rois5_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>((const float4*)rois, count, B, R, (float)grid_w, (float)grid_h,
+                                                               rois5);
     count_launch();
-    FRR_CHECK_LAUNCH("rois5_sized_kernel");
-    return FRR_OK;
-}
-
-int frr_rois5(const float* rois, const int32_t* count, int B, int R, float fw, float fh, float* rois5, frr_stream_t stream) {
-    using namespace frr;
-    FRR_CHECK_ARG(B >= 0 && R >= 0, "frr_rois5: bad sizes");
-    if (B == 0 || R == 0) return FRR_OK;
-    FRR_CHECK_ARG(rois && rois5 && aligned16(rois), "frr_rois5: rois must be non-null and 16-byte aligned");
-    rois5_kernel<<<(B * R + 255) / 256, 256, 0, (cudaStream_t)stream>>>((const float4*)rois, count, B, R, fw, fh, rois5);
-    count_launch();
-    FRR_CHECK_LAUNCH("rois5_kernel");
+    FRR_CHECK_LAUNCH(image_hw ? "rois5_sized_kernel" : "rois5_kernel");
     return FRR_OK;
 }
 
@@ -634,15 +629,11 @@ int frr_fpn_level_rois(const float* rois5, int K, int k_min, int k_max, int cano
 }
 
 int frr_roi_pool_fwd(const float* feat, const float* rois, int K, int B, int C, int H, int W, int PH, int PW,
-                     float spatial_scale, int channels_last, float* out, int32_t* argmax, frr_stream_t stream) {
-    return frr::roi_forward<false>(feat, rois, K, B, C, H, W, PH, PW, spatial_scale, 0, 0, channels_last, out, argmax, stream);
-}
-int frr_roi_pool_fwd_sized(const float* feat, const float* rois, int K, int B, int C, int H, int W, int PH, int PW,
-                           float spatial_scale, int channels_last, const int32_t* image_hw, int stride, float* out,
-                           int32_t* argmax, frr_stream_t stream) {
+                     float spatial_scale, int channels_last, const int32_t* image_hw, int stride, float* out,
+                     int32_t* argmax, frr_stream_t stream) {
     using namespace frr;
-    FRR_CHECK_ARG(image_hw && aligned8(image_hw) && stride > 0,
-                  "frr_roi_pool_fwd_sized: image_hw must be non-null and 8-byte aligned, stride > 0");
+    FRR_CHECK_ARG(image_hw == nullptr || (aligned8(image_hw) && stride > 0),
+                  "frr_roi_pool_fwd: image_hw must be 8-byte aligned, stride > 0");
     return roi_forward<false>(feat, rois, K, B, C, H, W, PH, PW, spatial_scale, 0, 0, channels_last, out, argmax, stream,
                               image_hw, stride);
 }

@@ -405,17 +405,11 @@ static int roi_backward_det(const float* grad_out, const int32_t* argmax, const 
 extern "C" {
 
 int frr_roi_pool_bwd_deterministic(const float* grad_out, const int32_t* argmax, const float* rois, int K, int B, int C,
-                                   int H, int W, int PH, int PW, float spatial_scale, int channels_last, float* grad_in,
-                                   frr_stream_t stream) {
-    return frr::roi_backward_det<false>(grad_out, argmax, rois, K, B, C, H, W, PH, PW, spatial_scale, 0, 0, channels_last,
-                                        grad_in, stream);
-}
-int frr_roi_pool_bwd_deterministic_sized(const float* grad_out, const int32_t* argmax, const float* rois, int K, int B,
-                                         int C, int H, int W, int PH, int PW, float spatial_scale, int channels_last,
-                                         const int32_t* image_hw, int stride, float* grad_in, frr_stream_t stream) {
+                                   int H, int W, int PH, int PW, float spatial_scale, int channels_last,
+                                   const int32_t* image_hw, int stride, float* grad_in, frr_stream_t stream) {
     using namespace frr;
-    FRR_CHECK_ARG(image_hw && aligned8(image_hw) && stride > 0,
-                  "frr_roi_pool_bwd_deterministic_sized: image_hw must be non-null and 8-byte aligned, stride > 0");
+    FRR_CHECK_ARG(image_hw == nullptr || (aligned8(image_hw) && stride > 0),
+                  "frr_roi_pool_bwd_deterministic: image_hw must be 8-byte aligned, stride > 0");
     return roi_backward_det<false>(grad_out, argmax, rois, K, B, C, H, W, PH, PW, spatial_scale, 0, 0, channels_last,
                                    grad_in, stream, image_hw, stride);
 }

@@ -456,29 +456,22 @@ static size_t frcnn_assign_smem(int Gmax, int M) {
     return 256 + (size_t)Gmax * 16 + (size_t)((Gmax + 3) & ~3) * 4 + 2 * (size_t)((M + 31) / 32) * 4 + 16;
 }
 
+// anchors given, or generated for the (img_h / stride) x (img_w / stride) grid (with image_hw: the padded grid)
 static int anchor_args(AnchorTable* tab, int* fw, const float* anchors, const float* base_table_host, int A, int img_h,
-                       int img_w, int stride, int N) {
+                       int img_w, const int32_t* image_hw, int stride, int N) {
     tab->A = 1;
     *fw = 1;
+    FRR_CHECK_ARG(image_hw == nullptr || (anchors == nullptr && aligned8(image_hw)),
+                  "rpn targets: with image_hw, anchors must be NULL and image_hw 8-byte aligned");
     if (anchors == nullptr) {
         FRR_CHECK_ARG(img_h > 0 && img_w > 0 && stride > 0, "rpn targets: bad image size");
         int rc = fill_anchor_table(tab, base_table_host, A, stride);
         if (rc) return rc;
         *fw = img_w / stride;
-        FRR_CHECK_ARG((img_h / stride) * (*fw) * tab->A == N, "rpn targets: N=%d does not match the image size", N);
+        FRR_CHECK_ARG((long long)(img_h / stride) * (*fw) * tab->A == N, "rpn targets: N=%d does not match the image size", N);
     } else {
         FRR_CHECK_ARG(aligned16(anchors), "rpn targets: anchors must be 16-byte aligned");
     }
-    return FRR_OK;
-}
-
-// anchors generated for a padded grid of grid_h x grid_w cells (the *_sized target entry points)
-static int sized_anchor_args(AnchorTable* tab, const float* base_table_host, int A, int grid_h, int grid_w, int stride, int N) {
-    FRR_CHECK_ARG(grid_h >= 0 && grid_w > 0 && stride > 0, "rpn targets: bad grid %dx%d / stride %d", grid_h, grid_w, stride);
-    int rc = fill_anchor_table(tab, base_table_host, A, stride);
-    if (rc) return rc;
-    FRR_CHECK_ARG((long long)grid_h * grid_w * tab->A == N, "rpn targets: N=%d does not match a %dx%d grid", N, grid_h,
-                  grid_w);
     return FRR_OK;
 }
 
@@ -520,69 +513,31 @@ static int finalize_slabs(int B, int N) {
 extern "C" {
 
 int frr_rpn_targets_assign(const float* gt, const int32_t* gt_count, int B, int Gmax, const float* anchors,
-                           const float* base_table_host, int A, int img_h, int img_w, int stride, int N, float neg_thr,
-                           float pos_thr, float iou_eps_, int inside_only, int tie_inclusive, float* iou_max,
-                           int32_t* argmax, int8_t* label8, int32_t* pos_list, int32_t* neg_list, int32_t* counts,
-                           frr_stream_t stream) {
+                           const float* base_table_host, int A, int img_h, int img_w, const int32_t* image_hw, int stride,
+                           int N, float neg_thr, float pos_thr, float iou_eps_, int inside_only, int tie_inclusive,
+                           float* iou_max, int32_t* argmax, int8_t* label8, int32_t* pos_list, int32_t* neg_list,
+                           int32_t* counts, frr_stream_t stream) {
     using namespace frr;
     FRR_CHECK_ARG(gt && iou_max && argmax && label8 && pos_list && neg_list && counts, "frr_rpn_targets_assign: null pointer");
     FRR_CHECK_ARG(B >= 0 && Gmax >= 1 && N >= 1, "frr_rpn_targets_assign: bad sizes (G = 0 is an error in the reference too)");
     FRR_CHECK_ARG(aligned16(gt), "frr_rpn_targets_assign: gt must be 16-byte aligned");
     AnchorTable tab;
     int fw;
-    int rc = anchor_args(&tab, &fw, anchors, base_table_host, A, img_h, img_w, stride, N);
+    int rc = anchor_args(&tab, &fw, anchors, base_table_host, A, img_h, img_w, image_hw, stride, N);
     if (rc) return rc;
     if (B == 0) return FRR_OK;
+    if (image_hw)
+        return launch_rpn_assign(rpn_assign_sized_kernel, B, N, Gmax, stream, (const float4*)gt, gt_count, Gmax, tab, N,
+                                 img_h / stride, fw, (float)stride, image_hw, neg_thr, pos_thr, iou_eps_, inside_only,
+                                 tie_inclusive, iou_max, argmax, label8, pos_list, neg_list, counts);
     return launch_rpn_assign(rpn_assign_kernel, B, N, Gmax, stream, (const float4*)gt, gt_count, Gmax, (const float4*)anchors,
                              tab, N, fw, (float)stride, (float)img_w, (float)img_h, neg_thr, pos_thr, iou_eps_, inside_only,
                              tie_inclusive, iou_max, argmax, label8, pos_list, neg_list, counts);
 }
 
-int frr_rpn_targets_assign_sized(const float* gt, const int32_t* gt_count, int B, int Gmax, const float* base_table_host,
-                                 int A, const int32_t* image_hw, int grid_h, int grid_w, int stride, int N, float neg_thr,
-                                 float pos_thr, float iou_eps_, int inside_only, int tie_inclusive, float* iou_max,
-                                 int32_t* argmax, int8_t* label8, int32_t* pos_list, int32_t* neg_list, int32_t* counts,
-                                 frr_stream_t stream) {
-    using namespace frr;
-    FRR_CHECK_ARG(gt && iou_max && argmax && label8 && pos_list && neg_list && counts && image_hw,
-                  "frr_rpn_targets_assign_sized: null pointer");
-    FRR_CHECK_ARG(B >= 0 && Gmax >= 1 && N >= 1, "frr_rpn_targets_assign_sized: bad sizes");
-    FRR_CHECK_ARG(aligned16(gt) && aligned8(image_hw), "frr_rpn_targets_assign_sized: gt / image_hw must be 16 / 8-byte aligned");
-    AnchorTable tab;
-    int rc = sized_anchor_args(&tab, base_table_host, A, grid_h, grid_w, stride, N);
-    if (rc) return rc;
-    if (B == 0) return FRR_OK;
-    return launch_rpn_assign(rpn_assign_sized_kernel, B, N, Gmax, stream, (const float4*)gt, gt_count, Gmax, tab, N, grid_h,
-                             grid_w, (float)stride, image_hw, neg_thr, pos_thr, iou_eps_, inside_only, tie_inclusive, iou_max,
-                             argmax, label8, pos_list, neg_list, counts);
-}
-
-int frr_rpn_targets_finalize_sized(const float* gt, int B, int Gmax, const float* base_table_host, int A,
-                                   const int32_t* image_hw, int grid_h, int grid_w, int stride, int N, const int32_t* argmax,
-                                   int8_t* label8, const int32_t* pos_list, const int32_t* neg_list, const int32_t* disable,
-                                   const int32_t* disable_off, int64_t* labels, float* reg, frr_stream_t stream) {
-    using namespace frr;
-    FRR_CHECK_ARG(gt && argmax && label8 && pos_list && neg_list && labels && reg && image_hw,
-                  "frr_rpn_targets_finalize_sized: null pointer");
-    FRR_CHECK_ARG((disable == nullptr) == (disable_off == nullptr), "frr_rpn_targets_finalize_sized: disable/disable_off mismatch");
-    FRR_CHECK_ARG(aligned16(gt) && aligned16(reg) && aligned8(image_hw),
-                  "frr_rpn_targets_finalize_sized: gt/reg must be 16-byte aligned, image_hw 8-byte aligned");
-    AnchorTable tab;
-    int rc = sized_anchor_args(&tab, base_table_host, A, grid_h, grid_w, stride, N);
-    if (rc) return rc;
-    if (B == 0) return FRR_OK;
-    FRR_CHECK_ARG(B <= 65535, "frr_rpn_targets_finalize_sized: B=%d exceeds the grid limit", B);
-    rpn_finalize_sized_kernel<<<dim3((unsigned)finalize_slabs(B, N), (unsigned)B), kTgtThreads, 0, (cudaStream_t)stream>>>(
-        (const float4*)gt, Gmax, tab, N, grid_w, (float)stride, image_hw, argmax, label8, pos_list, neg_list, disable,
-        disable_off, labels, (float4*)reg);
-    count_launch();
-    FRR_CHECK_LAUNCH("rpn_finalize_sized_kernel");
-    return FRR_OK;
-}
-
 int frr_rpn_targets_finalize(const float* gt, int B, int Gmax, const float* anchors, const float* base_table_host, int A,
-                             int img_h, int img_w, int stride, int N, const int32_t* argmax, int8_t* label8,
-                             const int32_t* pos_list, const int32_t* neg_list, const int32_t* disable,
+                             int img_h, int img_w, const int32_t* image_hw, int stride, int N, const int32_t* argmax,
+                             int8_t* label8, const int32_t* pos_list, const int32_t* neg_list, const int32_t* disable,
                              const int32_t* disable_off, int64_t* labels, float* reg, frr_stream_t stream) {
     using namespace frr;
     FRR_CHECK_ARG(gt && argmax && label8 && pos_list && neg_list && labels && reg, "frr_rpn_targets_finalize: null pointer");
@@ -590,15 +545,21 @@ int frr_rpn_targets_finalize(const float* gt, int B, int Gmax, const float* anch
     FRR_CHECK_ARG(aligned16(gt) && aligned16(reg), "frr_rpn_targets_finalize: gt/reg must be 16-byte aligned");
     AnchorTable tab;
     int fw;
-    int rc = anchor_args(&tab, &fw, anchors, base_table_host, A, img_h, img_w, stride, N);
+    int rc = anchor_args(&tab, &fw, anchors, base_table_host, A, img_h, img_w, image_hw, stride, N);
     if (rc) return rc;
     if (B == 0) return FRR_OK;
     FRR_CHECK_ARG(B <= 65535, "frr_rpn_targets_finalize: B=%d exceeds the grid limit", B);
-    rpn_finalize_kernel<<<dim3((unsigned)finalize_slabs(B, N), (unsigned)B), kTgtThreads, 0, (cudaStream_t)stream>>>(
-        (const float4*)gt, Gmax, (const float4*)anchors, tab, N, fw, (float)stride, (float)img_w, (float)img_h, argmax,
-        label8, pos_list, neg_list, disable, disable_off, labels, (float4*)reg);
+    const dim3 grid((unsigned)finalize_slabs(B, N), (unsigned)B);
+    if (image_hw)
+        rpn_finalize_sized_kernel<<<grid, kTgtThreads, 0, (cudaStream_t)stream>>>(
+            (const float4*)gt, Gmax, tab, N, fw, (float)stride, image_hw, argmax, label8, pos_list, neg_list, disable,
+            disable_off, labels, (float4*)reg);
+    else
+        rpn_finalize_kernel<<<grid, kTgtThreads, 0, (cudaStream_t)stream>>>(
+            (const float4*)gt, Gmax, (const float4*)anchors, tab, N, fw, (float)stride, (float)img_w, (float)img_h, argmax,
+            label8, pos_list, neg_list, disable, disable_off, labels, (float4*)reg);
     count_launch();
-    FRR_CHECK_LAUNCH("rpn_finalize_kernel");
+    FRR_CHECK_LAUNCH(image_hw ? "rpn_finalize_sized_kernel" : "rpn_finalize_kernel");
     return FRR_OK;
 }
 

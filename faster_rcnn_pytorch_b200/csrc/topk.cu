@@ -231,12 +231,6 @@ int topk_desc_impl(const float* scores, const uint8_t* valid, const float* boxes
 
 }  // namespace frr
 
-extern "C" int frr_topk_desc(const float* scores, const uint8_t* valid, const float* boxes, int B, int N, int k,
-                             float* out_scores, int32_t* out_idx, int32_t* out_cidx, float* out_boxes,
-                             int32_t* out_count, frr_stream_t stream) {
-    return frr::topk_desc_impl(scores, valid, boxes, B, N, k, out_scores, out_idx, out_cidx, out_boxes, out_count, 0, stream);
-}
-
 extern "C" int frr_topk_desc_opt(const float* scores, const uint8_t* valid, const float* boxes, int B, int N, int k,
                                  float* out_scores, int32_t* out_idx, int32_t* out_cidx, float* out_boxes,
                                  int32_t* out_count, int ctas_per_image, frr_stream_t stream) {
@@ -250,12 +244,12 @@ int frr::topk_desc_impl(const float* scores, const uint8_t* valid, const float* 
                         int32_t* out_idx, int32_t* out_cidx, float* out_boxes, int32_t* out_count, int cluster_hint,
                         frr_stream_t stream) {
     using namespace frr;
-    FRR_CHECK_ARG(scores && out_idx && out_count, "frr_topk_desc: null pointer");
-    FRR_CHECK_ARG(B >= 0 && N >= 0 && k >= 0, "frr_topk_desc: bad sizes B=%d N=%d k=%d", B, N, k);
+    FRR_CHECK_ARG(scores && out_idx && out_count, "frr_topk_desc_opt: null pointer");
+    FRR_CHECK_ARG(B >= 0 && N >= 0 && k >= 0, "frr_topk_desc_opt: bad sizes B=%d N=%d k=%d", B, N, k);
     FRR_CHECK_ARG((out_boxes == nullptr) || (boxes != nullptr && aligned16(boxes) && aligned16(out_boxes)),
-                  "frr_topk_desc: boxes must be given and 16-byte aligned when out_boxes is requested");
+                  "frr_topk_desc_opt: boxes must be given and 16-byte aligned when out_boxes is requested");
     if (B == 0 || k == 0) return FRR_OK;
-    FRR_CHECK_ARG(k <= 16384, "frr_topk_desc: k=%d exceeds the in-smem sort capacity 16384", k);
+    FRR_CHECK_ARG(k <= 16384, "frr_topk_desc_opt: k=%d exceeds the in-smem sort capacity 16384", k);
     {   // fast path: shared-memory bucket top-k (topk_radix.cu); shapes outside it take the bitonic kernel below
         const int rc = topk_radix_launch(scores, valid, boxes, B, N, k, out_scores, out_idx, out_cidx, out_boxes, out_count,
                                          stream, cluster_hint);
@@ -265,7 +259,7 @@ int frr::topk_desc_impl(const float* scores, const uint8_t* valid, const float* 
     while (P < k) P <<= 1;
     const int nchunks = (N + 31) / 32;
     const size_t smem = topk_smem_bytes(nchunks, P);
-    FRR_CHECK_ARG(smem <= 227 * 1024, "frr_topk_desc: N=%d k=%d needs %zu B shared memory (> 227 KB)", N, k, smem);
+    FRR_CHECK_ARG(smem <= 227 * 1024, "frr_topk_desc_opt: N=%d k=%d needs %zu B shared memory (> 227 KB)", N, k, smem);
     // per device attribute: set before every launch (a process may drive several GPUs)
     FRR_CUDA(cudaFuncSetAttribute(topk_bitonic_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
     topk_bitonic_kernel<<<B, kTopkThreads, smem, (cudaStream_t)stream>>>(scores, valid, (const float4*)boxes, N, k, P,

@@ -38,7 +38,7 @@ def nms(boxes: torch.Tensor, scores: torch.Tensor, iou_threshold: float) -> torc
         return torch.empty((0,), dtype=torch.int64, device=boxes.device)
     b = boxes.detach().to(torch.float32).contiguous()
     if n > 16384:
-        # beyond the in-shared-memory sort of frr_topk_desc (the reference never passes more than 12000 boxes,
+        # beyond the in-shared-memory sort of frr_topk_desc_opt (the reference never passes more than 12000 boxes,
         # models/model.py:24-28): the ordering falls to torch's stable device sort, the NMS itself stays frr_nms_sorted
         order = torch.argsort(scores.detach().to(torch.float32), descending=True, stable=True)
         keep, cnt, _ = ops.nms_sorted(b.index_select(0, order).reshape(1, n, 4), float(iou_threshold), gather=False)

@@ -197,8 +197,7 @@ def nms_sorted(boxes, iou_threshold: float, max_keep: int | None = None, counts=
     """N1 on score-sorted boxes [B,n,4].  Returns keep int32 [B,max_keep] (-1 padded), count int32 [B],
     rois [B,max_keep,4] (zero padded) or None.  ``unit_boxes``: the caller guarantees coordinates in [0,1]
     (enables a cheaper, result-identical screening test).  ``first_chunk``, ``max_chunk``, ``lanes_screen``,
-    ``lanes_pairs``: settings of the bucketed variant, 0 = automatic (frr_nms_sorted_tuned); results do not
-    depend on them."""
+    ``lanes_pairs``: settings of the bucketed variant, 0 = automatic; results do not depend on them."""
     lib = _lib.load()
     boxes = _req(boxes, "boxes")
     if boxes.dim() != 3 or boxes.shape[-1] != 4:
@@ -212,10 +211,10 @@ def nms_sorted(boxes, iou_threshold: float, max_keep: int | None = None, counts=
         keep = torch.empty((B, mk), dtype=torch.int32, device=dev)
         cnt = torch.empty((B,), dtype=torch.int32, device=dev)
         rois = torch.empty((B, mk, 4), dtype=torch.float32, device=dev) if gather else None
-        _lib.check(lib.frr_nms_sorted_tuned(boxes.data_ptr(), _ptr(counts), B, n, float(iou_threshold), mk,
-                                            keep.data_ptr(), cnt.data_ptr(), _ptr(rois), int(cluster_size), int(threads),
-                                            int(first_chunk), int(max_chunk), int(lanes_screen), int(lanes_pairs),
-                                            int(bool(unit_boxes)), _stream()), "frr_nms_sorted")
+        _lib.check(lib.frr_nms_sorted(boxes.data_ptr(), _ptr(counts), B, n, float(iou_threshold), mk, keep.data_ptr(),
+                                      cnt.data_ptr(), _ptr(rois), int(cluster_size), int(threads), int(first_chunk),
+                                      int(max_chunk), int(lanes_screen), int(lanes_pairs), int(bool(unit_boxes)), _stream()),
+                   "frr_nms_sorted")
     return keep, cnt, rois
 
 
@@ -300,13 +299,9 @@ def rois5(rois, count, feat_hw, out=None, image_hw=None, stride: int = 16):
     with torch.cuda.device(rois.device):
         if out is None:
             out = torch.empty((B * R, 5), dtype=torch.float32, device=rois.device)
-        if image_hw is not None:
-            hw = sized_hw(image_hw, B, feat_hw, stride, rois.device)
-            _lib.check(lib.frr_rois5_sized(rois.data_ptr(), _ptr(count), B, R, hw.data_ptr(), int(stride), int(feat_hw[0]),
-                                           int(feat_hw[1]), out.data_ptr(), _stream()), "frr_rois5_sized")
-            return out
-        _lib.check(lib.frr_rois5(rois.data_ptr(), _ptr(count), B, R, float(feat_hw[1]), float(feat_hw[0]), out.data_ptr(),
-                                 _stream()), "frr_rois5")
+        hw = None if image_hw is None else sized_hw(image_hw, B, feat_hw, stride, rois.device)
+        _lib.check(lib.frr_rois5(rois.data_ptr(), _ptr(count), B, R, int(feat_hw[0]), int(feat_hw[1]), _ptr(hw), int(stride),
+                                 out.data_ptr(), _stream()), "frr_rois5")
     return out
 
 
@@ -326,14 +321,9 @@ def roi_pool_forward(feat, rois5, output_size=(7, 7), spatial_scale: float = 1.0
     with torch.cuda.device(feat.device):
         out = torch.empty((K, C, PH, PW), dtype=torch.float32, device=feat.device)
         arg = torch.empty((K, C, PH, PW), dtype=torch.int32, device=feat.device) if want_argmax else None
-        if image_hw is not None:
-            hw = sized_hw(image_hw, B, (H, W), stride, feat.device)
-            _lib.check(lib.frr_roi_pool_fwd_sized(feat.data_ptr(), rois5.data_ptr(), K, B, C, H, W, PH, PW,
-                                                  float(spatial_scale), cl, hw.data_ptr(), int(stride), out.data_ptr(),
-                                                  _ptr(arg), _stream()), "frr_roi_pool_fwd_sized")
-            return out, arg
+        hw = None if image_hw is None else sized_hw(image_hw, B, (H, W), stride, feat.device)
         _lib.check(lib.frr_roi_pool_fwd(feat.data_ptr(), rois5.data_ptr(), K, B, C, H, W, PH, PW, float(spatial_scale), cl,
-                                        out.data_ptr(), _ptr(arg), _stream()), "frr_roi_pool_fwd")
+                                        _ptr(hw), int(stride), out.data_ptr(), _ptr(arg), _stream()), "frr_roi_pool_fwd")
     return out, arg
 
 
@@ -349,7 +339,6 @@ def roi_pool_backward(grad_out, argmax, rois5, feat_shape, spatial_scale: float 
     clips each bin window to the image's own grid.  The padding region of the gradient is zero either way."""
     lib = _lib.load()
     det = _deterministic(deterministic)
-    fn = lib.frr_roi_pool_bwd_deterministic if det else lib.frr_roi_pool_bwd
     grad_out = _req(grad_out, "grad_out")
     argmax = _req(argmax, "argmax", torch.int32)
     rois5 = _req(rois5, "rois")
@@ -358,15 +347,14 @@ def roi_pool_backward(grad_out, argmax, rois5, feat_shape, spatial_scale: float 
     with torch.cuda.device(grad_out.device):
         gin = torch.empty((B, C, H, W), dtype=torch.float32, device=grad_out.device,
                           memory_format=torch.channels_last if channels_last else torch.contiguous_format)
-        if det and image_hw is not None:
-            hw = sized_hw(image_hw, B, (H, W), stride, grad_out.device)
-            _lib.check(lib.frr_roi_pool_bwd_deterministic_sized(grad_out.data_ptr(), argmax.data_ptr(), rois5.data_ptr(), K, B,
-                                                                C, H, W, PH, PW, float(spatial_scale), int(channels_last),
-                                                                hw.data_ptr(), int(stride), gin.data_ptr(), _stream()),
-                       "frr_roi_pool_bwd_deterministic_sized")
-            return gin
-        _lib.check(fn(grad_out.data_ptr(), argmax.data_ptr(), rois5.data_ptr(), K, B, C, H, W, PH, PW, float(spatial_scale),
-                      int(channels_last), gin.data_ptr(), _stream()), fn.__name__)
+        args = (grad_out.data_ptr(), argmax.data_ptr(), rois5.data_ptr(), K, B, C, H, W, PH, PW, float(spatial_scale),
+                int(channels_last))
+        if det:
+            hw = None if image_hw is None else sized_hw(image_hw, B, (H, W), stride, grad_out.device)
+            _lib.check(lib.frr_roi_pool_bwd_deterministic(*args, _ptr(hw), int(stride), gin.data_ptr(), _stream()),
+                       "frr_roi_pool_bwd_deterministic")
+        else:
+            _lib.check(lib.frr_roi_pool_bwd(*args, gin.data_ptr(), _stream()), "frr_roi_pool_bwd")
     return gin
 
 
@@ -496,7 +484,7 @@ def rpn_targets_assign(gt, gt_count, N, image_hw=None, anchors=None, stride=16, 
         if anchors is not None or grid_hw is None:
             raise ValueError("rpn_targets_assign: per-image sizes need grid_hw and generated anchors")
         hw = sized_hw(image_hw, B, grid_hw, stride, gt.device)
-        H, W = int(grid_hw[0]), int(grid_hw[1])      # with hw set: the padded grid in cells
+        H, W = int(grid_hw[0]) * stride, int(grid_hw[1]) * stride      # with hw set: the padded size in pixels
     elif anchors is not None:
         anchors = _req(anchors, "anchors")
         H = W = 0
@@ -513,12 +501,8 @@ def rpn_targets_assign(gt, gt_count, N, image_hw=None, anchors=None, stride=16, 
         outs = (ws["iou_max"].data_ptr(), ws["argmax"].data_ptr(), ws["label8"].data_ptr(), ws["pos_list"].data_ptr(),
                 ws["neg_list"].data_ptr(), ws["counts"].data_ptr(), _stream())
         thr = (float(np.float32(neg_thr)), float(np.float32(pos_thr)), eps, inside_only, tie_inclusive)
-        if hw is not None:
-            _lib.check(lib.frr_rpn_targets_assign_sized(gt.data_ptr(), _ptr(gt_count), B, G, tptr, A, hw.data_ptr(), H, W,
-                                                        stride, N, *thr, *outs), "frr_rpn_targets_assign_sized")
-        else:
-            _lib.check(lib.frr_rpn_targets_assign(gt.data_ptr(), _ptr(gt_count), B, G, _ptr(anchors), tptr, A, H, W, stride, N,
-                                                  *thr, *outs), "frr_rpn_targets_assign")
+        _lib.check(lib.frr_rpn_targets_assign(gt.data_ptr(), _ptr(gt_count), B, G, _ptr(anchors), tptr, A, H, W, _ptr(hw),
+                                              stride, N, *thr, *outs), "frr_rpn_targets_assign")
     ws.update(gt=gt, anchors=anchors, geom=(H, W, stride, table, N), image_hw=hw)
     return ws
 
@@ -535,12 +519,8 @@ def rpn_targets_finalize(ws, disable=None, disable_off=None):
         reg = torch.empty((B, N, 4), dtype=torch.float32, device=dev)
         rest = (ws["argmax"].data_ptr(), ws["label8"].data_ptr(), ws["pos_list"].data_ptr(), ws["neg_list"].data_ptr(),
                 _ptr(disable), _ptr(disable_off), labels.data_ptr(), reg.data_ptr(), _stream())
-        if ws.get("image_hw") is not None:
-            _lib.check(lib.frr_rpn_targets_finalize_sized(gt.data_ptr(), B, G, tptr, A, ws["image_hw"].data_ptr(), H, W,
-                                                          stride, N, *rest), "frr_rpn_targets_finalize_sized")
-        else:
-            _lib.check(lib.frr_rpn_targets_finalize(gt.data_ptr(), B, G, _ptr(anchors), tptr, A, H, W, stride, N, *rest),
-                       "frr_rpn_targets_finalize")
+        _lib.check(lib.frr_rpn_targets_finalize(gt.data_ptr(), B, G, _ptr(anchors), tptr, A, H, W, _ptr(ws["image_hw"]),
+                                                stride, N, *rest), "frr_rpn_targets_finalize")
     return labels, reg
 
 

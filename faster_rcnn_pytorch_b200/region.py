@@ -109,22 +109,16 @@ class ProposalPlan:
             raise ValueError("ProposalPlan.run: shape mismatch with the plan")
         rois = self.rois if rois is None else rois
         count = self.count if count is None else count
+        hw = None
         if image_hw is not None:
             if self.anchors is not None:
                 raise ValueError("ProposalPlan.run: per-image sizes need generated anchors (a plan built with image_hw)")
             hw = ops.sized_hw(image_hw, self.B, self.grid_hw, self.stride, self.device)
-            _lib.check(self.lib.frr_rpn_proposals_sized(reg.data_ptr(), cls.data_ptr(), int(self.logits), self._tptr, self.A,
-                                                        hw.data_ptr(), self.grid_hw[0], self.grid_hw[1], self.stride,
-                                                        self.min_size, self.B, self.N, self.pre_k, self.post_k, self.thr,
-                                                        rois.data_ptr(), count.data_ptr(), self._ws_ptr, self.ws_bytes,
-                                                        self.nms_cluster_size, torch.cuda.current_stream().cuda_stream),
-                       "frr_rpn_proposals_sized")
-            return rois, count
-        _lib.check(self.lib.frr_rpn_proposals_opt(reg.data_ptr(), cls.data_ptr(), int(self.logits), ops._ptr(self.anchors),
-                                                  self._tptr, self.A, self.H, self.W, self.stride, self.min_size, self.B,
-                                                  self.N, self.pre_k, self.post_k, self.thr, rois.data_ptr(),
-                                                  count.data_ptr(), self._ws_ptr, self.ws_bytes, self.nms_cluster_size,
-                                                  torch.cuda.current_stream().cuda_stream), "frr_rpn_proposals_opt")
+        _lib.check(self.lib.frr_rpn_proposals(reg.data_ptr(), cls.data_ptr(), int(self.logits), ops._ptr(self.anchors),
+                                              self._tptr, self.A, self.H, self.W, ops._ptr(hw), self.stride, self.min_size,
+                                              self.B, self.N, self.pre_k, self.post_k, self.thr, rois.data_ptr(),
+                                              count.data_ptr(), self._ws_ptr, self.ws_bytes, self.nms_cluster_size,
+                                              torch.cuda.current_stream().cuda_stream), "frr_rpn_proposals")
         return rois, count
 
 

@@ -30,7 +30,7 @@ extern "C" {
 #pragma GCC visibility push(default)
 #endif
 
-#define FRR_ABI_VERSION 2
+#define FRR_ABI_VERSION 3
 
 #define FRR_OK 0
 #define FRR_E_INVALID (-1)   /* bad argument (shape, alignment, range)        */
@@ -83,11 +83,13 @@ int frr_rpn_decode(const float* reg /* [B,N,4] */, const float* cls /* [B,N,2] l
  *     scales rois by each image's own feature grid (:104-110).  A batch of differently sized images is padded to one grid
  *     of grid_h x grid_w cells (N = grid_h * grid_w * A anchors per image, cell-major / anchor-minor over the PADDED grid);
  *     image_hw int32 [B,2] (device, 8-byte aligned) holds each image's (H_b, W_b) in pixels.  Image b covers the cells
- *     y < fh_b = H_b / stride, x < fw_b = W_b / stride; the rest of the grid is padding.  Every *_sized entry point gives
- *     image b exactly what its uniform form gives for image b alone at (H_b, W_b) on the cropped inputs, with indices
- *     mapped by (y * grid_w + x) * A + a <-> (y * fw_b + x) * A + a.  The sizes are read on the device at run time (one
- *     CUDA graph serves every mix of sizes that fits the grid), so the host cannot check them: fh_b / fw_b are clamped to
- *     [0, grid_h] / [0, grid_w], and an image with an empty grid has no valid anchor, no proposal (count 0) and no rois.
+ *     y < fh_b = H_b / stride, x < fw_b = W_b / stride; the rest of the grid is padding.  Every entry point that takes
+ *     image_hw gives, when it is set, image b exactly what it gives with image_hw == NULL for image b alone at (H_b, W_b)
+ *     on the cropped inputs, with indices mapped by (y * grid_w + x) * A + a <-> (y * fw_b + x) * A + a; its size
+ *     parameters then describe the padded batch, anchors must be NULL (generated) and stride > 0.  The sizes are read on
+ *     the device at run time (one CUDA graph serves every mix of sizes that fits the grid), so the host cannot check
+ *     them: fh_b / fw_b are clamped to [0, grid_h] / [0, grid_w], and an image with an empty grid has no valid anchor, no
+ *     proposal (count 0) and no rois.
  * frr_rpn_decode_sized: anchors divided by each image's own (W_b, H_b) (the __fdiv_rn recipe of frr_rpn_decode);
  *     padding cells get box 0, score 0, valid 0 whatever reg / cls hold there (NaN included).                        */
 int frr_rpn_decode_sized(const float* reg /* [B,N,4] */, const float* cls /* [B,N,2] logits or [B,N] scores */,
@@ -103,13 +105,8 @@ int frr_rpn_decode_sized(const float* reg /* [B,N,4] */, const float* cls /* [B,
  *     (idx -1, score -inf, box 0).  out_cidx = index into the min-size-compacted array (what
  *     the reference's sort returns), out_idx = index into the full N.  k <= 16384.
  * ------------------------------------------------------------------------------------- */
-int frr_topk_desc(const float* scores /* [B,N] */, const uint8_t* valid /* [B,N] or NULL */,
-                  const float* boxes /* [B,N,4] or NULL */, int B, int N, int k,
-                  float* out_scores /* [B,k] or NULL */, int32_t* out_idx /* [B,k] */,
-                  int32_t* out_cidx /* [B,k] or NULL */, float* out_boxes /* [B,k,4] or NULL */,
-                  int32_t* out_count /* [B] */, frr_stream_t stream);
-/* The same with the CTAs per image chosen by the caller: 0 = automatic (a 2-CTA cluster per image when B * 2 CTAs fit the
- * SMs: lowest latency), 1 = one CTA per image (least SM time: several batches in flight).  Identical results.        */
+/* ctas_per_image: 0 = automatic (a 2-CTA cluster per image when B * 2 CTAs fit the SMs: lowest latency), 1 = one CTA per
+ * image (least SM time: several batches in flight).  Identical results.                                                */
 int frr_topk_desc_opt(const float* scores /* [B,N] */, const uint8_t* valid /* [B,N] or NULL */,
                   const float* boxes /* [B,N,4] or NULL */, int B, int N, int k,
                   float* out_scores /* [B,k] or NULL */, int32_t* out_idx /* [B,k] */,
@@ -123,20 +120,17 @@ int frr_topk_desc_opt(const float* scores /* [B,N] */, const uint8_t* valid /* [
  *     stops at max_keep.  keep = positions in the sorted list, ascending, -1 padded.
  *     cluster_size: 0 = auto, else 1,2,4,8,16.
  * ------------------------------------------------------------------------------------- */
+/* threads per CTA (0 = auto, 256, 512 or 1024); the settings of the bucketed variant (3 in frr_nms_variant), each
+ * 0 = automatic: first_chunk / max_chunk = candidates in the first / the largest chunk (multiples of 256 in [256, 2048];
+ * automatic 1024 / 2048), lanes_screen / lanes_pairs = lanes per candidate of its screen / pair phases (powers of two
+ * <= 32; automatic: lanes_screen 2 with 1-2 CTAs per image, else 4; lanes_pairs 4); unit_boxes != 0 = the caller
+ * guarantees every coordinate lies in [0,1] (true for the clamped RPN / detection boxes of models/model.py:34,378),
+ * which enables a cheaper screening test.  Results are identical for every setting.                                    */
 int frr_nms_sorted(const float* boxes /* [B,n,4] */, const int32_t* counts /* [B] or NULL (=n) */, int B,
                    int n, double iou_thr, int max_keep, int32_t* keep /* [B,max_keep] */,
                    int32_t* keep_count /* [B] */, float* out_boxes /* [B,max_keep,4] or NULL */,
-                   int cluster_size, frr_stream_t stream);
-/* Same, with tuning knobs: threads per CTA (0 = auto, 256, 512 or 1024); the settings of the bucketed variant (3 in
- * frr_nms_variant), each 0 = automatic: first_chunk / max_chunk = candidates in the first / the largest chunk
- * (multiples of 256 in [256, 2048]; automatic 1024 / 2048), lanes_screen / lanes_pairs = lanes per candidate of its
- * screen / pair phases (powers of two <= 32; automatic: lanes_screen 2 with 1-2 CTAs per image, else 4; lanes_pairs 4);
- * unit_boxes != 0 = the caller guarantees every coordinate lies in [0,1] (true for the clamped RPN / detection boxes of
- * models/model.py:34,378), which enables a cheaper screening test.  Results are identical for every setting.         */
-int frr_nms_sorted_tuned(const float* boxes, const int32_t* counts, int B, int n, double iou_thr, int max_keep,
-                         int32_t* keep, int32_t* keep_count, float* out_boxes, int cluster_size, int threads,
-                         int first_chunk, int max_chunk, int lanes_screen, int lanes_pairs, int unit_boxes,
-                         frr_stream_t stream);
+                   int cluster_size, int threads, int first_chunk, int max_chunk, int lanes_screen, int lanes_pairs,
+                   int unit_boxes, frr_stream_t stream);
 
 /* Which kernel variant and launch geometry the NMS entry points pick for a problem (host only, launches nothing;
  * tests and bench.py assert through it that the variant they mean to exercise is the one that runs):
@@ -146,7 +140,7 @@ int frr_nms_variant(int B, int n, double iou_thr, int max_keep, int cluster_size
                     int32_t* out4);
 
 /* Same, with the score order given as indices into an unsorted array: candidate i of image b is
- * boxes_src[b][order[b][i]] (boxes_src [B,src_n,4]; order int32 [B,n] = out_idx of frr_topk_desc).  Only the
+ * boxes_src[b][order[b][i]] (boxes_src [B,src_n,4]; order int32 [B,n] = out_idx of frr_topk_desc_opt).  Only the
  * candidates NMS visits are gathered; the top-k kernel then need not write sorted boxes at all.          */
 int frr_nms_sorted_indirect(const float* boxes_src, int src_n, const int32_t* order, const int32_t* counts, int B,
                             int n, double iou_thr, int max_keep, int32_t* keep, int32_t* keep_count,
@@ -164,30 +158,20 @@ size_t frr_rpn_proposals_workspace_bytes(int B, int N, int pre_nms_top_k, int po
  * offsets[0..5] = decoded boxes [B,N,4] f32, scores [B,N] f32, valid [B,N] u8, top-k order [B,k] i32 (indices into
  * N), top-k count [B] i32, NMS keep list [B,post] i32 (positions in the top-k order, -1 padded).                */
 int frr_rpn_proposals_workspace_layout(int B, int N, int pre_nms_top_k, int post_nms_top_k, size_t* offsets6);
+/* nms_cluster_size = CTAs per image of the NMS (1, 2, 4, 8, 16; 0 = automatic, the lowest latency of ONE call: 2 at 64
+ * images, 8-16 for a single image).  1 spends the least SM time per image (9.4 k vs 15.5 k SM-microseconds per 64
+ * images): the setting for several batches in flight on different streams (region.ProposalPipeline), where the other
+ * batches' kernels fill the SMs a single CTA per image leaves idle.  Results are identical for every setting.
+ * image_hw set: a mixed-size batch padded to (img_h / stride) x (img_w / stride) cells (see frr_rpn_decode_sized); the
+ * decode is frr_rpn_decode_sized, top-k and NMS are unchanged (padding cells are invalid; the row-major order of the
+ * padded grid keeps each image's relative anchor order, so ties break as for the image alone).  The workspace and the
+ * top-k order are those of the padded N.                                                                           */
 int frr_rpn_proposals(const float* reg /* [B,N,4] */, const float* cls /* [B,N,2] logits or [B,N] scores */,
                       int cls_is_logits, const float* anchors /* [N,4] or NULL */, const float* base_table_host, int A,
-                      int img_h, int img_w, int stride, float min_size, int B, int N, int pre_nms_top_k,
-                      int post_nms_top_k, double iou_thr, float* rois, int32_t* roi_count, void* workspace,
-                      size_t workspace_bytes, frr_stream_t stream);
-/* The same call with the NMS launch geometry chosen by the caller: nms_cluster_size = CTAs per image (1, 2, 4, 8, 16;
- * 0 = automatic, the lowest latency of ONE call: 2 at 64 images, 8-16 for a single image).  1 spends the least SM time
- * per image (9.4 k vs 15.5 k SM-microseconds per 64 images): the setting for several batches in flight on different
- * streams (region.ProposalPipeline), where the other batches' kernels fill the SMs a single CTA per image leaves idle.
- * Results are identical for every setting.                                                                        */
-int frr_rpn_proposals_opt(const float* reg, const float* cls, int cls_is_logits, const float* anchors,
-                          const float* base_table_host, int A, int img_h, int img_w, int stride, float min_size, int B,
-                          int N, int pre_nms_top_k, int post_nms_top_k, double iou_thr, float* rois, int32_t* roi_count,
-                          void* workspace, size_t workspace_bytes, int nms_cluster_size, frr_stream_t stream);
-
-/* frr_rpn_proposals_opt for a mixed-size batch padded to grid_h x grid_w cells (see frr_rpn_decode_sized): the decode
- * is the sized one, top-k and NMS are unchanged (padding cells are invalid; the row-major order of the padded grid keeps
- * each image's relative anchor order, so ties break as for the image alone).  Workspace size and layout are those of
- * frr_rpn_proposals_workspace_bytes / _layout for the padded N; the top-k order holds indices into the padded N.      */
-int frr_rpn_proposals_sized(const float* reg, const float* cls, int cls_is_logits, const float* base_table_host, int A,
-                            const int32_t* image_hw /* [B,2] device */, int grid_h, int grid_w, int stride, float min_size,
-                            int B, int N, int pre_nms_top_k, int post_nms_top_k, double iou_thr, float* rois,
-                            int32_t* roi_count, void* workspace, size_t workspace_bytes, int nms_cluster_size,
-                            frr_stream_t stream);
+                      int img_h, int img_w, const int32_t* image_hw /* [B,2] device, or NULL */, int stride,
+                      float min_size, int B, int N, int pre_nms_top_k, int post_nms_top_k, double iou_thr, float* rois,
+                      int32_t* roi_count, void* workspace, size_t workspace_bytes, int nms_cluster_size,
+                      frr_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------
  * R1-R3  RoIPool -- torchvision.ops.RoIPool((7,7), 1.0) at models/model.py:97,113 and its autograd
@@ -203,26 +187,22 @@ int frr_rpn_proposals_sized(const float* reg, const float* cls, int cls_is_logit
  * ------------------------------------------------------------------------------------- */
 /* R1 glue -- models/model.py:104-110 (roi * [fw,fh,fw,fh]) + TV ops/_utils.py:18-25 (list of per-image rois ->
  * Tensor[K,5] with the batch index): rois [B,R,4] normalised (e.g. the output of frr_rpn_proposals), count [B] or
- * NULL -> rois5 [B*R,5]; rows r >= count[b] get batch index -1 = masked: the RoI kernels skip masked rois (their
- * output rows are not written) and rois whose index is >= B. */
-int frr_rois5(const float* rois, const int32_t* count, int B, int R, float fw, float fh, float* rois5,
-              frr_stream_t stream);
+ * NULL -> rois5 [B*R,5] scaled by the feature grid (fw, fh) = (grid_w, grid_h); rows r >= count[b] get batch index
+ * -1 = masked: the RoI kernels skip masked rois (their output rows are not written) and rois whose index is >= B.
+ * image_hw set (mixed-size batch, see frr_rpn_decode_sized; grid_h x grid_w = the padded grid): image b's rois are
+ * scaled by its own grid (fw_b, fh_b), and the rows of an image with an empty grid are masked. */
+int frr_rois5(const float* rois, const int32_t* count, int B, int R, int grid_h, int grid_w,
+              const int32_t* image_hw /* [B,2] device, or NULL */, int stride, float* rois5, frr_stream_t stream);
+/* image_hw set (mixed-size batch, see frr_rpn_decode_sized; features padded to H x W cells): every bin window of a roi
+ * of image b is clipped to [0, fh_b) x [0, fw_b) instead of the padded map, as torchvision does on that image alone: a
+ * roi clamped to the image edge has round(x2 * fw_b) == fw_b and loses its last window column there, while the padded
+ * map holds padding values in that column.  argmax stays h * W + w, an index into the padded plane, and never points
+ * at padding.  fh_b = image_hw[b,0] / stride and fw_b = image_hw[b,1] / stride, clamped to [0, H] / [0, W] (stride 1:
+ * image_hw holds the feature extents themselves).  The kernel choice (frr_roi_variant) does not depend on image_hw.
+ * frr_roi_pool_bwd needs no extent: it follows argmax, so the padding region of grad_in comes out zero. */
 int frr_roi_pool_fwd(const float* feat, const float* rois, int K, int B, int C, int H, int W, int PH, int PW,
-                     float spatial_scale, int channels_last, float* out, int32_t* argmax, frr_stream_t stream);
-/* Mixed-size batches (see frr_rpn_decode_sized), features padded to H x W cells.  frr_rois5_sized scales image b's rois
- * by its own grid (fw_b, fh_b) (models/model.py:104-110) and masks the rows of an image with an empty grid.
- * frr_roi_pool_fwd_sized clips every bin window of a roi of image b to [0, fh_b) x [0, fw_b) instead of the padded map,
- * as torchvision does on that image alone: a roi clamped to the image edge has round(x2 * fw_b) == fw_b and loses its
- * last window column there, while the padded map holds padding values in that column.  argmax stays h * W + w, an index
- * into the padded plane, and never points at padding.  fh_b = image_hw[b,0] / stride and fw_b = image_hw[b,1] / stride,
- * clamped to [0, H] / [0, W] (stride 1: image_hw holds the feature extents themselves).  Same kernel choice as
- * frr_roi_pool_fwd (frr_roi_variant).  frr_roi_pool_bwd needs no extent: it follows argmax, so the padding region of
- * grad_in comes out zero. */
-int frr_rois5_sized(const float* rois, const int32_t* count, int B, int R, const int32_t* image_hw /* [B,2] device */,
-                    int stride, int grid_h, int grid_w, float* rois5, frr_stream_t stream);
-int frr_roi_pool_fwd_sized(const float* feat, const float* rois, int K, int B, int C, int H, int W, int PH, int PW,
-                           float spatial_scale, int channels_last, const int32_t* image_hw /* [B,2] device */, int stride,
-                           float* out, int32_t* argmax, frr_stream_t stream);
+                     float spatial_scale, int channels_last, const int32_t* image_hw /* [B,2] device, or NULL */,
+                     int stride, float* out, int32_t* argmax, frr_stream_t stream);
 /* grad_in [B,C,H,W] (same memory format as feat) is fully written (no pre-zeroing needed).  Rois of at least 6 feature
  * pixels per side are accumulated in shared memory in a fixed order (bit-reproducible); smaller rois, and every roi on maps
  * whose 8 planes do not fit twice per SM, are added with global fp32 atomics (same sums, order not fixed).  argmax must be
@@ -243,8 +223,8 @@ int frr_roi_align_bwd(const float* grad_out, const float* rois, int K, int B, in
                       frr_stream_t stream);
 
 /* Deterministic backward, bit-exact with torchvision's CPU kernels (torchvision::_roi_pool_backward /
- * _roi_align_backward on CPU): the same arguments as frr_roi_pool_bwd / frr_roi_align_bwd, for callers that need the
- * same gradient bits on every run (torch.use_deterministic_algorithms).
+ * _roi_align_backward on CPU): the arguments of frr_roi_pool_bwd (plus image_hw, stride) / frr_roi_align_bwd, for callers
+ * that need the same gradient bits on every run (torch.use_deterministic_algorithms).
  * grad_in[b,c,p] is the fp32 sum, starting at +0.0, of the following terms, added in this order.  Only rois with
  * 0 <= (int)rois[k,0] < B count, taken in ascending k.
  *  - RoIPool: for each k, then ph, then pw (row-major): grad_out[k,c,ph,pw] if argmax[k,c,ph,pw] == p and p lies inside
@@ -258,15 +238,12 @@ int frr_roi_align_bwd(const float* grad_out, const float* rois, int K, int B, in
  * runs; no atomic touches a value.  NaN / Inf in grad_out reach the same elements as in the CPU loop.  grad_in is fully
  * written (no pre-zeroing needed), NCHW or channels_last like the entry points above.  grad_out / argmax must be
  * 4-byte aligned; PH and PW up to about 70 (a one-channel ring of four rois must fit shared memory). */
+/* image_hw set (mixed-size batch): "p lies inside that bin's clipped window" uses image b's extent, exactly as
+ * frr_roi_pool_fwd clips with the same image_hw and stride; the padding region of grad_in is written as +0.0. */
 int frr_roi_pool_bwd_deterministic(const float* grad_out, const int32_t* argmax, const float* rois, int K, int B, int C,
-                                   int H, int W, int PH, int PW, float spatial_scale, int channels_last, float* grad_in,
+                                   int H, int W, int PH, int PW, float spatial_scale, int channels_last,
+                                   const int32_t* image_hw /* [B,2] device, or NULL */, int stride, float* grad_in,
                                    frr_stream_t stream);
-/* The same for a mixed-size batch: "p lies inside that bin's clipped window" uses image b's extent, exactly as
- * frr_roi_pool_fwd_sized clips (image_hw, stride as there); the padding region of grad_in is written as +0.0. */
-int frr_roi_pool_bwd_deterministic_sized(const float* grad_out, const int32_t* argmax, const float* rois, int K, int B,
-                                         int C, int H, int W, int PH, int PW, float spatial_scale, int channels_last,
-                                         const int32_t* image_hw /* [B,2] device */, int stride, float* grad_in,
-                                         frr_stream_t stream);
 int frr_roi_align_bwd_deterministic(const float* grad_out, const float* rois, int K, int B, int C, int H, int W, int PH,
                                     int PW, float spatial_scale, int sampling_ratio, int aligned, int channels_last,
                                     float* grad_in, frr_stream_t stream);
@@ -305,30 +282,23 @@ int frr_roi_variant(int op, int K, int B, int C, int H, int W, int PH, int PW, i
  *     (0, 0, 1) is RPNTargetMaker of the FPN variant, models/new_model.py:299-349 (box_iou without eps,
  *     util/box_ops.py:24-37; no inside-image filter; every anchor tied at a GT's best IoU becomes positive, :316-318).
  * ------------------------------------------------------------------------------------- */
+/* image_hw set: a mixed-size batch (see frr_rpn_decode_sized) padded to img_h x img_w pixels, anchors generated: image
+ * b's anchors are divided by its own (W_b, H_b) and the inside-image test is its own; its padding cells behave like
+ * anchors outside the image (label8 -2, then label -1 and a zero target).  pos_list / neg_list hold padded indices in
+ * the same order as the image's own lists, and counts are the image's own, so the host randperm path and
+ * frr_sample_targets draw the same numbers as for the image alone.  iou_max / argmax / label8 / lists / labels / reg
+ * are [B,N] of the padded N.  Pass the same image_hw to both calls. */
 int frr_rpn_targets_assign(const float* gt, const int32_t* gt_count, int B, int Gmax, const float* anchors,
-                           const float* base_table_host, int A, int img_h, int img_w, int stride, int N,
+                           const float* base_table_host, int A, int img_h, int img_w,
+                           const int32_t* image_hw /* [B,2] device, or NULL */, int stride, int N,
                            float neg_thr, float pos_thr, float iou_eps, int inside_only, int tie_inclusive,
                            float* iou_max, int32_t* argmax, int8_t* label8,
                            int32_t* pos_list, int32_t* neg_list, int32_t* counts, frr_stream_t stream);
 int frr_rpn_targets_finalize(const float* gt, int B, int Gmax, const float* anchors, const float* base_table_host,
-                             int A, int img_h, int img_w, int stride, int N, const int32_t* argmax, int8_t* label8,
-                             const int32_t* pos_list, const int32_t* neg_list, const int32_t* disable,
-                             const int32_t* disable_off, int64_t* labels, float* reg, frr_stream_t stream);
-/* The same for a mixed-size batch padded to grid_h x grid_w cells (see frr_rpn_decode_sized), anchors generated: image b's
- * anchors are divided by its own (W_b, H_b) and the inside-image test is its own; its padding cells behave like anchors
- * outside the image (label8 -2, then label -1 and a zero target).  pos_list / neg_list hold padded indices in the same
- * order as the image's own lists, and counts are the image's own, so the host randperm path and frr_sample_targets draw
- * the same numbers as for the image alone.  iou_max / argmax / label8 / lists / labels / reg are [B,N] of the padded N. */
-int frr_rpn_targets_assign_sized(const float* gt, const int32_t* gt_count, int B, int Gmax, const float* base_table_host,
-                                 int A, const int32_t* image_hw /* [B,2] device */, int grid_h, int grid_w, int stride, int N,
-                                 float neg_thr, float pos_thr, float iou_eps, int inside_only, int tie_inclusive,
-                                 float* iou_max, int32_t* argmax, int8_t* label8, int32_t* pos_list, int32_t* neg_list,
-                                 int32_t* counts, frr_stream_t stream);
-int frr_rpn_targets_finalize_sized(const float* gt, int B, int Gmax, const float* base_table_host, int A,
-                                   const int32_t* image_hw /* [B,2] device */, int grid_h, int grid_w, int stride, int N,
-                                   const int32_t* argmax, int8_t* label8, const int32_t* pos_list, const int32_t* neg_list,
-                                   const int32_t* disable, const int32_t* disable_off, int64_t* labels, float* reg,
-                                   frr_stream_t stream);
+                             int A, int img_h, int img_w, const int32_t* image_hw /* [B,2] device, or NULL */, int stride,
+                             int N, const int32_t* argmax, int8_t* label8, const int32_t* pos_list,
+                             const int32_t* neg_list, const int32_t* disable, const int32_t* disable_off, int64_t* labels,
+                             float* reg, frr_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------
  * T3  Fast R-CNN target maker -- FastRcnnTargetMaker.forward, models/model.py:127-179.
@@ -418,7 +388,7 @@ int frr_pack_detections(const float* det_boxes /* [B,cap,4] */, const int32_t* d
  * Only the rows frr_class_nms kept are ranked: leave its cap at R*(C-1) for a complete ranking.
  * min(max_det, cap) <= 16384, and the top-k's shared-memory limit on cap applies (cap <= 65536 always fits).
  * Workspace from frr_pack_detections_ranked_workspace_bytes, 256-byte aligned.  Three launches: eligibility mask,
- * the top-k of frr_topk_desc over the masked scores, gather into the packed rows. */
+ * the top-k of frr_topk_desc_opt over the masked scores, gather into the packed rows. */
 size_t frr_pack_detections_ranked_workspace_bytes(int B, int cap, int max_det);
 int frr_pack_detections_ranked(const float* det_boxes /* [B,cap,4] */, const int32_t* det_labels /* [B,cap] */,
                                const float* det_scores /* [B,cap] */, const int32_t* det_count /* [B] */, int B,

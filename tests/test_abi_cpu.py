@@ -1,6 +1,7 @@
 """CPU-side checks of the drop-in boundary: libfrr.so loads without a GPU and exports exactly the
 entry points include/frr.h declares; the product refuses CPU tensors (no fallback)."""
 import ctypes
+import re
 import subprocess
 
 import numpy as np
@@ -10,7 +11,7 @@ import torch
 from faster_rcnn_pytorch_b200 import _lib, ops
 
 
-def test_library_builds_loads_and_exports_every_declared_symbol_at_abi_version_2():
+def test_library_builds_loads_and_exports_every_declared_symbol_at_abi_version_3():
     from faster_rcnn_pytorch_b200 import build
     build.build()
     lib = _lib.load()
@@ -20,7 +21,37 @@ def test_library_builds_loads_and_exports_every_declared_symbol_at_abi_version_2
         assert hasattr(lib, n), n
         assert n in _lib.SIGNATURES, f"{n} declared in frr.h but not bound in _lib.SIGNATURES"
     assert set(_lib.SIGNATURES) == set(names)
-    assert lib.frr_abi_version() == 2
+    assert lib.frr_abi_version() == 3
+
+
+_CTYPES = {"int": ctypes.c_int, "float": ctypes.c_float, "double": ctypes.c_double, "size_t": ctypes.c_size_t,
+           "uint64_t": ctypes.c_uint64}
+
+
+def _ctype(decl: str):
+    """ctypes type of a C parameter or return type as frr.h spells it (a trailing parameter name is ignored)."""
+    decl = decl.strip()
+    if decl.startswith("const char*"):
+        return ctypes.c_char_p
+    if "*" in decl or decl.split()[0] == "frr_stream_t":
+        return ctypes.c_void_p
+    return _CTYPES[decl.split()[0]]
+
+
+def test_signatures_match_the_header_prototypes():
+    """Every prototype of include/frr.h against its _lib.SIGNATURES row: the restype and each argtype, in order."""
+    with open(_lib.HEADER) as fh:
+        text = fh.read()
+    text = re.sub(r"/\*.*?\*/", "", text, flags=re.S)
+    text = re.sub(r"^\s*#.*$", "", text, flags=re.M)
+    protos = re.findall(r"([A-Za-z_][\w ]*\**)\s*\b(frr_\w+)\s*\(([^)]*)\)\s*;", text)
+    assert sorted(name for _, name, _ in protos) == _lib.declared_symbols()
+    for ret, name, params in protos:
+        params = params.strip()
+        want = [] if params in ("", "void") else [_ctype(p) for p in params.split(",")]
+        restype, argtypes = _lib.SIGNATURES[name]
+        assert restype is _ctype(ret), f"{name}: restype {restype} vs {ret!r}"
+        assert list(argtypes) == want, f"{name}: argtypes {argtypes} vs ({params})"
 
 
 def test_library_reads_no_environment_variables():
@@ -32,10 +63,10 @@ def test_library_reads_no_environment_variables():
 
 
 @pytest.mark.parametrize("tune", [(128, 0, 0, 0), (0, 4096, 0, 0), (0, 0, 3, 0), (0, 0, 0, 64), (0, 0, -2, 0)])
-def test_nms_tuning_settings_are_range_checked(tune):
+def test_nms_sorted_settings_are_range_checked(tune):
     lib = _lib.load()
-    rc = lib.frr_nms_sorted_tuned(None, None, 1, 0, 0.7, 0, None, None, None, 0, 0, *tune, 1, None)
-    assert rc == -1 and b"frr_nms_sorted_tuned" in lib.frr_last_error()
+    rc = lib.frr_nms_sorted(None, None, 1, 0, 0.7, 0, None, None, None, 0, 0, *tune, 1, None)
+    assert rc == -1 and b"frr_nms_sorted" in lib.frr_last_error()
 
 
 def test_anchor_base_host_matches_oracle(oracle):

@@ -70,7 +70,7 @@ def test_headline_config1_every_image_eager_and_graph(oracle):
 
 def test_proposal_pipeline_batches_in_flight(oracle):
     """region.ProposalPipeline (the bench's throughput mode): four batches in flight on four streams, NMS with one CTA per
-    image (frr_rpn_proposals_opt, nms_cluster_size = 1), graph replays.  Every image of every batch against the oracle,
+    image (frr_rpn_proposals with nms_cluster_size = 1), graph replays.  Every image of every batch against the oracle,
     and bit-equal to the single-plan / automatic-cluster result."""
     B, n = 64, synth.num_anchors(HW)
     v = ops.nms_variant(B, 12000, 0.7, 2000, cluster_size=1, unit_boxes=True)

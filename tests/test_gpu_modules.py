@@ -47,7 +47,7 @@ def test_nms_drop_in_unsorted_input(oracle, key):
 
 
 def test_nms_drop_in_more_boxes_than_the_reference_path(oracle):
-    """torchvision.ops.nms has no size limit: 20 000 boxes (beyond frr_topk_desc's 16 384) still give the CPU kernel's list."""
+    """torchvision.ops.nms has no size limit: 20 000 boxes (beyond frr_topk_desc_opt's 16 384) still give the CPU kernel's list."""
     b, s = synth.random_boxes(123, 20000, cluster=False)
     b = (b * np.float32(0.2) + np.float32(0.4) * np.random.RandomState(3).uniform(size=(20000, 1)).astype(np.float32)).astype(np.float32)
     keep = modules.nms(dev(b), dev(s), 0.5)

@@ -310,7 +310,7 @@ def pool_fwd_abi(feat, rois, osz, scale, want_argmax):
     K = rois.shape[0]
     out = torch.full((K, C) + tuple(osz), float("nan"), device=DEV)
     arg = torch.full((K, C) + tuple(osz), -7, dtype=torch.int32, device=DEV) if want_argmax else None
-    _lib.check(lib.frr_roi_pool_fwd(f.data_ptr(), rois.data_ptr(), K, B, C, H, W, osz[0], osz[1], float(scale), cl,
+    _lib.check(lib.frr_roi_pool_fwd(f.data_ptr(), rois.data_ptr(), K, B, C, H, W, osz[0], osz[1], float(scale), cl, None, 0,
                                     out.data_ptr(), arg.data_ptr() if want_argmax else None, ops._stream()),
                "frr_roi_pool_fwd")
     return out.cpu().numpy(), (arg.cpu().numpy() if want_argmax else None)
@@ -327,7 +327,7 @@ ALIGN_RUNS = [(c, sr, al, cl) for c in ALIGN_CASES for sr in c[7] for al in (Fal
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("case,channels_last", POOL_RUNS, ids=[f"{c[0]}-{'nhwc' if cl else 'nchw'}" for c, cl in POOL_RUNS])
-def test_roi_pool_variant(oracle, case, channels_last):
+def test_roi_pool_variant_uniform(oracle, case, channels_last):
     name, B, C, H, W, K, osz, scale, want_fwd, want_bwd, _ = case
     assert pool_picks(case) == (want_fwd, want_bwd)
     feat = make_feat(seed_of(name) + 900, B, C, H, W, specials=True)

@@ -1,4 +1,4 @@
-"""Developer tool: bucketed NMS with ONE CTA per image (the throughput geometry) over the per-call settings of frr_nms_sorted_tuned."""
+"""Developer tool: bucketed NMS with ONE CTA per image (the throughput geometry) over the per-call settings of frr_nms_sorted."""
 import sys, os, json
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch

@@ -23,14 +23,34 @@ def _ptr(t):
     return 0 if t is None else t.data_ptr()
 
 
-def _req(t: torch.Tensor, name: str, dtype=torch.float32):
+def _check(t: torch.Tensor, name: str, dtype=torch.float32, shape=None, device=None, contiguous: bool = False):
+    """The contract of a tensor handed to libfrr as a bare pointer: a CUDA tensor of ``dtype``, on ``device`` (the launch
+    device) and of ``shape`` (a tuple of ints, None = any size in that dimension) when given, and already contiguous when
+    ``contiguous`` is set (where a copy would be wrong: a tensor written in place, whose copy would not reach the caller,
+    or the input of a plan that allocates nothing).  Returns ``t``; raises TypeError for a non-tensor, ValueError for any
+    other mismatch."""
     if not isinstance(t, torch.Tensor):
         raise TypeError(f"{name} must be a torch.Tensor")
-    if not t.is_cuda:
-        raise ValueError(f"{name} must be a CUDA tensor: the region stage has no CPU path")
+    if device is None or t.device != device:              # on the CUDA ``device``: CUDA needs no test of its own
+        if not t.is_cuda:
+            raise ValueError(f"{name} must be a CUDA tensor: the region stage has no CPU path")
+        if device is not None:
+            raise ValueError(f"{name} must be on {device}, the device of the launch, got {t.device}")
     if t.dtype != dtype:
         raise ValueError(f"{name} must be {dtype}, got {t.dtype}")
-    return t.contiguous()
+    if shape is not None:
+        s = t.shape                                       # a full tuple matches in one comparison
+        if s != shape and (len(s) != len(shape) or [d for d, w in zip(s, shape) if w is not None and d != w]):
+            want = ",".join("*" if w is None else str(w) for w in shape)
+            raise ValueError(f"{name} must be [{want}], got {list(s)}")
+    if contiguous and not t.is_contiguous():
+        raise ValueError(f"{name} must be contiguous")
+    return t
+
+
+def _req(t: torch.Tensor, name: str, dtype=torch.float32, shape=None, device=None):
+    """An input a kernel reads: ``t`` checked by ``_check`` and made contiguous."""
+    return _check(t, name, dtype, shape, device).contiguous()
 
 
 def anchor_base_table(base_size: int = 16) -> np.ndarray:
@@ -103,12 +123,10 @@ def sized_hw(image_hw, B: int, grid_hw, stride: int, device) -> torch.Tensor:
     image's grid must fit ``grid_hw``, else ValueError, and they are copied to ``device``."""
     gh, gw = int(grid_hw[0]), int(grid_hw[1])
     if isinstance(image_hw, torch.Tensor) and image_hw.is_cuda:
-        if image_hw.dtype != torch.int32 or tuple(image_hw.shape) != (B, 2):
-            raise ValueError(f"image_hw must be an int32 [{B},2] tensor of (H, W) per image")
         dev = torch.device(device)
-        if dev.type != "cuda" or (dev.index is not None and image_hw.device.index != dev.index):
-            raise ValueError("image_hw must be on the device of the batch")
-        return image_hw.contiguous()
+        if dev.index is None:                  # "cuda": the current device, where torch allocates for it
+            dev = torch.device(dev.type, torch.cuda.current_device())
+        return _req(image_hw, "image_hw", torch.int32, (B, 2), dev)
     hw = np.asarray(image_hw.numpy() if isinstance(image_hw, torch.Tensor) else image_hw, dtype=np.int64)
     if hw.shape != (B, 2):
         raise ValueError(f"image_hw must be [{B},2] (H, W) per image, got shape {hw.shape}")
@@ -126,40 +144,34 @@ def rpn_decode(reg, cls, image_hw=None, anchors=None, stride: int = 16, table=No
     cells, N = grid_h * grid_w * A.  Each image is decoded exactly as alone at its own size; its padding cells get
     box 0, score 0, valid 0."""
     lib = _lib.load()
-    reg = _req(reg, "reg")
-    cls = _req(cls, "cls")
-    if reg.dim() != 3 or reg.shape[-1] != 4:
-        raise ValueError("reg must be [B,N,4]")
-    B, N = reg.shape[0], reg.shape[1]
-    logits = cls.dim() == 3
-    if tuple(cls.shape) != ((B, N, 2) if logits else (B, N)):
-        raise ValueError("cls must be [B,N,2] logits or [B,N] scores")
+    reg = _req(reg, "reg", shape=(None, None, 4))
+    B, N, dev = reg.shape[0], reg.shape[1], reg.device
+    logits = isinstance(cls, torch.Tensor) and cls.dim() == 3
+    cls = _req(cls, "cls", shape=(B, N, 2) if logits else (B, N), device=dev)
     keep, tptr, A = _table_arg(table)
     if is_sized(image_hw):
         if anchors is not None or grid_hw is None:
             raise ValueError("rpn_decode: per-image sizes need grid_hw and generated anchors")
-        hw = sized_hw(image_hw, B, grid_hw, stride, reg.device)
-        with torch.cuda.device(reg.device):
-            boxes = torch.empty((B, N, 4), dtype=torch.float32, device=reg.device)
-            scores = torch.empty((B, N), dtype=torch.float32, device=reg.device)
-            valid = torch.empty((B, N), dtype=torch.uint8, device=reg.device)
+        hw = sized_hw(image_hw, B, grid_hw, stride, dev)
+        with torch.cuda.device(dev):
+            boxes = torch.empty((B, N, 4), dtype=torch.float32, device=dev)
+            scores = torch.empty((B, N), dtype=torch.float32, device=dev)
+            valid = torch.empty((B, N), dtype=torch.uint8, device=dev)
             _lib.check(lib.frr_rpn_decode_sized(reg.data_ptr(), cls.data_ptr(), int(logits), tptr, A, hw.data_ptr(),
                                                 int(grid_hw[0]), int(grid_hw[1]), stride, float(min_size), boxes.data_ptr(),
                                                 scores.data_ptr(), valid.data_ptr(), B, N, _stream()), "frr_rpn_decode_sized")
         return boxes, scores, valid
     if anchors is not None:
-        anchors = _req(anchors, "anchors")
-        if tuple(anchors.shape) != (N, 4):
-            raise ValueError("anchors must be [N,4]")
+        anchors = _req(anchors, "anchors", shape=(N, 4), device=dev)
         H = W = 0
     else:
         if image_hw is None:
             raise ValueError("image_hw is required when anchors are generated in-kernel")
         H, W = int(image_hw[0]), int(image_hw[1])
-    with torch.cuda.device(reg.device):
-        boxes = torch.empty((B, N, 4), dtype=torch.float32, device=reg.device)
-        scores = torch.empty((B, N), dtype=torch.float32, device=reg.device)
-        valid = torch.empty((B, N), dtype=torch.uint8, device=reg.device)
+    with torch.cuda.device(dev):
+        boxes = torch.empty((B, N, 4), dtype=torch.float32, device=dev)
+        scores = torch.empty((B, N), dtype=torch.float32, device=dev)
+        valid = torch.empty((B, N), dtype=torch.uint8, device=dev)
         _lib.check(lib.frr_rpn_decode(reg.data_ptr(), cls.data_ptr(), int(logits), _ptr(anchors), tptr, A, H, W, stride,
                                       float(min_size), boxes.data_ptr(), scores.data_ptr(), valid.data_ptr(), B, N,
                                       _stream()), "frr_rpn_decode")
@@ -170,15 +182,12 @@ def topk_desc(scores, k: int, valid=None, boxes=None, want_cidx: bool = False, c
     """P4.  scores [B,N] -> dict(scores [B,k], idx int32 [B,k], cidx, boxes [B,k,4], count int32 [B]).
     ``ctas_per_image``: 0 = automatic (a 2-CTA cluster per image for small batches), 1 = one CTA per image."""
     lib = _lib.load()
-    scores = _req(scores, "scores")
-    if scores.dim() != 2:
-        raise ValueError("scores must be [B,N]")
-    B, N = scores.shape
+    scores = _req(scores, "scores", shape=(None, None))
+    (B, N), dev = scores.shape, scores.device
     if valid is not None:
-        valid = _req(valid, "valid", torch.uint8)
+        valid = _req(valid, "valid", torch.uint8, (B, N), dev)
     if boxes is not None:
-        boxes = _req(boxes, "boxes")
-    dev = scores.device
+        boxes = _req(boxes, "boxes", shape=(B, N, 4), device=dev)
     with torch.cuda.device(dev):
         o_s = torch.empty((B, k), dtype=torch.float32, device=dev)
         o_i = torch.empty((B, k), dtype=torch.int32, device=dev)
@@ -199,14 +208,11 @@ def nms_sorted(boxes, iou_threshold: float, max_keep: int | None = None, counts=
     (enables a cheaper, result-identical screening test).  ``first_chunk``, ``max_chunk``, ``lanes_screen``,
     ``lanes_pairs``: settings of the bucketed variant, 0 = automatic; results do not depend on them."""
     lib = _lib.load()
-    boxes = _req(boxes, "boxes")
-    if boxes.dim() != 3 or boxes.shape[-1] != 4:
-        raise ValueError("boxes must be [B,n,4]")
-    B, n = boxes.shape[0], boxes.shape[1]
+    boxes = _req(boxes, "boxes", shape=(None, None, 4))
+    B, n, dev = boxes.shape[0], boxes.shape[1], boxes.device
     mk = n if max_keep is None else int(max_keep)
     if counts is not None:
-        counts = _req(counts, "counts", torch.int32)
-    dev = boxes.device
+        counts = _req(counts, "counts", torch.int32, (B,), dev)
     with torch.cuda.device(dev):
         keep = torch.empty((B, mk), dtype=torch.int32, device=dev)
         cnt = torch.empty((B,), dtype=torch.int32, device=dev)
@@ -259,11 +265,11 @@ def roi_variant(op: str, K: int, B: int, C: int, H: int, W: int, output_size=(7,
 # ------------------------------------------------------------------------------------------------
 # RoIPool / RoIAlign (R1-R4): raw kernels + autograd functions
 # ------------------------------------------------------------------------------------------------
-def _feat_layout(feat: torch.Tensor):
-    """Returns (tensor usable in place, channels_last flag).  NCHW-contiguous and channels_last memory are both
-    consumed without a copy; anything else is made NCHW-contiguous."""
-    if feat.dim() != 4:
-        raise ValueError("features must be [B,C,H,W]")
+def _feat_layout(feat: torch.Tensor, name: str = "features", shape=(None, None, None, None), device=None):
+    """Checks a CUDA fp32 [B,C,H,W] map (of ``shape``, on ``device``: see ``_check``) and returns (tensor usable in place,
+    channels_last flag).  NCHW-contiguous and channels_last memory are both consumed without a copy; anything else is
+    made NCHW-contiguous."""
+    _check(feat, name, torch.float32, shape, device)
     if feat.is_contiguous():
         return feat, 0
     if feat.is_contiguous(memory_format=torch.channels_last):
@@ -290,16 +296,16 @@ def rois5(rois, count, feat_hw, out=None, image_hw=None, stride: int = 16):
     ``image_hw`` [B,2] (mixed-size batch, ``feat_hw`` = the padded grid): image b is scaled by its own grid
     (W_b // stride, H_b // stride)."""
     lib = _lib.load()
-    rois = _req(rois, "rois")
-    if rois.dim() != 3 or rois.shape[-1] != 4:
-        raise ValueError("rois must be [B,R,4]")
-    B, R = rois.shape[0], rois.shape[1]
+    rois = _req(rois, "rois", shape=(None, None, 4))
+    B, R, dev = rois.shape[0], rois.shape[1], rois.device
     if count is not None:
-        count = _req(count, "count", torch.int32)
-    with torch.cuda.device(rois.device):
+        count = _req(count, "count", torch.int32, (B,), dev)
+    if out is not None:
+        _check(out, "out", shape=(B * R, 5), device=dev, contiguous=True)
+    with torch.cuda.device(dev):
         if out is None:
-            out = torch.empty((B * R, 5), dtype=torch.float32, device=rois.device)
-        hw = None if image_hw is None else sized_hw(image_hw, B, feat_hw, stride, rois.device)
+            out = torch.empty((B * R, 5), dtype=torch.float32, device=dev)
+        hw = None if image_hw is None else sized_hw(image_hw, B, feat_hw, stride, dev)
         _lib.check(lib.frr_rois5(rois.data_ptr(), _ptr(count), B, R, int(feat_hw[0]), int(feat_hw[1]), _ptr(hw), int(stride),
                                  out.data_ptr(), _stream()), "frr_rois5")
     return out
@@ -310,18 +316,15 @@ def roi_pool_forward(feat, rois5, output_size=(7, 7), spatial_scale: float = 1.0
     """``image_hw`` [B,2] (mixed-size batch padded to the map's H x W cells): every bin window of a roi of image b is
     clipped to that image's own grid (H_b // stride, W_b // stride) -- stride 1 when ``image_hw`` holds feature extents."""
     lib = _lib.load()
-    feat = _req(feat, "features") if feat.is_contiguous() else feat
-    if not feat.is_cuda or feat.dtype != torch.float32:
-        raise ValueError("features must be a CUDA fp32 tensor: the region stage has no CPU path")
     feat, cl = _feat_layout(feat)
-    rois5 = _req(rois5, "rois")
-    B, C, H, W = feat.shape
+    (B, C, H, W), dev = feat.shape, feat.device
+    rois5 = _req(rois5, "rois", shape=(None, 5), device=dev)
     K = rois5.shape[0]
     PH, PW = int(output_size[0]), int(output_size[1])
-    with torch.cuda.device(feat.device):
-        out = torch.empty((K, C, PH, PW), dtype=torch.float32, device=feat.device)
-        arg = torch.empty((K, C, PH, PW), dtype=torch.int32, device=feat.device) if want_argmax else None
-        hw = None if image_hw is None else sized_hw(image_hw, B, (H, W), stride, feat.device)
+    with torch.cuda.device(dev):
+        out = torch.empty((K, C, PH, PW), dtype=torch.float32, device=dev)
+        arg = torch.empty((K, C, PH, PW), dtype=torch.int32, device=dev) if want_argmax else None
+        hw = None if image_hw is None else sized_hw(image_hw, B, (H, W), stride, dev)
         _lib.check(lib.frr_roi_pool_fwd(feat.data_ptr(), rois5.data_ptr(), K, B, C, H, W, PH, PW, float(spatial_scale), cl,
                                         _ptr(hw), int(stride), out.data_ptr(), _ptr(arg), _stream()), "frr_roi_pool_fwd")
     return out, arg
@@ -339,18 +342,19 @@ def roi_pool_backward(grad_out, argmax, rois5, feat_shape, spatial_scale: float 
     clips each bin window to the image's own grid.  The padding region of the gradient is zero either way."""
     lib = _lib.load()
     det = _deterministic(deterministic)
-    grad_out = _req(grad_out, "grad_out")
-    argmax = _req(argmax, "argmax", torch.int32)
-    rois5 = _req(rois5, "rois")
     B, C, H, W = feat_shape
-    K, _, PH, PW = grad_out.shape
-    with torch.cuda.device(grad_out.device):
-        gin = torch.empty((B, C, H, W), dtype=torch.float32, device=grad_out.device,
+    rois5 = _req(rois5, "rois", shape=(None, 5))
+    K, dev = rois5.shape[0], rois5.device
+    grad_out = _req(grad_out, "grad_out", shape=(K, C, None, None), device=dev)
+    PH, PW = grad_out.shape[2], grad_out.shape[3]
+    argmax = _req(argmax, "argmax", torch.int32, (K, C, PH, PW), dev)
+    with torch.cuda.device(dev):
+        gin = torch.empty((B, C, H, W), dtype=torch.float32, device=dev,
                           memory_format=torch.channels_last if channels_last else torch.contiguous_format)
         args = (grad_out.data_ptr(), argmax.data_ptr(), rois5.data_ptr(), K, B, C, H, W, PH, PW, float(spatial_scale),
                 int(channels_last))
         if det:
-            hw = None if image_hw is None else sized_hw(image_hw, B, (H, W), stride, grad_out.device)
+            hw = None if image_hw is None else sized_hw(image_hw, B, (H, W), stride, dev)
             _lib.check(lib.frr_roi_pool_bwd_deterministic(*args, _ptr(hw), int(stride), gin.data_ptr(), _stream()),
                        "frr_roi_pool_bwd_deterministic")
         else:
@@ -362,18 +366,16 @@ def roi_align_forward(feat, rois5, output_size=(7, 7), spatial_scale: float = 1.
                       aligned: bool = False, out=None):
     """``out``: write into an existing [K,C,PH,PW] tensor (rows of rois with a negative batch index are left untouched)."""
     lib = _lib.load()
-    if not feat.is_cuda or feat.dtype != torch.float32:
-        raise ValueError("features must be a CUDA fp32 tensor: the region stage has no CPU path")
     feat, cl = _feat_layout(feat)
-    rois5 = _req(rois5, "rois")
-    B, C, H, W = feat.shape
+    (B, C, H, W), dev = feat.shape, feat.device
+    rois5 = _req(rois5, "rois", shape=(None, 5), device=dev)
     K = rois5.shape[0]
     PH, PW = int(output_size[0]), int(output_size[1])
-    with torch.cuda.device(feat.device):
+    if out is not None:
+        _check(out, "out", shape=(K, C, PH, PW), device=dev, contiguous=True)
+    with torch.cuda.device(dev):
         if out is None:
-            out = torch.empty((K, C, PH, PW), dtype=torch.float32, device=feat.device)
-        elif tuple(out.shape) != (K, C, PH, PW) or not out.is_contiguous() or out.dtype != torch.float32:
-            raise ValueError("roi_align_forward: out must be a contiguous fp32 [K,C,PH,PW] tensor")
+            out = torch.empty((K, C, PH, PW), dtype=torch.float32, device=dev)
         _lib.check(lib.frr_roi_align_fwd(feat.data_ptr(), rois5.data_ptr(), K, B, C, H, W, PH, PW, float(spatial_scale),
                                          int(sampling_ratio), int(aligned), cl, out.data_ptr(), _stream()),
                    "frr_roi_align_fwd")
@@ -385,12 +387,13 @@ def roi_align_backward(grad_out, rois5, feat_shape, spatial_scale: float = 1.0, 
     """``deterministic``: as for ``roi_pool_backward``."""
     lib = _lib.load()
     fn = lib.frr_roi_align_bwd_deterministic if _deterministic(deterministic) else lib.frr_roi_align_bwd
-    grad_out = _req(grad_out, "grad_out")
-    rois5 = _req(rois5, "rois")
     B, C, H, W = feat_shape
-    K, _, PH, PW = grad_out.shape
-    with torch.cuda.device(grad_out.device):
-        gin = torch.empty((B, C, H, W), dtype=torch.float32, device=grad_out.device,
+    rois5 = _req(rois5, "rois", shape=(None, 5))
+    K, dev = rois5.shape[0], rois5.device
+    grad_out = _req(grad_out, "grad_out", shape=(K, C, None, None), device=dev)
+    PH, PW = grad_out.shape[2], grad_out.shape[3]
+    with torch.cuda.device(dev):
+        gin = torch.empty((B, C, H, W), dtype=torch.float32, device=dev,
                           memory_format=torch.channels_last if channels_last else torch.contiguous_format)
         _lib.check(fn(grad_out.data_ptr(), rois5.data_ptr(), K, B, C, H, W, PH, PW, float(spatial_scale),
                       int(sampling_ratio), int(aligned), int(channels_last), gin.data_ptr(), _stream()), fn.__name__)
@@ -470,27 +473,24 @@ def rpn_targets_assign(gt, gt_count, N, image_hw=None, anchors=None, stride=16, 
     test are its own, its padding cells are labelled like anchors outside the image."""
     lib = _lib.load()
     eps, inside_only, tie_inclusive = VARIANTS[variant]
-    gt = _req(gt, "gt")
-    if gt.dim() != 3 or gt.shape[-1] != 4:
-        raise ValueError("gt must be [B,Gmax,4]")
-    B, G = gt.shape[0], gt.shape[1]
+    gt = _req(gt, "gt", shape=(None, None, 4))
+    B, G, dev = gt.shape[0], gt.shape[1], gt.device
     if G == 0:
         raise IndexError("max(): Expected reduction dim 1 to have non-zero size")   # models/model.py:199
     if gt_count is not None:
-        gt_count = _req(gt_count, "gt_count", torch.int32)
+        gt_count = _req(gt_count, "gt_count", torch.int32, (B,), dev)
     keep, tptr, A = _table_arg(table)
     hw = None
     if is_sized(image_hw):
         if anchors is not None or grid_hw is None:
             raise ValueError("rpn_targets_assign: per-image sizes need grid_hw and generated anchors")
-        hw = sized_hw(image_hw, B, grid_hw, stride, gt.device)
+        hw = sized_hw(image_hw, B, grid_hw, stride, dev)
         H, W = int(grid_hw[0]) * stride, int(grid_hw[1]) * stride      # with hw set: the padded size in pixels
     elif anchors is not None:
-        anchors = _req(anchors, "anchors")
+        anchors = _req(anchors, "anchors", shape=(N, 4), device=dev)
         H = W = 0
     else:
         H, W = int(image_hw[0]), int(image_hw[1])
-    dev = gt.device
     with torch.cuda.device(dev):
         ws = dict(iou_max=torch.empty((B, N), dtype=torch.float32, device=dev),
                   argmax=torch.empty((B, N), dtype=torch.int32, device=dev),
@@ -509,36 +509,46 @@ def rpn_targets_assign(gt, gt_count, N, image_hw=None, anchors=None, stride=16, 
 
 def rpn_targets_finalize(ws, disable=None, disable_off=None):
     lib = _lib.load()
-    gt, anchors = ws["gt"], ws["anchors"]
     H, W, stride, table, N = ws["geom"]
     keep, tptr, A = _table_arg(table)
-    B, G = gt.shape[0], gt.shape[1]
-    dev = gt.device
+    gt = _req(ws["gt"], "ws['gt']", shape=(None, None, 4))
+    B, G, dev = gt.shape[0], gt.shape[1], gt.device
+    anchors, hw = ws["anchors"], ws["image_hw"]
+    if anchors is not None:
+        anchors = _req(anchors, "ws['anchors']", shape=(N, 4), device=dev)
+    if hw is not None:
+        hw = _req(hw, "ws['image_hw']", torch.int32, (B, 2), dev)
+    argmax = _req(ws["argmax"], "ws['argmax']", torch.int32, (B, N), dev)
+    label8 = _check(ws["label8"], "ws['label8']", torch.int8, (B, N), dev, contiguous=True)
+    pos_list = _req(ws["pos_list"], "ws['pos_list']", torch.int32, (B, N), dev)
+    neg_list = _req(ws["neg_list"], "ws['neg_list']", torch.int32, (B, N), dev)
+    if disable is not None or disable_off is not None:
+        disable = _req(disable, "disable", torch.int32, (None,), dev)
+        disable_off = _req(disable_off, "disable_off", torch.int32, (3 * B,), dev)
     with torch.cuda.device(dev):
         labels = torch.empty((B, N), dtype=torch.int64, device=dev)
         reg = torch.empty((B, N, 4), dtype=torch.float32, device=dev)
-        rest = (ws["argmax"].data_ptr(), ws["label8"].data_ptr(), ws["pos_list"].data_ptr(), ws["neg_list"].data_ptr(),
-                _ptr(disable), _ptr(disable_off), labels.data_ptr(), reg.data_ptr(), _stream())
-        _lib.check(lib.frr_rpn_targets_finalize(gt.data_ptr(), B, G, _ptr(anchors), tptr, A, H, W, _ptr(ws["image_hw"]),
-                                                stride, N, *rest), "frr_rpn_targets_finalize")
+        rest = (argmax.data_ptr(), label8.data_ptr(), pos_list.data_ptr(), neg_list.data_ptr(), _ptr(disable),
+                _ptr(disable_off), labels.data_ptr(), reg.data_ptr(), _stream())
+        _lib.check(lib.frr_rpn_targets_finalize(gt.data_ptr(), B, G, _ptr(anchors), tptr, A, H, W, _ptr(hw), stride, N,
+                                                *rest), "frr_rpn_targets_finalize")
     return labels, reg
 
 
 def frcnn_targets_assign(rois, roi_count, gt, gt_count, fg_thr=0.5, variant: str = "vgg"):
     lib = _lib.load()
     eps = VARIANTS[variant][0]
-    rois = _req(rois, "rois")
-    gt = _req(gt, "gt")
-    B, R = rois.shape[0], rois.shape[1]
+    rois = _req(rois, "rois", shape=(None, None, 4))
+    B, R, dev = rois.shape[0], rois.shape[1], rois.device
+    gt = _req(gt, "gt", shape=(B, None, 4), device=dev)
     G = gt.shape[1]
     if G == 0:
         raise IndexError("max(): Expected reduction dim 1 to have non-zero size")
     if roi_count is not None:
-        roi_count = _req(roi_count, "roi_count", torch.int32)
+        roi_count = _req(roi_count, "roi_count", torch.int32, (B,), dev)
     if gt_count is not None:
-        gt_count = _req(gt_count, "gt_count", torch.int32)
+        gt_count = _req(gt_count, "gt_count", torch.int32, (B,), dev)
     M = R + G
-    dev = rois.device
     with torch.cuda.device(dev):
         ws = dict(iou_max=torch.empty((B, M), dtype=torch.float32, device=dev),
                   argmax=torch.empty((B, M), dtype=torch.int32, device=dev),
@@ -556,21 +566,29 @@ def frcnn_targets_assign(rois, roi_count, gt, gt_count, fg_thr=0.5, variant: str
 
 def frcnn_targets_finalize(ws, gt_label, sel, sel_n, std=_STD4, label_offset: int = 1):
     lib = _lib.load()
-    rois, gt = ws["rois"], ws["gt"]
-    gt_label = _req(gt_label, "gt_label", torch.int64)
-    sel = _req(sel, "sel", torch.int32)
-    sel_n = _req(sel_n, "sel_n", torch.int32)
-    B, R, G, S = rois.shape[0], rois.shape[1], gt.shape[1], sel.shape[1]
+    rois = _req(ws["rois"], "ws['rois']", shape=(None, None, 4))
+    B, R, dev = rois.shape[0], rois.shape[1], rois.device
+    gt = _req(ws["gt"], "ws['gt']", shape=(B, None, 4), device=dev)
+    G = gt.shape[1]
+    roi_count = ws["roi_count"]
+    if roi_count is not None:
+        roi_count = _req(roi_count, "ws['roi_count']", torch.int32, (B,), dev)
+    argmax = _req(ws["argmax"], "ws['argmax']", torch.int32, (B, R + G), dev)
+    pos_list = _req(ws["pos_list"], "ws['pos_list']", torch.int32, (B, R + G), dev)
+    neg_list = _req(ws["neg_list"], "ws['neg_list']", torch.int32, (B, R + G), dev)
+    gt_label = _req(gt_label, "gt_label", torch.int64, (B, G), dev)
+    sel = _req(sel, "sel", torch.int32, (B, None), dev)
+    S = sel.shape[1]
+    sel_n = _req(sel_n, "sel_n", torch.int32, (B, 2), dev)
     std = np.ascontiguousarray(std, dtype=np.float32)
-    dev = rois.device
     with torch.cuda.device(dev):
         cls = torch.empty((B, S), dtype=torch.int64, device=dev)
         reg = torch.empty((B, S, 4), dtype=torch.float32, device=dev)
         srois = torch.empty((B, S, 4), dtype=torch.float32, device=dev)
         kidx = torch.empty((B, S), dtype=torch.int32, device=dev)
-        _lib.check(lib.frr_frcnn_targets_finalize(rois.data_ptr(), _ptr(ws["roi_count"]), B, R, gt.data_ptr(),
-                                                  gt_label.data_ptr(), G, ws["argmax"].data_ptr(), ws["pos_list"].data_ptr(),
-                                                  ws["neg_list"].data_ptr(), sel.data_ptr(), sel_n.data_ptr(), S,
+        _lib.check(lib.frr_frcnn_targets_finalize(rois.data_ptr(), _ptr(roi_count), B, R, gt.data_ptr(),
+                                                  gt_label.data_ptr(), G, argmax.data_ptr(), pos_list.data_ptr(),
+                                                  neg_list.data_ptr(), sel.data_ptr(), sel_n.data_ptr(), S,
                                                   std.ctypes.data, int(label_offset), cls.data_ptr(), reg.data_ptr(), srois.data_ptr(),
                                                   kidx.data_ptr(), _stream()), "frr_frcnn_targets_finalize")
     return cls, reg, srois, kidx
@@ -585,11 +603,19 @@ def sample_targets(mt_state, ws_rpn=None, ws_frcnn=None, rpn_batch: int = 256, r
     lib = _lib.load()
     if ws_rpn is None and ws_frcnn is None:
         raise ValueError("sample_targets: nothing to sample")
-    ref = ws_rpn if ws_rpn is not None else ws_frcnn
-    dev = ref["counts"].device
-    B = ref["counts"].shape[0]
-    if mt_state.device != dev or mt_state.dtype != torch.int32 or mt_state.numel() != 626:
-        raise ValueError("mt_state must be an int32 [626] tensor on the device of the targets")
+    mt_state = _check(mt_state, "mt_state", torch.int32, (626,), contiguous=True)       # advanced in place
+    dev, B, N = mt_state.device, None, 0
+    rpn_counts = frcnn_counts = label8 = pos_list = neg_list = None
+    if ws_rpn is not None:
+        rpn_counts = _req(ws_rpn["counts"], "ws_rpn['counts']", torch.int32, (None, 2), dev)
+        B = rpn_counts.shape[0]
+        label8 = _check(ws_rpn["label8"], "ws_rpn['label8']", torch.int8, (B, None), dev, contiguous=True)   # edited in place
+        N = label8.shape[1]
+        pos_list = _req(ws_rpn["pos_list"], "ws_rpn['pos_list']", torch.int32, (B, N), dev)
+        neg_list = _req(ws_rpn["neg_list"], "ws_rpn['neg_list']", torch.int32, (B, N), dev)
+    if ws_frcnn is not None:
+        frcnn_counts = _req(ws_frcnn["counts"], "ws_frcnn['counts']", torch.int32, (B, 2), dev)     # the same B
+        B = frcnn_counts.shape[0]
     S = max(rpn_batch if ws_rpn is not None else 0, frcnn_batch if ws_frcnn is not None else 0)
     with torch.cuda.device(dev):
         jobs = torch.empty((B, 4, 4), dtype=torch.int32, device=dev)
@@ -598,15 +624,10 @@ def sample_targets(mt_state, ws_rpn=None, ws_frcnn=None, rpn_batch: int = 256, r
         if ws_frcnn is not None:
             sel = torch.zeros((B, frcnn_batch), dtype=torch.int32, device=dev)
             sel_n = torch.zeros((B, 2), dtype=torch.int32, device=dev)
-        N = ws_rpn["label8"].shape[1] if ws_rpn is not None else 0
-        _lib.check(lib.frr_sample_targets(_ptr(ws_rpn["counts"]) if ws_rpn is not None else None,
-                                          _ptr(ws_frcnn["counts"]) if ws_frcnn is not None else None, B, int(rpn_batch),
-                                          int(rpn_max_pos), int(frcnn_batch), int(frcnn_max_pos), mt_state.data_ptr(), N,
-                                          _ptr(ws_rpn["label8"]) if ws_rpn is not None else None,
-                                          _ptr(ws_rpn["pos_list"]) if ws_rpn is not None else None,
-                                          _ptr(ws_rpn["neg_list"]) if ws_rpn is not None else None, _ptr(sel), _ptr(sel_n),
-                                          int(frcnn_batch), jobs.data_ptr(), draws.data_ptr(), S, _stream()),
-                   "frr_sample_targets")
+        _lib.check(lib.frr_sample_targets(_ptr(rpn_counts), _ptr(frcnn_counts), B, int(rpn_batch), int(rpn_max_pos),
+                                          int(frcnn_batch), int(frcnn_max_pos), mt_state.data_ptr(), N, _ptr(label8),
+                                          _ptr(pos_list), _ptr(neg_list), _ptr(sel), _ptr(sel_n), int(frcnn_batch),
+                                          jobs.data_ptr(), draws.data_ptr(), S, _stream()), "frr_sample_targets")
     return sel, sel_n
 
 
@@ -673,26 +694,25 @@ def region_loss_args(rpn_cls=None, rpn_reg=None, rpn_target_cls=None, rpn_target
     (rpn_cls, rpn_reg, frcnn_cls, frcnn_reg, rpn_target_cls, rpn_target_reg, frcnn_target_cls, frcnn_target_reg)."""
     if rpn_cls is None and frcnn_cls is None:
         raise ValueError("region_loss: nothing to compute")
+    B = dev = None                                        # taken from the RPN half, when given, for both halves
     if rpn_cls is not None:
-        rpn_cls, rpn_reg, rpn_target_reg = _req(rpn_cls, "rpn_cls"), _req(rpn_reg, "rpn_reg"), _req(rpn_target_reg, "rpn_target_reg")
-        rpn_target_cls = _req(rpn_target_cls, "rpn_target_cls", torch.int64)
-        B, N = rpn_cls.shape[0], rpn_cls.shape[1]
-        if tuple(rpn_cls.shape) != (B, N, 2) or tuple(rpn_reg.shape) != (B, N, 4) or tuple(rpn_target_cls.shape) != (B, N) \
-                or tuple(rpn_target_reg.shape) != (B, N, 4):
-            raise ValueError("region_loss: RPN tensors must be [B,N,2], [B,N,4], [B,N], [B,N,4]")
+        rpn_cls = _req(rpn_cls, "rpn_cls", shape=(None, None, 2))
+        B, N, dev = rpn_cls.shape[0], rpn_cls.shape[1], rpn_cls.device
+        rpn_reg = _req(rpn_reg, "rpn_reg", shape=(B, N, 4), device=dev)
+        rpn_target_cls = _req(rpn_target_cls, "rpn_target_cls", torch.int64, (B, N), dev)
+        rpn_target_reg = _req(rpn_target_reg, "rpn_target_reg", shape=(B, N, 4), device=dev)
     if frcnn_cls is not None:
-        frcnn_cls, frcnn_reg = _req(frcnn_cls, "frcnn_cls"), _req(frcnn_reg, "frcnn_reg")
-        frcnn_target_cls = _req(frcnn_target_cls, "frcnn_target_cls", torch.int64)
-        frcnn_target_reg = _req(frcnn_target_reg, "frcnn_target_reg")
-        B, S, C = frcnn_cls.shape
+        frcnn_cls = _req(frcnn_cls, "frcnn_cls", shape=(B, None, None), device=dev)
+        (B, S, C), dev = frcnn_cls.shape, frcnn_cls.device
+        frcnn_reg = _req(frcnn_reg, "frcnn_reg", device=dev)
         if frcnn_reg.numel() == B * S * C * 4:
             frcnn_reg = frcnn_reg.reshape(B, S, C, 4)
         elif frcnn_reg.numel() == B * S * 4:
             frcnn_reg = frcnn_reg.reshape(B, S, 1, 4)
         else:
             raise ValueError("region_loss: frcnn_reg must hold C or 1 rows of 4 per sample")
-        if tuple(frcnn_target_cls.shape) != (B, S) or tuple(frcnn_target_reg.shape) != (B, S, 4):
-            raise ValueError("region_loss: Fast R-CNN targets must be [B,S] and [B,S,4]")
+        frcnn_target_cls = _req(frcnn_target_cls, "frcnn_target_cls", torch.int64, (B, S), dev)
+        frcnn_target_reg = _req(frcnn_target_reg, "frcnn_target_reg", shape=(B, S, 4), device=dev)
     return rpn_cls, rpn_reg, frcnn_cls, frcnn_reg, rpn_target_cls, rpn_target_reg, frcnn_target_cls, frcnn_target_reg
 
 
@@ -713,14 +733,14 @@ def region_loss(rpn_cls=None, rpn_reg=None, rpn_target_cls=None, rpn_target_reg=
 def decode_classwise(cls_logits, reg, rois, num_classes: int, std=_STD4):
     """cls [rows,C], reg [rows,4C], rois [rows,4] -> prob [rows,C], boxes [rows,4C] (clamped to [0,1])."""
     lib = _lib.load()
-    cls_logits = _req(cls_logits, "cls_logits")
-    reg = _req(reg, "reg")
-    rois = _req(rois, "rois")
-    rows, C = cls_logits.shape[0], int(num_classes)
-    if cls_logits.shape[1] != C or reg.numel() != rows * C * 4 or rois.numel() != rows * 4:
-        raise ValueError("decode_classwise: shape mismatch")
+    C = int(num_classes)
+    cls_logits = _req(cls_logits, "cls_logits", shape=(None, C))
+    rows, dev = cls_logits.shape[0], cls_logits.device
+    rois = _req(rois, "rois", shape=(rows, 4), device=dev)
+    reg = _req(reg, "reg", device=dev)
+    if reg.numel() != rows * C * 4:
+        raise ValueError(f"decode_classwise: reg must hold {C} rows of 4 per roi ([rows,{4 * C}] or [rows,{C},4])")
     std = np.ascontiguousarray(std, dtype=np.float32)
-    dev = cls_logits.device
     with torch.cuda.device(dev):
         prob = torch.empty((rows, C), dtype=torch.float32, device=dev)
         boxes = torch.empty((rows, C * 4), dtype=torch.float32, device=dev)
@@ -732,15 +752,15 @@ def decode_classwise(cls_logits, reg, rois, num_classes: int, std=_STD4):
 def class_nms(prob, boxes, num_classes: int, score_thres: float = 0.05, iou_thr: float = 0.3, roi_count=None, cap=None):
     """prob [B,R,C], boxes [B,R,4C] -> det_boxes [B,cap,4], det_labels int32 [B,cap], det_scores [B,cap], count [B]."""
     lib = _lib.load()
-    prob = _req(prob, "prob")
-    boxes = _req(boxes, "boxes")
-    B, R, C = prob.shape[0], prob.shape[1], int(num_classes)
-    if prob.shape[2] != C or boxes.numel() != B * R * C * 4:
-        raise ValueError("class_nms: shape mismatch")
+    C = int(num_classes)
+    prob = _req(prob, "prob", shape=(None, None, C))
+    B, R, dev = prob.shape[0], prob.shape[1], prob.device
+    boxes = _req(boxes, "boxes", device=dev)
+    if boxes.numel() != B * R * C * 4:
+        raise ValueError(f"class_nms: boxes must hold {C} boxes per roi ([B,R,{4 * C}] or [B,R,{C},4])")
     if roi_count is not None:
-        roi_count = _req(roi_count, "roi_count", torch.int32)
+        roi_count = _req(roi_count, "roi_count", torch.int32, (B,), dev)
     cap = R * (C - 1) if cap is None else int(cap)
-    dev = prob.device
     with torch.cuda.device(dev):
         nbytes = int(lib.frr_class_nms_workspace_bytes(B, R, C))
         ws = torch.empty((nbytes + 256,), dtype=torch.uint8, device=dev)
@@ -784,14 +804,15 @@ def pack_detections(det_boxes, det_labels, det_scores, det_count, max_det: int, 
     ``workspace``: from ``pack_ranked_workspace`` (allocated here when None)."""
     check_rank(rank, per_class_max)
     lib = _lib.load()
-    det_boxes = _req(det_boxes, "det_boxes")
-    det_labels = _req(det_labels, "det_labels", torch.int32)
-    det_scores = _req(det_scores, "det_scores")
-    det_count = _req(det_count, "det_count", torch.int32)
+    det_labels = _req(det_labels, "det_labels", torch.int32, (None, None))
+    (B, cap), dev = det_labels.shape, det_labels.device
+    det_boxes = _req(det_boxes, "det_boxes", shape=(B, cap, 4), device=dev)
+    det_scores = _req(det_scores, "det_scores", shape=(B, cap), device=dev)
+    det_count = _req(det_count, "det_count", torch.int32, (B,), dev)
     if image_wh is not None:
-        image_wh = _req(image_wh, "image_wh")
-    B, cap = det_labels.shape
-    dev = det_boxes.device
+        image_wh = _req(image_wh, "image_wh", shape=(B, 2), device=dev)
+    if workspace is not None:
+        workspace = _req(workspace, "workspace", torch.uint8, device=dev)
     with torch.cuda.device(dev):
         out = torch.empty((B, int(max_det), 6), dtype=torch.float32, device=dev)
         cnt = torch.empty((B,), dtype=torch.int32, device=dev)
@@ -802,7 +823,6 @@ def pack_detections(det_boxes, det_labels, det_scores, det_count, max_det: int, 
             return out, cnt
         if workspace is None:
             workspace = pack_ranked_workspace(B, cap, max_det, dev)
-        workspace = _req(workspace, "workspace", torch.uint8)
         off = (-workspace.data_ptr()) % 256
         _lib.check(lib.frr_pack_detections_ranked(det_boxes.data_ptr(), det_labels.data_ptr(), det_scores.data_ptr(),
                                                   det_count.data_ptr(), B, cap, int(max_det), int(per_class_max),
@@ -830,11 +850,11 @@ def infer_scales(features, image_shapes):
 def fpn_level_rois(rois5, k_min: int, k_max: int, canonical_scale: float = 224.0, canonical_level: int = 4):
     """LevelMapper on the device: (levels int32 [K], rois_per_level [L,K,5] with foreign rois masked by batch index -1)."""
     lib = _lib.load()
-    rois5 = _req(rois5, "rois")
-    K, L = rois5.shape[0], k_max - k_min + 1
-    with torch.cuda.device(rois5.device):
-        levels = torch.empty((K,), dtype=torch.int32, device=rois5.device)
-        per = torch.empty((L, K, 5), dtype=torch.float32, device=rois5.device)
+    rois5 = _req(rois5, "rois", shape=(None, 5))
+    K, L, dev = rois5.shape[0], k_max - k_min + 1, rois5.device
+    with torch.cuda.device(dev):
+        levels = torch.empty((K,), dtype=torch.int32, device=dev)
+        per = torch.empty((L, K, 5), dtype=torch.float32, device=dev)
         _lib.check(lib.frr_fpn_level_rois(rois5.data_ptr(), K, int(k_min), int(k_max), int(canonical_level),
                                           float(canonical_scale), L, levels.data_ptr(), per.data_ptr(), _stream()),
                    "frr_fpn_level_rois")
@@ -845,15 +865,17 @@ def multiscale_roi_align_forward(feats, rois5, output_size, sampling_ratio: int,
                                  canonical_scale: float = 224.0, canonical_level: int = 4):
     """The kernels of ``multiscale_roi_align`` for given per-level ``scales`` (see ``infer_scales``): returns (out
     [K,C,PH,PW], levels int32 [K], the per-level rois [L,K,5] the backward reads, channels_last flag per level)."""
-    K, C = rois5.shape[0], feats[0].shape[1]
+    if len(feats) != k_max - k_min + 1:
+        raise ValueError(f"multiscale_roi_align: one feature map per level {k_min}..{k_max}, got {len(feats)} maps")
+    maps = [_feat_layout(feats[0], "features[0]")]
+    C, dev = maps[0][0].shape[1], maps[0][0].device
+    maps += [_feat_layout(f, f"features[{l}]", (None, C, None, None), dev) for l, f in enumerate(feats[1:], 1)]
+    rois5 = _req(rois5, "rois", shape=(None, 5), device=dev)
     levels, per = fpn_level_rois(rois5, k_min, k_max, canonical_scale, canonical_level)
-    out = torch.empty((K, C, output_size[0], output_size[1]), dtype=torch.float32, device=rois5.device)
-    lay = []
-    for l, f in enumerate(feats):
-        f_l, cl = _feat_layout(f)
-        lay.append(bool(cl))
+    out = torch.empty((rois5.shape[0], C, output_size[0], output_size[1]), dtype=torch.float32, device=dev)
+    for l, (f_l, _) in enumerate(maps):
         roi_align_forward(f_l, per[l], output_size, scales[l], sampling_ratio, False, out=out)
-    return out, levels, per, lay
+    return out, levels, per, [bool(cl) for _, cl in maps]
 
 
 def multiscale_roi_align_backward(grad_out, per, shapes, scales, sampling_ratio: int, lay):

@@ -79,10 +79,14 @@ class ProposalPlan:
         self.B, self.N, self.device = int(B), int(N), torch.device(device)
         self.logits, self.stride, self.thr, self.min_size = bool(logits), int(stride), float(nms_thresh), float(min_size)
         self._table, self._tptr, self.A = ops._table_arg(table)
+        with torch.cuda.device(self.device):
+            self.ws_bytes = int(self.lib.frr_rpn_proposals_workspace_bytes(self.B, self.N, self.pre_k, self.post_k))
+            self._ws = torch.empty((self.ws_bytes + 256,), dtype=torch.uint8, device=self.device)
+            self._ws_ptr = self._ws.data_ptr() + ((-self._ws.data_ptr()) % 256)
+            self.rois = torch.empty((self.B, self.post_k, 4), dtype=torch.float32, device=self.device)
+            self.count = torch.empty((self.B,), dtype=torch.int32, device=self.device)
         if anchors is not None:
-            self.anchors = ops._req(anchors, "anchors")
-            if tuple(self.anchors.shape) != (self.N, 4):
-                raise ValueError("anchors must be [N,4]")
+            self.anchors = ops._req(anchors, "anchors", shape=(self.N, 4), device=self._ws.device)
             self.H = self.W = 0
         else:
             if image_hw is None:
@@ -90,30 +94,22 @@ class ProposalPlan:
             self.anchors = None
             self.H, self.W = int(image_hw[0]), int(image_hw[1])
         self.grid_hw = (self.H // self.stride, self.W // self.stride)   # padded grid of a mixed-size batch
-        with torch.cuda.device(self.device):
-            self.ws_bytes = int(self.lib.frr_rpn_proposals_workspace_bytes(self.B, self.N, self.pre_k, self.post_k))
-            self._ws = torch.empty((self.ws_bytes + 256,), dtype=torch.uint8, device=self.device)
-            self._ws_ptr = self._ws.data_ptr() + ((-self._ws.data_ptr()) % 256)
-            self.rois = torch.empty((self.B, self.post_k, 4), dtype=torch.float32, device=self.device)
-            self.count = torch.empty((self.B,), dtype=torch.int32, device=self.device)
 
     def run(self, cls, reg, rois=None, count=None, image_hw=None):
         """cls [B,N,2] logits / [B,N] scores and reg [B,N,4]: CUDA fp32 contiguous.  Returns (rois, count) --
         the plan's own output buffers unless ``rois`` / ``count`` are given (overwritten by the next run).
         ``image_hw``: per-image sizes (see the class doc); host sizes are checked and copied, so pass a device tensor
         where the call is captured into a graph."""
-        if not (cls.is_cuda and reg.is_cuda and cls.dtype == torch.float32 and reg.dtype == torch.float32):
-            raise ValueError("ProposalPlan.run: cls / reg must be CUDA fp32 tensors: the region stage has no CPU path")
-        if tuple(reg.shape) != (self.B, self.N, 4) or not reg.is_contiguous() or not cls.is_contiguous() or \
-                tuple(cls.shape) != ((self.B, self.N, 2) if self.logits else (self.B, self.N)):
-            raise ValueError("ProposalPlan.run: shape mismatch with the plan")
-        rois = self.rois if rois is None else rois
-        count = self.count if count is None else count
+        B, N, dev = self.B, self.N, self._ws.device
+        ops._check(cls, "cls", shape=(B, N, 2) if self.logits else (B, N), device=dev, contiguous=True)
+        ops._check(reg, "reg", shape=(B, N, 4), device=dev, contiguous=True)
+        rois = self.rois if rois is None else ops._check(rois, "rois", shape=(B, self.post_k, 4), device=dev, contiguous=True)
+        count = self.count if count is None else ops._check(count, "count", torch.int32, (B,), dev, contiguous=True)
         hw = None
         if image_hw is not None:
             if self.anchors is not None:
                 raise ValueError("ProposalPlan.run: per-image sizes need generated anchors (a plan built with image_hw)")
-            hw = ops.sized_hw(image_hw, self.B, self.grid_hw, self.stride, self.device)
+            hw = ops.sized_hw(image_hw, B, self.grid_hw, self.stride, dev)
         _lib.check(self.lib.frr_rpn_proposals(reg.data_ptr(), cls.data_ptr(), int(self.logits), ops._ptr(self.anchors),
                                               self._tptr, self.A, self.H, self.W, ops._ptr(hw), self.stride, self.min_size,
                                               self.B, self.N, self.pre_k, self.post_k, self.thr, rois.data_ptr(),

@@ -359,7 +359,7 @@ static int nms_pick(int B, int n, double iou_thr, int max_keep, int cluster_size
         out->threads = threads != 0 ? threads : 1024;
         out->slice_cap = 0;
         out->bucketed = 1;
-        out->smem = nms_bucket_smem_bytes(out->threads);
+        out->smem = nms_bucket_smem_bytes(out->threads, S);
         return FRR_OK;
     }
     // a CTA whose slice of the kept list is short (one image spread over 16 CTAs) is bound by its per-chunk barriers:

@@ -1,5 +1,5 @@
 // Shared by the NMS kernels (nms.cu: keep-list kernel; nms_bucket.cu: bucketed large-chunk kernel): the decision
-// arithmetic of torchvision's CPU kernel, the division-free screen, and the (area class, x bin) bucket keys.
+// arithmetic of torchvision's CPU kernel, the division-free screen, and the (x bin, y bin, area class) bucket keys.
 #pragma once
 #include <math.h>
 
@@ -21,15 +21,9 @@ struct NmsThr {
     float up;  // smallest fp32 with (double)up > thr
     float c2;  // up/(1+up) * (1 - 2^-19): screening constant
     float alo, ahi;  // a box of area A can only be suppressed by boxes with area in [alo * A, ahi * A] (IoU <= min/max area)
-    float fx;        // ... and only by boxes whose x-centre is within fx * (its width) of its own
+    float fx;        // ... and only by boxes whose x-centre is within fx * (its width) of its own, y-centre likewise
     int fast;  // screening usable (1e-6 <= thr, finite)
 };
-
-constexpr int kStrips = 88;         // area classes of the sorted kept slice (4 per octave, 2^-22 .. 1)
-constexpr int kXBins = 8;           // x-centre bins inside an area class
-constexpr int kKeys = kStrips * kXBins;  // bucket keys; key kKeys = boxes that must always be tested
-constexpr int kKeyPer = ((kKeys + 2 + 31) / 32 + 3) & ~3;  // keys scanned per lane (a multiple of 4: uint4 accesses)
-constexpr int kKeyCap = 32 * kKeyPer;                       // padded length of the per-key arrays
 
 __device__ __forceinline__ float box_area(const float4& b) {
     return __fmul_rn(__fsub_rn(b.z, b.x), __fsub_rn(b.w, b.y));
@@ -67,22 +61,34 @@ __device__ __forceinline__ bool suppress_screen(const float4& a, float sa, const
     return !(__fmul_rn(w, h) < __fadd_rn(sa, sb));
 }
 
-// Bucket key of a box = (area class, x bin).
+// Bucket key of a box = (x bin, y bin, area class) of the bucketed kernel, area class minor: the admissible area classes
+// of one cell are ONE contiguous run of a bucketed array, so a walk is one range per admissible cell.
 // Area class: the top bits of the fp32 area (exponent + 2 mantissa bits = 4 classes per octave), an exactly monotone
-// integer function of the area.  IoU <= min(area) / max(area) (in fp32 as well: w <= both widths and RN is monotone, so
-// inter <= both areas), hence only kept boxes whose area lies within [thr, 1/thr] of the candidate's can suppress it: for
-// RPN proposals (three anchor scales, a factor 4 apart in area) that alone removes 3/4 of the pairs.
-// x bin: kXBins equal strips of the x-centre; IoU >= thr also needs |cx_K - cx_c| <= fx * w_c, which is sharp exactly
-// where the area cut is not -- the many small boxes of the most populated classes.
+// integer function of the area, clamped to [2^-15, 1) (clamping keeps it monotone, so the admissible classes of a box
+// still contain every class that can suppress it).  IoU <= min(area) / max(area) (in fp32 as well: w <= both widths and
+// RN is monotone, so inter <= both areas), hence only kept boxes whose area lies within [thr, 1/thr] of the
+// candidate's can suppress it: for RPN proposals (three anchor scales, a factor 4 apart in area) that alone removes 3/4
+// of the pairs.
+// Cell: kX x kY equal bins of the x- and y-centre; IoU >= thr also needs |cx_a - cx_b| <= fx * w and, the same rule
+// with the axes swapped, |cy_a - cy_b| <= fx * h of either box, which is sharp exactly where the area cut is not -- the
+// many small boxes of the most populated classes.  kY = 1 is the x-only key (nms_bucket.cu: bk_ybins).
 // Boxes without a usable screening area (degenerate / malformed, NaN sa) get the extra key kKeys and are tested
 // against everything.
-__device__ __forceinline__ int strip_of_area(float a) {
-    return min(kStrips - 1, max(0, (__float_as_int(a) >> 21) - ((127 - 22) << 2)));
-}
-__device__ __forceinline__ int xbin_of(float cx) { return min(kXBins - 1, max(0, (int)(cx * (float)kXBins))); }
-__device__ __forceinline__ int strip_of(const float4& b, float sa) {
-    return (sa != sa) ? kKeys : strip_of_area(box_area(b)) * kXBins + xbin_of(0.5f * (b.x + b.z));
-}
+template <int kYBins>
+struct BkGrid {
+    static constexpr int kX = 8, kY = kYBins;
+    static constexpr int kClasses = 60;                   // 4 per octave, 2^-15 .. 1
+    static constexpr int kKeys = kX * kY * kClasses;      // key kKeys: boxes that must always be tested
+    static __device__ __forceinline__ int cls(float a) {
+        return min(kClasses - 1, max(0, (__float_as_int(a) >> 21) - ((127 - 15) << 2)));
+    }
+    static __device__ __forceinline__ int xbin(float cx) { return min(kX - 1, max(0, (int)(cx * (float)kX))); }
+    static __device__ __forceinline__ int ybin(float cy) { return min(kY - 1, max(0, (int)(cy * (float)kY))); }
+    static __device__ __forceinline__ int key(const float4& b, float sa) {
+        return (sa != sa) ? kKeys
+                          : (xbin(0.5f * (b.x + b.z)) * kY + ybin(0.5f * (b.y + b.w))) * kClasses + cls(box_area(b));
+    }
+};
 
 inline NmsThr make_thr(double thr) {
     NmsThr t;
@@ -97,9 +103,10 @@ inline NmsThr make_thr(double thr) {
     const double u = (double)t.up;
     t.c2 = t.fast ? (float)(u / (1.0 + u) * (1.0 - 1.9073486328125e-06)) : 0.f;
     // IoU >= thr needs min(area) / max(area) >= thr; thr is lowered by 2^-17 relative to cover the fp32 roundings of the
-    // exact IoU (<= 2^-20, see strip_of_area) and of the two products below
+    // exact IoU (<= 2^-20) and of the two products below
     const double tl = thr * (1.0 - 7.62939453125e-06);
-    // ... and |cx_a - cx_b| <= max(1 - thr, (1 - thr) / (2 thr)) * w of EITHER box (DESIGN.md)
+    // ... and |cx_a - cx_b| <= max(1 - thr, (1 - thr) / (2 thr)) * w of EITHER box, |cy_a - cy_b| the same with h
+    // (DESIGN.md)
     t.fx = t.fast ? (float)(fmax(1.0 - tl, (1.0 - tl) / (2.0 * tl)) * (1.0 + 1.0e-6)) : 0.f;
     t.alo = t.fast ? (float)(tl * (1.0 - 1.0e-6)) : 0.f;
     t.ahi = t.fast ? (float)(1.0 / tl * (1.0 + 1.0e-6)) : 0.f;
@@ -113,7 +120,7 @@ int nms_launch(const float* boxes, const int32_t* counts, int B, int n, double i
 
 // nms_bucket.cu: eligibility + launch of the bucketed kernel (unit-range boxes, screenable threshold, kept list <= 2047)
 bool nms_bucket_eligible(int n, int max_keep, const NmsThr& thr, int unit_boxes);
-size_t nms_bucket_smem_bytes(int threads);  // dynamic shared memory of a launch with `threads` threads per CTA
+size_t nms_bucket_smem_bytes(int threads, int S);  // dynamic shared memory of a launch: threads per CTA, CTAs per image
 int nms_bucket_launch(const float* boxes, const int32_t* counts, int B, int n, const NmsThr& thr, int max_keep, int32_t* keep,
                       int32_t* keep_count, float* out_boxes, int S, int threads, const NmsTune& tune, frr_stream_t stream,
                       const int32_t* gather_idx, int src_n);

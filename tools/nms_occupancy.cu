@@ -16,22 +16,23 @@ void set_error(const char* fmt, ...) {
 }
 }  // namespace frr
 
-template <int kThreads>
+template <int kThreads, int S>
 static int report() {
-    auto kern = frr::nms_bucket_kernel<kThreads>;
-    const size_t smem = frr::nms_bucket_smem_bytes(kThreads);
+    constexpr int kYBins = frr::bk_ybins(kThreads, S);
+    auto kern = frr::nms_bucket_kernel<kThreads, kYBins>;
+    const size_t smem = frr::nms_bucket_smem_bytes(kThreads, S);
     FRR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     FRR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     cudaFuncAttributes fa;
     FRR_CUDA(cudaFuncGetAttributes(&fa, kern));
     int blocks = 0;
     FRR_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, kern, kThreads, smem));
-    printf("{\"kernel\": \"nms_bucket_kernel<%d>\", \"dynamic_smem\": %zu, \"registers\": %d, \"local_bytes\": %zu, "
-           "\"ctas_per_sm\": %d}\n", kThreads, smem, fa.numRegs, fa.localSizeBytes, blocks);
+    printf("{\"kernel\": \"nms_bucket_kernel<%d, %d>\", \"dynamic_smem\": %zu, \"registers\": %d, \"local_bytes\": %zu, "
+           "\"ctas_per_sm\": %d}\n", kThreads, kYBins, smem, fa.numRegs, fa.localSizeBytes, blocks);
     return 0;
 }
 
 int main() {
-    if (report<256>() || report<512>() || report<1024>()) return 1;
+    if (report<256, 1>() || report<512, 1>() || report<1024, 1>() || report<1024, 8>()) return 1;
     return 0;
 }

@@ -203,7 +203,11 @@ __device__ __forceinline__ void rpn_assign_body(const float4* __restrict__ gt, c
             for (int g = 0; g < G; ++g) {
                 const float v = iou_eps(a, aa, sgt[g], sga[g], eps);
                 if (v > mx) { mx = v; arg = g; }
-                const unsigned long long key = ((unsigned long long)__float_as_uint(v) << 32) | (unsigned int)(~(unsigned int)i);
+                // key on v + 0: a GT inverted in one axis has IoU -0.0 with the anchors smaller than its |area| (0 over
+                // a negative union), whose sign bit would outrank every positive IoU; the reference's argmax takes
+                // -0.0 == 0.0 and the first anchor
+                const unsigned long long key =
+                    ((unsigned long long)__float_as_uint(__fadd_rn(v, 0.f)) << 32) | (unsigned int)(~(unsigned int)i);
                 if (key > best[g]) atomicMax(&best[g], key);
             }
             l = (mx < neg_thr) ? 0 : -1;
@@ -568,7 +572,7 @@ int frr_frcnn_targets_assign(const float* rois, const int32_t* roi_count, int B,
                              int32_t* argmax, int8_t* label8, int32_t* pos_list, int32_t* neg_list, int32_t* counts,
                              frr_stream_t stream) {
     using namespace frr;
-    FRR_CHECK_ARG(rois && gt && iou_max && argmax && label8 && pos_list && neg_list && counts,
+    FRR_CHECK_ARG((rois || Rmax == 0) && gt && iou_max && argmax && label8 && pos_list && neg_list && counts,
                   "frr_frcnn_targets_assign: null pointer");
     FRR_CHECK_ARG(B >= 0 && Rmax >= 0 && Gmax >= 1, "frr_frcnn_targets_assign: bad sizes");
     FRR_CHECK_ARG(aligned16(rois) && aligned16(gt), "frr_frcnn_targets_assign: rois/gt must be 16-byte aligned");
@@ -590,7 +594,7 @@ int frr_frcnn_targets_finalize(const float* rois, const int32_t* roi_count, int 
                                const float* std4_host, int label_offset, int64_t* cls, float* reg, float* sample_rois,
                                int32_t* keep_index, frr_stream_t stream) {
     using namespace frr;
-    FRR_CHECK_ARG(rois && gt && gt_label && argmax && pos_list && neg_list && sel && sel_n && cls && reg && sample_rois &&
+    FRR_CHECK_ARG((rois || Rmax == 0) && gt && gt_label && argmax && pos_list && neg_list && sel && sel_n && cls && reg && sample_rois &&
                       keep_index && std4_host,
                   "frr_frcnn_targets_finalize: null pointer");
     FRR_CHECK_ARG(B >= 0 && S >= 1, "frr_frcnn_targets_finalize: bad sizes");

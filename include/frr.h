@@ -345,6 +345,11 @@ int frr_sample_targets(const int32_t* rpn_counts, const int32_t* frcnn_counts, i
  *     frcnn_target_cls int64 [B,S] (negative = padding of a short sample), frcnn_target_reg [B,S,4].
  *     loss [B,5] = (total, rpn_cls, rpn_reg, frcnn_cls, frcnn_reg).  The grad_* tensors (same shapes as the predictions,
  *     any may be NULL) receive d loss_component / d prediction for a unit upstream gradient.  Either half may be NULL.
+ *     An image with no sampled anchor (or no non-padding row) gets NaN for that half's two losses, like the
+ *     reference's 0 / 0, and zero gradients.  A Fast R-CNN class >= C is not checked (a host-side check would
+ *     synchronise a captured or compiled step): the row counts in the normaliser and adds no loss term and no
+ *     gradient, where the reference raises.  Non-finite logits give what the reference's fp32 cross entropy gives:
+ *     NaN for a row with +inf or with every logit -inf, +inf for -inf in the target class only.
  * ------------------------------------------------------------------------------------- */
 int frr_region_loss(const float* rpn_cls, const float* rpn_reg, const int64_t* rpn_target_cls, const float* rpn_target_reg,
                     int B, int N, const float* frcnn_cls, const float* frcnn_reg, const int64_t* frcnn_target_cls,
